@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (one process per GPU under torchrun)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU algorithm (oracle port) on the host cores
+    python bench.py --steps K --dump-outputs DIR            # also writes what the last timed step computed to DIR/*.npy
 
 A "step" is one pass of the hot path -- PQMF.forward then PQMF.inverse -- over one batch of synthetic audio.
 Workload = BASELINE.json configs[1]: 64 x 2^20 mono samples per GPU, n_band 16, attenuation 100, polyphase.
@@ -25,6 +26,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark may run from a read-only checkout: it leaves nothing in the tree
 
 METRIC = "PQMF analyze+inverse throughput (n_band=16)"
 UNIT = "Msamples/s"
@@ -191,7 +193,7 @@ def run_gpu(args):
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         dist.init_process_group("nccl", device_id=dev)
     n_gpus = world if distributed else 1
-    steps, warmup = max(1, args.steps), max(3, args.warmup)
+    steps, warmup = args.steps, max(3, args.warmup)
 
     # rows are independent: each rank owns its own 64 x 2^20 shard (weak scaling), no collective on the data path
     gen = torch.Generator(device=dev).manual_seed(1234 + rank)
@@ -227,6 +229,8 @@ def run_gpu(args):
     sampler.sample_now()  # the launches above only queue work: the GPU is still inside the timed region here
     torch.cuda.synchronize()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, y, out)
     if distributed:
         dist.barrier()
     launches = pq.launch_count() - launches0
@@ -352,6 +356,23 @@ def run_gpu(args):
     if distributed:
         dist.destroy_process_group()
     return 0
+
+
+DUMP_ROWS = 4  # whole rows of the batch: sub-bands + reconstruction of 4 rows are 32 MiB, inside the 64 MB a dump may take
+
+
+def dump_outputs(dirname: str, y, out):
+    """Writes what the timed step returns to its caller -- the sub-bands of PQMF.forward [rows, 16, 65536] and the reconstruction of
+    PQMF.inverse [rows, 1, 2^20] -- for a fixed, seeded sample of DUMP_ROWS rows (the same rows on every run) as float32 .npy files, so
+    that two builds run with the same arguments can be compared output for output."""
+    import numpy as np
+    import torch
+
+    rows = np.sort(np.random.default_rng(0).choice(BATCH, DUMP_ROWS, replace=False))
+    idx = torch.from_numpy(rows).to(y.device)
+    os.makedirs(dirname, exist_ok=True)
+    for name, t in (("subbands", y), ("reconstruction", out)):
+        np.save(os.path.join(dirname, f"{name}.npy"), t.index_select(0, idx).to(torch.float32).cpu().numpy())
 
 
 def _max_over_ranks(torch, dist, dev, ms: float, distributed: bool) -> float:
@@ -544,18 +565,23 @@ def main():
     ap.add_argument("--impl", choices=("b200", "reference"), default="b200")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true", help="skip the sustained runs of configs 3 / 4 / 5 that are appended to the line")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the sub-bands and reconstruction of the last step (rank 0, a fixed sample of rows) to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.gpus > 1 and world == 1:
-        # convenience: re-launch ourselves under torchrun (the driver launches torchrun itself)
+        # convenience: re-launch ourselves under torchrun (a launcher may also start torchrun itself)
         import subprocess
 
         cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={args.gpus}", "--master-addr", "127.0.0.1",
                "--master-port", os.environ.get("MASTER_PORT", "29533"), os.path.abspath(__file__), "--gpus", str(args.gpus), "--steps",
                str(args.steps), "--warmup", str(args.warmup)] + (["--no-cpu-baseline"] if args.no_cpu_baseline else []) + (
-                   ["--no-other-configs"] if args.no_other_configs else [])
+                   ["--no-other-configs"] if args.no_other_configs else []) + (
+                   ["--dump-outputs", os.path.abspath(args.dump_outputs)] if args.dump_outputs else [])
         return subprocess.call(cmd)
     return run_gpu(args)
 

@@ -87,6 +87,9 @@ def main():
     import scipy
 
     meta["scipy"] = scipy.__version__
+    # CPU conv1d bits also depend on these: tests/test_oracle.py reproduces the thread count and checks the level
+    meta["cpu_capability"] = torch.backends.cpu.get_cpu_capability()
+    meta["threads"] = torch.get_num_threads()
 
     # ---- banks: h, hk for every n_band the configs name (attenuation 100) + attenuation sweep at M=16
     for m in (2, 4, 8, 16, 32, 64):

@@ -121,13 +121,17 @@ def test_torchscript_script_save_load(pq, tmp_path):
     assert "pqmf_b200::synthesis" in str(scripted_plain.inverse.graph)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference checkout not mounted")
+REFERENCE = os.environ.get("PQMF_REFERENCE", "")  # a checkout of the original project (not part of this repository)
+
+
+@pytest.mark.skipif(not os.path.isfile(os.path.join(REFERENCE, "PQMFWrapper.py")),
+                    reason="set PQMF_REFERENCE to a checkout of the original project to run its PQMFWrapper.py")
 def test_reference_wrapper_scripts_unchanged_against_dropin(tmp_path):
     """The reference's own PQMFWrapper.py, byte for byte, with dropin/ on sys.path instead of the reference's pqmf.py.
-    (Copied to a temp dir at test time only because the reference mount is read-only and the file mkdirs next to itself.)"""
+    (Copied to a temp dir at test time only because the reference checkout may be read-only and the file mkdirs next to itself.)"""
     import shutil
 
-    shutil.copy("/root/reference/PQMFWrapper.py", tmp_path / "PQMFWrapper.py")
+    shutil.copy(os.path.join(REFERENCE, "PQMFWrapper.py"), tmp_path / "PQMFWrapper.py")
     code = (
         "import sys; sys.path[:0] = [%r, %r, %r]\n"
         "import torch, PQMFWrapper as W\n"
