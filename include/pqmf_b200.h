@@ -11,7 +11,8 @@
  *
  * Conventions
  *   - every data pointer is a DEVICE pointer to row-contiguous float32 unless the name ends
- *     in _host; the caller owns all buffers (including streaming state);
+ *     in _host (host pointers) or _x (`void*` data of the element type `dtype`: float32, float16
+ *     or bfloat16); the caller owns all buffers (including streaming state);
  *   - functions never allocate device memory, never synchronise, never throw: they enqueue
  *     on `stream` (a cudaStream_t passed as void*) and return 0 on success, a negative
  *     PQMF_ERR_* code for rejected arguments, or a positive cudaError_t value
@@ -178,6 +179,29 @@ int pqmf_roundtrip_f32(const float* x, float* y, float* out, const float* hk, co
 size_t pqmf_reconstruct_scratch_bytes(int B, long T, long n_frames, int M);
 int pqmf_reconstruct_f32(const float* x, float* out, float* scratch, size_t scratch_bytes, const float* hk, const float* tables, int B, long T,
                          long n_frames, int M, int L, int delay_frames, unsigned flags, pqmf_stream_t stream);
+
+/* ---- half-precision signals and sub-bands (PyTorch's float16 / bfloat16 tensors) ----
+ * pqmf_analysis_x, pqmf_synthesis_x, pqmf_roundtrip_x and pqmf_reconstruct_x are the _f32 entry points above with `void*` data
+ * pointers whose element type is `dtype` (input and output alike).  With PQMF_DTYPE_F32 each one IS the _f32 entry.  With
+ * PQMF_DTYPE_F16 / PQMF_DTYPE_BF16 the samples are widened to fp32 exactly in the kernels' loads, processed by the same kernels with
+ * the same fp32 accumulation, and rounded to nearest even in the stores: bit-identical to the _f32 call on the widened input followed
+ * by a round-to-nearest-even cast of its output, at half the bytes.  Native half-precision kernels exist for the offline Hankel-4
+ * family only: a call runs natively where the _f32 call would run those kernels with an unsplit bank (no PQMF_FLAG_H4_SPLIT) as CTA
+ * pairs, and its buffers are 16-byte aligned.  Every other call (small batches, ragged lengths, frame counts not a multiple of 4,
+ * the fold / Hankel-16 / direct-form families, split banks, misaligned buffers) returns PQMF_ERR_UNSUPPORTED before anything is
+ * launched; the caller then widens, calls the _f32 entry and rounds (torch_ops.cpp does).  pqmf_roundtrip_x and pqmf_reconstruct_x
+ * run only when every launch they make is native.  pqmf_reconstruct_x's scratch is sized by pqmf_reconstruct_scratch_bytes. */
+#define PQMF_DTYPE_F32 0
+#define PQMF_DTYPE_F16 1
+#define PQMF_DTYPE_BF16 2
+int pqmf_analysis_x(const void* x, void* y, const float* hk, const float* tables, int B, long T, long n_frames, int M, int L, unsigned flags,
+                    int dtype, pqmf_stream_t stream);
+int pqmf_synthesis_x(const void* s, void* out, const float* hk, const float* tables, int B, long n_frames, int M, int L, int delay_frames,
+                     unsigned flags, int dtype, pqmf_stream_t stream);
+int pqmf_roundtrip_x(const void* x, void* y, void* out, const float* hk, const float* tables, int B, long T, long n_frames, int M, int L,
+                     int delay_frames, unsigned flags, int dtype, pqmf_stream_t stream);
+int pqmf_reconstruct_x(const void* x, void* out, void* scratch, size_t scratch_bytes, const float* hk, const float* tables, int B, long T,
+                       long n_frames, int M, int L, int delay_frames, unsigned flags, int dtype, pqmf_stream_t stream);
 
 /* ---- end-to-end host entry (what a non-torch host -- e.g. the Pure Data external that loads the
  *      reference's .ts, README.md:16 -- would call): host buffers in, host buffers out.

@@ -26,6 +26,9 @@ PQMF_FLAG_NO_PAIR = 8
 PQMF_FLAG_FP32 = 16
 PQMF_FLAG_NO_FOLD = 32
 PQMF_FLAG_H4_SPLIT = 1 << 23
+PQMF_DTYPE_F32 = 0
+PQMF_DTYPE_F16 = 1
+PQMF_DTYPE_BF16 = 2
 
 
 def _load():
@@ -92,6 +95,21 @@ cabi.pqmf_roundtrip_host_pcm16.argtypes = [_vp, _vp, _vp, _vp, _vp, ctypes.c_int
 cabi.pqmf_roundtrip_host_multi_f32.restype = ctypes.c_int
 cabi.pqmf_roundtrip_host_multi_f32.argtypes = [_vp, _vp, _vp, _vp, _vp, ctypes.c_int, ctypes.c_long, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                                ctypes.c_uint, ctypes.POINTER(ctypes.c_int), ctypes.c_int]
+# half-precision I/O (dtype: PQMF_DTYPE_*); PQMF_ERR_UNSUPPORTED where no native kernel exists
+cabi.pqmf_analysis_x.restype = ctypes.c_int
+cabi.pqmf_analysis_x.argtypes = [_vp, _vp, _vp, _vp, ctypes.c_int, ctypes.c_long, ctypes.c_long, ctypes.c_int, ctypes.c_int, ctypes.c_uint,
+                                 ctypes.c_int, _vp]
+cabi.pqmf_synthesis_x.restype = ctypes.c_int
+cabi.pqmf_synthesis_x.argtypes = [_vp, _vp, _vp, _vp, ctypes.c_int, ctypes.c_long, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_uint,
+                                  ctypes.c_int, _vp]
+cabi.pqmf_roundtrip_x.restype = ctypes.c_int
+cabi.pqmf_roundtrip_x.argtypes = [_vp, _vp, _vp, _vp, _vp, ctypes.c_int, ctypes.c_long, ctypes.c_long, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                  ctypes.c_uint, ctypes.c_int, _vp]
+cabi.pqmf_reconstruct_scratch_bytes.restype = ctypes.c_size_t
+cabi.pqmf_reconstruct_scratch_bytes.argtypes = [ctypes.c_int, ctypes.c_long, ctypes.c_long, ctypes.c_int]
+cabi.pqmf_reconstruct_x.restype = ctypes.c_int
+cabi.pqmf_reconstruct_x.argtypes = [_vp, _vp, _vp, ctypes.c_size_t, _vp, _vp, ctypes.c_int, ctypes.c_long, ctypes.c_long, ctypes.c_int, ctypes.c_int,
+                                    ctypes.c_int, ctypes.c_uint, ctypes.c_int, _vp]
 
 if cabi.pqmf_abi_version() != 2:  # pragma: no cover
     raise ImportError("pqmf_b200: libpqmf_b200.so ABI version mismatch; rebuild")

@@ -15,6 +15,8 @@
 // Roles: worker warps convert fp32 -> 2 x fp16 planes (swizzled STS) and drain TMEM; ONE warp only issues the MMAs
 // (tcgen05.mma issue blocks the issuing thread while the tensor queue is full).  With PAIR the kernel runs as clusters of two
 // CTAs sharing the bank operand (cta_group::2).  DESIGN.md section 5 has the measurements behind each of these choices.
+// IO (half_io.cuh) is the sample format at the kernel's edge -- fp32, fp16 / bf16 (widened exactly in the loads, rounded to nearest
+// even in the stores) or int16 PCM (pcm.cuh); everything between the loads and the stores is the same for all of them.
 //
 // Round 2: the second fp16 term of every sample and the second term of the bank are scaled by 2^11 (h2' = 2^11 (x - h1),
 // c2' = 2^11 (2^10 hk - c1)) and accumulate in their own TMEM columns: D[:, 0:64] = h1 c1, D[:, 64:128] = h1 c2' + h2' c1, result =
@@ -34,6 +36,7 @@
 
 #include <atomic>
 
+#include "half_io.cuh"
 #include "hankel16.cuh"
 #include "pcm.cuh"
 #include "ptx.cuh"
@@ -253,9 +256,9 @@ __device__ __forceinline__ void h4_publish(const H4Smem& s, uint32_t pfull_leade
 // analysis
 // =============================================================================================
 struct H4AnalysisParams {
-  const float* x;        // [B, T]
+  const float* x;        // [B, T]; half-precision instantiations: raw fp16 / bf16 bits (the launch's H4Io)
   PcmIn in;              // PCM instantiation: the rows come from interleaved int16 WAV frames (x unused)
-  float* y;              // [B, M, F]
+  float* y;              // [B, M, F]; half-precision instantiations: raw fp16 / bf16 bits
   const uint16_t* bank;  // fp16 image(s), see hankel4_build_banks / hankel4_pair_image
   long T, F;
   int off;               // L / 2 (offline only: streaming blocks are far smaller than a tile)
@@ -270,8 +273,9 @@ struct H4AnalysisParams {
 #endif
 };
 
-template <int M, bool PAIR, bool PCM>
+template <int M, bool PAIR, H4Io IO>
 __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_kernel(H4AnalysisParams p) {
+  constexpr bool PCM = IO == H4Io::PCM, HALF = h4_io_half(IO);
   constexpr int FR = 64 / M;                                               // frames per 64-sample row
   constexpr int HB = M / 2;                                                // bands per epilogue thread
   constexpr int NO = (kH4MaxPlaneRows * 8 + kH4Workers - 1) / kH4Workers;  // 8-sample loads per thread per tile (a row is 8 of them)
@@ -306,13 +310,20 @@ __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_kernel(H4AnalysisPa
     auto load_window = [&](unsigned bb, unsigned cc) {
       const long s0 = (long)cc * kH4TileSamples + g.jlo - p.off;
       const float* xrow = p.x + (size_t)bb * p.T;
+      const uint16_t* xhrow = reinterpret_cast<const uint16_t*>(p.x) + (size_t)bb * p.T;
 #pragma unroll
       for (int r = 0; r < NO; ++r) {
         const int o = tid + kH4Workers * r;
         const long s = s0 + 8L * o;
         if (bb < n_rows && o < n_octs && s >= 0 && s < p.T) {
-          if constexpr (PCM) pcm_load8_raw(p.in, bb, s, p.T, x0[r]);   // raw int16 words: converted when the tile is consumed
-          else ptx::ldg256_na(xrow + s, x0[r]);
+          if constexpr (PCM) {
+            pcm_load8_raw(p.in, bb, s, p.T, x0[r]);   // raw int16 words: converted when the tile is consumed
+          } else if constexpr (HALF) {                // eight half samples = 16 bytes, kept raw in x0[r][0..3] until the tile is consumed
+            const float4 raw = ptx::ldg128_na(reinterpret_cast<const float4*>(xhrow + s));
+            x0[r][0] = raw.x; x0[r][1] = raw.y; x0[r][2] = raw.z; x0[r][3] = raw.w;
+          } else {
+            ptx::ldg256_na(xrow + s, x0[r]);
+          }
         } else {
 #pragma unroll
           for (int e = 0; e < 8; ++e) x0[r][e] = 0.f;
@@ -332,6 +343,7 @@ __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_kernel(H4AnalysisPa
             const long s = (long)cc * kH4TileSamples + g.jlo - p.off + 8L * o;
             if (bb < n_rows && s >= 0 && s < p.T) pcm_convert8(p.in, bb, x0[r]);
           }
+          if constexpr (HALF) h4_widen8<IO>(x0[r]);  // exact; zero words (padding) widen to zeros
           uint4 a, bq;
           split2_f16s(x0[r][0], x0[r][1], a.x, bq.x);
           split2_f16s(x0[r][2], x0[r][3], a.y, bq.y);
@@ -375,6 +387,39 @@ __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_kernel(H4AnalysisPa
           v[dl][kk] = t.x;
           v[dl][kk + 1] = __uint_as_float(__float_as_uint(t.y) ^ flip);
         }
+      }
+      if constexpr (HALF) {  // round to nearest even; FR consecutive frames = 2 FR bytes per band (no accumulation: split banks are not native)
+        uint16_t* yp = reinterpret_cast<uint16_t*>(p.y) + ((size_t)bb * M + HB * hb) * p.F + n;
+        if (n + FR - 1 < p.F && (p.F % (FR >= 8 ? 8 : FR)) == 0) {
+#pragma unroll
+          for (int kk = 0; kk < HB; ++kk) {
+            uint16_t* q = yp + (size_t)kk * p.F;
+            if constexpr (FR >= 8) {
+#pragma unroll
+              for (int d8 = 0; d8 < FR; d8 += 8) {
+                const uint4 w = make_uint4(h4_narrow2<IO>(v[d8][kk], v[d8 + 1][kk]), h4_narrow2<IO>(v[d8 + 2][kk], v[d8 + 3][kk]),
+                                           h4_narrow2<IO>(v[d8 + 4][kk], v[d8 + 5][kk]), h4_narrow2<IO>(v[d8 + 6][kk], v[d8 + 7][kk]));
+                if (p.keep_in_l2) *reinterpret_cast<uint4*>(q + d8) = w;
+                else __stcs(reinterpret_cast<uint4*>(q + d8), w);
+              }
+            } else if constexpr (FR == 4) {
+              const uint2 w = make_uint2(h4_narrow2<IO>(v[0][kk], v[1][kk]), h4_narrow2<IO>(v[2][kk], v[3][kk]));
+              if (p.keep_in_l2) *reinterpret_cast<uint2*>(q) = w;
+              else __stcs(reinterpret_cast<uint2*>(q), w);
+            } else if constexpr (FR == 2) {
+              __stcs(reinterpret_cast<unsigned int*>(q), h4_narrow2<IO>(v[0][kk], v[1][kk]));
+            } else {
+              __stcs(reinterpret_cast<unsigned short*>(q), h4_narrow1<IO>(v[0][kk]));
+            }
+          }
+        } else {
+#pragma unroll
+          for (int kk = 0; kk < HB; ++kk)
+#pragma unroll
+            for (int dl = 0; dl < FR; ++dl)
+              if (n + dl < p.F) yp[(size_t)kk * p.F + dl] = h4_narrow1<IO>(v[dl][kk]);
+        }
+        return;
       }
       float* yp = p.y + ((size_t)bb * M + HB * hb) * p.F + n;
       if (n + FR - 1 < p.F && (p.F % (FR >= 4 ? 4 : FR)) == 0) {
@@ -458,8 +503,8 @@ __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_kernel(H4AnalysisPa
 // synthesis
 // =============================================================================================
 struct H4SynthesisParams {
-  const float* s;        // [B, M, F]
-  float* out;            // [B, M F]
+  const float* s;        // [B, M, F]; half-precision instantiations: raw fp16 / bf16 bits (the launch's H4Io)
+  float* out;            // [B, M F]; half-precision instantiations: raw fp16 / bf16 bits
   int16_t* pcm_out;      // PCM instantiation: interleaved int16 WAV frames [B / C, M F, C] (out unused)
   int C;
   int duo;               // PCM stereo: the launch walks CLIPS; a CTA runs the left and the right row of a tile back to back and its
@@ -478,8 +523,9 @@ struct H4SynthesisParams {
 #endif
 };
 
-template <int M, bool PAIR, bool PCM>
+template <int M, bool PAIR, H4Io IO>
 __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_kernel(H4SynthesisParams p) {
+  constexpr bool PCM = IO == H4Io::PCM, HALF = h4_io_half(IO);
   constexpr int FR = 64 / M;       // frames per 128-byte plane row ([frame][band] fp16)
   constexpr int NBG = M >= 8 ? M / 8 : 1;     // band groups: a 16-byte chunk is 8 bands of one frame, or (n_band 4) all bands of two frames
   constexpr int FPI = M >= 8 ? 4 : 32 / M;   // frames per load/convert item (four chunks)
@@ -515,7 +561,12 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_kernel(H4Synthe
     const int n_fq = (g.rows * FR + FPI - 1) / FPI;          // items per band group (the last one may run into the plane's padding)
     const int bg = tid / n_fq, fq = tid - bg * n_fq;
     const bool has_item = tid < n_fq * NBG;
-    float4 v0[8];  // prefetched one tile ahead
+    float4 v0[8];  // prefetched one tile ahead (half instantiations: four raw frames in .x / .y, widened when the tile is consumed)
+    auto load4h = [&](const uint16_t* at, bool ok) {  // four half frames of one band
+      if (!ok) return make_float4(0.f, 0.f, 0.f, 0.f);
+      const float2 raw = ptx::ldg64_na(at);
+      return make_float4(raw.x, raw.y, 0.f, 0.f);
+    };
     auto load_frames = [&](float4 (&v)[8], unsigned bb, unsigned cc, unsigned hh) {
       if (p.reverse && bb < n_rows) {
         bb = n_rows - 1 - bb;
@@ -524,7 +575,21 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_kernel(H4Synthe
       const long n = (long)cc * (kH4Rows * FR) + nbase + FPI * fq;
       const bool live = bb < n_rows && has_item;
       const size_t row = (size_t)bb * G + hh;
-      if constexpr (M >= 8) {  // v[kk] = frames n .. n + 3 of band 8 bg + kk
+      if constexpr (HALF) {    // the same frames as below, 8 bytes per load
+        if constexpr (M >= 8) {
+          const uint16_t* sp = reinterpret_cast<const uint16_t*>(p.s) + (row * M + 8 * bg) * p.F + n;
+          const bool ok = live && n >= 0 && n + 3 < p.F;
+#pragma unroll
+          for (int kk = 0; kk < 8; ++kk) v[kk] = load4h(sp + (size_t)kk * p.F, ok);
+        } else {
+          const uint16_t* sp = reinterpret_cast<const uint16_t*>(p.s) + row * M * p.F + n;
+#pragma unroll
+          for (int kk = 0; kk < 8; ++kk) {
+            const int b4 = kk >> 1, h = kk & 1;
+            v[kk] = load4h(sp + (size_t)b4 * p.F + 4 * h, live && n + 4 * h >= 0 && n + 4 * h + 3 < p.F);
+          }
+        }
+      } else if constexpr (M >= 8) {  // v[kk] = frames n .. n + 3 of band 8 bg + kk
         const float* sp = p.s + (row * M + 8 * bg) * p.F + n;
         const bool ok = live && n >= 0 && n + 3 < p.F;
 #pragma unroll
@@ -659,6 +724,17 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_kernel(H4Synthe
           if (t0 + 64 * q + 7 < total) pcm_store8(p.pcm_out, p.C, (long)row, t0 + 64 * q, total, val[q]);
         return;
       }
+      if constexpr (HALF) {  // round to nearest even: eight samples = one 16-byte store per slot, a lane quad covers 64 contiguous bytes
+        uint16_t* op = reinterpret_cast<uint16_t*>(p.out) + row * total + t0;
+#pragma unroll
+        for (int q = 0; q < 4; ++q)
+          if (t0 + 64 * q + 7 < total) {
+            const uint4 w = make_uint4(h4_narrow2<IO>(val[q][0], val[q][1]), h4_narrow2<IO>(val[q][2], val[q][3]), h4_narrow2<IO>(val[q][4], val[q][5]),
+                                       h4_narrow2<IO>(val[q][6], val[q][7]));
+            __stcs(reinterpret_cast<uint4*>(op + (size_t)q * 64), w);
+          }
+        return;
+      }
       float* op = p.out + row * total + t0;
 #pragma unroll
       for (int q = 0; q < 4; ++q)
@@ -686,7 +762,14 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_kernel(H4Synthe
     for (unsigned it = 0; it < n_iter; ++it) {
       const int pb = (int)(it & 1);
       H4_STAMP(0);
-      convert(v0, pb);
+      if constexpr (HALF) {
+        float4 w[8];
+#pragma unroll
+        for (int kk = 0; kk < 8; ++kk) w[kk] = h4_widen4<IO>(v0[kk]);  // exact
+        convert(w, pb);
+      } else {
+        convert(v0, pb);
+      }
       H4_STAMP(1);
       h4_publish<PAIR>(sm, pfull_leader, it, pb, tid);
       if (it + 1 < n_iter) load_frames(v0, b1, c1, h1);
@@ -784,29 +867,47 @@ inline int h4_launch(Kern kern, Params p, int B, long row_samples, int threads, 
   }
 }
 
-// the PCM instantiations exist as CTA pairs only (the single-CTA launch is a fallback for contexts that cannot co-schedule pairs)
+// the PCM and half-precision instantiations exist as CTA pairs only (the single-CTA launch is a fallback for contexts that cannot
+// co-schedule pairs)
 template <int M, bool PAIR>
-int h4_launch_analysis(H4AnalysisParams p, int B, cudaStream_t st) {
-  static H4Configured configured[2];
-  if (p.in.pcm != nullptr) {
-    if constexpr (PAIR) return h4_launch<PAIR>(h4_analysis_kernel<M, PAIR, true>, p, B, p.F * M, kH4Threads, configured[1], st);
-    else return -2;
-  }
-  return h4_launch<PAIR>(h4_analysis_kernel<M, PAIR, false>, p, B, p.F * M, kH4Threads, configured[0], st);
-}
-
-template <int M, bool PAIR>
-int h4_launch_synthesis(H4SynthesisParams p, int B, cudaStream_t st) {
-  static H4Configured configured[2];
-  if (p.pcm_out != nullptr) {
+int h4_launch_analysis(H4AnalysisParams p, int B, cudaStream_t st, H4Io io = H4Io::F32) {
+  static H4Configured configured[4];
+  if (p.in.pcm != nullptr) io = H4Io::PCM;
+  if (io != H4Io::F32) {
     if constexpr (PAIR) {
-      p.duo = (p.C == 2 && B % 2 == 0) ? 1 : 0;  // stereo: the tiles of a launch are (clip, chunk), each visited once per channel
-      return h4_launch<PAIR>(h4_synthesis_kernel<M, PAIR, true>, p, p.duo ? B / 2 : B, p.F * M, kH4SynThreads, configured[1], st);
+      switch (io) {
+        case H4Io::PCM: return h4_launch<PAIR>(h4_analysis_kernel<M, PAIR, H4Io::PCM>, p, B, p.F * M, kH4Threads, configured[1], st);
+        case H4Io::F16: return h4_launch<PAIR>(h4_analysis_kernel<M, PAIR, H4Io::F16>, p, B, p.F * M, kH4Threads, configured[2], st);
+        case H4Io::BF16: return h4_launch<PAIR>(h4_analysis_kernel<M, PAIR, H4Io::BF16>, p, B, p.F * M, kH4Threads, configured[3], st);
+        default: return -2;
+      }
     } else {
       return -2;
     }
   }
-  return h4_launch<PAIR>(h4_synthesis_kernel<M, PAIR, false>, p, B, p.F * M, kH4SynThreads, configured[0], st);
+  return h4_launch<PAIR>(h4_analysis_kernel<M, PAIR, H4Io::F32>, p, B, p.F * M, kH4Threads, configured[0], st);
+}
+
+template <int M, bool PAIR>
+int h4_launch_synthesis(H4SynthesisParams p, int B, cudaStream_t st, H4Io io = H4Io::F32) {
+  static H4Configured configured[4];
+  if (p.pcm_out != nullptr) {
+    if constexpr (PAIR) {
+      p.duo = (p.C == 2 && B % 2 == 0) ? 1 : 0;  // stereo: the tiles of a launch are (clip, chunk), each visited once per channel
+      return h4_launch<PAIR>(h4_synthesis_kernel<M, PAIR, H4Io::PCM>, p, p.duo ? B / 2 : B, p.F * M, kH4SynThreads, configured[1], st);
+    } else {
+      return -2;
+    }
+  }
+  if (h4_io_half(io)) {
+    if constexpr (PAIR) {
+      if (io == H4Io::F16) return h4_launch<PAIR>(h4_synthesis_kernel<M, PAIR, H4Io::F16>, p, B, p.F * M, kH4SynThreads, configured[2], st);
+      return h4_launch<PAIR>(h4_synthesis_kernel<M, PAIR, H4Io::BF16>, p, B, p.F * M, kH4SynThreads, configured[3], st);
+    } else {
+      return -2;
+    }
+  }
+  return h4_launch<PAIR>(h4_synthesis_kernel<M, PAIR, H4Io::F32>, p, B, p.F * M, kH4SynThreads, configured[0], st);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -168,12 +168,6 @@ long h4_tables_floats(int M, int L) {
 bool use_h4(int B, long F, int M, const float* hist) {
   return hist == nullptr && (long)B * (((long)F * M + pqmf::kH4TileSamples - 1) / pqmf::kH4TileSamples) >= 96;
 }
-bool h4_analysis_ok(const float* x, const float* y, long T, long F, int M) {
-  return T > 0 && (T % M) == 0 && (T % 8) == 0 && F == T / M && ((uintptr_t)x % 32) == 0 && ((uintptr_t)y % 16) == 0;  // 256-bit loads
-}
-bool h4_synthesis_ok(const float* s, const float* out, long F) {
-  return F > 0 && (F & 3) == 0 && ((uintptr_t)s % 16) == 0 && ((uintptr_t)out % 32) == 0;
-}
 // taps kept by the images in `tables` (PQMF_FLAG_TAPS from pqmf_build_tables_f32); kt == 0: the caller did not pass them.
 // With PQMF_FLAG_H4_SPLIT the field holds half the span.
 void h4_taps(unsigned flags, int& jlo, int& kt) {
@@ -182,7 +176,7 @@ void h4_taps(unsigned flags, int& jlo, int& kt) {
 }
 
 template <int M>
-int h4_analysis_m(pqmf::H4AnalysisParams p, const float* tables, int jlo, int kt, int B, int L, unsigned flags, cudaStream_t st) {
+int h4_analysis_m(pqmf::H4AnalysisParams p, const float* tables, int jlo, int kt, int B, int L, unsigned flags, cudaStream_t st, pqmf::H4Io io) {
   const int trim = (flags & PQMF_FLAG_EXACT) ? 0 : (int)PQMF_FLAG_H4_TRIM_A(flags);  // exact mode: every correction term
   if (flags & PQMF_FLAG_H4_SPLIT) {  // two tap ranges, two launches; only the outer edge of each range may skip the corrections
     for (int half = 0; half < 2; ++half) {
@@ -191,7 +185,7 @@ int h4_analysis_m(pqmf::H4AnalysisParams p, const float* tables, int jlo, int kt
       p.trim_lo = half ? 0 : trim;
       p.trim_hi = half ? trim : 0;
       p.accumulate = half;
-      if (const int e = pqmf::h4_launch_analysis<M, true>(p, B, st)) {
+      if (const int e = pqmf::h4_launch_analysis<M, true>(p, B, st, io)) {
         if (half) return e;
         (void)cudaGetLastError();  // nothing was launched: the caller falls back to the direct form, which must not see this error
         return PQMF_ERR_UNSUPPORTED;
@@ -203,7 +197,7 @@ int h4_analysis_m(pqmf::H4AnalysisParams p, const float* tables, int jlo, int kt
   if (!(flags & PQMF_FLAG_NO_PAIR)) {
     p.g = pqmf::h4_shape(M, jlo, kt, true, false);
     p.bank = reinterpret_cast<const uint16_t*>(tables + h4_pair_offset(M, L));
-    const int e = pqmf::h4_launch_analysis<M, true>(p, B, st);
+    const int e = pqmf::h4_launch_analysis<M, true>(p, B, st, io);
     if (e == 0) return 0;
     (void)cudaGetLastError();  // a context that cannot co-schedule CTA pairs (e.g. an SM partition): same arithmetic, one CTA per SM
   }
@@ -213,28 +207,29 @@ int h4_analysis_m(pqmf::H4AnalysisParams p, const float* tables, int jlo, int kt
     if (!pqmf::hankel16_supported(M, L)) return PQMF_ERR_UNSUPPORTED;
     p.g = pqmf::h4_shape(M, jlo, kt, false, false);
     p.bank = reinterpret_cast<const uint16_t*>(tables + kH4TableOffset);
-    return pqmf::h4_launch_analysis<M, false>(p, B, st);
+    return pqmf::h4_launch_analysis<M, false>(p, B, st, io);
   }
 }
-int h4_analysis(const float* x, float* y, const float* tables, int B, long T, long F, int M, int L, unsigned flags, cudaStream_t st,
-                pqmf::PcmIn pcm = pqmf::PcmIn{nullptr, 1, 0}) {
+// x / y: float32 rows and sub-bands, or raw half bits when io is F16 / BF16 (x unused with PCM input)
+int h4_analysis(const void* x, void* y, const float* tables, int B, long T, long F, int M, int L, unsigned flags, cudaStream_t st,
+                pqmf::PcmIn pcm = pqmf::PcmIn{nullptr, 1, 0}, pqmf::H4Io io = pqmf::H4Io::F32) {
   int jlo, kt;
   h4_taps(flags, jlo, kt);
   if (kt == 0) return PQMF_ERR_UNSUPPORTED;
   pqmf::H4AnalysisParams p{};
-  p.x = x; p.in = pcm; p.y = y; p.T = T; p.F = F; p.off = L / 2; p.parity = 0; p.keep_in_l2 = 1;
+  p.x = static_cast<const float*>(x); p.in = pcm; p.y = static_cast<float*>(y); p.T = T; p.F = F; p.off = L / 2; p.parity = 0; p.keep_in_l2 = 1;
   switch (M) {
-    case 4: return h4_analysis_m<4>(p, tables, jlo, kt, B, L, flags, st);
-    case 8: return h4_analysis_m<8>(p, tables, jlo, kt, B, L, flags, st);
-    case 16: return h4_analysis_m<16>(p, tables, jlo, kt, B, L, flags, st);
-    case 32: return h4_analysis_m<32>(p, tables, jlo, kt, B, L, flags, st);
-    case 64: return h4_analysis_m<64>(p, tables, jlo, kt, B, L, flags, st);
+    case 4: return h4_analysis_m<4>(p, tables, jlo, kt, B, L, flags, st, io);
+    case 8: return h4_analysis_m<8>(p, tables, jlo, kt, B, L, flags, st, io);
+    case 16: return h4_analysis_m<16>(p, tables, jlo, kt, B, L, flags, st, io);
+    case 32: return h4_analysis_m<32>(p, tables, jlo, kt, B, L, flags, st, io);
+    case 64: return h4_analysis_m<64>(p, tables, jlo, kt, B, L, flags, st, io);
     default: return PQMF_ERR_UNSUPPORTED;
   }
 }
 
 template <int M>
-int h4_synthesis_m(pqmf::H4SynthesisParams p, const float* tables, int jlo, int kt, int B, int L, unsigned flags, cudaStream_t st) {
+int h4_synthesis_m(pqmf::H4SynthesisParams p, const float* tables, int jlo, int kt, int B, int L, unsigned flags, cudaStream_t st, pqmf::H4Io io) {
   const int trim = (flags & PQMF_FLAG_EXACT) ? 0 : (int)PQMF_FLAG_H4_TRIM_S(flags);
   if ((flags & PQMF_FLAG_H4_SPLIT) && p.pcm_out != nullptr) return PQMF_ERR_UNSUPPORTED;  // the second launch accumulates: not in int16
   if (flags & PQMF_FLAG_H4_SPLIT) {
@@ -245,7 +240,7 @@ int h4_synthesis_m(pqmf::H4SynthesisParams p, const float* tables, int jlo, int 
       p.trim_lo = half ? trim : 0;
       p.trim_hi = half ? 0 : trim;
       p.accumulate = half;
-      if (const int e = pqmf::h4_launch_synthesis<M, true>(p, B, st)) {
+      if (const int e = pqmf::h4_launch_synthesis<M, true>(p, B, st, io)) {
         if (half) return e;
         (void)cudaGetLastError();
         return PQMF_ERR_UNSUPPORTED;
@@ -261,7 +256,7 @@ int h4_synthesis_m(pqmf::H4SynthesisParams p, const float* tables, int jlo, int 
     if (variant) p.trim_lo = p.trim_hi = trim > 0 ? trim - 1 : 0;
     p.g = pqmf::h4_shape(M, jlo, kt + variant * M, true, true);
     p.bank = reinterpret_cast<const uint16_t*>(tables + h4_pair_offset(M, L) + (1 + variant) * h4_pair_floats(M, L));
-    const int e = pqmf::h4_launch_synthesis<M, true>(p, B, st);
+    const int e = pqmf::h4_launch_synthesis<M, true>(p, B, st, io);
     if (e == 0) return 0;
     (void)cudaGetLastError();
   }
@@ -271,22 +266,23 @@ int h4_synthesis_m(pqmf::H4SynthesisParams p, const float* tables, int jlo, int 
     if (!pqmf::hankel16_supported(M, L)) return PQMF_ERR_UNSUPPORTED;
     p.g = pqmf::h4_shape(M, jlo, kt, false, true);
     p.bank = reinterpret_cast<const uint16_t*>(tables + kH4TableOffset + kH4ImageFloats);
-    return pqmf::h4_launch_synthesis<M, false>(p, B, st);
+    return pqmf::h4_launch_synthesis<M, false>(p, B, st, io);
   }
 }
-int h4_synthesis(const float* s, float* out, const float* tables, int B, long F, int off2, int M, int L, unsigned flags, cudaStream_t st,
-                 int16_t* pcm_out = nullptr, int C = 1) {
+// s / out: float32 sub-bands and rows, or raw half bits when io is F16 / BF16 (out unused with PCM output)
+int h4_synthesis(const void* s, void* out, const float* tables, int B, long F, int off2, int M, int L, unsigned flags, cudaStream_t st,
+                 int16_t* pcm_out = nullptr, int C = 1, pqmf::H4Io io = pqmf::H4Io::F32) {
   int jlo, kt;
   h4_taps(flags, jlo, kt);
   if (kt == 0 || off2 % M != 0) return PQMF_ERR_UNSUPPORTED;
   pqmf::H4SynthesisParams p{};
-  p.s = s; p.out = out; p.pcm_out = pcm_out; p.C = C; p.F = F; p.o = off2 / M; p.parity = 0; p.reverse = 1;
+  p.s = static_cast<const float*>(s); p.out = static_cast<float*>(out); p.pcm_out = pcm_out; p.C = C; p.F = F; p.o = off2 / M; p.parity = 0; p.reverse = 1;
   switch (M) {
-    case 4: return h4_synthesis_m<4>(p, tables, jlo, kt, B, L, flags, st);
-    case 8: return h4_synthesis_m<8>(p, tables, jlo, kt, B, L, flags, st);
-    case 16: return h4_synthesis_m<16>(p, tables, jlo, kt, B, L, flags, st);
-    case 32: return h4_synthesis_m<32>(p, tables, jlo, kt, B, L, flags, st);
-    case 64: return h4_synthesis_m<64>(p, tables, jlo, kt, B, L, flags, st);
+    case 4: return h4_synthesis_m<4>(p, tables, jlo, kt, B, L, flags, st, io);
+    case 8: return h4_synthesis_m<8>(p, tables, jlo, kt, B, L, flags, st, io);
+    case 16: return h4_synthesis_m<16>(p, tables, jlo, kt, B, L, flags, st, io);
+    case 32: return h4_synthesis_m<32>(p, tables, jlo, kt, B, L, flags, st, io);
+    case 64: return h4_synthesis_m<64>(p, tables, jlo, kt, B, L, flags, st, io);
     default: return PQMF_ERR_UNSUPPORTED;
   }
 }
@@ -388,22 +384,15 @@ int exact_tc_synthesis(const float* s, const float* hist, float* out, float* his
   return trimmed ? pqmf::h16_launch_synthesis<64, 384>(p, st) : pqmf::h16_launch_synthesis<0, 512>(p, st);
 }
 
+// (offline calls try the Hankel-4 kernels before these: h4_route_analysis / h4_route_synthesis)
 int fast_analysis(const float* x, const float* hist, float* y, float* hist_out, const float* tables, int B, long T, long F, int off,
                   int parity, unsigned flags, cudaStream_t st) {
-  if (!(flags & PQMF_FLAG_FOLD) && use_h4(B, F, 16, hist) && h4_analysis_ok(x, y, T, F, 16) && off == 256) {
-    const int e = h4_analysis(x, y, tables, B, T, F, 16, 512, flags, st);
-    if (e != PQMF_ERR_UNSUPPORTED) return e;
-  }
   if (flags & (PQMF_FLAG_EXACT | PQMF_FLAG_NO_FOLD)) return exact_tc_analysis(x, hist, y, hist_out, tables, B, T, F, off, parity, flags, st);
   return pqmf::fast16_analysis(x, hist, y, hist_out, tables, B, T, F, off, parity, flags, st);
 }
 
 int fast_synthesis(const float* s, const float* hist, float* out, float* hist_out, const float* tables, int B, long F, int off2,
                    int parity, unsigned flags, cudaStream_t st) {
-  if (!(flags & PQMF_FLAG_FOLD) && use_h4(B, F, 16, hist) && h4_synthesis_ok(s, out, F)) {
-    const int e = h4_synthesis(s, out, tables, B, F, off2, 16, 512, flags, st);
-    if (e != PQMF_ERR_UNSUPPORTED) return e;
-  }
   if (flags & (PQMF_FLAG_EXACT | PQMF_FLAG_NO_FOLD)) return exact_tc_synthesis(s, hist, out, hist_out, tables, B, F, off2, parity, flags, st);
   return pqmf::fast16_synthesis(s, hist, out, hist_out, tables, B, F, off2, parity, flags, st);
 }
@@ -415,6 +404,39 @@ bool use_fast(int M, int L, const float* tables, unsigned flags) {
 // functions use the direct form); PQMF_FLAG_EXACT keeps them but runs every correction term
 bool use_h4_family(int M, int L, const float* tables, unsigned flags) {
   return tables != nullptr && !(flags & (PQMF_FLAG_NO_SIGN | PQMF_FLAG_FOLD | PQMF_FLAG_FP32)) && h4_family(M, L);
+}
+
+// ---- which kernels an offline call runs: the offline Hankel-4 kernels exactly when these say so and the buffers are aligned for
+//      them; everything else (n_band 16: the fold / Hankel-16 kernels; other band counts: the direct form) comes after.  The fp32 and
+//      the half-precision entry points both decide here, so a half-precision call runs natively exactly where the fp32 call on its
+//      widened input runs the same kernels with the same trims -- which is what makes the two bit-identical.
+//      (n_band 16 / L 512: fast_analysis's shape checks, hankel16_analysis_ok, are implied.) ----
+bool h4_route_analysis(int B, long T, long F, int M, int L, const float* tables, unsigned flags) {
+  const bool shape = T > 0 && (T % M) == 0 && (T % 8) == 0 && F == T / M && use_h4(B, F, M, nullptr);
+  if (use_fast(M, L, tables, flags)) return shape && !(flags & PQMF_FLAG_FOLD);
+  return !pqmf::hankel16_supported(M, L) && use_h4_family(M, L, tables, flags) && shape;
+}
+bool h4_route_synthesis(int B, long F, int M, int L, const float* tables, unsigned flags) {
+  const bool shape = F > 0 && (F & 3) == 0 && use_h4(B, F, M, nullptr);
+  if (use_fast(M, L, tables, flags)) return shape && !(flags & PQMF_FLAG_FOLD);
+  return !pqmf::hankel16_supported(M, L) && use_h4_family(M, L, tables, flags) && shape;
+}
+// fp32 buffers: 256-bit signal loads / stores, 128-bit sub-band loads / stores
+bool h4_aligned_f32(const void* signal, const void* bands) { return ((uintptr_t)signal % 32) == 0 && ((uintptr_t)bands % 16) == 0; }
+// half-precision buffers: 128-bit signal loads / stores; 64-bit sub-band loads, up to 128-bit sub-band stores
+bool h4_aligned_half(const void* signal, const void* bands) { return (((uintptr_t)signal | (uintptr_t)bands) % 16) == 0; }
+// the half-precision instantiations exist for the unsplit banks, as CTA pairs
+bool half_analysis_native(const void* x, const void* y, int B, long T, long F, int M, int L, const float* tables, unsigned flags) {
+  return h4_route_analysis(B, T, F, M, L, tables, flags) && !(flags & PQMF_FLAG_H4_SPLIT) && h4_aligned_half(x, y);
+}
+bool half_synthesis_native(const void* s, const void* out, int B, long F, int M, int L, const float* tables, unsigned flags) {
+  return h4_route_synthesis(B, F, M, L, tables, flags) && !(flags & PQMF_FLAG_H4_SPLIT) && h4_aligned_half(out, s);
+}
+bool half_io_of(int dtype, pqmf::H4Io& io) {
+  if (dtype == PQMF_DTYPE_F16) io = pqmf::H4Io::F16;
+  else if (dtype == PQMF_DTYPE_BF16) io = pqmf::H4Io::BF16;
+  else return false;
+  return true;
 }
 
 // ---- chunk schedule of the host-buffer entry points (host arithmetic only; exported as pqmf_host_chunk_plan for the tests) ----
@@ -739,12 +761,12 @@ int pqmf_analysis_f32(const float* x, float* y, const float* hk, const float* ta
   if (B == 0 || n_frames == 0) return PQMF_OK;
   if (!x || !y || !hk) return PQMF_ERR_ARG;
   cudaStream_t st = (cudaStream_t)stream;
-  if (use_fast(M, L, tables, flags) && pqmf::hankel16_analysis_ok(x, y, T, n_frames)) {
-    int e = fast_analysis(x, nullptr, y, nullptr, tables, B, T, n_frames, L / 2, 0, flags, st);
+  if (h4_route_analysis(B, T, n_frames, M, L, tables, flags) && h4_aligned_f32(x, y)) {
+    int e = h4_analysis(x, y, tables, B, T, n_frames, M, L, flags, st);
     if (e != PQMF_ERR_UNSUPPORTED) { g_launches += (e == 0); return e; }
   }
-  if (!pqmf::hankel16_supported(M, L) && use_h4_family(M, L, tables, flags) && h4_analysis_ok(x, y, T, n_frames, M) && use_h4(B, n_frames, M, nullptr)) {
-    int e = h4_analysis(x, y, tables, B, T, n_frames, M, L, flags, st);
+  if (use_fast(M, L, tables, flags) && pqmf::hankel16_analysis_ok(x, y, T, n_frames)) {
+    int e = fast_analysis(x, nullptr, y, nullptr, tables, B, T, n_frames, L / 2, 0, flags, st);
     if (e != PQMF_ERR_UNSUPPORTED) { g_launches += (e == 0); return e; }
   }
   return analysis_direct(x, nullptr, y, hk, B, T, n_frames, M, L, L / 2, 0, (flags & PQMF_FLAG_NO_SIGN) ? 1 : 0, st);
@@ -757,12 +779,12 @@ int pqmf_synthesis_f32(const float* s, float* out, const float* hk, const float*
   if (!s || !out || !hk) return PQMF_ERR_ARG;
   cudaStream_t st = (cudaStream_t)stream;
   const int off2 = L / 2 - delay_frames * M;
-  if (use_fast(M, L, tables, flags) && pqmf::hankel16_synthesis_ok(s, out, n_frames)) {
-    int e = fast_synthesis(s, nullptr, out, nullptr, tables, B, n_frames, off2, 0, flags, st);
+  if (h4_route_synthesis(B, n_frames, M, L, tables, flags) && h4_aligned_f32(out, s)) {
+    int e = h4_synthesis(s, out, tables, B, n_frames, off2, M, L, flags, st);
     if (e != PQMF_ERR_UNSUPPORTED) { g_launches += (e == 0); return e; }
   }
-  if (!pqmf::hankel16_supported(M, L) && use_h4_family(M, L, tables, flags) && h4_synthesis_ok(s, out, n_frames) && use_h4(B, n_frames, M, nullptr)) {
-    int e = h4_synthesis(s, out, tables, B, n_frames, off2, M, L, flags, st);
+  if (use_fast(M, L, tables, flags) && pqmf::hankel16_synthesis_ok(s, out, n_frames)) {
+    int e = fast_synthesis(s, nullptr, out, nullptr, tables, B, n_frames, off2, 0, flags, st);
     if (e != PQMF_ERR_UNSUPPORTED) { g_launches += (e == 0); return e; }
   }
   return synthesis_direct(s, nullptr, out, hk, B, n_frames, M, L, off2, 0, (flags & PQMF_FLAG_NO_SIGN) ? 1 : 0, st);
@@ -950,6 +972,83 @@ int pqmf_reconstruct_f32(const float* x, float* out, float* scratch, size_t scra
     int e = pqmf_analysis_f32(x + (size_t)r0 * T, scratch, hk, tables, n, T, n_frames, M, L, flags, stream);
     if (e) return e;
     e = pqmf_synthesis_f32(scratch, out + (size_t)r0 * M * n_frames, hk, tables, n, n_frames, M, L, delay_frames, flags, stream);
+    if (e) return e;
+  }
+  return PQMF_OK;
+}
+
+// ---- half-precision I/O: the offline Hankel-4 kernels with fp16 / bf16 loads and stores (half_io.cuh), wherever the fp32 call
+//      would run them (h4_route_*); every other call is refused before anything is launched ----
+int pqmf_analysis_x(const void* x, void* y, const float* hk, const float* tables, int B, long T, long n_frames, int M, int L, unsigned flags,
+                    int dtype, pqmf_stream_t stream) {
+  if (dtype == PQMF_DTYPE_F32)
+    return pqmf_analysis_f32(static_cast<const float*>(x), static_cast<float*>(y), hk, tables, B, T, n_frames, M, L, flags, stream);
+  pqmf::H4Io io;
+  if (!half_io_of(dtype, io) || bad_dims(B, T, M, L) || n_frames < 0) return PQMF_ERR_ARG;
+  if (B == 0 || n_frames == 0) return PQMF_OK;
+  if (!x || !y || !hk) return PQMF_ERR_ARG;
+  if (!half_analysis_native(x, y, B, T, n_frames, M, L, tables, flags)) return PQMF_ERR_UNSUPPORTED;
+  const int e = h4_analysis(x, y, tables, B, T, n_frames, M, L, flags, (cudaStream_t)stream, pqmf::PcmIn{nullptr, 1, 0}, io);
+  g_launches += (e == 0);
+  return e;
+}
+
+int pqmf_synthesis_x(const void* s, void* out, const float* hk, const float* tables, int B, long n_frames, int M, int L, int delay_frames,
+                     unsigned flags, int dtype, pqmf_stream_t stream) {
+  if (dtype == PQMF_DTYPE_F32)
+    return pqmf_synthesis_f32(static_cast<const float*>(s), static_cast<float*>(out), hk, tables, B, n_frames, M, L, delay_frames, flags, stream);
+  pqmf::H4Io io;
+  if (!half_io_of(dtype, io) || bad_dims(B, n_frames, M, L) || delay_frames < 0 || delay_frames > 1) return PQMF_ERR_ARG;
+  if (B == 0 || n_frames == 0) return PQMF_OK;
+  if (!s || !out || !hk) return PQMF_ERR_ARG;
+  if (!half_synthesis_native(s, out, B, n_frames, M, L, tables, flags)) return PQMF_ERR_UNSUPPORTED;
+  const int e = h4_synthesis(s, out, tables, B, n_frames, L / 2 - delay_frames * M, M, L, flags, (cudaStream_t)stream, nullptr, 1, io);
+  g_launches += (e == 0);
+  return e;
+}
+
+int pqmf_roundtrip_x(const void* x, void* y, void* out, const float* hk, const float* tables, int B, long T, long n_frames, int M, int L,
+                     int delay_frames, unsigned flags, int dtype, pqmf_stream_t stream) {
+  if (dtype == PQMF_DTYPE_F32)
+    return pqmf_roundtrip_f32(static_cast<const float*>(x), static_cast<float*>(y), static_cast<float*>(out), hk, tables, B, T, n_frames, M, L,
+                              delay_frames, flags, stream);
+  pqmf::H4Io io;
+  if (!half_io_of(dtype, io) || bad_dims(B, T, M, L) || n_frames < 0 || delay_frames < 0 || delay_frames > 1) return PQMF_ERR_ARG;
+  if (B == 0 || n_frames == 0) return PQMF_OK;
+  if (!x || !y || !out || !hk) return PQMF_ERR_ARG;
+  // both directions native, or neither is launched
+  if (!half_analysis_native(x, y, B, T, n_frames, M, L, tables, flags) || !half_synthesis_native(y, out, B, n_frames, M, L, tables, flags))
+    return PQMF_ERR_UNSUPPORTED;
+  const int e = pqmf_analysis_x(x, y, hk, tables, B, T, n_frames, M, L, flags, dtype, stream);
+  if (e) return e;
+  return pqmf_synthesis_x(y, out, hk, tables, B, n_frames, M, L, delay_frames, flags, dtype, stream);
+}
+
+// the sub-bands of a chunk are half-width here: the scratch sized for fp32 sub-bands holds them with room to spare
+int pqmf_reconstruct_x(const void* x, void* out, void* scratch, size_t scratch_bytes, const float* hk, const float* tables, int B, long T,
+                       long n_frames, int M, int L, int delay_frames, unsigned flags, int dtype, pqmf_stream_t stream) {
+  if (dtype == PQMF_DTYPE_F32)
+    return pqmf_reconstruct_f32(static_cast<const float*>(x), static_cast<float*>(out), static_cast<float*>(scratch), scratch_bytes, hk, tables, B, T,
+                                n_frames, M, L, delay_frames, flags, stream);
+  pqmf::H4Io io;
+  if (!half_io_of(dtype, io) || bad_dims(B, T, M, L) || n_frames < 0 || delay_frames < 0 || delay_frames > 1) return PQMF_ERR_ARG;
+  if (B == 0 || n_frames == 0) return PQMF_OK;
+  if (!x || !out || !hk || !scratch || scratch_bytes < pqmf_reconstruct_scratch_bytes(B, T, n_frames, M)) return PQMF_ERR_ARG;
+  const long rows = recon_chunk_rows(B, T);
+  const uint16_t* xh = static_cast<const uint16_t*>(x);
+  uint16_t* oh = static_cast<uint16_t*>(out);
+  // every chunk native in both directions (a short last chunk may have too few tiles), or nothing is launched
+  for (long r0 = 0; r0 < B; r0 += rows) {
+    const int n = (int)(B - r0 < rows ? B - r0 : rows);
+    if (!half_analysis_native(xh + (size_t)r0 * T, scratch, n, T, n_frames, M, L, tables, flags) ||
+        !half_synthesis_native(scratch, oh + (size_t)r0 * M * n_frames, n, n_frames, M, L, tables, flags))
+      return PQMF_ERR_UNSUPPORTED;
+  }
+  for (long r0 = 0; r0 < B; r0 += rows) {
+    const int n = (int)(B - r0 < rows ? B - r0 : rows);
+    int e = pqmf_analysis_x(xh + (size_t)r0 * T, scratch, hk, tables, n, T, n_frames, M, L, flags, dtype, stream);
+    if (e) return e;
+    e = pqmf_synthesis_x(scratch, oh + (size_t)r0 * M * n_frames, hk, tables, n, n_frames, M, L, delay_frames, flags, dtype, stream);
     if (e) return e;
   }
   return PQMF_OK;

@@ -246,6 +246,12 @@ __device__ __forceinline__ float4 ldg128_na(const float4* p) {
   asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p));
   return v;
 }
+// the same, 64 bits (four half-precision frames); p must be 8-byte aligned
+__device__ __forceinline__ float2 ldg64_na(const void* p) {
+  float2 v;
+  asm volatile("ld.global.nc.L1::no_allocate.v2.f32 {%0,%1}, [%2];" : "=f"(v.x), "=f"(v.y) : "l"(p));
+  return v;
+}
 
 // 128-bit load through L2 (no L1): data written earlier by THIS kernel (the fused streaming step reads back its own sub-bands)
 __device__ __forceinline__ float4 ldg128_cg(const float4* p) {

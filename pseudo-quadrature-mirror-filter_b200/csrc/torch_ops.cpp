@@ -26,6 +26,21 @@ void check_f32_cuda(const at::Tensor& t, const char* name) {
   TORCH_CHECK(t.scalar_type() == at::kFloat, name, " must be float32, got ", t.scalar_type());
 }
 
+// element type of a signal / sub-band tensor of the offline ops: float32, or a half-precision type (the _x entry points of the C ABI)
+int io_dtype(const at::Tensor& t, const char* name) {
+  TORCH_CHECK(t.is_cuda(), name, " must be a CUDA tensor (pqmf_b200 has no CPU fallback)");
+  switch (t.scalar_type()) {
+    case at::kFloat: return PQMF_DTYPE_F32;
+    case at::kHalf: return PQMF_DTYPE_F16;
+    case at::kBFloat16: return PQMF_DTYPE_BF16;
+    default: TORCH_CHECK(false, name, " must be float32, float16 or bfloat16, got ", t.scalar_type());
+  }
+  return -1;
+}
+// a half-precision call the library has no native kernel for (PQMF_ERR_UNSUPPORTED, nothing launched): the caller widens to fp32, runs
+// the fp32 op and rounds the result -- bit-identical to the native path by construction
+bool staged(int rc, int dtype) { return rc == PQMF_ERR_UNSUPPORTED && dtype != PQMF_DTYPE_F32; }
+
 const float* tables_ptr(const at::Tensor& tables, const at::Tensor& like) {
   if (tables.numel() == 0) return nullptr;
   check_f32_cuda(tables, "tables");
@@ -46,8 +61,9 @@ Bank bank_of(const at::Tensor& hk, const at::Tensor& like) {
 }
 
 // x [B, C, T] -> [B, C*M, n_frames]      (reference: C == 1; C > 1 is folded into the batch)
+// float32 / float16 / bfloat16 in, the same type out
 at::Tensor analysis(const at::Tensor& x, const at::Tensor& hk, const at::Tensor& tables, int64_t n_frames, int64_t flags) {
-  check_f32_cuda(x, "x");
+  const int dtype = io_dtype(x, "x");
   TORCH_CHECK(x.dim() == 3, "pqmf analysis expects [batch, channels, time], got ", x.dim(), " dims");
   const Bank bank = bank_of(hk, x);
   c10::cuda::CUDAGuard guard(x.device());
@@ -56,16 +72,16 @@ at::Tensor analysis(const at::Tensor& x, const at::Tensor& hk, const at::Tensor&
   TORCH_CHECK(n_frames >= 0 && B < (1LL << 31), "bad sizes");
   at::Tensor y = at::empty({xc.size(0), xc.size(1) * bank.M, n_frames}, xc.options());
   if (y.numel() == 0) return y;
-  check_rc(pqmf_analysis_f32(xc.data_ptr<float>(), y.data_ptr<float>(), bank.ptr, tables_ptr(tables, x), (int)B, (long)T,
-                             (long)n_frames, (int)bank.M, (int)bank.L, (unsigned)flags,
-                             (pqmf_stream_t)at::cuda::getCurrentCUDAStream().stream()),
-           "pqmf_analysis_f32");
+  const int rc = pqmf_analysis_x(xc.data_ptr(), y.data_ptr(), bank.ptr, tables_ptr(tables, x), (int)B, (long)T, (long)n_frames, (int)bank.M,
+                                 (int)bank.L, (unsigned)flags, dtype, (pqmf_stream_t)at::cuda::getCurrentCUDAStream().stream());
+  if (staged(rc, dtype)) return analysis(xc.to(at::kFloat), hk, tables, n_frames, flags).to(x.scalar_type());
+  check_rc(rc, "pqmf_analysis_x");
   return y;
 }
 
 // s [B, C*M, F] -> [B, C, M*F]
 at::Tensor synthesis(const at::Tensor& s, const at::Tensor& hk, const at::Tensor& tables, int64_t delay_frames, int64_t flags) {
-  check_f32_cuda(s, "s");
+  const int dtype = io_dtype(s, "s");
   TORCH_CHECK(s.dim() == 3, "pqmf synthesis expects [batch, n_band, frames], got ", s.dim(), " dims");
   const Bank bank = bank_of(hk, s);
   TORCH_CHECK(s.size(1) % bank.M == 0, "sub-band tensor has ", s.size(1), " channels, expected a multiple of n_band=", bank.M);
@@ -75,17 +91,17 @@ at::Tensor synthesis(const at::Tensor& s, const at::Tensor& hk, const at::Tensor
   TORCH_CHECK(B < (1LL << 31), "bad sizes");
   at::Tensor out = at::empty({sc.size(0), C, bank.M * F}, sc.options());
   if (out.numel() == 0) return out;
-  check_rc(pqmf_synthesis_f32(sc.data_ptr<float>(), out.data_ptr<float>(), bank.ptr, tables_ptr(tables, s), (int)B, (long)F,
-                              (int)bank.M, (int)bank.L, (int)delay_frames, (unsigned)flags,
-                              (pqmf_stream_t)at::cuda::getCurrentCUDAStream().stream()),
-           "pqmf_synthesis_f32");
+  const int rc = pqmf_synthesis_x(sc.data_ptr(), out.data_ptr(), bank.ptr, tables_ptr(tables, s), (int)B, (long)F, (int)bank.M, (int)bank.L,
+                                  (int)delay_frames, (unsigned)flags, dtype, (pqmf_stream_t)at::cuda::getCurrentCUDAStream().stream());
+  if (staged(rc, dtype)) return synthesis(sc.to(at::kFloat), hk, tables, delay_frames, flags).to(s.scalar_type());
+  check_rc(rc, "pqmf_synthesis_x");
   return out;
 }
 
 // x [B, C, T] -> (out [B, C, M*n_frames], y [B, C*M, n_frames]): forward then inverse in one call (pqmf_roundtrip_f32)
 std::tuple<at::Tensor, at::Tensor> roundtrip(const at::Tensor& x, const at::Tensor& hk, const at::Tensor& tables, int64_t n_frames,
                                              int64_t delay_frames, int64_t flags) {
-  check_f32_cuda(x, "x");
+  const int dtype = io_dtype(x, "x");
   TORCH_CHECK(x.dim() == 3, "pqmf roundtrip expects [batch, channels, time], got ", x.dim(), " dims");
   const Bank bank = bank_of(hk, x);
   c10::cuda::CUDAGuard guard(x.device());
@@ -95,10 +111,14 @@ std::tuple<at::Tensor, at::Tensor> roundtrip(const at::Tensor& x, const at::Tens
   at::Tensor y = at::empty({xc.size(0), xc.size(1) * bank.M, n_frames}, xc.options());
   at::Tensor out = at::empty({xc.size(0), xc.size(1), bank.M * n_frames}, xc.options());
   if (y.numel() == 0) return {out, y};
-  check_rc(pqmf_roundtrip_f32(xc.data_ptr<float>(), y.data_ptr<float>(), out.data_ptr<float>(), bank.ptr, tables_ptr(tables, x), (int)B,
-                              (long)T, (long)n_frames, (int)bank.M, (int)bank.L, (int)delay_frames, (unsigned)flags,
-                              (pqmf_stream_t)at::cuda::getCurrentCUDAStream().stream()),
-           "pqmf_roundtrip_f32");
+  const int rc = pqmf_roundtrip_x(xc.data_ptr(), y.data_ptr(), out.data_ptr(), bank.ptr, tables_ptr(tables, x), (int)B, (long)T, (long)n_frames,
+                                  (int)bank.M, (int)bank.L, (int)delay_frames, (unsigned)flags, dtype,
+                                  (pqmf_stream_t)at::cuda::getCurrentCUDAStream().stream());
+  if (staged(rc, dtype)) {  // direction by direction (each native where it can be); the synthesis reads the rounded sub-bands
+    at::Tensor ys = analysis(xc, hk, tables, n_frames, flags);
+    return {synthesis(ys, hk, tables, delay_frames, flags), ys};
+  }
+  check_rc(rc, "pqmf_roundtrip_x");
   return {out, y};
 }
 
@@ -140,7 +160,7 @@ at::Tensor synthesis_pcm16(const at::Tensor& s, const at::Tensor& hk, const at::
 
 // x [B, C, T] -> out [B, C, M * n_frames] only (pqmf_reconstruct_f32): the sub-bands live in a scratch buffer of one row chunk
 at::Tensor reconstruct(const at::Tensor& x, const at::Tensor& hk, const at::Tensor& tables, int64_t n_frames, int64_t delay_frames, int64_t flags) {
-  check_f32_cuda(x, "x");
+  const int dtype = io_dtype(x, "x");
   TORCH_CHECK(x.dim() == 3, "pqmf reconstruct expects [batch, channels, time], got ", x.dim(), " dims");
   const Bank bank = bank_of(hk, x);
   c10::cuda::CUDAGuard guard(x.device());
@@ -150,11 +170,15 @@ at::Tensor reconstruct(const at::Tensor& x, const at::Tensor& hk, const at::Tens
   at::Tensor out = at::empty({xc.size(0), xc.size(1), bank.M * n_frames}, xc.options());
   if (out.numel() == 0) return out;
   const size_t bytes = pqmf_reconstruct_scratch_bytes((int)B, (long)T, (long)n_frames, (int)bank.M);
-  at::Tensor scratch = at::empty({(int64_t)(bytes / sizeof(float))}, xc.options());
-  check_rc(pqmf_reconstruct_f32(xc.data_ptr<float>(), out.data_ptr<float>(), scratch.data_ptr<float>(), bytes, bank.ptr, tables_ptr(tables, x), (int)B,
-                                (long)T, (long)n_frames, (int)bank.M, (int)bank.L, (int)delay_frames, (unsigned)flags,
-                                (pqmf_stream_t)at::cuda::getCurrentCUDAStream().stream()),
-           "pqmf_reconstruct_f32");
+  at::Tensor scratch = at::empty({(int64_t)(bytes / sizeof(float))}, xc.options().dtype(at::kFloat));  // sized for fp32 sub-bands: holds either width
+  const int rc = pqmf_reconstruct_x(xc.data_ptr(), out.data_ptr(), scratch.data_ptr(), bytes, bank.ptr, tables_ptr(tables, x), (int)B, (long)T,
+                                    (long)n_frames, (int)bank.M, (int)bank.L, (int)delay_frames, (unsigned)flags, dtype,
+                                    (pqmf_stream_t)at::cuda::getCurrentCUDAStream().stream());
+  if (staged(rc, dtype)) {  // what process() computes: the synthesis of the rounded sub-bands
+    scratch.reset();
+    return synthesis(analysis(xc, hk, tables, n_frames, flags), hk, tables, delay_frames, flags);
+  }
+  check_rc(rc, "pqmf_reconstruct_x");
   return out;
 }
 
@@ -301,11 +325,18 @@ at::Tensor call_synthesis(const at::Tensor& s, const at::Tensor& hk, const at::T
 struct GradScale {
   at::Tensor down, up;  // 0-dim fp32 tensors 2^-e, 2^e
 };
+// (the scale is computed in fp32 whatever g's type -- the clamp bounds do not exist in fp16 -- and multiplies g as a 0-dim tensor, so the
+// scaled gradient keeps g's type)
 GradScale grad_scale(const at::Tensor& g) {
-  const at::Tensor amax = at::clamp(g.detach().abs().amax(), 1e-30, 1e30);
+  const at::Tensor amax = at::clamp(g.detach().abs().amax().to(at::kFloat), 1e-30, 1e30);
   const at::Tensor e = at::floor(at::log2(amax));
   return {at::exp2(-e), at::exp2(e)};
 }
+
+// The backward passes below normalise the gradient so that the kernels' outputs are near 1, and scale back afterwards.  In float32 and
+// bfloat16 the scaling back is exact (fp32's exponent range); in float16 it can pass through the subnormal range, where a result already
+// rounded at the kernel's output would lose bits.  So fp16 gradients are widened here and the fp32 result is rounded once at the end.
+at::Tensor backward_in(const at::Tensor& g) { return g.scalar_type() == at::kHalf ? g.to(at::kFloat) : g; }
 
 struct AnalysisFn : public torch::autograd::Function<AnalysisFn> {
   static at::Tensor forward(torch::autograd::AutogradContext* ctx, const at::Tensor& x, const at::Tensor& hk, const at::Tensor& tables,
@@ -320,17 +351,18 @@ struct AnalysisFn : public torch::autograd::Function<AnalysisFn> {
     const auto saved = ctx->get_saved_variables();
     const at::Tensor &hk = saved[0], &tables = saved[1];
     const int64_t T = ctx->saved_data["T"].toInt(), flags = ctx->saved_data["flags"].toInt(), M = hk.size(0);
-    at::Tensor gy = grads[0].contiguous();
+    const auto dtype = grads[0].scalar_type();
+    at::Tensor gy = backward_in(grads[0].contiguous());
     const int64_t F = gy.size(-1), need = (T + M - 1) / M;   // frames whose synthesis output covers [0, T)
     if (need > F) gy = at::constant_pad_nd(gy, {0, need - F});
     if (flags & PQMF_FLAG_FP32) {
       at::Tensor gx = call_synthesis(gy, hk, tables, 0, flags);
-      return {gx.slice(-1, 0, T) * (1.0 / (double)M), at::Tensor(), at::Tensor(), at::Tensor(), at::Tensor()};
+      return {(gx.slice(-1, 0, T) * (1.0 / (double)M)).to(dtype), at::Tensor(), at::Tensor(), at::Tensor(), at::Tensor()};
     }
     const GradScale sc = grad_scale(gy);
     at::Tensor gx = call_synthesis(gy * sc.down, hk, tables, 0, flags);
     gx = gx.slice(-1, 0, T) * (sc.up * (1.0 / (double)M));
-    return {gx, at::Tensor(), at::Tensor(), at::Tensor(), at::Tensor()};
+    return {gx.to(dtype), at::Tensor(), at::Tensor(), at::Tensor(), at::Tensor()};
   }
 };
 
@@ -347,7 +379,8 @@ struct SynthesisFn : public torch::autograd::Function<SynthesisFn> {
     const auto saved = ctx->get_saved_variables();
     const at::Tensor &hk = saved[0], &tables = saved[1];
     const int64_t d = ctx->saved_data["delay"].toInt(), flags = ctx->saved_data["flags"].toInt(), M = hk.size(0);
-    const at::Tensor g = grads[0].contiguous();          // [B, C, M F]
+    const auto dtype = grads[0].scalar_type();
+    const at::Tensor g = backward_in(grads[0].contiguous());          // [B, C, M F]
     const int64_t F = g.size(-1) / M;
     const bool plain = (flags & PQMF_FLAG_FP32) != 0;
     GradScale sc;
@@ -356,12 +389,14 @@ struct SynthesisFn : public torch::autograd::Function<SynthesisFn> {
     if (d > 0) {
       a = a.slice(-1, d, F + d);
       if (!(flags & PQMF_FLAG_NO_SIGN) && (d & 1)) {
-        const at::Tensor sign = 1.0 - 2.0 * at::arange(a.size(1), a.options()).remainder((double)M).remainder(2.0);
+        // counted in fp32 (bf16 cannot count past 256), applied in a's type
+        const at::Tensor sign =
+            (1.0 - 2.0 * at::arange(a.size(1), a.options().dtype(at::kFloat)).remainder((double)M).remainder(2.0)).to(a.scalar_type());
         a = a * sign.view({1, -1, 1});
       }
     }
     a = plain ? a * (double)M : a * (sc.up * (double)M);
-    return {a, at::Tensor(), at::Tensor(), at::Tensor(), at::Tensor()};
+    return {a.to(dtype), at::Tensor(), at::Tensor(), at::Tensor(), at::Tensor()};
   }
 };
 

@@ -13,6 +13,13 @@ Differences that are deliberate (SURVEY.md A.6):
 * both classes are TorchScript-scriptable (the reference's plain PQMF is not);
 * ``CachedPQMF`` has an explicit streaming mode with caller-visible state instead of the hidden
   global switch of the third-party ``cached_conv`` package (``streaming=True`` / ``forward_stream``).
+
+Precision: ``forward`` / ``inverse`` / ``process`` / ``reconstruct`` and the free functions accept float32, float16 and bfloat16
+signals and sub-bands and return the input's dtype: ``forward(x_d)`` is bit-equal to ``forward(x_d.float()).to(d)`` (exact widening,
+fp32 accumulation, round-to-nearest-even output; the large offline calls run on half-precision kernels, the rest widen, run the
+fp32 kernels and round).  The input dtype and the module's dtype are independent: ``.half()`` / ``.to(torch.bfloat16)`` cast ``hk`` and
+``h`` as the reference's module casts its buffers, and the arithmetic then uses that rounded bank, accumulated in fp32.  Other dtypes
+(float64 included) raise.  The streaming, int16-PCM and per-band entry points take float32 sub-bands / signals only.
 """
 from __future__ import annotations
 
@@ -27,6 +34,8 @@ from . import _lib
 from .design import center_pad_next_pow_2, get_prototype, get_qmf_bank, make_odd
 
 _EMPTY = torch.zeros(0)
+# fp32 buffers that are not numbers of the bank: module casts move them to the new device but never change their dtype (PQMF._apply)
+_FP32_BUFFERS = ("_tables", "_x_state", "_s_state")
 
 # largest |hk - g (x) C| accepted for the fold + modulation factorisation (SURVEY.md A.3: 1.7e-7 for the
 # reference's own banks).  A bank that fails it (e.g. a hand-edited hk) silently uses the direct-form kernels.
@@ -59,23 +68,23 @@ def polyphase_forward(x: torch.Tensor, hk: torch.Tensor, rearrange_filter: bool 
     hk = _bank_2d(hk, rearrange_filter, False)
     if x.shape[-1] % hk.shape[0] != 0:
         raise RuntimeError(f"polyphase_forward: T={x.shape[-1]} is not a multiple of n_band={hk.shape[0]}")
-    return torch.ops.pqmf_b200.analysis(x, hk, _EMPTY, x.shape[-1] // hk.shape[0], _lib.PQMF_FLAG_NO_SIGN)
+    return torch.ops.pqmf_b200.analysis(x, hk.float(), _EMPTY, x.shape[-1] // hk.shape[0], _lib.PQMF_FLAG_NO_SIGN)
 
 
 def classic_forward(x: torch.Tensor, hk: torch.Tensor) -> torch.Tensor:
     """Analysis WITHOUT the sign mask, any T (reference pqmf.py:160-177). x [B,1,T] -> [B,M,floor(T/M)]."""
-    return torch.ops.pqmf_b200.analysis(x, hk, _EMPTY, x.shape[-1] // hk.shape[0], _lib.PQMF_FLAG_NO_SIGN)
+    return torch.ops.pqmf_b200.analysis(x, hk.float(), _EMPTY, x.shape[-1] // hk.shape[0], _lib.PQMF_FLAG_NO_SIGN)
 
 
 def polyphase_inverse(x: torch.Tensor, hk: torch.Tensor, rearrange_filter: bool = True) -> torch.Tensor:
     """Synthesis WITHOUT the sign mask (reference pqmf.py:133-157). x [B,M,F] -> [B,1,M*F]."""
     hk = _bank_2d(hk, rearrange_filter, True)
-    return torch.ops.pqmf_b200.synthesis(x, hk, _EMPTY, 0, _lib.PQMF_FLAG_NO_SIGN)
+    return torch.ops.pqmf_b200.synthesis(x, hk.float(), _EMPTY, 0, _lib.PQMF_FLAG_NO_SIGN)
 
 
 def classic_inverse(x: torch.Tensor, hk: torch.Tensor) -> torch.Tensor:
     """Synthesis WITHOUT the sign mask (reference pqmf.py:180-199; same function as polyphase_inverse)."""
-    return torch.ops.pqmf_b200.synthesis(x, hk, _EMPTY, 0, _lib.PQMF_FLAG_NO_SIGN)
+    return torch.ops.pqmf_b200.synthesis(x, hk.float(), _EMPTY, 0, _lib.PQMF_FLAG_NO_SIGN)
 
 
 def _refresh_after_load(module, _incompatible_keys):
@@ -98,6 +107,8 @@ class PQMF(nn.Module):
                   reference's ``conv1d`` -- no range limit, fp32's relative accuracy at any signal level, ~20x slower
     check_range : debug aid.  The tensor-core kernels assume audio-like magnitudes; with ``check_range=True`` every call first checks
                   max|x| (one host sync) and routes inputs beyond +-6e4 or entirely below 1e-6 to the fp32 kernels
+
+    Signals and sub-bands may be float32, float16 or bfloat16; every output has its input's dtype (see the module docstring).
     """
 
     def __init__(self, attenuation, n_band, polyphase=True, n_channels=1, exact=False, fp32=False, check_range=False):
@@ -120,9 +131,25 @@ class PQMF(nn.Module):
         self.refresh_tables()
         self.register_load_state_dict_post_hook(_refresh_after_load)
 
+    def _apply(self, fn, recurse=True):
+        """Module casts and moves.  ``hk`` and ``h`` follow a cast (``.half()``, ``.to(torch.bfloat16)``), as the reference's buffers
+        do, and the tables are then re-derived from the bank as it now is.  The fp32 buffers that are not numbers of the bank follow
+        the device only: ``_tables`` holds packed fp16 images, which a numeric cast would corrupt, and the streaming state stays fp32.
+        A pure device move keeps the tables as they are (bit-equal, not rebuilt)."""
+        hk_dtype = self.hk.dtype
+        keep = {name: self._buffers[name] for name in _FP32_BUFFERS if self._buffers.get(name) is not None}
+        super()._apply(fn, recurse)
+        for name, buf in keep.items():
+            moved = self._buffers[name]
+            if moved is not None and moved.dtype != buf.dtype:
+                self._buffers[name] = buf.to(moved.device)
+        if self.hk.dtype != hk_dtype:
+            self.refresh_tables()
+        return self
+
     @torch.jit.unused
     def refresh_tables(self) -> None:
-        """(Re)derive the fast-path coefficient tables from the current ``hk`` / ``h`` buffers."""
+        """(Re)derive the fast-path coefficient tables from the current ``hk`` / ``h`` buffers (as fp32: the tables are always fp32)."""
         tables, residual, fast_flags = _lib.build_tables(self.hk, self.h)
         if tables.numel() and not (residual <= _FOLD_RESIDUAL_LIMIT):
             # bank is not window x cosine (e.g. a hand-edited hk was loaded): the fold + modulation kernels do not apply, the
@@ -150,7 +177,7 @@ class PQMF(nn.Module):
         t = x.shape[-1]
         if self.polyphase and t % self.n_band != 0:
             raise RuntimeError("polyphase PQMF needs the number of samples to be a multiple of n_band")
-        return torch.ops.pqmf_b200.analysis(x, self.hk, self._tables, t // self.n_band, self._call_flags(x))
+        return torch.ops.pqmf_b200.analysis(x, self.hk.float(), self._tables, t // self.n_band, self._call_flags(x))
 
     @torch.jit.export
     def inverse(self, x: torch.Tensor) -> torch.Tensor:
@@ -159,7 +186,7 @@ class PQMF(nn.Module):
             raise RuntimeError("PQMF.inverse expects a 3-D tensor [batch, n_band, frames]")
         if self.n_band == 1:
             return x
-        return torch.ops.pqmf_b200.synthesis(x, self.hk, self._tables, 0, self._call_flags(x))
+        return torch.ops.pqmf_b200.synthesis(x, self.hk.float(), self._tables, 0, self._call_flags(x))
 
     @torch.jit.export
     def reconstruct(self, x: torch.Tensor) -> torch.Tensor:
@@ -173,7 +200,7 @@ class PQMF(nn.Module):
             return x
         if torch.is_grad_enabled() and x.requires_grad:
             return self.inverse(self.forward(x))
-        return torch.ops.pqmf_b200.reconstruct(x, self.hk, self._tables, self._n_frames_of(x.shape[-1]), self._inverse_delay(), self._flags)
+        return torch.ops.pqmf_b200.reconstruct(x, self.hk.float(), self._tables, self._n_frames_of(x.shape[-1]), self._inverse_delay(), self._flags)
 
     def _n_frames_of(self, t: int) -> int:
         if self.polyphase and t % self.n_band != 0:
@@ -191,7 +218,7 @@ class PQMF(nn.Module):
         t = pcm.shape[1]
         if self.polyphase and t % self.n_band != 0:
             raise RuntimeError("polyphase PQMF needs the number of samples to be a multiple of n_band")
-        return torch.ops.pqmf_b200.analysis_pcm16(pcm, self.hk, self._tables, t // self.n_band, downmix, self._flags)
+        return torch.ops.pqmf_b200.analysis_pcm16(pcm, self.hk.float(), self._tables, t // self.n_band, downmix, self._flags)
 
     @torch.jit.export
     def inverse_pcm16(self, x: torch.Tensor) -> torch.Tensor:
@@ -200,7 +227,7 @@ class PQMF(nn.Module):
         interleave fused into the kernel's stores."""
         if x.dim() != 3:
             raise RuntimeError("inverse_pcm16 expects a 3-D tensor [batch, channels * n_band, frames]")
-        return torch.ops.pqmf_b200.synthesis_pcm16(x, self.hk, self._tables, self._inverse_delay(), self._flags)
+        return torch.ops.pqmf_b200.synthesis_pcm16(x, self.hk.float(), self._tables, self._inverse_delay(), self._flags)
 
     def _inverse_delay(self) -> int:
         return 0
@@ -214,7 +241,7 @@ class PQMF(nn.Module):
         is centre-cropped / zero-padded to ``n_frames``, and the bands are synthesised -- all inside the kernel's loads, without the
         ``cat(dim=1)`` tensor.  Returns ``(signal [B, 1, n_band * n_frames], new prev_tail [n_band, Lx])``.  Pass an empty ``prev_tail``
         (``numel() == 0``) for no cross-fade."""
-        return torch.ops.pqmf_b200.synthesis_bands(bands, self.hk, n_frames, self._inverse_delay(), prev_tail, fade_out, fade_in, self._flags)
+        return torch.ops.pqmf_b200.synthesis_bands(bands, self.hk.float(), n_frames, self._inverse_delay(), prev_tail, fade_out, fade_in, self._flags)
 
     @torch.jit.export
     def process(self, x: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
@@ -231,7 +258,7 @@ class PQMF(nn.Module):
         if torch.is_grad_enabled() and x.requires_grad:  # the fused op has no autograd kernel: same result through the two ops
             y = self.forward(x)
             return self.inverse(y), y
-        return torch.ops.pqmf_b200.roundtrip(x, self.hk, self._tables, t // self.n_band, 0, self._flags)
+        return torch.ops.pqmf_b200.roundtrip(x, self.hk.float(), self._tables, t // self.n_band, 0, self._flags)
 
 
 class _BankConv(nn.Module):
@@ -313,7 +340,7 @@ class CachedPQMF(PQMF):
         if self.streaming:
             return self.forward_stream(x)
         n_frames = (x.shape[-1] + self.n_band - 1) // self.n_band
-        return torch.ops.pqmf_b200.analysis(x, self.hk, self._tables, n_frames, self._call_flags(x))
+        return torch.ops.pqmf_b200.analysis(x, self.hk.float(), self._tables, n_frames, self._call_flags(x))
 
     @torch.jit.export
     def inverse(self, x: torch.Tensor) -> torch.Tensor:
@@ -323,7 +350,7 @@ class CachedPQMF(PQMF):
             return x
         if self.streaming:
             return self.inverse_stream(x)
-        return torch.ops.pqmf_b200.synthesis(x, self.hk, self._tables, 1, self._call_flags(x))
+        return torch.ops.pqmf_b200.synthesis(x, self.hk.float(), self._tables, 1, self._call_flags(x))
 
     @torch.jit.export
     def process(self, x: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
@@ -337,7 +364,7 @@ class CachedPQMF(PQMF):
             y = self.forward(x)
             return self.inverse(y), y
         n_frames = (x.shape[-1] + self.n_band - 1) // self.n_band
-        return torch.ops.pqmf_b200.roundtrip(x, self.hk, self._tables, n_frames, 1, self._flags)
+        return torch.ops.pqmf_b200.roundtrip(x, self.hk.float(), self._tables, n_frames, 1, self._flags)
 
     @torch.jit.export
     def process_stream(self, x: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
@@ -354,7 +381,7 @@ class CachedPQMF(PQMF):
             self._s_state = torch.zeros(2, rows, length, device=x.device)
             self._s_slot = 0
             self._frames_out = 0
-        out, y = torch.ops.pqmf_b200.stream_step(x, self.hk, self._tables, self._x_state[self._x_slot], self._x_state[1 - self._x_slot],
+        out, y = torch.ops.pqmf_b200.stream_step(x, self.hk.float(), self._tables, self._x_state[self._x_slot], self._x_state[1 - self._x_slot],
                                                  self._s_state[self._s_slot], self._s_state[1 - self._s_slot], self._frames_in % 2,
                                                  self._frames_out % 2, self._flags)
         self._x_slot = 1 - self._x_slot
@@ -372,7 +399,7 @@ class CachedPQMF(PQMF):
             self._x_state = torch.zeros(2, rows, length, device=x.device)
             self._x_slot = 0
             self._frames_in = 0
-        y = torch.ops.pqmf_b200.analysis_stream(x, self.hk, self._tables, self._x_state[self._x_slot],
+        y = torch.ops.pqmf_b200.analysis_stream(x, self.hk.float(), self._tables, self._x_state[self._x_slot],
                                                 self._x_state[1 - self._x_slot], self._frames_in % 2, self._flags)
         self._x_slot = 1 - self._x_slot
         self._frames_in += x.shape[-1] // self.n_band
@@ -387,7 +414,7 @@ class CachedPQMF(PQMF):
             self._s_state = torch.zeros(2, rows, length, device=s.device)
             self._s_slot = 0
             self._frames_out = 0
-        out = torch.ops.pqmf_b200.synthesis_stream(s, self.hk, self._tables, self._s_state[self._s_slot],
+        out = torch.ops.pqmf_b200.synthesis_stream(s, self.hk.float(), self._tables, self._s_state[self._s_slot],
                                                    self._s_state[1 - self._s_slot], self._frames_out % 2, self._flags)
         self._s_slot = 1 - self._s_slot
         self._frames_out += s.shape[-1]
