@@ -108,16 +108,19 @@ for case in range(int(sys.argv[3]) if len(sys.argv) > 3 else 12):
     if not ok:
         print("HOST ENTRY MISMATCH", dict(m=m, c=c, t=t, b=b, rc=rc)); sys.exit(1)
 # half-precision I/O: bit-identical to the fp32 call on the widened input, rounded -- on random shapes around the boundary between the
-# native half-precision kernels and the staged path (T % 8, frames % 4, tile count near 96, base pointer offset)
+# native half-precision kernels and the staged path (T % 8, frames % 4, tile count near 96, base pointer offset), on every bank the
+# half-precision kernels serve (attenuation 50 .. 140), and from one tile per CTA up to ~10 (the steady state of the persistent loop)
 for case in range(int(sys.argv[4]) if len(sys.argv) > 4 else 40):
     m = random.choice((4, 8, 16, 16, 32, 64))
+    att = random.choice((50, 60, 80, 100, 100, 120, 140))
     dt = random.choice((torch.float16, torch.bfloat16))
     cls = random.choice((pq.PQMF, pq.CachedPQMF))
-    mod = cls(100, m, exact=random.random() < 0.25).cuda()
+    mod = cls(att, m, exact=random.random() < 0.25).cuda()
     tpr = random.choice((1, 2, 3, 8))
     t = tpr * 8192 - random.choice((0, 0, 8 * m, 4 * m, 2 * m, m, 4, 3))
     if cls is pq.PQMF: t -= t % m  # polyphase: whole frames
-    rows = max(1, -(-96 // -(-t // 8192)) + random.choice((-1, 0, 0, 1)))
+    tiles = random.choice((96, 96, 97, 149, 297, 601, 1221, 1480))
+    rows = max(1, -(-tiles // -(-t // 8192)) + random.choice((-1, 0, 0, 1)))
     offset = random.choice((0, 0, 0, 1, 8))
     flat = (0.5 * torch.randn(rows * t + offset, device="cuda")).clamp_(-1, 1).to(dt)
     x = flat[offset:offset + rows * t].view(rows, 1, t)
@@ -125,5 +128,5 @@ for case in range(int(sys.argv[4]) if len(sys.argv) > 4 else 40):
     o = mod.inverse(y)
     if not (torch.equal(y.view(torch.int16), mod(x.float()).to(dt).view(torch.int16)) and
             torch.equal(o.view(torch.int16), mod.inverse(y.float()).to(dt).view(torch.int16)) and y.dtype == dt and o.dtype == dt):
-        print("HALF MISMATCH", dict(m=m, dtype=str(dt), cls=cls.__name__, rows=rows, t=t, offset=offset)); sys.exit(1)
+        print("HALF MISMATCH", dict(m=m, att=att, dtype=str(dt), cls=cls.__name__, rows=rows, t=t, offset=offset)); sys.exit(1)
 print("fuzz ok; worst |hankel - direct| per (n_band, attenuation):", {k: (f"{v[0]:.1e}", f"{v[1]:.1e}") for k, v in sorted(worst.items())})
