@@ -149,13 +149,108 @@ __device__ __forceinline__ void h4_tmem_ld(uint32_t taddr, uint32_t (&r)[N]) {
   else ptx::tmem_ld32(taddr, r);
 }
 
+// eight samples -> their two fp16 terms: one 16-byte chunk at (swizzled) byte `off` of each plane of a pair, the second plane `plane` bytes
+// after the first
+__device__ __forceinline__ void h4_split_store8(const float (&w)[8], unsigned char* p1, int plane, uint32_t off) {
+  uint4 a, bq;
+  split2_f16s(w[0], w[1], a.x, bq.x);
+  split2_f16s(w[2], w[3], a.y, bq.y);
+  split2_f16s(w[4], w[5], a.z, bq.z);
+  split2_f16s(w[6], w[7], a.w, bq.w);
+  unsigned char* p2 = p1 + plane;
+  *reinterpret_cast<uint4*>(p1 + off) = a;
+  *reinterpret_cast<uint4*>(p2 + off) = bq;
+}
+
+// synthesis convert, n_band >= 8: v[kk] = four frames of band 8 bg + kk; chunk j = frame j of them, odd bands sign-flipped by fl
+__device__ __forceinline__ void h4_synthesis_chunk8(const float4 (&v)[8], int j, uint32_t fl, float (&w)[8]) {
+#pragma unroll
+  for (int kk = 0; kk < 8; ++kk) {
+    const float t = j == 0 ? v[kk].x : j == 1 ? v[kk].y : j == 2 ? v[kk].z : v[kk].w;
+    w[kk] = (kk & 1) ? __uint_as_float(__float_as_uint(t) ^ fl) : t;
+  }
+}
+
+// analysis drain, D (TMEM) -> v: worker thread (row i = tid & 127, band half hb = tid >> 7) gets frames FR i .. FR i + FR - 1 of bands
+// HB hb .. HB hb + HB - 1 with the sign applied.  sigma(k, n): odd bands flip on even frames.  A row's first frame is a multiple of FR,
+// even for FR > 1, so there the frame parity is dl's; `first` is the parity of the row's first frame, used at FR = 1 only.
+template <int M>
+__device__ __forceinline__ void h4_drain_analysis(uint32_t tmem, int dbuf, int tid, int first, int parity, float (&v)[64 / M][M / 2]) {
+  constexpr int FR = 64 / M, HB = M / 2;
+  const uint32_t taddr = tmem + ((uint32_t)(((tid >> 5) & 3) * 32) << 16) + (uint32_t)(dbuf * 128 + HB * (tid >> 7));
+  uint32_t r0[FR][HB], r1[FR][HB];
+#pragma unroll
+  for (int dl = 0; dl < FR; ++dl) {
+    h4_tmem_ld<HB>(taddr + dl * M, r0[dl]);
+    h4_tmem_ld<HB>(taddr + 64 + dl * M, r1[dl]);
+  }
+  ptx::tmem_ld_wait();
+#pragma unroll
+  for (int dl = 0; dl < FR; ++dl) {
+    const uint32_t flip = (((FR > 1 ? dl : first) + parity) & 1) == 0 ? 0x80000000u : 0u;
+#pragma unroll
+    for (int kk = 0; kk < HB; kk += 2) {
+      const float2 t = h4_combine2(r0[dl][kk], r0[dl][kk + 1], r1[dl][kk], r1[dl][kk + 1]);
+      v[dl][kk] = t.x;
+      v[dl][kk + 1] = __uint_as_float(__float_as_uint(t.y) ^ flip);
+    }
+  }
+}
+
+// synthesis drain, D (TMEM) -> val.  Worker thread (row i, half hb) reads 32 consecutive output samples = four 32-byte chunks, but rows
+// are 256 B apart: stored like that, every warp store would touch 32 lines.  A 4 x 4 chunk transpose inside each lane quad (two shuffle
+// stages) leaves lane r with chunk r & 3 of the quad's four rows: val[q] = samples 32 hb + 8 (lane & 3) .. + 7 of row (i & ~3) | q, so
+// one STG.256 per slot covers eight whole 128-byte lines.
+__device__ __forceinline__ void h4_drain_synthesis(uint32_t tmem, int dbuf, int tid, float (&val)[4][8]) {
+  const int hb = tid >> 7, lane = tid & 31;
+  const uint32_t taddr = tmem + ((uint32_t)(((tid >> 5) & 3) * 32) << 16) + (uint32_t)(dbuf * 128 + 2 * hb * 16);
+  uint32_t r0[2][16], r1[2][16];
+  ptx::tmem_ld16(taddr, r0[0]);
+  ptx::tmem_ld16(taddr + 64, r1[0]);
+  ptx::tmem_ld16(taddr + 16, r0[1]);
+  ptx::tmem_ld16(taddr + 80, r1[1]);
+  ptx::tmem_ld_wait();
+#pragma unroll
+  for (int q = 0; q < 4; ++q)  // chunk q = samples 32 hb + 8 q .. + 7 of the row
+#pragma unroll
+    for (int e = 0; e < 8; e += 2) {
+      const int c0 = 8 * (q & 1) + e;
+      const float2 t = h4_combine2(r0[q >> 1][c0], r0[q >> 1][c0 + 1], r1[q >> 1][c0], r1[q >> 1][c0 + 1]);
+      val[q][e] = t.x;
+      val[q][e + 1] = t.y;
+    }
+  const bool b0 = lane & 1, b1 = lane & 2;
+#pragma unroll
+  for (int pr = 0; pr < 2; ++pr)  // lanes r, r ^ 1 swap the off-diagonal chunks of (2 pr, 2 pr + 1)
+#pragma unroll
+    for (int e = 0; e < 8; ++e) {
+      const float recv = __shfl_xor_sync(0xffffffffu, b0 ? val[2 * pr][e] : val[2 * pr + 1][e], 1);
+      val[2 * pr + 1][e] = b0 ? val[2 * pr + 1][e] : recv;
+      val[2 * pr][e] = b0 ? recv : val[2 * pr][e];
+    }
+#pragma unroll
+  for (int u = 0; u < 2; ++u)  // lanes r, r ^ 2 swap the off-diagonal chunks of (u, u + 2)
+#pragma unroll
+    for (int e = 0; e < 8; ++e) {
+      const float recv = __shfl_xor_sync(0xffffffffu, b1 ? val[u][e] : val[u + 2][e], 2);
+      val[u + 2][e] = b1 ? val[u + 2][e] : recv;
+      val[u][e] = b1 ? recv : val[u][e];
+    }
+}
+
+// PQMF_H4_TRACE (experiments/trace_h4.cu): `trace` = [iterations][8 warps][8] clock64 stamps of CTA 0 at the phase boundaries of the
+// worker loop, then per CTA its lifetime in cycles and ns.  Kernels without a trace buffer pass nullptr.
 #ifdef PQMF_H4_TRACE
-#define H4_STAMP(k) do { if (blockIdx.x == 0 && (tid & 31) == 0 && it < 64) p.trace[((size_t)it * 8 + warp) * 8 + (k)] = clock64(); } while (0)
+#define H4_TRACE_PARAM , long long* trace
+#define H4_TRACE(x) , x
+#define H4_STAMP(k) do { if (trace && blockIdx.x == 0 && (tid & 31) == 0 && it < 64) trace[((size_t)it * 8 + (tid >> 5)) * 8 + (k)] = clock64(); } while (0)
 #else
+#define H4_TRACE_PARAM
+#define H4_TRACE(x)
 #define H4_STAMP(k) do { } while (0)
 #endif
 
-// shared-memory carve-up common to both kernels
+// shared-memory carve-up common to all Hankel-4 kernels
 struct H4Smem {
   unsigned char *bank, *planes;
   uint64_t *pfull, *mma_bar, *bankfull;
@@ -222,9 +317,9 @@ __device__ __forceinline__ void h4_teardown(uint32_t tmem, int warp) {
 // the issuing thread for ~3200 cycles), so this warp does nothing else and the pipe never waits for a converting thread
 template <bool PAIR>
 __device__ __forceinline__ void h4_issuer_loop(const H4Smem& s, const H4Shape& g, uint32_t tmem, unsigned n_iter, int pad_bytes, int tlo,
-                                               int thi, unsigned it0 = 0) {
+                                               int thi) {
   const uint32_t bank_addr = ptx::smem_u32(s.bank), plane_addr = ptx::smem_u32(s.planes);
-  for (unsigned it = it0; it < it0 + n_iter; ++it) {   // it0 > 0: a second phase of the same kernel continues the barrier sequence
+  for (unsigned it = 0; it < n_iter; ++it) {
     const int pb = (int)(it & 1);
     ptx::mbar_wait(&s.pfull[pb], (it >> 1) & 1);
     ptx::tc_fence_after();
@@ -238,18 +333,81 @@ __device__ __forceinline__ void h4_issuer_loop(const H4Smem& s, const H4Shape& g
   }
 }
 
-// a worker warp publishes its share of planes[pb]: one arrival per warp, after this CTA's bank image has landed (the first tile of a
-// phase waits for it: bank_phase = how many images were loaded before this one)
+// a worker warp publishes its share of planes[pb]: one arrival per warp, after this CTA's bank image has landed (the first tile waits
+// for it)
 template <bool PAIR>
-__device__ __forceinline__ void h4_publish(const H4Smem& s, uint32_t pfull_leader, unsigned it, int pb, int tid, unsigned it0 = 0, unsigned bank_phase = 0) {
+__device__ __forceinline__ void h4_publish(const H4Smem& s, uint32_t pfull_leader, unsigned it, int pb, int tid) {
   ptx::fence_proxy_async();
   ptx::tc_fence_before();
   __syncwarp();
   if ((tid & 31) == 0) {
-    if (it == it0) ptx::mbar_wait(s.bankfull, bank_phase & 1);
+    if (it == 0) ptx::mbar_wait(s.bankfull, 0);
     if constexpr (PAIR) ptx::mbar_arrive_cluster(pfull_leader + 8u * pb);
     else ptx::mbar_arrive(&s.pfull[pb]);
   }
+}
+
+// the worker warps' tile loop.  Iteration it converts tile it into planes[it & 1] and publishes it, loads tile it + 1 into registers
+// (one tile ahead), then waits for the MMAs of tile it - 1 -- after which planes[(it - 1) & 1] may be rewritten -- and drains their
+// accumulator.  The kernel supplies the steps: convert(pb) the current tile, load_next() the tile after it, drain(dbuf) the previous
+// tile, advance() the cursors (current -> previous, next -> current).
+template <bool PAIR, typename Convert, typename LoadNext, typename Drain, typename Advance>
+__device__ __forceinline__ void h4_worker_loop(const H4Smem& s, uint32_t pfull_leader, unsigned n_iter, int tid, Convert&& convert,
+                                               LoadNext&& load_next, Drain&& drain, Advance&& advance H4_TRACE_PARAM) {
+  for (unsigned it = 0; it < n_iter; ++it) {
+    const int pb = (int)(it & 1);
+    H4_STAMP(0);
+    convert(pb);
+    H4_STAMP(1);
+    h4_publish<PAIR>(s, pfull_leader, it, pb, tid);
+    if (it + 1 < n_iter) load_next();  // consumed at the top of the next iteration
+    H4_STAMP(2);
+    if (it > 0) {
+      ptx::mbar_wait(&s.mma_bar[(it - 1) & 1], ((it - 1) >> 1) & 1);
+      ptx::tc_fence_after();
+      drain((int)((it - 1) & 1));
+    }
+    H4_STAMP(5);
+    advance();
+  }
+  ptx::mbar_wait(&s.mma_bar[(n_iter - 1) & 1], ((n_iter - 1) >> 1) & 1);
+  ptx::tc_fence_after();
+  drain((int)((n_iter - 1) & 1));
+}
+
+// the frame of every Hankel-4 kernel: shared-memory carve-up, prologue, the issuer warp (warp WORKERS / 32, leader CTA only) and the
+// teardown.  Each CTA (pair) runs visits x its share of the n_tiles tiles; the worker warps run
+// workers(smem, tmem, pfull_leader, n_iter).
+template <bool PAIR, int WORKERS, typename Workers>
+__device__ __forceinline__ void h4_kernel(const H4Shape& g, const uint16_t* bank, long n_tiles, unsigned visits, int pad_bytes, int trim_lo,
+                                          int trim_hi, Workers&& workers H4_TRACE_PARAM) {
+  extern __shared__ __align__(1024) unsigned char h4_smem[];
+  const H4Smem sm = h4_carve(h4_smem, g);
+  const int tid = threadIdx.x, warp = tid >> 5;
+  const uint32_t rank = PAIR ? ptx::cluster_ctarank() : 0u;
+  const uint32_t tmem = h4_prologue<PAIR>(sm, g, bank, rank, WORKERS / 32, tid);
+  const uint32_t pfull_leader = PAIR ? ptx::mapa_shared(ptx::smem_u32(sm.pfull), 0) : 0u;
+  const unsigned first_tile = PAIR ? (blockIdx.x & ~1u) : blockIdx.x;  // both CTAs of a pair run the same number of tiles
+  const unsigned n_iter = visits * (unsigned)((n_tiles - first_tile + gridDim.x - 1) / gridDim.x);
+#ifdef PQMF_H4_TRACE
+  long long cta_c0 = clock64(), cta_t0;
+  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(cta_t0));
+#endif
+  if (warp == WORKERS / 32) {
+    if (rank == 0) h4_issuer_loop<PAIR>(sm, g, tmem, n_iter, pad_bytes, trim_lo, trim_hi);
+  } else {
+    workers(sm, tmem, pfull_leader, n_iter);
+  }
+#ifdef PQMF_H4_TRACE
+  __syncthreads();
+  if (trace && tid == 0) {
+    long long t1;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t1));
+    trace[64 * 64 + 2 * blockIdx.x] = clock64() - cta_c0;
+    trace[64 * 64 + 2 * blockIdx.x + 1] = t1 - cta_t0;
+  }
+#endif
+  h4_teardown<PAIR>(tmem, warp);
 }
 
 // =============================================================================================
@@ -275,33 +433,28 @@ struct H4AnalysisParams {
 
 template <int M, bool PAIR, H4Io IO>
 __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_kernel(H4AnalysisParams p) {
-  constexpr bool PCM = IO == H4Io::PCM, HALF = h4_io_half(IO);
-  constexpr int FR = 64 / M;                                               // frames per 64-sample row
-  constexpr int HB = M / 2;                                                // bands per epilogue thread
-  constexpr int NO = (kH4MaxPlaneRows * 8 + kH4Workers - 1) / kH4Workers;  // 8-sample loads per thread per tile (a row is 8 of them)
-  extern __shared__ __align__(1024) unsigned char h4_smem[];
-  const H4Shape g = p.g;
-  const H4Smem sm = h4_carve(h4_smem, g);
-  const int tid = threadIdx.x, warp = tid >> 5;
-  constexpr int kMmaWarp = kH4Workers / 32;
-  const uint32_t rank = PAIR ? ptx::cluster_ctarank() : 0u;
-  const uint32_t tmem = h4_prologue<PAIR>(sm, g, p.bank, rank, kH4Workers / 32, tid);
-  const uint32_t pfull_leader = PAIR ? ptx::mapa_shared(ptx::smem_u32(sm.pfull), 0) : 0u;
-
-  const unsigned tpr = (unsigned)p.tiles_per_row;
-  const unsigned step_b = gridDim.x / tpr, step_c = gridDim.x % tpr;
-  unsigned b = blockIdx.x / tpr, c = blockIdx.x % tpr;
-  const unsigned first_tile = PAIR ? (blockIdx.x & ~1u) : blockIdx.x;  // both CTAs of a pair run the same number of tiles:
-  const unsigned n_iter = (unsigned)((p.n_tiles - first_tile + gridDim.x - 1) / gridDim.x);
-  const unsigned n_rows = (unsigned)(p.n_tiles / p.tiles_per_row);     // a tile with b >= n_rows is padding (zeros in, nothing out)
-#ifdef PQMF_H4_TRACE
-  long long cta_c0 = clock64(), cta_t0;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(cta_t0));
-#endif
-
-  if (warp == kMmaWarp) {
-    if (rank == 0) h4_issuer_loop<PAIR>(sm, g, tmem, n_iter, 0, p.trim_lo, p.trim_hi);
-  } else {
+  h4_kernel<PAIR, kH4Workers>(p.g, p.bank, p.n_tiles, 1u, 0, p.trim_lo, p.trim_hi, [&](const H4Smem& sm, uint32_t tmem, uint32_t pfull_leader, unsigned n_iter) {
+    constexpr bool PCM = IO == H4Io::PCM, HALF = h4_io_half(IO);
+    constexpr int FR = 64 / M;                                               // frames per 64-sample row
+    constexpr int HB = M / 2;                                                // bands per epilogue thread
+    constexpr int NO = (kH4MaxPlaneRows * 8 + kH4Workers - 1) / kH4Workers;  // 8-sample loads per thread per tile (a row is 8 of them)
+    const H4Shape& g = p.g;
+    const int tid = threadIdx.x;
+    const unsigned tpr = (unsigned)p.tiles_per_row;
+    const unsigned step_b = gridDim.x / tpr, step_c = gridDim.x % tpr;
+    const unsigned n_rows = (unsigned)(p.n_tiles / p.tiles_per_row);  // a tile with b >= n_rows is padding (zeros in, nothing out)
+    auto advance = [&](unsigned& bb, unsigned& cc) {
+      bb += step_b;
+      cc += step_c;
+      if (cc >= tpr) {
+        cc -= tpr;
+        ++bb;
+      }
+    };
+    unsigned b = blockIdx.x / tpr, c = blockIdx.x % tpr;  // tile it
+    unsigned b1 = b, c1 = c;                              // tile it + 1
+    advance(b1, c1);
+    unsigned prev_b = 0, prev_c = 0;                      // tile it - 1
     const int n_octs = g.rows * 8;
     // this thread's share of the fp32 window of a tile (8 consecutive samples per 256-bit load), prefetched one tile ahead straight
     // from global memory.  (Two tiles ahead in two register sets was measured on the same box: 6 % slower in bursts and sustained --
@@ -332,64 +485,31 @@ __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_kernel(H4AnalysisPa
     };
     // fp32 window -> two fp16 planes (SWIZZLE_128B rows of 64 samples, one 16-byte chunk per load).  planes[pb] were last read by
     // the MMAs of tile it-2, whose completion this thread observed before draining tile it-2.
-    auto convert = [&](int pb, unsigned bb, unsigned cc) {
+    auto convert = [&](int pb) {
       unsigned char* p1 = sm.planes + (2 * pb) * g.plane;
-      unsigned char* p2 = p1 + g.plane;
 #pragma unroll
       for (int r = 0; r < NO; ++r) {
         const int o = tid + kH4Workers * r;
         if (o < n_octs) {
           if constexpr (PCM) {  // the registers hold raw PCM words where the load was live (zeros stay zeros: 0 is not a valid raw mono / stereo pattern to convert)
-            const long s = (long)cc * kH4TileSamples + g.jlo - p.off + 8L * o;
-            if (bb < n_rows && s >= 0 && s < p.T) pcm_convert8(p.in, bb, x0[r]);
+            const long s = (long)c * kH4TileSamples + g.jlo - p.off + 8L * o;
+            if (b < n_rows && s >= 0 && s < p.T) pcm_convert8(p.in, b, x0[r]);
           }
           if constexpr (HALF) h4_widen8<IO>(x0[r]);  // exact; zero words (padding) widen to zeros
-          uint4 a, bq;
-          split2_f16s(x0[r][0], x0[r][1], a.x, bq.x);
-          split2_f16s(x0[r][2], x0[r][3], a.y, bq.y);
-          split2_f16s(x0[r][4], x0[r][5], a.z, bq.z);
-          split2_f16s(x0[r][6], x0[r][7], a.w, bq.w);
-          const uint32_t off = sw128_offset((uint32_t)o * 16u);
-          *reinterpret_cast<uint4*>(p1 + off) = a;
-          *reinterpret_cast<uint4*>(p2 + off) = bq;
+          h4_split_store8(x0[r], p1, g.plane, sw128_offset((uint32_t)o * 16u));
         }
-      }
-    };
-    auto advance = [&](unsigned& bb, unsigned& cc) {
-      bb += step_b;
-      cc += step_c;
-      if (cc >= tpr) {
-        cc -= tpr;
-        ++bb;
       }
     };
     // D (TMEM) -> y: thread (row i, band half hb) owns frames FR i .. FR i + FR - 1 of bands HB hb .. HB hb + HB - 1:
     // FR consecutive frames per band (32 / 16 / 8 bytes at n_band 8 / 16 / 32), consecutive rows in consecutive lanes
-    auto epilogue = [&](unsigned bb, unsigned cc, int dbuf) {
+    auto drain = [&](int dbuf) {
+      if (prev_b >= n_rows) return;
       const int i = tid & 127, hb = tid >> 7;
-      const uint32_t taddr = tmem + ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)(dbuf * 128 + HB * hb);
-      const long n = ((long)cc * kH4Rows + i) * FR;
-      uint32_t r0[FR][HB], r1[FR][HB];
-#pragma unroll
-      for (int dl = 0; dl < FR; ++dl) {
-        h4_tmem_ld<HB>(taddr + dl * M, r0[dl]);
-        h4_tmem_ld<HB>(taddr + 64 + dl * M, r1[dl]);
-      }
-      ptx::tmem_ld_wait();
+      const long n = ((long)prev_c * kH4Rows + i) * FR;
       float v[FR][HB];
-#pragma unroll
-      for (int dl = 0; dl < FR; ++dl) {
-        // sigma(k, n): odd bands flip on even frames; n (a multiple of FR) is even for FR > 1, so the frame parity is dl's
-        const uint32_t flip = (((FR > 1 ? dl : (int)(n & 1)) + p.parity) & 1) == 0 ? 0x80000000u : 0u;
-#pragma unroll
-        for (int kk = 0; kk < HB; kk += 2) {
-          const float2 t = h4_combine2(r0[dl][kk], r0[dl][kk + 1], r1[dl][kk], r1[dl][kk + 1]);
-          v[dl][kk] = t.x;
-          v[dl][kk + 1] = __uint_as_float(__float_as_uint(t.y) ^ flip);
-        }
-      }
+      h4_drain_analysis<M>(tmem, dbuf, tid, (int)(n & 1), p.parity, v);
       if constexpr (HALF) {  // round to nearest even; FR consecutive frames = 2 FR bytes per band (no accumulation: split banks are not native)
-        uint16_t* yp = reinterpret_cast<uint16_t*>(p.y) + ((size_t)bb * M + HB * hb) * p.F + n;
+        uint16_t* yp = reinterpret_cast<uint16_t*>(p.y) + ((size_t)prev_b * M + HB * hb) * p.F + n;
         if (n + FR - 1 < p.F && (p.F % (FR >= 8 ? 8 : FR)) == 0) {
 #pragma unroll
           for (int kk = 0; kk < HB; ++kk) {
@@ -421,7 +541,7 @@ __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_kernel(H4AnalysisPa
         }
         return;
       }
-      float* yp = p.y + ((size_t)bb * M + HB * hb) * p.F + n;
+      float* yp = p.y + ((size_t)prev_b * M + HB * hb) * p.F + n;
       if (n + FR - 1 < p.F && (p.F % (FR >= 4 ? 4 : FR)) == 0) {
         if (p.accumulate) {  // second tap range of a split bank: all the reads first, so they overlap instead of alternating with the stores
           float prev[FR][HB];
@@ -459,44 +579,15 @@ __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_kernel(H4AnalysisPa
       }
     };
 
-    unsigned b1 = b, c1 = c;  // tile it + 1
-    advance(b1, c1);
     load_window(b, c);
-    unsigned prev_b = 0, prev_c = 0;
-    for (unsigned it = 0; it < n_iter; ++it) {
-      const int pb = (int)(it & 1);
-      H4_STAMP(0);
-      convert(pb, b, c);
-      H4_STAMP(1);
-      h4_publish<PAIR>(sm, pfull_leader, it, pb, tid);
-      if (it + 1 < n_iter) load_window(b1, c1);  // consumed at the top of the next iteration
-      H4_STAMP(2);
-      if (it > 0) {
-        ptx::mbar_wait(&sm.mma_bar[(it - 1) & 1], ((it - 1) >> 1) & 1);
-        ptx::tc_fence_after();
-        if (prev_b < n_rows) epilogue(prev_b, prev_c, (int)((it - 1) & 1));
-      }
-      H4_STAMP(5);
+    h4_worker_loop<PAIR>(sm, pfull_leader, n_iter, tid, convert, [&] { load_window(b1, c1); }, drain, [&] {
       prev_b = b;
       prev_c = c;
       b = b1;
       c = c1;
       advance(b1, c1);
-    }
-    ptx::mbar_wait(&sm.mma_bar[(n_iter - 1) & 1], ((n_iter - 1) >> 1) & 1);
-    ptx::tc_fence_after();
-    if (prev_b < n_rows) epilogue(prev_b, prev_c, (int)((n_iter - 1) & 1));
-  }  // workers
-#ifdef PQMF_H4_TRACE
-  __syncthreads();
-  if (tid == 0) {
-    long long t1;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t1));
-    p.trace[64 * 64 + 2 * blockIdx.x] = clock64() - cta_c0;
-    p.trace[64 * 64 + 2 * blockIdx.x + 1] = t1 - cta_t0;
-  }
-#endif
-  h4_teardown<PAIR>(tmem, warp);
+    } H4_TRACE(p.trace));
+  } H4_TRACE(p.trace));
 }
 
 // =============================================================================================
@@ -526,39 +617,41 @@ struct H4SynthesisParams {
 template <int M, bool PAIR, H4Io IO>
 __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_kernel(H4SynthesisParams p) {
   constexpr bool PCM = IO == H4Io::PCM, HALF = h4_io_half(IO);
-  constexpr int FR = 64 / M;       // frames per 128-byte plane row ([frame][band] fp16)
-  constexpr int NBG = M >= 8 ? M / 8 : 1;     // band groups: a 16-byte chunk is 8 bands of one frame, or (n_band 4) all bands of two frames
-  constexpr int FPI = M >= 8 ? 4 : 32 / M;   // frames per load/convert item (four chunks)
-  extern __shared__ __align__(1024) unsigned char h4s_smem[];
-  const H4Shape g = p.g;
-  const H4Smem sm = h4_carve(h4s_smem, g);
-  const int tid = threadIdx.x, warp = tid >> 5;
-  constexpr int kMmaWarp = kH4SynWorkers / 32;
-  const uint32_t rank = PAIR ? ptx::cluster_ctarank() : 0u;
-  const uint32_t tmem = h4_prologue<PAIR>(sm, g, p.bank, rank, kH4SynWorkers / 32, tid);
-  const uint32_t pfull_leader = PAIR ? ptx::mapa_shared(ptx::smem_u32(sm.pfull), 0) : 0u;
-
-  const unsigned tpr = (unsigned)p.tiles_per_row;
-  const unsigned step_b = gridDim.x / tpr, step_c = gridDim.x % tpr;
-  unsigned b = blockIdx.x / tpr, c = blockIdx.x % tpr;
-  const unsigned first_tile = PAIR ? (blockIdx.x & ~1u) : blockIdx.x;
-  const unsigned G = (PCM && p.duo) ? 2u : 1u;  // rows per tile visit (see H4SynthesisParams::duo): b counts clips then, row = G b + channel
-  const unsigned n_iter = G * (unsigned)((p.n_tiles - first_tile + gridDim.x - 1) / gridDim.x);
-  const unsigned n_rows = (unsigned)(p.n_tiles / p.tiles_per_row);
-
   // plane frame m <-> sub-band frame n = 128 FR c + (o - ehi - pad) + m, ehi = largest frame lag with a non-zero tap,
   // pad = (o - ehi) mod 4, so that frame quads are 16-byte aligned in global memory; K-step s of row i then starts
   // 32 s + 2 M pad bytes into the row.
-  const int ehi = (g.jlo + g.kt) / M - 1;
+  const int ehi = (p.g.jlo + p.g.kt) / M - 1;
   const int pad = (p.o - ehi) & 3;
-  const int nbase = p.o - ehi - pad;  // multiple of 4 (may be negative)
-  if (warp == kMmaWarp) {
-    if (rank == 0) h4_issuer_loop<PAIR>(sm, g, tmem, n_iter, 2 * M * pad, p.trim_lo, p.trim_hi);
-  } else {
-    // ---- workers.  Item (fq, bg): frames 4 fq .. 4 fq + 3 of bands 8 bg .. 8 bg + 7 = eight float4 loads (prefetched one
-    //      tile ahead) -> four 16-byte chunks per fp16 plane.  bg-major thread order keeps a quarter-warp on eight consecutive
-    //      frame quads of one band group: their SWIZZLE_128B images hit eight different bank groups at n_band 8 and 16.
-    const int n_fq = (g.rows * FR + FPI - 1) / FPI;          // items per band group (the last one may run into the plane's padding)
+  const unsigned G = (PCM && p.duo) ? 2u : 1u;  // rows per tile visit (see H4SynthesisParams::duo): b counts clips then, row = G b + channel
+  h4_kernel<PAIR, kH4SynWorkers>(p.g, p.bank, p.n_tiles, G, 2 * M * pad, p.trim_lo, p.trim_hi, [&](const H4Smem& sm, uint32_t tmem, uint32_t pfull_leader, unsigned n_iter) {
+    constexpr int FR = 64 / M;                // frames per 128-byte plane row ([frame][band] fp16)
+    constexpr int NBG = M >= 8 ? M / 8 : 1;   // band groups: a 16-byte chunk is 8 bands of one frame, or (n_band 4) all bands of two frames
+    constexpr int FPI = M >= 8 ? 4 : 32 / M;  // frames per load/convert item (four chunks)
+    const H4Shape& g = p.g;
+    const int tid = threadIdx.x, warp = tid >> 5;
+    const int nbase = p.o - ehi - pad;  // multiple of 4 (may be negative)
+    const unsigned tpr = (unsigned)p.tiles_per_row;
+    const unsigned step_b = gridDim.x / tpr, step_c = gridDim.x % tpr;
+    const unsigned n_rows = (unsigned)(p.n_tiles / p.tiles_per_row);
+    auto next_visit = [&](unsigned& bb, unsigned& cc, unsigned& hh) {  // the tile's next row, or the CTA's next tile
+      if (++hh == G) {
+        hh = 0;
+        bb += step_b;
+        cc += step_c;
+        if (cc >= tpr) {
+          cc -= tpr;
+          ++bb;
+        }
+      }
+    };
+    unsigned b = blockIdx.x / tpr, c = blockIdx.x % tpr, h = 0;  // visit it
+    unsigned b1 = b, c1 = c, h1 = 0;                             // visit it + 1
+    next_visit(b1, c1, h1);
+    unsigned prev_b = 0, prev_c = 0, prev_h = 0;                 // visit it - 1
+    // ---- Item (fq, bg): frames 4 fq .. 4 fq + 3 of bands 8 bg .. 8 bg + 7 = eight float4 loads (prefetched one tile ahead) -> four
+    //      16-byte chunks per fp16 plane.  bg-major thread order keeps a quarter-warp on eight consecutive frame quads of one band
+    //      group: their SWIZZLE_128B images hit eight different bank groups at n_band 8 and 16.
+    const int n_fq = (g.rows * FR + FPI - 1) / FPI;  // items per band group (the last one may run into the plane's padding)
     const int bg = tid / n_fq, fq = tid - bg * n_fq;
     const bool has_item = tid < n_fq * NBG;
     float4 v0[8];  // prefetched one tile ahead (half instantiations: four raw frames in .x / .y, widened when the tile is consumed)
@@ -567,7 +660,7 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_kernel(H4Synthe
       const float2 raw = ptx::ldg64_na(at);
       return make_float4(raw.x, raw.y, 0.f, 0.f);
     };
-    auto load_frames = [&](float4 (&v)[8], unsigned bb, unsigned cc, unsigned hh) {
+    auto load_frames = [&](unsigned bb, unsigned cc, unsigned hh) {
       if (p.reverse && bb < n_rows) {
         bb = n_rows - 1 - bb;
         cc = tpr - 1 - cc;
@@ -580,120 +673,73 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_kernel(H4Synthe
           const uint16_t* sp = reinterpret_cast<const uint16_t*>(p.s) + (row * M + 8 * bg) * p.F + n;
           const bool ok = live && n >= 0 && n + 3 < p.F;
 #pragma unroll
-          for (int kk = 0; kk < 8; ++kk) v[kk] = load4h(sp + (size_t)kk * p.F, ok);
+          for (int kk = 0; kk < 8; ++kk) v0[kk] = load4h(sp + (size_t)kk * p.F, ok);
         } else {
           const uint16_t* sp = reinterpret_cast<const uint16_t*>(p.s) + row * M * p.F + n;
 #pragma unroll
           for (int kk = 0; kk < 8; ++kk) {
-            const int b4 = kk >> 1, h = kk & 1;
-            v[kk] = load4h(sp + (size_t)b4 * p.F + 4 * h, live && n + 4 * h >= 0 && n + 4 * h + 3 < p.F);
+            const int b4 = kk >> 1, hf = kk & 1;
+            v0[kk] = load4h(sp + (size_t)b4 * p.F + 4 * hf, live && n + 4 * hf >= 0 && n + 4 * hf + 3 < p.F);
           }
         }
-      } else if constexpr (M >= 8) {  // v[kk] = frames n .. n + 3 of band 8 bg + kk
+      } else if constexpr (M >= 8) {  // v0[kk] = frames n .. n + 3 of band 8 bg + kk
         const float* sp = p.s + (row * M + 8 * bg) * p.F + n;
         const bool ok = live && n >= 0 && n + 3 < p.F;
 #pragma unroll
-        for (int kk = 0; kk < 8; ++kk) v[kk] = ok ? ptx::ldg128_na(reinterpret_cast<const float4*>(sp + (size_t)kk * p.F)) : make_float4(0.f, 0.f, 0.f, 0.f);
-      } else {                 // n_band 4: v[2 b + h] = frames n + 4 h .. n + 4 h + 3 of band b
+        for (int kk = 0; kk < 8; ++kk) v0[kk] = ok ? ptx::ldg128_na(reinterpret_cast<const float4*>(sp + (size_t)kk * p.F)) : make_float4(0.f, 0.f, 0.f, 0.f);
+      } else {                 // n_band 4: v0[2 b + h] = frames n + 4 h .. n + 4 h + 3 of band b
         const float* sp = p.s + row * M * p.F + n;
 #pragma unroll
         for (int kk = 0; kk < 8; ++kk) {
-          const int b4 = kk >> 1, h = kk & 1;
-          const bool ok = live && n + 4 * h >= 0 && n + 4 * h + 3 < p.F;
-          v[kk] = ok ? ptx::ldg128_na(reinterpret_cast<const float4*>(sp + (size_t)b4 * p.F + 4 * h)) : make_float4(0.f, 0.f, 0.f, 0.f);
+          const int b4 = kk >> 1, hf = kk & 1;
+          const bool ok = live && n + 4 * hf >= 0 && n + 4 * hf + 3 < p.F;
+          v0[kk] = ok ? ptx::ldg128_na(reinterpret_cast<const float4*>(sp + (size_t)b4 * p.F + 4 * hf)) : make_float4(0.f, 0.f, 0.f, 0.f);
         }
       }
     };
     // sigma(k, n): odd bands (odd kk) flip on even global frames; quads start on multiples of 4, so the parity is j's
     const uint32_t flip_even = (p.parity & 1) ? 0u : 0x80000000u, flip_odd = flip_even ^ 0x80000000u;
-    auto advance = [&](unsigned& bb, unsigned& cc) {
-      bb += step_b;
-      cc += step_c;
-      if (cc >= tpr) {
-        cc -= tpr;
-        ++bb;
-      }
-    };
-    auto convert = [&](const float4 (&v)[8], int pb) {
+    auto convert = [&](int pb) {
+      float4 v[8];  // the tile's frames as fp32
+#pragma unroll
+      for (int kk = 0; kk < 8; ++kk) v[kk] = HALF ? h4_widen4<IO>(v0[kk]) : v0[kk];  // exact
       if (!has_item) return;
       unsigned char* p1 = sm.planes + (2 * pb) * g.plane;
-      auto comp = [](const float4& q, int c) { return c == 0 ? q.x : c == 1 ? q.y : c == 2 ? q.z : q.w; };
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
         float w[8];
         uint32_t o;
         if constexpr (M >= 8) {  // chunk j = frame 4 fq + j, bands 8 bg .. 8 bg + 7
-          const uint32_t fl = (j & 1) ? flip_odd : flip_even;
-#pragma unroll
-          for (int kk = 0; kk < 8; ++kk) {
-            const float t = comp(v[kk], j);
-            w[kk] = (kk & 1) ? __uint_as_float(__float_as_uint(t) ^ fl) : t;
-          }
+          h4_synthesis_chunk8(v, j, (j & 1) ? flip_odd : flip_even, w);
           o = sw128_offset((uint32_t)(4 * fq + j) * (2u * M) + 16u * bg);
         } else {                 // n_band 4: chunk j = frames 8 fq + 2 j (even) and + 1 (odd), four bands each
 #pragma unroll
           for (int kk = 0; kk < 8; ++kk) {
             const int b4 = kk & 3, odd = kk >> 2;
-            const float t = comp(v[2 * b4 + (j >> 1)], 2 * (j & 1) + odd);
+            const float4& q = v[2 * b4 + (j >> 1)];
+            const int cmp = 2 * (j & 1) + odd;
+            const float t = cmp == 0 ? q.x : cmp == 1 ? q.y : cmp == 2 ? q.z : q.w;
             w[kk] = (b4 & 1) ? __uint_as_float(__float_as_uint(t) ^ (odd ? flip_odd : flip_even)) : t;
           }
           o = sw128_offset((uint32_t)(8 * fq + 2 * j) * (2u * M));
         }
-        uint4 h1, h2;
-        split2_f16s(w[0], w[1], h1.x, h2.x);
-        split2_f16s(w[2], w[3], h1.y, h2.y);
-        split2_f16s(w[4], w[5], h1.z, h2.z);
-        split2_f16s(w[6], w[7], h1.w, h2.w);
-        *reinterpret_cast<uint4*>(p1 + o) = h1;
-        *reinterpret_cast<uint4*>(p1 + g.plane + o) = h2;
+        h4_split_store8(w, p1, g.plane, o);
       }
     };
-    // D (TMEM) -> out.  Thread (row i, half hb) drains 32 consecutive output samples = four 32-byte chunks, but rows are 256 B
-    // apart: stored like that, every warp store would touch 32 lines.  A 4 x 4 chunk transpose inside each lane quad (two shuffle
-    // stages) leaves lane r with chunk r & 3 of the quad's four rows, so one STG.256 covers eight whole 128-byte lines.
+    // D (TMEM) -> out: h4_drain_synthesis leaves slot q with 8 samples of row (i & ~3) | q; one 32-byte store each
     uint32_t held[4][4];  // duo: the left channel's quantised samples of this thread's four chunks, kept for the right channel's visit
-    auto epilogue = [&](unsigned bb, unsigned cc, unsigned hh, int dbuf) {
+    auto drain = [&](int dbuf) {
+      if (warp >= 8 || prev_b >= n_rows) return;  // every worker waited for the MMAs; the ninth warp has no TMEM rows to drain
+      unsigned bb = prev_b, cc = prev_c;
       if (p.reverse) {
         bb = n_rows - 1 - bb;
         cc = tpr - 1 - cc;
       }
-      const size_t row = (size_t)bb * G + hh;
+      const size_t row = (size_t)bb * G + prev_h;
       const int i = tid & 127, hb = tid >> 7, lane = tid & 31;
-      const uint32_t taddr = tmem + ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)(dbuf * 128 + 2 * hb * 16);
-      uint32_t r0[2][16], r1[2][16];
-      ptx::tmem_ld16(taddr, r0[0]);
-      ptx::tmem_ld16(taddr + 64, r1[0]);
-      ptx::tmem_ld16(taddr + 16, r0[1]);
-      ptx::tmem_ld16(taddr + 80, r1[1]);
-      ptx::tmem_ld_wait();
-      float val[4][8];  // chunk q = samples 32 hb + 8 q .. + 7 of the row
-#pragma unroll
-      for (int q = 0; q < 4; ++q)
-#pragma unroll
-        for (int e = 0; e < 8; e += 2) {
-          const int c0 = 8 * (q & 1) + e;
-          const float2 t = h4_combine2(r0[q >> 1][c0], r0[q >> 1][c0 + 1], r1[q >> 1][c0], r1[q >> 1][c0 + 1]);
-          val[q][e] = t.x;
-          val[q][e + 1] = t.y;
-        }
-      const bool b0 = lane & 1, b1 = lane & 2;
-#pragma unroll
-      for (int pr = 0; pr < 2; ++pr)  // lanes r, r ^ 1 swap the off-diagonal chunks of (2 pr, 2 pr + 1)
-#pragma unroll
-        for (int e = 0; e < 8; ++e) {
-          const float recv = __shfl_xor_sync(0xffffffffu, b0 ? val[2 * pr][e] : val[2 * pr + 1][e], 1);
-          val[2 * pr + 1][e] = b0 ? val[2 * pr + 1][e] : recv;
-          val[2 * pr][e] = b0 ? recv : val[2 * pr][e];
-        }
-#pragma unroll
-      for (int u = 0; u < 2; ++u)  // lanes r, r ^ 2 swap the off-diagonal chunks of (u, u + 2)
-#pragma unroll
-        for (int e = 0; e < 8; ++e) {
-          const float recv = __shfl_xor_sync(0xffffffffu, b1 ? val[u][e] : val[u + 2][e], 2);
-          val[u + 2][e] = b1 ? val[u + 2][e] : recv;
-          val[u][e] = b1 ? recv : val[u][e];
-        }
-      // slot q now holds chunk (lane & 3) of row (i & ~3) | q: samples 64 row + 32 hb + 8 (lane & 3) .. + 7 of the tile
+      float val[4][8];
+      h4_drain_synthesis(tmem, dbuf, tid, val);
+      // slot q holds samples 64 row + 32 hb + 8 (lane & 3) .. + 7 of the tile, row = (i & ~3) | q
       const long total = p.F * M;  // samples per output row (a multiple of 8: the dispatcher requires F % 4 == 0)
       const long t0 = (long)cc * kH4TileSamples + 64 * (i & ~3) + 32 * hb + 8 * (lane & 3);
       if constexpr (PCM) {
@@ -704,7 +750,7 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_kernel(H4Synthe
 #pragma unroll
             for (int k = 0; k < 4; ++k)
               w[k] = (uint32_t)(uint16_t)pcm_quantise(val[q][2 * k]) | ((uint32_t)(uint16_t)pcm_quantise(val[q][2 * k + 1]) << 16);
-            if (hh == 0) {
+            if (prev_h == 0) {
 #pragma unroll
               for (int k = 0; k < 4; ++k) held[q][k] = w[k];
             } else if (t0 + 64 * q + 7 < total) {
@@ -749,38 +795,8 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_kernel(H4Synthe
         }
     };
 
-    auto next_visit = [&](unsigned& bb, unsigned& cc, unsigned& hh) {  // the tile's next row, or the CTA's next tile
-      if (++hh == G) {
-        hh = 0;
-        advance(bb, cc);
-      }
-    };
-    unsigned h = 0, b1 = b, c1 = c, h1 = 0;
-    next_visit(b1, c1, h1);
-    load_frames(v0, b, c, h);
-    unsigned prev_b = 0, prev_c = 0, prev_h = 0;
-    for (unsigned it = 0; it < n_iter; ++it) {
-      const int pb = (int)(it & 1);
-      H4_STAMP(0);
-      if constexpr (HALF) {
-        float4 w[8];
-#pragma unroll
-        for (int kk = 0; kk < 8; ++kk) w[kk] = h4_widen4<IO>(v0[kk]);  // exact
-        convert(w, pb);
-      } else {
-        convert(v0, pb);
-      }
-      H4_STAMP(1);
-      h4_publish<PAIR>(sm, pfull_leader, it, pb, tid);
-      if (it + 1 < n_iter) load_frames(v0, b1, c1, h1);
-      H4_STAMP(2);
-      if (it > 0) {
-        // every worker waits (planes[pb ^ 1] are rewritten next iteration); the ninth warp has no TMEM rows to drain
-        ptx::mbar_wait(&sm.mma_bar[(it - 1) & 1], ((it - 1) >> 1) & 1);
-        ptx::tc_fence_after();
-        if (warp < 8 && prev_b < n_rows) epilogue(prev_b, prev_c, prev_h, (int)((it - 1) & 1));
-      }
-      H4_STAMP(5);
+    load_frames(b, c, h);
+    h4_worker_loop<PAIR>(sm, pfull_leader, n_iter, tid, convert, [&] { load_frames(b1, c1, h1); }, drain, [&] {
       prev_b = b;
       prev_c = c;
       prev_h = h;
@@ -788,12 +804,8 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_kernel(H4Synthe
       c = c1;
       h = h1;
       next_visit(b1, c1, h1);
-    }
-    ptx::mbar_wait(&sm.mma_bar[(n_iter - 1) & 1], ((n_iter - 1) >> 1) & 1);
-    ptx::tc_fence_after();
-    if (warp < 8 && prev_b < n_rows) epilogue(prev_b, prev_c, prev_h, (int)((n_iter - 1) & 1));
-  }  // workers
-  h4_teardown<PAIR>(tmem, warp);
+    } H4_TRACE(p.trace));
+  } H4_TRACE(p.trace));
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -833,15 +845,21 @@ inline int h4_configure(Kern kern, int bytes, H4Configured& configured, int& sm_
   return 0;
 }
 
-// one CTA (or CTA pair) per SM, static round-robin over the tiles; PAIR launches clusters of two
+// the tiles of an offline launch: B rows of row_samples samples (analysis: input, synthesis: output); false: too many for the kernels'
+// 32-bit tile cursors
+template <typename Params>
+inline bool h4_set_tiles(Params& p, int B, long row_samples) {
+  p.tiles_per_row = (row_samples + kH4TileSamples - 1) / kH4TileSamples;
+  p.n_tiles = p.tiles_per_row * B;
+  return p.tiles_per_row < (1L << 31) && p.n_tiles < (1L << 40);
+}
+
+// one CTA (or CTA pair) per SM, static round-robin over the caller's p.n_tiles tiles; PAIR launches clusters of two
 template <bool PAIR, typename Kern, typename Params>
-inline int h4_launch(Kern kern, Params p, int B, long row_samples, int threads, H4Configured& configured, cudaStream_t st) {
+inline int h4_launch(Kern kern, const Params& p, int threads, H4Configured& configured, cudaStream_t st) {
   int sms = 0;
   if (!h4_shape_fits(p.g)) return -2;
   if (int e = h4_configure(kern, p.g.bytes, configured, sms)) return e;
-  p.tiles_per_row = (row_samples + kH4TileSamples - 1) / kH4TileSamples;
-  p.n_tiles = p.tiles_per_row * B;
-  if (p.tiles_per_row >= (1L << 31) || p.n_tiles >= (1L << 40)) return -2;
   long grid = PAIR ? (sms & ~1) : sms;
   const long want = PAIR ? ((p.n_tiles + 1) & ~1L) : p.n_tiles;
   if (grid > want) grid = want;
@@ -872,20 +890,21 @@ inline int h4_launch(Kern kern, Params p, int B, long row_samples, int threads, 
 template <int M, bool PAIR>
 int h4_launch_analysis(H4AnalysisParams p, int B, cudaStream_t st, H4Io io = H4Io::F32) {
   static H4Configured configured[4];
+  if (!h4_set_tiles(p, B, p.F * M)) return -2;
   if (p.in.pcm != nullptr) io = H4Io::PCM;
   if (io != H4Io::F32) {
     if constexpr (PAIR) {
       switch (io) {
-        case H4Io::PCM: return h4_launch<PAIR>(h4_analysis_kernel<M, PAIR, H4Io::PCM>, p, B, p.F * M, kH4Threads, configured[1], st);
-        case H4Io::F16: return h4_launch<PAIR>(h4_analysis_kernel<M, PAIR, H4Io::F16>, p, B, p.F * M, kH4Threads, configured[2], st);
-        case H4Io::BF16: return h4_launch<PAIR>(h4_analysis_kernel<M, PAIR, H4Io::BF16>, p, B, p.F * M, kH4Threads, configured[3], st);
+        case H4Io::PCM: return h4_launch<PAIR>(h4_analysis_kernel<M, PAIR, H4Io::PCM>, p, kH4Threads, configured[1], st);
+        case H4Io::F16: return h4_launch<PAIR>(h4_analysis_kernel<M, PAIR, H4Io::F16>, p, kH4Threads, configured[2], st);
+        case H4Io::BF16: return h4_launch<PAIR>(h4_analysis_kernel<M, PAIR, H4Io::BF16>, p, kH4Threads, configured[3], st);
         default: return -2;
       }
     } else {
       return -2;
     }
   }
-  return h4_launch<PAIR>(h4_analysis_kernel<M, PAIR, H4Io::F32>, p, B, p.F * M, kH4Threads, configured[0], st);
+  return h4_launch<PAIR>(h4_analysis_kernel<M, PAIR, H4Io::F32>, p, kH4Threads, configured[0], st);
 }
 
 template <int M, bool PAIR>
@@ -894,20 +913,22 @@ int h4_launch_synthesis(H4SynthesisParams p, int B, cudaStream_t st, H4Io io = H
   if (p.pcm_out != nullptr) {
     if constexpr (PAIR) {
       p.duo = (p.C == 2 && B % 2 == 0) ? 1 : 0;  // stereo: the tiles of a launch are (clip, chunk), each visited once per channel
-      return h4_launch<PAIR>(h4_synthesis_kernel<M, PAIR, H4Io::PCM>, p, p.duo ? B / 2 : B, p.F * M, kH4SynThreads, configured[1], st);
+      if (!h4_set_tiles(p, p.duo ? B / 2 : B, p.F * M)) return -2;
+      return h4_launch<PAIR>(h4_synthesis_kernel<M, PAIR, H4Io::PCM>, p, kH4SynThreads, configured[1], st);
     } else {
       return -2;
     }
   }
+  if (!h4_set_tiles(p, B, p.F * M)) return -2;
   if (h4_io_half(io)) {
     if constexpr (PAIR) {
-      if (io == H4Io::F16) return h4_launch<PAIR>(h4_synthesis_kernel<M, PAIR, H4Io::F16>, p, B, p.F * M, kH4SynThreads, configured[2], st);
-      return h4_launch<PAIR>(h4_synthesis_kernel<M, PAIR, H4Io::BF16>, p, B, p.F * M, kH4SynThreads, configured[3], st);
+      if (io == H4Io::F16) return h4_launch<PAIR>(h4_synthesis_kernel<M, PAIR, H4Io::F16>, p, kH4SynThreads, configured[2], st);
+      return h4_launch<PAIR>(h4_synthesis_kernel<M, PAIR, H4Io::BF16>, p, kH4SynThreads, configured[3], st);
     } else {
       return -2;
     }
   }
-  return h4_launch<PAIR>(h4_synthesis_kernel<M, PAIR, H4Io::F32>, p, B, p.F * M, kH4SynThreads, configured[0], st);
+  return h4_launch<PAIR>(h4_synthesis_kernel<M, PAIR, H4Io::F32>, p, kH4SynThreads, configured[0], st);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -43,183 +43,123 @@ struct H4AnalysisStreamParams {
   long n_tiles;
 };
 
-// the worker warps' part of streaming analysis (warps 0-7): tiles blockIdx.x, + gridDim.x, ...; `it0` / `bank_phase` continue the
-// barrier sequence when this is a phase of the fused block-step kernel
-template <int M, bool PAIR>
-__device__ __forceinline__ void h4_analysis_stream_workers(const H4AnalysisStreamParams& p, const H4Smem& sm, uint32_t tmem, uint32_t pfull_leader,
-                                                           unsigned n_iter, unsigned it0, unsigned bank_phase, int tid) {
-  constexpr int FR = 64 / M, HB = M / 2;  // frames per 64-sample row, bands per epilogue thread
-  constexpr int NO = (kH4Rows * 8 + kH4Workers - 1) / kH4Workers;  // 4 x 8 samples per thread cover the 128 region rows of a tile
-  const H4Shape& g = p.g;
-  const H4StreamGeom& sg = p.s;
-  const int warp = tid >> 5;
-  // rows past the last region are read by MMA rows whose results are never stored: make them finite once
-  for (int u = sg.spt * sg.pitch * 32 + tid; u < g.rows * 32; u += kH4Workers)
+// streaming analysis: tiles blockIdx.x, + gridDim.x, ... of spt streams each
+template <int M>
+__global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_stream_kernel(H4AnalysisStreamParams p) {
+  h4_kernel<true, kH4Workers>(p.g, p.bank, p.n_tiles, 1u, p.pad_bytes, p.trim_lo, p.trim_hi, [&](const H4Smem& sm, uint32_t tmem, uint32_t pfull_leader, unsigned n_iter) {
+    constexpr int FR = 64 / M, HB = M / 2;  // frames per 64-sample row, bands per epilogue thread
+    constexpr int NO = (kH4Rows * 8 + kH4Workers - 1) / kH4Workers;  // 4 x 8 samples per thread cover the 128 region rows of a tile
+    const H4Shape& g = p.g;
+    const H4StreamGeom& sg = p.s;
+    const int tid = threadIdx.x;
+    // rows past the last region are read by MMA rows whose results are never stored: make them finite once
+    for (int u = sg.spt * sg.pitch * 32 + tid; u < g.rows * 32; u += kH4Workers)
 #pragma unroll
-    for (int pl = 0; pl < 4; ++pl) reinterpret_cast<float*>(sm.planes + pl * g.plane)[u] = 0.f;
-  // tile-invariant plan of this thread's 8-sample groups, made once: the stream slot, RUNNING pointers to the group's source (history or
-  // block) and -- for the groups that hold the tail of a block -- to its place in the next history, and what a tile step adds to them.
-  // The loop below then only tests the slot against the live streams of the tile and bumps pointers (no per-tile index arithmetic).
-  const int region_octs = sg.pitch * 8, n_octs = sg.spt * region_octs;
-  const long F = p.T / M;
-  const size_t step_x = (size_t)gridDim.x * sg.spt * p.T, step_h = (size_t)gridDim.x * sg.spt * p.L;
-  constexpr int kDead = 1 << 20;  // slot of padding rows: never below the live-stream count
-  int q_slot[NO];
-  const float* src[NO];
-  size_t src_step[NO];
-  float* roll[NO];  // where the group goes in hist_out (nullptr: it is not part of the last L samples)
-#pragma unroll
-  for (int r = 0; r < NO; ++r) {
-    const int u = tid + kH4Workers * r;
-    q_slot[r] = kDead;
-    src[r] = p.x;
-    src_step[r] = 0;
-    roll[r] = nullptr;
-    if (u < n_octs) {
-      const int t = u / region_octs, w = u - t * region_octs, q = w >> 3, col = w & 7;
-      const size_t stream0 = (size_t)blockIdx.x * sg.spt + t;  // the stream this group belongs to in this CTA's first tile
-      if (q < sg.hrows) {
-        q_slot[r] = t;
-        src[r] = p.hist_in + stream0 * p.L + ((p.L - sg.hrows * 64) + q * 64 + 8 * col);
-        src_step[r] = step_h;
-      } else if (q - sg.hrows < sg.rows_b) {
-        const long off = (q - sg.hrows) * 64 + 8 * col;
-        q_slot[r] = t;
-        src[r] = p.x + stream0 * p.T + off;
-        src_step[r] = step_x;
-        if (off >= p.T - p.L) roll[r] = p.hist_out + stream0 * p.L + (off - (p.T - p.L));
-      }
-    }
-  }
-  float xr[NO][8];
-  int nlive = 0;  // live streams of the tile held in xr
-  auto load_tile = [&](long tile) {
-    nlive = (int)min((long)sg.spt, (long)p.B - tile * sg.spt);
-#pragma unroll
-    for (int r = 0; r < NO; ++r) {
-      if (q_slot[r] < nlive) {
-        ptx::ldg256_na(src[r], xr[r]);
-      } else {
-#pragma unroll
-        for (int e = 0; e < 8; ++e) xr[r][e] = 0.f;
-      }
-      src[r] += src_step[r];
-    }
-  };
-  // fp32 -> fp16 planes; the threads that hold the last L samples of a block also roll the history (here, where the data is
-  // needed anyway: a store next to the load would make every prefetch wait for its own data)
-  auto convert = [&](int pb) {
-    unsigned char* p1 = sm.planes + (2 * pb) * g.plane;
-    unsigned char* p2 = p1 + g.plane;
+      for (int pl = 0; pl < 4; ++pl) reinterpret_cast<float*>(sm.planes + pl * g.plane)[u] = 0.f;
+    // tile-invariant plan of this thread's 8-sample groups, made once: the stream slot, RUNNING pointers to the group's source (history or
+    // block) and -- for the groups that hold the tail of a block -- to its place in the next history, and what a tile step adds to them.
+    // The loop below then only tests the slot against the live streams of the tile and bumps pointers (no per-tile index arithmetic).
+    const int region_octs = sg.pitch * 8, n_octs = sg.spt * region_octs;
+    const long F = p.T / M;
+    const size_t step_x = (size_t)gridDim.x * sg.spt * p.T, step_h = (size_t)gridDim.x * sg.spt * p.L;
+    constexpr int kDead = 1 << 20;  // slot of padding rows: never below the live-stream count
+    int q_slot[NO];
+    const float* src[NO];
+    size_t src_step[NO];
+    float* roll[NO];  // where the group goes in hist_out (nullptr: it is not part of the last L samples)
 #pragma unroll
     for (int r = 0; r < NO; ++r) {
       const int u = tid + kH4Workers * r;
+      q_slot[r] = kDead;
+      src[r] = p.x;
+      src_step[r] = 0;
+      roll[r] = nullptr;
       if (u < n_octs) {
-        uint4 a, bq;
-        split2_f16s(xr[r][0], xr[r][1], a.x, bq.x);
-        split2_f16s(xr[r][2], xr[r][3], a.y, bq.y);
-        split2_f16s(xr[r][4], xr[r][5], a.z, bq.z);
-        split2_f16s(xr[r][6], xr[r][7], a.w, bq.w);
-        const uint32_t o = sw128_offset((uint32_t)u * 16u);
-        *reinterpret_cast<uint4*>(p1 + o) = a;
-        *reinterpret_cast<uint4*>(p2 + o) = bq;
-        if (roll[r] != nullptr) {
-          if (q_slot[r] < nlive) {
-            *reinterpret_cast<float4*>(roll[r]) = make_float4(xr[r][0], xr[r][1], xr[r][2], xr[r][3]);
-            *reinterpret_cast<float4*>(roll[r] + 4) = make_float4(xr[r][4], xr[r][5], xr[r][6], xr[r][7]);
-          }
-          roll[r] += step_h;
+        const int t = u / region_octs, w = u - t * region_octs, q = w >> 3, col = w & 7;
+        const size_t stream0 = (size_t)blockIdx.x * sg.spt + t;  // the stream this group belongs to in this CTA's first tile
+        if (q < sg.hrows) {
+          q_slot[r] = t;
+          src[r] = p.hist_in + stream0 * p.L + ((p.L - sg.hrows * 64) + q * 64 + 8 * col);
+          src_step[r] = step_h;
+        } else if (q - sg.hrows < sg.rows_b) {
+          const long off = (q - sg.hrows) * 64 + 8 * col;
+          q_slot[r] = t;
+          src[r] = p.x + stream0 * p.T + off;
+          src_step[r] = step_x;
+          if (off >= p.T - p.L) roll[r] = p.hist_out + stream0 * p.L + (off - (p.T - p.L));
         }
       }
     }
-  };
-  // D (TMEM) -> y: MMA row i = region t, row q: block row q (frames FR q .. FR q + FR - 1) of stream tile * spt + t when q < rows_b
-  const int i = tid & 127, hb = tid >> 7;
-  const int et = i / sg.pitch, eq = i - et * sg.pitch;
-  const bool e_row = et < sg.spt && eq < sg.rows_b;
-  float* yrun = p.y + (((size_t)blockIdx.x * sg.spt + et) * M + HB * hb) * F + FR * eq;  // this thread's rows of the CTA's first tile
-  const size_t y_step = (size_t)gridDim.x * sg.spt * M * F;
-  auto epilogue = [&](long tile, int dbuf) {
-    const uint32_t taddr = tmem + ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)(dbuf * 128 + HB * hb);
-    uint32_t r0[FR][HB], r1[FR][HB];
+    float xr[NO][8];
+    int nlive = 0;  // live streams of the tile held in xr
+    auto load_tile = [&](long tile) {
+      nlive = (int)min((long)sg.spt, (long)p.B - tile * sg.spt);
 #pragma unroll
-    for (int dl = 0; dl < FR; ++dl) {
-      h4_tmem_ld<HB>(taddr + dl * M, r0[dl]);
-      h4_tmem_ld<HB>(taddr + 64 + dl * M, r1[dl]);
-    }
-    ptx::tmem_ld_wait();
-    float* yp = yrun;
-    yrun += y_step;
-    if (!e_row || tile * sg.spt + et >= p.B) return;
-    float v[FR][HB];
+      for (int r = 0; r < NO; ++r) {
+        if (q_slot[r] < nlive) {
+          ptx::ldg256_na(src[r], xr[r]);
+        } else {
 #pragma unroll
-    for (int dl = 0; dl < FR; ++dl) {
-      // global frame parity = parity of (FR eq + dl) + frame_parity; FR eq is even for FR > 1: odd bands flip on even frames
-      const uint32_t flip = ((((FR > 1 ? dl : eq) + p.parity) & 1) == 0) ? 0x80000000u : 0u;
-#pragma unroll
-      for (int kk = 0; kk < HB; kk += 2) {
-        const float2 t = h4_combine2(r0[dl][kk], r0[dl][kk + 1], r1[dl][kk], r1[dl][kk + 1]);
-        v[dl][kk] = t.x;
-        v[dl][kk + 1] = __uint_as_float(__float_as_uint(t.y) ^ flip);
+          for (int e = 0; e < 8; ++e) xr[r][e] = 0.f;
+        }
+        src[r] += src_step[r];
       }
-    }
+    };
+    // fp32 -> fp16 planes; the threads that hold the last L samples of a block also roll the history (here, where the data is
+    // needed anyway: a store next to the load would make every prefetch wait for its own data)
+    auto convert = [&](int pb) {
+      unsigned char* p1 = sm.planes + (2 * pb) * g.plane;
 #pragma unroll
-    for (int kk = 0; kk < HB; ++kk) {
-      float w[FR];
-#pragma unroll
-      for (int dl = 0; dl < FR; ++dl) w[dl] = v[dl][kk];
-      float* q = yp + (size_t)kk * F;
-      if constexpr (FR >= 4) {
-#pragma unroll
-        for (int d4 = 0; d4 < FR; d4 += 4) __stcs(reinterpret_cast<float4*>(q + d4), make_float4(w[d4], w[d4 + 1], w[d4 + 2], w[d4 + 3]));
-      } else if constexpr (FR == 2) {
-        __stcs(reinterpret_cast<float2*>(q), make_float2(w[0], w[1]));
-      } else {
-        __stcs(q, w[0]);
+      for (int r = 0; r < NO; ++r) {
+        const int u = tid + kH4Workers * r;
+        if (u < n_octs) {
+          h4_split_store8(xr[r], p1, g.plane, sw128_offset((uint32_t)u * 16u));
+          if (roll[r] != nullptr) {
+            if (q_slot[r] < nlive) {
+              *reinterpret_cast<float4*>(roll[r]) = make_float4(xr[r][0], xr[r][1], xr[r][2], xr[r][3]);
+              *reinterpret_cast<float4*>(roll[r] + 4) = make_float4(xr[r][4], xr[r][5], xr[r][6], xr[r][7]);
+            }
+            roll[r] += step_h;
+          }
+        }
       }
-    }
-  };
+    };
+    // D (TMEM) -> y: MMA row i = region t, row q: block row q (frames FR q .. FR q + FR - 1) of stream tile * spt + t when q < rows_b
+    const int i = tid & 127, hb = tid >> 7;
+    const int et = i / sg.pitch, eq = i - et * sg.pitch;
+    const bool e_row = et < sg.spt && eq < sg.rows_b;
+    float* yrun = p.y + (((size_t)blockIdx.x * sg.spt + et) * M + HB * hb) * F + FR * eq;  // this thread's rows of the CTA's first tile
+    const size_t y_step = (size_t)gridDim.x * sg.spt * M * F;
+    long tile = blockIdx.x, prev_tile = 0;
+    auto drain = [&](int dbuf) {
+      float v[FR][HB];
+      h4_drain_analysis<M>(tmem, dbuf, tid, eq, p.parity, v);  // the first frame of block row eq is FR eq
+      float* yp = yrun;
+      yrun += y_step;
+      if (!e_row || prev_tile * sg.spt + et >= p.B) return;
+#pragma unroll
+      for (int kk = 0; kk < HB; ++kk) {
+        float w[FR];
+#pragma unroll
+        for (int dl = 0; dl < FR; ++dl) w[dl] = v[dl][kk];
+        float* q = yp + (size_t)kk * F;
+        if constexpr (FR >= 4) {
+#pragma unroll
+          for (int d4 = 0; d4 < FR; d4 += 4) __stcs(reinterpret_cast<float4*>(q + d4), make_float4(w[d4], w[d4 + 1], w[d4 + 2], w[d4 + 3]));
+        } else if constexpr (FR == 2) {
+          __stcs(reinterpret_cast<float2*>(q), make_float2(w[0], w[1]));
+        } else {
+          __stcs(q, w[0]);
+        }
+      }
+    };
 
-  long tile = blockIdx.x;
-  load_tile(tile);
-  long prev_tile = 0;
-  for (unsigned it = it0; it < it0 + n_iter; ++it) {
-    const int pb = (int)(it & 1);
-    convert(pb);
-    h4_publish<PAIR>(sm, pfull_leader, it, pb, tid, it0, bank_phase);
-    if (it + 1 < it0 + n_iter) load_tile(tile + gridDim.x);
-    if (it > it0) {
-      ptx::mbar_wait(&sm.mma_bar[(it - 1) & 1], ((it - 1) >> 1) & 1);
-      ptx::tc_fence_after();
-      epilogue(prev_tile, (int)((it - 1) & 1));
-    }
-    prev_tile = tile;
-    tile += gridDim.x;
-  }
-  const unsigned last = it0 + n_iter - 1;
-  ptx::mbar_wait(&sm.mma_bar[last & 1], (last >> 1) & 1);
-  ptx::tc_fence_after();
-  epilogue(prev_tile, (int)(last & 1));
-}
-
-template <int M, bool PAIR>
-__global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_stream_kernel(H4AnalysisStreamParams p) {
-  extern __shared__ __align__(1024) unsigned char h4as_smem[];
-  const H4Shape g = p.g;
-  const H4Smem sm = h4_carve(h4as_smem, g);
-  const int tid = threadIdx.x, warp = tid >> 5;
-  constexpr int kMmaWarp = kH4Workers / 32;
-  const uint32_t rank = PAIR ? ptx::cluster_ctarank() : 0u;
-  const uint32_t tmem = h4_prologue<PAIR>(sm, g, p.bank, rank, kH4Workers / 32, tid);
-  const uint32_t pfull_leader = PAIR ? ptx::mapa_shared(ptx::smem_u32(sm.pfull), 0) : 0u;
-  const unsigned first_tile = PAIR ? (blockIdx.x & ~1u) : blockIdx.x;
-  const unsigned n_iter = (unsigned)((p.n_tiles - first_tile + gridDim.x - 1) / gridDim.x);
-  if (warp == kMmaWarp) {
-    if (rank == 0) h4_issuer_loop<PAIR>(sm, g, tmem, n_iter, p.pad_bytes, p.trim_lo, p.trim_hi);
-  } else {
-    h4_analysis_stream_workers<M, PAIR>(p, sm, tmem, pfull_leader, n_iter, 0, 0, tid);
-  }
-  h4_teardown<PAIR>(tmem, warp);
+    load_tile(tile);
+    h4_worker_loop<true>(sm, pfull_leader, n_iter, tid, convert, [&] { load_tile(tile + gridDim.x); }, drain, [&] {
+      prev_tile = tile;
+      tile += gridDim.x;
+    } H4_TRACE(nullptr));
+  } H4_TRACE(nullptr));
 }
 
 struct H4SynthesisStreamParams {
@@ -237,220 +177,117 @@ struct H4SynthesisStreamParams {
   long n_tiles;
 };
 
-// the worker warps' part of streaming synthesis (warps 0-8).  OWN: the sub-bands were written by an earlier phase of this kernel
-// (by this very CTA: same tile -> stream map), so they are read through L2 instead of the non-coherent path.
-template <int M, bool PAIR, bool OWN>
-__device__ __forceinline__ void h4_synthesis_stream_workers(const H4SynthesisStreamParams& p, const H4Smem& sm, uint32_t tmem, uint32_t pfull_leader,
-                                                            unsigned n_iter, unsigned it0, unsigned bank_phase, int tid) {
-  static_assert(M >= 8, "frame quads of 8-band groups (n_band 4 packs its chunks differently: offline kernels only)");
-  constexpr int FR = 64 / M, NBG = M / 8;  // frames per 128-byte plane row, 8-band groups
-  const H4Shape& g = p.g;
-  const H4StreamGeom& sg = p.sg;
-  const int warp = tid >> 5;
-  for (int u = sg.spt * sg.pitch * 32 + tid; u < g.rows * 32; u += kH4SynWorkers)
-#pragma unroll
-    for (int pl = 0; pl < 4; ++pl) reinterpret_cast<float*>(sm.planes + pl * g.plane)[u] = 0.f;
-  // item (frame quad wq of the tile, band group bg): four frames x eight bands = four 16-byte chunks per plane.  A region holds
-  // pitch * FR frames; its first hrows * FR frames are history (both multiples of 4: a quad never straddles the boundary)
-  const int n_fq = sg.spt * sg.pitch * FR / 4;
-  const int bg = tid / n_fq, wq = tid - bg * n_fq;
-  const bool has_item = tid < NBG * n_fq;
-  const int region_frames = sg.pitch * FR, hist_fr = sg.hrows * FR, block_fr = sg.rows_b * FR;
-  const int lt = (4 * wq) / region_frames, lf = 4 * wq - lt * region_frames;  // region, first frame of the quad within the region
-  const int fb = lf - hist_fr;  // first frame of this thread's quad within the block (negative: history)
-  // tile-invariant plan, made once: RUNNING pointers to the quad's eight band rows (in the state for history frames, in s for block
-  // frames), to its place in the next state when it is one of the block's last K frames, and what a tile step adds to them
-  constexpr int kDead = 1 << 20;
-  const size_t band0 = ((size_t)blockIdx.x * sg.spt + lt) * M + 8 * bg;  // first band row of the item in this CTA's first tile
-  const size_t step_state = (size_t)gridDim.x * sg.spt * M * p.K;
-  int slot = kDead;
-  const float* src = p.s;
-  size_t src_step = 0, src_pitch = 0;
-  float* roll = nullptr;
-  if (has_item) {
-    if (fb < 0) {
-      slot = lt;
-      src = p.state_in + band0 * p.K + (p.K - hist_fr) + lf;
-      src_step = step_state;
-      src_pitch = (size_t)p.K;
-    } else if (fb < block_fr) {
-      slot = lt;
-      src = p.s + band0 * p.F + fb;
-      src_step = (size_t)gridDim.x * sg.spt * M * p.F;
-      src_pitch = (size_t)p.F;
-      if (fb >= p.F - p.K) roll = p.state_out + band0 * p.K + (fb - (p.F - p.K));  // the last K frames of the block become the next history
-    }
-  }
-  float4 v[8];
-  int nlive = 0;  // live streams of the tile held in v
-  auto load_tile = [&](long tile) {
-    nlive = (int)min((long)sg.spt, (long)p.B - tile * sg.spt);
-    const bool live = slot < nlive;
-#pragma unroll
-    for (int kk = 0; kk < 8; ++kk) {
-      const float4* q = reinterpret_cast<const float4*>(src + (size_t)kk * src_pitch);
-      v[kk] = live ? (OWN ? ptx::ldg128_cg(q) : ptx::ldg128_na(q)) : make_float4(0.f, 0.f, 0.f, 0.f);
-    }
-    src += src_step;
-  };
-  // sigma(k, n): odd bands flip on even global frames; regions and history lengths are multiples of 4 frames, so the parity is j's
-  const uint32_t flip_even = (p.parity & 1) ? 0u : 0x80000000u, flip_odd = flip_even ^ 0x80000000u;
-  auto convert = [&](int pb) {
-    if (!has_item) return;
-    unsigned char* p1 = sm.planes + (2 * pb) * g.plane;
-    if (roll != nullptr) {
-      if (slot < nlive) {
-#pragma unroll
-        for (int kk = 0; kk < 8; ++kk) *reinterpret_cast<float4*>(roll + (size_t)kk * p.K) = v[kk];
-      }
-      roll += step_state;
-    }
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const uint32_t fl = (j & 1) ? flip_odd : flip_even;
-      float w[8];
-#pragma unroll
-      for (int kk = 0; kk < 8; ++kk) {
-        const float t = j == 0 ? v[kk].x : j == 1 ? v[kk].y : j == 2 ? v[kk].z : v[kk].w;
-        w[kk] = (kk & 1) ? __uint_as_float(__float_as_uint(t) ^ fl) : t;
-      }
-      uint4 h1, h2;
-      split2_f16s(w[0], w[1], h1.x, h2.x);
-      split2_f16s(w[2], w[3], h1.y, h2.y);
-      split2_f16s(w[4], w[5], h1.z, h2.z);
-      split2_f16s(w[6], w[7], h1.w, h2.w);
-      const uint32_t o = sw128_offset((uint32_t)(4 * wq + j) * (2u * M) + 16u * bg);
-      *reinterpret_cast<uint4*>(p1 + o) = h1;
-      *reinterpret_cast<uint4*>(p1 + g.plane + o) = h2;
-    }
-  };
-  // D (TMEM) -> out, with the 4 x 4 chunk transpose of the offline kernel.  pitch and rows_b are multiples of 4, so the four rows
-  // of a lane quad belong to one region and are valid or not together.
-  const int i = tid & 127, hb = tid >> 7, lane = tid & 31;
-  const int i0 = i & ~3, et = i0 / sg.pitch, eq0 = i0 - et * sg.pitch;
-  const bool e_rows = et < sg.spt && eq0 < sg.rows_b;
-  float* orun = p.out + ((size_t)blockIdx.x * sg.spt + et) * (size_t)(p.F * M) + 64 * eq0 + 32 * hb + 8 * (lane & 3);  // slot q: row eq0 + q of the block
-  const size_t out_step = (size_t)gridDim.x * sg.spt * (size_t)(p.F * M);
-  auto epilogue = [&](long tile, int dbuf) {
-    const uint32_t taddr = tmem + ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)(dbuf * 128 + 2 * hb * 16);
-    uint32_t r0[2][16], r1[2][16];
-    ptx::tmem_ld16(taddr, r0[0]);
-    ptx::tmem_ld16(taddr + 64, r1[0]);
-    ptx::tmem_ld16(taddr + 16, r0[1]);
-    ptx::tmem_ld16(taddr + 80, r1[1]);
-    ptx::tmem_ld_wait();
-    float val[4][8];
-#pragma unroll
-    for (int q = 0; q < 4; ++q)
-#pragma unroll
-      for (int e = 0; e < 8; e += 2) {
-        const int c0 = 8 * (q & 1) + e;
-        const float2 t = h4_combine2(r0[q >> 1][c0], r0[q >> 1][c0 + 1], r1[q >> 1][c0], r1[q >> 1][c0 + 1]);
-        val[q][e] = t.x;
-        val[q][e + 1] = t.y;
-      }
-    const bool b0 = lane & 1, b1 = lane & 2;
-#pragma unroll
-    for (int pr = 0; pr < 2; ++pr)
-#pragma unroll
-      for (int e = 0; e < 8; ++e) {
-        const float recv = __shfl_xor_sync(0xffffffffu, b0 ? val[2 * pr][e] : val[2 * pr + 1][e], 1);
-        val[2 * pr + 1][e] = b0 ? val[2 * pr + 1][e] : recv;
-        val[2 * pr][e] = b0 ? recv : val[2 * pr][e];
-      }
-#pragma unroll
-    for (int u = 0; u < 2; ++u)
-#pragma unroll
-      for (int e = 0; e < 8; ++e) {
-        const float recv = __shfl_xor_sync(0xffffffffu, b1 ? val[u][e] : val[u + 2][e], 2);
-        val[u + 2][e] = b1 ? val[u + 2][e] : recv;
-        val[u][e] = b1 ? recv : val[u][e];
-      }
-    float* op = orun;
-    orun += out_step;
-    if (!e_rows || tile * sg.spt + et >= p.B) return;
-#pragma unroll
-    for (int q = 0; q < 4; ++q) ptx::stg256_cs(op + (size_t)q * 64, val[q]);
-  };
-
-  long tile = blockIdx.x;
-  load_tile(tile);
-  long prev_tile = 0;
-  for (unsigned it = it0; it < it0 + n_iter; ++it) {
-    const int pb = (int)(it & 1);
-    convert(pb);
-    h4_publish<PAIR>(sm, pfull_leader, it, pb, tid, it0, bank_phase);
-    if (it + 1 < it0 + n_iter) load_tile(tile + gridDim.x);
-    if (it > it0) {
-      ptx::mbar_wait(&sm.mma_bar[(it - 1) & 1], ((it - 1) >> 1) & 1);
-      ptx::tc_fence_after();
-      if (warp < 8) epilogue(prev_tile, (int)((it - 1) & 1));
-    }
-    prev_tile = tile;
-    tile += gridDim.x;
-  }
-  const unsigned last = it0 + n_iter - 1;
-  ptx::mbar_wait(&sm.mma_bar[last & 1], (last >> 1) & 1);
-  ptx::tc_fence_after();
-  if (warp < 8) epilogue(prev_tile, (int)(last & 1));
-}
-
-template <int M, bool PAIR>
+// streaming synthesis: tiles blockIdx.x, + gridDim.x, ... of spt streams each
+template <int M>
 __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_stream_kernel(H4SynthesisStreamParams p) {
-  extern __shared__ __align__(1024) unsigned char h4ss_smem[];
-  const H4Shape g = p.g;
-  const H4Smem sm = h4_carve(h4ss_smem, g);
-  const int tid = threadIdx.x, warp = tid >> 5;
-  constexpr int kMmaWarp = kH4SynWorkers / 32;
-  const uint32_t rank = PAIR ? ptx::cluster_ctarank() : 0u;
-  const uint32_t tmem = h4_prologue<PAIR>(sm, g, p.bank, rank, kH4SynWorkers / 32, tid);
-  const uint32_t pfull_leader = PAIR ? ptx::mapa_shared(ptx::smem_u32(sm.pfull), 0) : 0u;
-  const unsigned first_tile = PAIR ? (blockIdx.x & ~1u) : blockIdx.x;
-  const unsigned n_iter = (unsigned)((p.n_tiles - first_tile + gridDim.x - 1) / gridDim.x);
-  if (warp == kMmaWarp) {
-    if (rank == 0) h4_issuer_loop<PAIR>(sm, g, tmem, n_iter, p.pad_bytes, p.trim_lo, p.trim_hi);
-  } else {
-    h4_synthesis_stream_workers<M, PAIR, false>(p, sm, tmem, pfull_leader, n_iter, 0, 0, tid);
-  }
-  h4_teardown<PAIR>(tmem, warp);
+  static_assert(M >= 8, "frame quads of 8-band groups (n_band 4 packs its chunks differently: offline kernels only)");
+  h4_kernel<true, kH4SynWorkers>(p.g, p.bank, p.n_tiles, 1u, p.pad_bytes, p.trim_lo, p.trim_hi, [&](const H4Smem& sm, uint32_t tmem, uint32_t pfull_leader, unsigned n_iter) {
+    constexpr int FR = 64 / M, NBG = M / 8;  // frames per 128-byte plane row, 8-band groups
+    const H4Shape& g = p.g;
+    const H4StreamGeom& sg = p.sg;
+    const int tid = threadIdx.x, warp = tid >> 5;
+    for (int u = sg.spt * sg.pitch * 32 + tid; u < g.rows * 32; u += kH4SynWorkers)
+#pragma unroll
+      for (int pl = 0; pl < 4; ++pl) reinterpret_cast<float*>(sm.planes + pl * g.plane)[u] = 0.f;
+    // item (frame quad wq of the tile, band group bg): four frames x eight bands = four 16-byte chunks per plane.  A region holds
+    // pitch * FR frames; its first hrows * FR frames are history (both multiples of 4: a quad never straddles the boundary)
+    const int n_fq = sg.spt * sg.pitch * FR / 4;
+    const int bg = tid / n_fq, wq = tid - bg * n_fq;
+    const bool has_item = tid < NBG * n_fq;
+    const int region_frames = sg.pitch * FR, hist_fr = sg.hrows * FR, block_fr = sg.rows_b * FR;
+    const int lt = (4 * wq) / region_frames, lf = 4 * wq - lt * region_frames;  // region, first frame of the quad within the region
+    const int fb = lf - hist_fr;  // first frame of this thread's quad within the block (negative: history)
+    // tile-invariant plan, made once: RUNNING pointers to the quad's eight band rows (in the state for history frames, in s for block
+    // frames), to its place in the next state when it is one of the block's last K frames, and what a tile step adds to them
+    constexpr int kDead = 1 << 20;
+    const size_t band0 = ((size_t)blockIdx.x * sg.spt + lt) * M + 8 * bg;  // first band row of the item in this CTA's first tile
+    const size_t step_state = (size_t)gridDim.x * sg.spt * M * p.K;
+    int slot = kDead;
+    const float* src = p.s;
+    size_t src_step = 0, src_pitch = 0;
+    float* roll = nullptr;
+    if (has_item) {
+      if (fb < 0) {
+        slot = lt;
+        src = p.state_in + band0 * p.K + (p.K - hist_fr) + lf;
+        src_step = step_state;
+        src_pitch = (size_t)p.K;
+      } else if (fb < block_fr) {
+        slot = lt;
+        src = p.s + band0 * p.F + fb;
+        src_step = (size_t)gridDim.x * sg.spt * M * p.F;
+        src_pitch = (size_t)p.F;
+        if (fb >= p.F - p.K) roll = p.state_out + band0 * p.K + (fb - (p.F - p.K));  // the last K frames of the block become the next history
+      }
+    }
+    float4 v[8];
+    int nlive = 0;  // live streams of the tile held in v
+    auto load_tile = [&](long tile) {
+      nlive = (int)min((long)sg.spt, (long)p.B - tile * sg.spt);
+      const bool live = slot < nlive;
+#pragma unroll
+      for (int kk = 0; kk < 8; ++kk)
+        v[kk] = live ? ptx::ldg128_na(reinterpret_cast<const float4*>(src + (size_t)kk * src_pitch)) : make_float4(0.f, 0.f, 0.f, 0.f);
+      src += src_step;
+    };
+    // sigma(k, n): odd bands flip on even global frames; regions and history lengths are multiples of 4 frames, so the parity is j's
+    const uint32_t flip_even = (p.parity & 1) ? 0u : 0x80000000u, flip_odd = flip_even ^ 0x80000000u;
+    auto convert = [&](int pb) {
+      if (!has_item) return;
+      unsigned char* p1 = sm.planes + (2 * pb) * g.plane;
+      if (roll != nullptr) {
+        if (slot < nlive) {
+#pragma unroll
+          for (int kk = 0; kk < 8; ++kk) *reinterpret_cast<float4*>(roll + (size_t)kk * p.K) = v[kk];
+        }
+        roll += step_state;
+      }
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        float w[8];
+        h4_synthesis_chunk8(v, j, (j & 1) ? flip_odd : flip_even, w);
+        h4_split_store8(w, p1, g.plane, sw128_offset((uint32_t)(4 * wq + j) * (2u * M) + 16u * bg));
+      }
+    };
+    // D (TMEM) -> out (h4_drain_synthesis).  pitch and rows_b are multiples of 4, so the four rows of a lane quad belong to one region
+    // and are valid or not together.
+    const int i = tid & 127, hb = tid >> 7, lane = tid & 31;
+    const int i0 = i & ~3, et = i0 / sg.pitch, eq0 = i0 - et * sg.pitch;
+    const bool e_rows = et < sg.spt && eq0 < sg.rows_b;
+    float* orun = p.out + ((size_t)blockIdx.x * sg.spt + et) * (size_t)(p.F * M) + 64 * eq0 + 32 * hb + 8 * (lane & 3);  // slot q: row eq0 + q of the block
+    const size_t out_step = (size_t)gridDim.x * sg.spt * (size_t)(p.F * M);
+    long tile = blockIdx.x, prev_tile = 0;
+    auto drain = [&](int dbuf) {
+      if (warp >= 8) return;  // every worker waited for the MMAs; the ninth warp has no TMEM rows to drain
+      float val[4][8];
+      h4_drain_synthesis(tmem, dbuf, tid, val);
+      float* op = orun;
+      orun += out_step;
+      if (!e_rows || prev_tile * sg.spt + et >= p.B) return;
+#pragma unroll
+      for (int q = 0; q < 4; ++q) ptx::stg256_cs(op + (size_t)q * 64, val[q]);
+    };
+
+    load_tile(tile);
+    h4_worker_loop<true>(sm, pfull_leader, n_iter, tid, convert, [&] { load_tile(tile + gridDim.x); }, drain, [&] {
+      prev_tile = tile;
+      tile += gridDim.x;
+    } H4_TRACE(nullptr));
+  } H4_TRACE(nullptr));
 }
 
 // launches (CTA pairs; the caller falls back to the fold kernels on any error)
-template <typename Kern, typename Params>
-inline int h4_stream_launch(Kern kern, Params p, int threads, H4Configured& configured, cudaStream_t st) {
-  int sms = 0;
-  if (!h4_shape_fits(p.g)) return -2;
-  if (int e = h4_configure(kern, p.g.bytes, configured, sms)) return e;
-  long grid = sms & ~1;
-  const long want = (p.n_tiles + 1) & ~1L;
-  if (grid > want) grid = want;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)grid);
-  cfg.blockDim = dim3((unsigned)threads);
-  cfg.dynamicSmemBytes = (size_t)p.g.bytes;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 2;
-  return (int)cudaLaunchKernelEx(&cfg, kern, p);
-}
 template <int M>
 inline int h4_launch_analysis_stream(H4AnalysisStreamParams p, cudaStream_t st) {
   static H4Configured configured;
   p.n_tiles = (p.B + p.s.spt - 1) / p.s.spt;
-  return h4_stream_launch(h4_analysis_stream_kernel<M, true>, p, kH4Threads, configured, st);
+  return h4_launch<true>(h4_analysis_stream_kernel<M>, p, kH4Threads, configured, st);
 }
 template <int M>
 inline int h4_launch_synthesis_stream(H4SynthesisStreamParams p, cudaStream_t st) {
   static H4Configured configured;
   p.n_tiles = (p.B + p.sg.spt - 1) / p.sg.spt;
-  return h4_stream_launch(h4_synthesis_stream_kernel<M, true>, p, kH4SynThreads, configured, st);
+  return h4_launch<true>(h4_synthesis_stream_kernel<M>, p, kH4SynThreads, configured, st);
 }
 
 }  // namespace pqmf

@@ -253,13 +253,6 @@ __device__ __forceinline__ float2 ldg64_na(const void* p) {
   return v;
 }
 
-// 128-bit load through L2 (no L1): data written earlier by THIS kernel (the fused streaming step reads back its own sub-bands)
-__device__ __forceinline__ float4 ldg128_cg(const float4* p) {
-  float4 v;
-  asm volatile("ld.global.cg.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p) : "memory");
-  return v;
-}
-
 // ---- packed fp32 (FFMA2) ----
 __device__ __forceinline__ float2 ffma2(float2 a, float2 b, float2 c) { return __ffma2_rn(a, b, c); }
 
