@@ -161,6 +161,27 @@ int pqmf_stream_step_f32(const float* x, float* y, float* out, const float* hk, 
                          const float* sstate_in, float* sstate_out, int B, long T, int M, int L, int parity_in, int parity_out, unsigned flags,
                          pqmf_stream_t stream);
 
+/* ---- stream pools: device-resident state of P independent streams, any n distinct of which are stepped by one call, in any order.
+ *      Each stream has its own history, ping-pong half and frame parity, all on the device (caller-owned, fp32, zeros = P fresh streams):
+ *        xpool [2, P, L]           analysis state;  spool [2, P, M, K], K = L / M   synthesis state
+ *        xphase [P] / sphase [P]   one int32 word per stream and direction: bit 0 = the half that holds the stream's current history,
+ *                                  bit 1 = the parity of the stream's next global frame index
+ *      ids [n] (device int32, distinct, in [0, P)): row r of x [n, T] / y [n, M, T/M] / s / out [n, T] is the next block of stream ids[r].
+ *      Per row the result is bit for bit that of pqmf_analysis_stream_f32 / pqmf_synthesis_stream_f32 with state_in = the stream's
+ *      current half, state_out = its other half, frame_parity = its parity bit, run on the same kernel family: the streaming Hankel-4
+ *      kernels exactly where a lockstep call with B = n runs them, the direct form everywhere else (also few-stream n_band 16, where a
+ *      lockstep call runs the fold kernels).  After the compute launches, one more launch on `stream` flips the half bit of every listed
+ *      stream and advances its parity by T / M (by n_frames for synthesis); streams not listed are untouched, state and phase word.
+ *      A row whose id is outside [0, P) gives zeros and touches no state.  ids must be distinct; one pool is stepped from one stream at a
+ *      time.  n == 0 returns 0.  The step runs both directions on the same ids (three launches). ---- */
+int pqmf_stream_pool_analysis_f32(const float* x, float* y, const float* hk, const float* tables, float* xpool, int* xphase, int P,
+                                  const int* ids, int n, long T, int M, int L, unsigned flags, pqmf_stream_t stream);
+int pqmf_stream_pool_synthesis_f32(const float* s, float* out, const float* hk, const float* tables, float* spool, int* sphase, int P,
+                                   const int* ids, int n, long n_frames, int M, int L, unsigned flags, pqmf_stream_t stream);
+int pqmf_stream_pool_step_f32(const float* x, float* y, float* out, const float* hk, const float* tables, float* xpool, int* xphase,
+                              float* spool, int* sphase, int P, const int* ids, int n, long T, int M, int L, unsigned flags,
+                              pqmf_stream_t stream);
+
 /* ---- fused round trip on device buffers: PQMFWrapper.process (PQMFWrapper.py:81-92: forward, then inverse of the same
  *      sub-bands) and the Pvoc wrapper's forward (1-PitchShifterWrapper.py:303-316) ----
  * pqmf_analysis_f32 followed by pqmf_synthesis_f32 on the same stream, as one call; the synthesis kernels walk their tiles

@@ -3,10 +3,10 @@ from .pqmf import (PQMF, CachedPQMF, classic_forward, classic_inverse, polyphase
 from . import _lib
 from ._lib import launch_count, library_paths
 from .sharding import shard_rows
-from .streaming import StreamGraph
+from .streaming import StreamGraph, StreamPool
 
 __all__ = [
     "PQMF", "CachedPQMF", "reverse_half", "polyphase_forward", "polyphase_inverse", "classic_forward", "classic_inverse",
     "get_prototype", "get_qmf_bank", "kaiser_filter", "loss_wc", "center_pad_next_pow_2", "make_odd", "launch_count",
-    "library_paths", "shard_rows", "StreamGraph",
+    "library_paths", "shard_rows", "StreamGraph", "StreamPool",
 ]

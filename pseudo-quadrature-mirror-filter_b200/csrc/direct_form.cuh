@@ -8,7 +8,9 @@
 //   synthesis: out[b,tau] = M * sum_k sum_n sigma(k, n+par) S[b,k,n] * hk[k, tau - n*M + off2]
 //
 // (closed forms of reference pqmf.py:115-130/160-177 and :133-157/180-199, SURVEY.md A.1.)
-// X / S are the block optionally preceded by caller-owned history (streaming mode).
+// X / S are the block optionally preceded by caller-owned history (streaming mode).  The POOL instantiations serve stream pools
+// (stream_pool.cuh): row b is the next block of stream ids[b], whose history, next history and frame parity come from the pool and the
+// stream's phase word; a row whose id is outside [0, P) gives zeros and touches no state.
 //
 // Both kernels are register-tiled correlations on a polyphase shared-memory layout:
 // lanes walk consecutive frames (conflict-free LDS, coalesced sub-band rows), each thread owns
@@ -20,7 +22,10 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <type_traits>
+
 #include "pcm.cuh"
+#include "stream_pool.cuh"
 
 namespace pqmf {
 
@@ -52,9 +57,13 @@ struct AnalysisDirectParams {
   PcmIn in;      // in.pcm != nullptr: the rows come from interleaved int16 PCM instead of x
   float* hist_out;  // streaming: the last L samples of (hist ++ x) per row (must not alias hist); the CTA of a row's last frame tile writes them
 };
+// POOL: hist and hist_out are both the pool [2, P, L]
+struct AnalysisDirectPoolParams : AnalysisDirectParams {
+  StreamPoolIndex pool;
+};
 
-template <int BG, int RF>
-__global__ void __launch_bounds__(kDirectThreads) analysis_direct_kernel(AnalysisDirectParams p) {
+template <int BG, int RF, bool POOL>
+__global__ void __launch_bounds__(kDirectThreads) analysis_direct_kernel(std::conditional_t<POOL, AnalysisDirectPoolParams, AnalysisDirectParams> p) {
   constexpr int FL = kDirectThreads / BG;  // frame lanes
   constexpr int FT = FL * RF;              // frames per CTA
   constexpr int NB = 4 * BG;               // bands per CTA
@@ -71,6 +80,22 @@ __global__ void __launch_bounds__(kDirectThreads) analysis_direct_kernel(Analysi
   const int M = p.M, L = p.L;
   const float* xrow = p.x + (size_t)b * p.T;
   const float* hrow = p.hist ? p.hist + (size_t)b * L : nullptr;
+  float* hout = nullptr;  // POOL: the stream's next history row
+  int parity = 0;         // POOL: the stream's frame parity
+  if constexpr (POOL) {
+    size_t cur, next;
+    if (!pool_row(p.pool, b, (size_t)L, cur, next, parity)) {  // dead row: zero sub-bands
+      float* yb = p.y + (size_t)b * M * p.n_frames;
+      for (int e = tid; e < FT * NB; e += kDirectThreads) {
+        const long n = n0 + e % FT;
+        const int k = kb + e / FT;
+        if (n < p.n_frames && k < M) yb[(size_t)k * p.n_frames + n] = 0.f;
+      }
+      return;
+    }
+    hrow = p.hist + cur;
+    hout = p.hist_out + next;
+  }
 
   float acc[RF][4];
 #pragma unroll
@@ -131,7 +156,9 @@ __global__ void __launch_bounds__(kDirectThreads) analysis_direct_kernel(Analysi
   if (p.hist_out != nullptr && blockIdx.x == gridDim.x - 1 && blockIdx.y == 0) {  // streaming: roll this row's history (no extra launch)
     for (int i = tid; i < L; i += kDirectThreads) {
       const long src = (long)i + p.T - L;  // position in the block; negative: still inside the old history
-      p.hist_out[(size_t)b * L + i] = src >= 0 ? __ldg(xrow + src) : (hrow != nullptr ? __ldg(hrow + i + p.T) : 0.f);
+      const float v = src >= 0 ? __ldg(xrow + src) : (hrow != nullptr ? __ldg(hrow + i + p.T) : 0.f);
+      if constexpr (POOL) hout[i] = v;
+      else p.hist_out[(size_t)b * L + i] = v;
     }
   }
   float* yb = p.y + (size_t)b * M * p.n_frames;
@@ -139,7 +166,7 @@ __global__ void __launch_bounds__(kDirectThreads) analysis_direct_kernel(Analysi
   for (int r = 0; r < RF; ++r) {
     const long n = n0 + tf + r * FL;
     if (n >= p.n_frames) continue;
-    const bool even = !p.nosign && ((n + p.parity) & 1) == 0;
+    const bool even = !p.nosign && ((n + (POOL ? parity : p.parity)) & 1) == 0;
 #pragma unroll
     for (int c = 0; c < 4; ++c) {
       const int k = kb + bg * 4 + c;
@@ -213,10 +240,15 @@ struct SynthesisDirectParams {
   BandTable bands;    // bands.enabled: the sub-bands come from n_band separate tensors (s unused)
   float* hist_out;    // streaming: the last K frames of (hist ++ s) per band row (must not alias hist), written by the row's last frame tile
 };
+// POOL: hist and hist_out are both the pool [2, P, M, K]
+struct SynthesisDirectPoolParams : SynthesisDirectParams {
+  StreamPoolIndex pool;
+};
 
 constexpr int kSynthBandsPerChunk = 4;
-template <int PG, int RF, bool VEC>
-__global__ void __launch_bounds__(kDirectThreads) synthesis_direct_kernel(SynthesisDirectParams p) {
+template <int PG, int RF, bool VEC, bool POOL>
+__global__ void __launch_bounds__(kDirectThreads)
+    synthesis_direct_kernel(std::conditional_t<POOL, SynthesisDirectPoolParams, SynthesisDirectParams> p) {
   constexpr int FL = kDirectThreads / PG;
   constexpr int FT = FL * RF;
   constexpr int NP = 4 * PG;  // output phases per CTA
@@ -238,6 +270,22 @@ __global__ void __launch_bounds__(kDirectThreads) synthesis_direct_kernel(Synthe
   const int jlo = p.dlo * M + p.off2;  // tap index of (d = dlo, phase 0)
   const float* sb = p.s + (size_t)b * M * p.F;
   const float* hb = p.hist ? p.hist + (size_t)b * M * p.K : nullptr;
+  float* hout = nullptr;  // POOL: the stream's next history row
+  int parity = 0;         // POOL: the stream's frame parity
+  if constexpr (POOL) {
+    size_t cur, next;
+    if (!pool_row(p.pool, b, (size_t)M * p.K, cur, next, parity)) {  // dead row: zero output
+      float* ob = p.out + (size_t)b * M * p.F;
+      for (int e = tid; e < FT * NP; e += kDirectThreads) {
+        const long f = f0 + e % FT;
+        const int ph = blockIdx.y * NP + e / FT;
+        if (f < p.F && ph < M) ob[f * M + ph] = 0.f;
+      }
+      return;
+    }
+    hb = p.hist + cur;
+    hout = p.hist_out + next;
+  }
 
   float acc[RF][4];
 #pragma unroll
@@ -264,7 +312,7 @@ __global__ void __launch_bounds__(kDirectThreads) synthesis_direct_kernel(Synthe
         } else if (hb != nullptr && n >= -(long)p.K) {
           v = __ldg(hb + (size_t)k * p.K + p.K + n);
         }
-        if (!p.nosign && (k & 1) && (((n + p.parity) & 1) == 0)) v = -v;
+        if (!p.nosign && (k & 1) && (((n + (POOL ? parity : p.parity)) & 1) == 0)) v = -v;
       }
       ss[kk * p.sstride + i] = v;
     }
@@ -299,7 +347,9 @@ __global__ void __launch_bounds__(kDirectThreads) synthesis_direct_kernel(Synthe
     for (int e = tid; e < M * p.K; e += kDirectThreads) {
       const int k = e / p.K, i = e - k * p.K;
       const long src = (long)i + p.F - p.K;
-      p.hist_out[((size_t)b * M + k) * p.K + i] = src >= 0 ? __ldg(sb + (size_t)k * p.F + src) : (hb != nullptr ? __ldg(hb + (size_t)k * p.K + i + p.F) : 0.f);
+      const float v = src >= 0 ? __ldg(sb + (size_t)k * p.F + src) : (hb != nullptr ? __ldg(hb + (size_t)k * p.K + i + p.F) : 0.f);
+      if constexpr (POOL) hout[(size_t)k * p.K + i] = v;
+      else p.hist_out[((size_t)b * M + k) * p.K + i] = v;
     }
   }
   const float gain = (float)M;

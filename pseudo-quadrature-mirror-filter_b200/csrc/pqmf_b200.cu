@@ -12,6 +12,7 @@
 #include <cstring>
 #include <mutex>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #include "direct_form.cuh"
@@ -44,14 +45,19 @@ int ensure_smem(K kernel, size_t bytes) {
   return (int)e;
 }
 
+// stream pools (stream_pool.cuh): the rows of a call are streams ids[0 .. n) of a pool of P
+using PoolRows = pqmf::StreamPoolIndex;
+
 // ------------------------------------------------------------------ direct-form launches
-template <int BG, int RF>
-int launch_analysis_direct(pqmf::AnalysisDirectParams p, int B, cudaStream_t st) {
+// Params: AnalysisDirectParams, or AnalysisDirectPoolParams for the POOL instantiations
+template <int BG, int RF, typename Params>
+int launch_analysis_direct(Params p, int B, cudaStream_t st) {
+  constexpr bool POOL = std::is_same_v<Params, pqmf::AnalysisDirectPoolParams>;
   constexpr int FL = pqmf::kDirectThreads / BG, FT = FL * RF, NB = 4 * BG;
   p.xstride = (FT + p.QC - 1) | 1;
   const size_t smem = ((size_t)p.JC * NB + (size_t)p.M * p.xstride) * sizeof(float);
   if (smem > 200 * 1024) return PQMF_ERR_UNSUPPORTED;
-  auto kern = pqmf::analysis_direct_kernel<BG, RF>;
+  auto kern = pqmf::analysis_direct_kernel<BG, RF, POOL>;
   if (int e = ensure_smem(kern, smem)) return e;
   dim3 grid((unsigned)((p.n_frames + FT - 1) / FT), (unsigned)((p.M + NB - 1) / NB), (unsigned)B);
   kern<<<grid, pqmf::kDirectThreads, smem, st>>>(p);
@@ -60,7 +66,8 @@ int launch_analysis_direct(pqmf::AnalysisDirectParams p, int B, cudaStream_t st)
 }
 
 int analysis_direct(const float* x, const float* hist, float* y, const float* hk, int B, long T, long n_frames, int M, int L,
-                    int off, int parity, int nosign, cudaStream_t st, pqmf::PcmIn pcm = pqmf::PcmIn{nullptr, 1, 0}, float* hist_out = nullptr) {
+                    int off, int parity, int nosign, cudaStream_t st, pqmf::PcmIn pcm = pqmf::PcmIn{nullptr, 1, 0}, float* hist_out = nullptr,
+                    const PoolRows* pool = nullptr) {
   if (n_frames == 0 || B == 0) return PQMF_OK;
   pqmf::AnalysisDirectParams p{};
   p.x = x; p.hist = hist; p.y = y; p.hk = hk; p.in = pcm; p.hist_out = hist_out;
@@ -72,6 +79,14 @@ int analysis_direct(const float* x, const float* hist, float* y, const float* hk
   if (jc > lceil) jc = lceil;
   p.JC = jc; p.QC = jc / M;
   if (B > 65535) return PQMF_ERR_UNSUPPORTED;
+  if (pool) {
+    const pqmf::AnalysisDirectPoolParams q{p, *pool};
+    if (M <= 4) return launch_analysis_direct<1, 4>(q, B, st);
+    if (M <= 8) return launch_analysis_direct<2, 4>(q, B, st);
+    if (M <= 32) return launch_analysis_direct<4, 4>(q, B, st);
+    if (M <= 64) return launch_analysis_direct<4, 2>(q, B, st);
+    return launch_analysis_direct<4, 1>(q, B, st);
+  }
   if (M <= 4) return launch_analysis_direct<1, 4>(p, B, st);
   if (M <= 8) return launch_analysis_direct<2, 4>(p, B, st);
   if (M <= 32) return launch_analysis_direct<4, 4>(p, B, st);
@@ -79,14 +94,16 @@ int analysis_direct(const float* x, const float* hist, float* y, const float* hk
   return launch_analysis_direct<4, 1>(p, B, st);
 }
 
-template <int PG, int RF, bool VEC>
-int launch_synthesis_direct(pqmf::SynthesisDirectParams p, int B, cudaStream_t st) {
+// Params: SynthesisDirectParams, or SynthesisDirectPoolParams for the POOL instantiations
+template <int PG, int RF, bool VEC, typename Params>
+int launch_synthesis_direct(Params p, int B, cudaStream_t st) {
+  constexpr bool POOL = std::is_same_v<Params, pqmf::SynthesisDirectPoolParams>;
   constexpr int FL = pqmf::kDirectThreads / PG, FT = FL * RF, NP = 4 * PG;
   p.hstride = p.ND * p.M + 16;
   p.sstride = (FT + p.ND - 1) | 1;
   const size_t smem = (size_t)pqmf::kSynthBandsPerChunk * ((size_t)p.hstride + p.sstride) * sizeof(float);
   if (smem > 200 * 1024) return PQMF_ERR_UNSUPPORTED;
-  auto kern = pqmf::synthesis_direct_kernel<PG, RF, VEC>;
+  auto kern = pqmf::synthesis_direct_kernel<PG, RF, VEC, POOL>;
   if (int e = ensure_smem(kern, smem)) return e;
   dim3 grid((unsigned)((p.F + FT - 1) / FT), (unsigned)((p.M + NP - 1) / NP), (unsigned)B);
   kern<<<grid, pqmf::kDirectThreads, smem, st>>>(p);
@@ -96,7 +113,7 @@ int launch_synthesis_direct(pqmf::SynthesisDirectParams p, int B, cudaStream_t s
 
 int synthesis_direct(const float* s, const float* hist, float* out, const float* hk, int B, long F, int M, int L, int off2,
                      int parity, int nosign, cudaStream_t st, int16_t* pcm_out = nullptr, int C = 1, const pqmf::BandTable* bands = nullptr,
-                     float* hist_out = nullptr) {
+                     float* hist_out = nullptr, const PoolRows* pool = nullptr) {
   if (F == 0 || B == 0) return PQMF_OK;
   pqmf::SynthesisDirectParams p{};
   p.s = s; p.hist = hist; p.out = out; p.hk = hk; p.pcm_out = pcm_out; p.C = C; p.hist_out = hist_out;
@@ -107,6 +124,13 @@ int synthesis_direct(const float* s, const float* hist, float* out, const float*
   p.ND = dhi - p.dlo + 1;
   if (B > 65535) return PQMF_ERR_UNSUPPORTED;
   const bool vec = (M % 4) == 0;
+  if (pool) {
+    const pqmf::SynthesisDirectPoolParams q{p, *pool};
+    if (!vec) return launch_synthesis_direct<4, 4, false>(q, B, st);
+    if (M <= 4) return launch_synthesis_direct<1, 4, true>(q, B, st);
+    if (M <= 8) return launch_synthesis_direct<2, 4, true>(q, B, st);
+    return launch_synthesis_direct<4, 4, true>(q, B, st);
+  }
   if (!vec) return launch_synthesis_direct<4, 4, false>(p, B, st);
   if (M <= 4) return launch_synthesis_direct<1, 4, true>(p, B, st);
   if (M <= 8) return launch_synthesis_direct<2, 4, true>(p, B, st);
@@ -289,8 +313,9 @@ int h4_synthesis(const void* s, void* out, const float* tables, int B, long F, i
 
 // ---- streaming blocks of n_band 16 on the Hankel kernels (hankel4_stream.cuh): several streams per MMA tile.  Any refusal
 //      (short blocks, few streams, odd sizes, a context without CTA pairs) returns UNSUPPORTED and the fold kernels run instead ----
+// pool != nullptr: the indexed (POOL) kernels, with state_in = state_out = the pool
 int h4_analysis_stream(const float* x, float* y, const float* tables, const float* state_in, float* state_out, int B, long T, int M, int L,
-                       int parity, unsigned flags, cudaStream_t st) {
+                       int parity, unsigned flags, cudaStream_t st, const PoolRows* pool = nullptr) {
   int jlo, kt;
   h4_taps(flags, jlo, kt);
   if (kt == 0 || (flags & (PQMF_FLAG_H4_SPLIT | PQMF_FLAG_NO_PAIR | PQMF_FLAG_FOLD))) return PQMF_ERR_UNSUPPORTED;
@@ -309,11 +334,21 @@ int h4_analysis_stream(const float* x, float* y, const float* tables, const floa
   p.s = sg;
   p.bank = reinterpret_cast<const uint16_t*>(tables + h4_pair_offset(M, L));
   int e = -2;
-  switch (M) {
-    case 8: e = pqmf::h4_launch_analysis_stream<8>(p, st); break;
-    case 16: e = pqmf::h4_launch_analysis_stream<16>(p, st); break;
-    case 32: e = pqmf::h4_launch_analysis_stream<32>(p, st); break;
-    default: break;
+  if (pool) {
+    const pqmf::H4AnalysisStreamPoolParams q{p, *pool};
+    switch (M) {
+      case 8: e = pqmf::h4_launch_analysis_stream<8>(q, st); break;
+      case 16: e = pqmf::h4_launch_analysis_stream<16>(q, st); break;
+      case 32: e = pqmf::h4_launch_analysis_stream<32>(q, st); break;
+      default: break;
+    }
+  } else {
+    switch (M) {
+      case 8: e = pqmf::h4_launch_analysis_stream<8>(p, st); break;
+      case 16: e = pqmf::h4_launch_analysis_stream<16>(p, st); break;
+      case 32: e = pqmf::h4_launch_analysis_stream<32>(p, st); break;
+      default: break;
+    }
   }
   if (e != 0) {
     (void)cudaGetLastError();
@@ -322,7 +357,7 @@ int h4_analysis_stream(const float* x, float* y, const float* tables, const floa
   return 0;
 }
 int h4_synthesis_stream(const float* s, float* out, const float* tables, const float* state_in, float* state_out, int B, long F, int M, int L,
-                        int parity, unsigned flags, cudaStream_t st) {
+                        int parity, unsigned flags, cudaStream_t st, const PoolRows* pool = nullptr) {
   int jlo, kt;
   h4_taps(flags, jlo, kt);
   if (kt == 0 || (flags & (PQMF_FLAG_H4_SPLIT | PQMF_FLAG_NO_PAIR | PQMF_FLAG_FOLD))) return PQMF_ERR_UNSUPPORTED;
@@ -342,11 +377,21 @@ int h4_synthesis_stream(const float* s, float* out, const float* tables, const f
   p.sg = sg;
   p.bank = reinterpret_cast<const uint16_t*>(tables + h4_pair_offset(M, L) + h4_pair_floats(M, L));
   int e = -2;
-  switch (M) {
-    case 8: e = pqmf::h4_launch_synthesis_stream<8>(p, st); break;
-    case 16: e = pqmf::h4_launch_synthesis_stream<16>(p, st); break;
-    case 32: e = pqmf::h4_launch_synthesis_stream<32>(p, st); break;
-    default: break;
+  if (pool) {
+    const pqmf::H4SynthesisStreamPoolParams q{p, *pool};
+    switch (M) {
+      case 8: e = pqmf::h4_launch_synthesis_stream<8>(q, st); break;
+      case 16: e = pqmf::h4_launch_synthesis_stream<16>(q, st); break;
+      case 32: e = pqmf::h4_launch_synthesis_stream<32>(q, st); break;
+      default: break;
+    }
+  } else {
+    switch (M) {
+      case 8: e = pqmf::h4_launch_synthesis_stream<8>(p, st); break;
+      case 16: e = pqmf::h4_launch_synthesis_stream<16>(p, st); break;
+      case 32: e = pqmf::h4_launch_synthesis_stream<32>(p, st); break;
+      default: break;
+    }
   }
   if (e != 0) {
     (void)cudaGetLastError();
@@ -605,6 +650,37 @@ int roundtrip_host(const Sample* x_host, float* y_host, Sample* out_host, const 
   }
   return rc;
 }
+
+// ---- stream pools.  One routing decision per direction: the indexed Hankel-4 kernels exactly where a lockstep call with B = n runs the
+//      Hankel-4 streaming kernels (the same family test as pqmf_*_stream_f32, and h4_*_stream's own shape, flag, alignment and tile-count
+//      checks); the indexed direct form everywhere else -- including few-stream n_band 16, where a lockstep call runs the fold kernels ----
+bool h4_stream_family(int M, int L, const float* tables, unsigned flags) {
+  if (use_fast(M, L, tables, flags)) return true;  // n_band 16 / L 512
+  return !pqmf::hankel16_supported(M, L) && use_h4_family(M, L, tables, flags) && (M == 8 || M == 32);
+}
+int pool_analysis(const float* x, float* y, const float* hk, const float* tables, float* xpool, const PoolRows& pool, int n, long T, int M, int L,
+                  unsigned flags, cudaStream_t st) {
+  if (h4_stream_family(M, L, tables, flags) && h4_analysis_stream(x, y, tables, xpool, xpool, n, T, M, L, 0, flags, st, &pool) == 0) {
+    ++g_launches;
+    return 0;
+  }
+  return analysis_direct(x, xpool, y, hk, n, T, T / M, M, L, L, 0, 0, st, pqmf::PcmIn{nullptr, 1, 0}, xpool, &pool);
+}
+int pool_synthesis(const float* s, float* out, const float* hk, const float* tables, float* spool, const PoolRows& pool, int n, long F, int M, int L,
+                   unsigned flags, cudaStream_t st) {
+  if (h4_stream_family(M, L, tables, flags) && h4_synthesis_stream(s, out, tables, spool, spool, n, F, M, L, 0, flags, st, &pool) == 0) {
+    ++g_launches;
+    return 0;
+  }
+  return synthesis_direct(s, spool, out, hk, n, F, M, L, -M, 0, 0, st, nullptr, 1, nullptr, spool, &pool);
+}
+// after the compute launches of a call: flip the half and advance the parity of every listed stream (one launch on the same stream)
+int pool_phase(const PoolRows& pool, int n, int* xphase, long x_frames, int* sphase, long s_frames, cudaStream_t st) {
+  pqmf::stream_pool_phase_kernel<<<(n + 255) / 256, 256, 0, st>>>(pool.ids, n, pool.P, xphase, (int)(x_frames & 1), sphase, (int)(s_frames & 1));
+  ++g_launches;
+  return cuda_status();
+}
+bool bad_pool(int P, int n) { return P < 1 || n < 0 || n > P; }
 
 }  // namespace
 
@@ -920,6 +996,41 @@ int pqmf_stream_step_f32(const float* x, float* y, float* out, const float* hk, 
   int e = pqmf_analysis_stream_f32(x, y, hk, tables, xstate_in, xstate_out, B, T, M, L, parity_in, flags, stream);
   if (e) return e;
   return pqmf_synthesis_stream_f32(y, out, hk, tables, sstate_in, sstate_out, B, T / M, M, L, parity_out, flags, stream);
+}
+
+int pqmf_stream_pool_analysis_f32(const float* x, float* y, const float* hk, const float* tables, float* xpool, int* xphase, int P,
+                                  const int* ids, int n, long T, int M, int L, unsigned flags, pqmf_stream_t stream) {
+  if (bad_dims(n, T, M, L) || bad_pool(P, n) || T <= 0 || (T % M) != 0) return PQMF_ERR_ARG;
+  if (n == 0) return PQMF_OK;
+  if (!x || !y || !hk || !xpool || !xphase || !ids) return PQMF_ERR_ARG;
+  cudaStream_t st = (cudaStream_t)stream;
+  const PoolRows pool{ids, xphase, P};
+  if (int e = pool_analysis(x, y, hk, tables, xpool, pool, n, T, M, L, flags, st)) return e;
+  return pool_phase(pool, n, xphase, T / M, nullptr, 0, st);
+}
+
+int pqmf_stream_pool_synthesis_f32(const float* s, float* out, const float* hk, const float* tables, float* spool, int* sphase, int P,
+                                   const int* ids, int n, long n_frames, int M, int L, unsigned flags, pqmf_stream_t stream) {
+  if (bad_dims(n, n_frames, M, L) || bad_pool(P, n) || n_frames <= 0 || (L % M) != 0) return PQMF_ERR_ARG;
+  if (n == 0) return PQMF_OK;
+  if (!s || !out || !hk || !spool || !sphase || !ids) return PQMF_ERR_ARG;
+  cudaStream_t st = (cudaStream_t)stream;
+  const PoolRows pool{ids, sphase, P};
+  if (int e = pool_synthesis(s, out, hk, tables, spool, pool, n, n_frames, M, L, flags, st)) return e;
+  return pool_phase(pool, n, nullptr, 0, sphase, n_frames, st);
+}
+
+int pqmf_stream_pool_step_f32(const float* x, float* y, float* out, const float* hk, const float* tables, float* xpool, int* xphase,
+                              float* spool, int* sphase, int P, const int* ids, int n, long T, int M, int L, unsigned flags,
+                              pqmf_stream_t stream) {
+  if (bad_dims(n, T, M, L) || bad_pool(P, n) || T <= 0 || (T % M) != 0 || (L % M) != 0) return PQMF_ERR_ARG;
+  if (n == 0) return PQMF_OK;
+  if (!x || !y || !out || !hk || !xpool || !xphase || !spool || !sphase || !ids || xphase == sphase) return PQMF_ERR_ARG;
+  cudaStream_t st = (cudaStream_t)stream;
+  const PoolRows xrows{ids, xphase, P}, srows{ids, sphase, P};
+  if (int e = pool_analysis(x, y, hk, tables, xpool, xrows, n, T, M, L, flags, st)) return e;
+  if (int e = pool_synthesis(y, out, hk, tables, spool, srows, n, T / M, M, L, flags, st)) return e;
+  return pool_phase(xrows, n, xphase, T / M, sphase, T / M, st);
 }
 
 int pqmf_roundtrip_f32(const float* x, float* y, float* out, const float* hk, const float* tables, int B, long T, long n_frames,

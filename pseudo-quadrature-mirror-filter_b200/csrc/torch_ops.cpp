@@ -300,6 +300,100 @@ std::tuple<at::Tensor, at::Tensor> stream_step(const at::Tensor& x, const at::Te
   return {out, y};
 }
 
+// ---- stream pools (pqmf_stream_pool_*_f32): pool [2, P, ...] and phase [P] are mutated in place; ids is a CUDA int32 tensor of n
+//      distinct stream numbers, trusted as it is (checking it would need a host synchronisation) ----
+struct Pool {
+  int64_t P;
+  float* state;
+  int* phase;
+};
+Pool pool_of(const at::Tensor& state, const at::Tensor& phase, const Bank& bank, const at::Tensor& like, const char* what) {
+  check_f32_cuda(state, what);
+  TORCH_CHECK(state.is_contiguous() && state.dim() >= 2 && state.size(0) == 2 && state.device() == like.device() &&
+                  state.numel() == 2 * state.size(1) * bank.L,
+              what, " must be a contiguous [2, P, ...] tensor of 2 * P * L float32 elements (L=", bank.L, ") on the input's device");
+  TORCH_CHECK(phase.is_cuda() && phase.scalar_type() == at::kInt && phase.is_contiguous() && phase.dim() == 1 && phase.size(0) == state.size(1) &&
+                  phase.device() == like.device(),
+              "phase words must be a contiguous int32 [P] tensor on the input's device (P=", state.size(1), ")");
+  TORCH_CHECK(state.size(1) >= 1 && state.size(1) < (1LL << 31), "bad pool size");
+  return {state.size(1), state.data_ptr<float>(), phase.data_ptr<int>()};
+}
+const int* ids_of(const at::Tensor& ids, int64_t n, const at::Tensor& like) {
+  TORCH_CHECK(ids.is_cuda() && ids.scalar_type() == at::kInt && ids.dim() == 1 && ids.is_contiguous() && ids.device() == like.device(),
+              "ids must be a contiguous 1-D int32 CUDA tensor on the input's device");
+  TORCH_CHECK(ids.size(0) == n, "ids has ", ids.size(0), " entries but the block has ", n, " rows");
+  return ids.data_ptr<int>();
+}
+
+// x [n, 1, T] -> y [n, M, T / M]
+at::Tensor stream_pool_analysis(const at::Tensor& x, const at::Tensor& hk, const at::Tensor& tables, at::Tensor xpool, at::Tensor xphase,
+                                const at::Tensor& ids, int64_t flags) {
+  check_f32_cuda(x, "x");
+  TORCH_CHECK(x.dim() == 3 && x.size(1) == 1, "pqmf stream pool analysis expects [streams, 1, block], got ", x.sizes());
+  const Bank bank = bank_of(hk, x);
+  c10::cuda::CUDAGuard guard(x.device());
+  const at::Tensor xc = x.contiguous();
+  const int64_t n = xc.size(0), T = xc.size(2);
+  TORCH_CHECK(T > 0 && T % bank.M == 0, "streaming block length ", T, " must be a positive multiple of n_band=", bank.M);
+  const Pool pool = pool_of(xpool, xphase, bank, x, "xpool");
+  const int* id = ids_of(ids, n, x);
+  TORCH_CHECK(n <= pool.P, "more rows (", n, ") than streams in the pool (", pool.P, ")");
+  at::Tensor y = at::empty({n, bank.M, T / bank.M}, xc.options());
+  if (n == 0) return y;
+  check_rc(pqmf_stream_pool_analysis_f32(xc.data_ptr<float>(), y.data_ptr<float>(), bank.ptr, tables_ptr(tables, x), pool.state, pool.phase, (int)pool.P,
+                                         id, (int)n, (long)T, (int)bank.M, (int)bank.L, (unsigned)flags,
+                                         (pqmf_stream_t)at::cuda::getCurrentCUDAStream().stream()),
+           "pqmf_stream_pool_analysis_f32");
+  return y;
+}
+
+// s [n, M, F] -> out [n, 1, M F]
+at::Tensor stream_pool_synthesis(const at::Tensor& s, const at::Tensor& hk, const at::Tensor& tables, at::Tensor spool, at::Tensor sphase,
+                                 const at::Tensor& ids, int64_t flags) {
+  check_f32_cuda(s, "s");
+  const Bank bank = bank_of(hk, s);
+  TORCH_CHECK(s.dim() == 3 && s.size(1) == bank.M, "pqmf stream pool synthesis expects [streams, n_band, frames], got ", s.sizes());
+  TORCH_CHECK(bank.L % bank.M == 0, "streaming synthesis needs L a multiple of n_band");
+  c10::cuda::CUDAGuard guard(s.device());
+  const at::Tensor sc = s.contiguous();
+  const int64_t n = sc.size(0), F = sc.size(2);
+  TORCH_CHECK(F > 0, "empty block");
+  const Pool pool = pool_of(spool, sphase, bank, s, "spool");
+  const int* id = ids_of(ids, n, s);
+  TORCH_CHECK(n <= pool.P, "more rows (", n, ") than streams in the pool (", pool.P, ")");
+  at::Tensor out = at::empty({n, 1, bank.M * F}, sc.options());
+  if (n == 0) return out;
+  check_rc(pqmf_stream_pool_synthesis_f32(sc.data_ptr<float>(), out.data_ptr<float>(), bank.ptr, tables_ptr(tables, s), pool.state, pool.phase,
+                                          (int)pool.P, id, (int)n, (long)F, (int)bank.M, (int)bank.L, (unsigned)flags,
+                                          (pqmf_stream_t)at::cuda::getCurrentCUDAStream().stream()),
+           "pqmf_stream_pool_synthesis_f32");
+  return out;
+}
+
+// one block step of the listed streams: (out [n, 1, T], y [n, M, T / M])
+std::tuple<at::Tensor, at::Tensor> stream_pool_step(const at::Tensor& x, const at::Tensor& hk, const at::Tensor& tables, at::Tensor xpool,
+                                                     at::Tensor xphase, at::Tensor spool, at::Tensor sphase, const at::Tensor& ids, int64_t flags) {
+  check_f32_cuda(x, "x");
+  TORCH_CHECK(x.dim() == 3 && x.size(1) == 1, "pqmf stream pool step expects [streams, 1, block], got ", x.sizes());
+  const Bank bank = bank_of(hk, x);
+  c10::cuda::CUDAGuard guard(x.device());
+  const at::Tensor xc = x.contiguous();
+  const int64_t n = xc.size(0), T = xc.size(2);
+  TORCH_CHECK(T > 0 && T % bank.M == 0 && bank.L % bank.M == 0, "streaming block length ", T, " must be a positive multiple of n_band=", bank.M);
+  const Pool xp = pool_of(xpool, xphase, bank, x, "xpool"), sp = pool_of(spool, sphase, bank, x, "spool");
+  TORCH_CHECK(xp.P == sp.P, "the analysis and synthesis pools hold different numbers of streams");
+  const int* id = ids_of(ids, n, x);
+  TORCH_CHECK(n <= xp.P, "more rows (", n, ") than streams in the pool (", xp.P, ")");
+  at::Tensor y = at::empty({n, bank.M, T / bank.M}, xc.options());
+  at::Tensor out = at::empty({n, 1, T}, xc.options());
+  if (n == 0) return {out, y};
+  check_rc(pqmf_stream_pool_step_f32(xc.data_ptr<float>(), y.data_ptr<float>(), out.data_ptr<float>(), bank.ptr, tables_ptr(tables, x), xp.state, xp.phase,
+                                     sp.state, sp.phase, (int)xp.P, id, (int)n, (long)T, (int)bank.M, (int)bank.L, (unsigned)flags,
+                                     (pqmf_stream_t)at::cuda::getCurrentCUDAStream().stream()),
+           "pqmf_stream_pool_step_f32");
+  return {out, y};
+}
+
 int64_t launch_count() { return (int64_t)pqmf_launch_count(); }
 
 // ---- autograd (SURVEY 8f-2: the reference path is differentiable, upstream users train through PQMF) --------------------
@@ -431,6 +525,35 @@ std::tuple<at::Tensor, at::Tensor> stream_step_autograd(const at::Tensor& x, con
   return op.call(x, hk, tables, xs_in, xs_out, ss_in, ss_out, parity_in, parity_out, flags);
 }
 
+at::Tensor stream_pool_analysis_autograd(const at::Tensor& x, const at::Tensor& hk, const at::Tensor& tables, at::Tensor xpool, at::Tensor xphase,
+                                         const at::Tensor& ids, int64_t flags) {
+  TORCH_CHECK(!(at::GradMode::is_enabled() && x.requires_grad()),
+              "pqmf_b200::stream_pool_analysis is not differentiable (a stream pool carries state across calls); use forward() for training "
+              "or wrap the call in torch.no_grad()");
+  at::AutoDispatchBelowADInplaceOrView guard;
+  static auto op = c10::Dispatcher::singleton().findSchemaOrThrow("pqmf_b200::stream_pool_analysis", "").typed<decltype(stream_pool_analysis)>();
+  return op.call(x, hk, tables, xpool, xphase, ids, flags);
+}
+at::Tensor stream_pool_synthesis_autograd(const at::Tensor& s, const at::Tensor& hk, const at::Tensor& tables, at::Tensor spool, at::Tensor sphase,
+                                          const at::Tensor& ids, int64_t flags) {
+  TORCH_CHECK(!(at::GradMode::is_enabled() && s.requires_grad()),
+              "pqmf_b200::stream_pool_synthesis is not differentiable (a stream pool carries state across calls); use inverse() for training "
+              "or wrap the call in torch.no_grad()");
+  at::AutoDispatchBelowADInplaceOrView guard;
+  static auto op = c10::Dispatcher::singleton().findSchemaOrThrow("pqmf_b200::stream_pool_synthesis", "").typed<decltype(stream_pool_synthesis)>();
+  return op.call(s, hk, tables, spool, sphase, ids, flags);
+}
+std::tuple<at::Tensor, at::Tensor> stream_pool_step_autograd(const at::Tensor& x, const at::Tensor& hk, const at::Tensor& tables, at::Tensor xpool,
+                                                             at::Tensor xphase, at::Tensor spool, at::Tensor sphase, const at::Tensor& ids,
+                                                             int64_t flags) {
+  TORCH_CHECK(!(at::GradMode::is_enabled() && x.requires_grad()),
+              "pqmf_b200::stream_pool_step is not differentiable (a stream pool carries state across calls); use forward() / inverse() for "
+              "training or wrap the call in torch.no_grad()");
+  at::AutoDispatchBelowADInplaceOrView guard;
+  static auto op = c10::Dispatcher::singleton().findSchemaOrThrow("pqmf_b200::stream_pool_step", "").typed<decltype(stream_pool_step)>();
+  return op.call(x, hk, tables, xpool, xphase, spool, sphase, ids, flags);
+}
+
 at::Tensor analysis_autograd(const at::Tensor& x, const at::Tensor& hk, const at::Tensor& tables, int64_t n_frames, int64_t flags) {
   return AnalysisFn::apply(x, hk, tables, n_frames, flags);
 }
@@ -457,6 +580,11 @@ TORCH_LIBRARY(pqmf_b200, m) {
   m.def("synthesis_bands(Tensor[] bands, Tensor hk, int n_frames, int delay_frames, Tensor prev_tail, Tensor fade_out, Tensor fade_in, int flags) -> (Tensor, Tensor)");
   m.def("analysis_pcm16(Tensor pcm, Tensor hk, Tensor tables, int n_frames, bool downmix, int flags) -> Tensor");
   m.def("synthesis_pcm16(Tensor s, Tensor hk, Tensor tables, int delay_frames, int flags) -> Tensor");
+  m.def("stream_pool_analysis(Tensor x, Tensor hk, Tensor tables, Tensor(a!) xpool, Tensor(b!) xphase, Tensor ids, int flags) -> Tensor");
+  m.def("stream_pool_synthesis(Tensor s, Tensor hk, Tensor tables, Tensor(a!) spool, Tensor(b!) sphase, Tensor ids, int flags) -> Tensor");
+  m.def(
+      "stream_pool_step(Tensor x, Tensor hk, Tensor tables, Tensor(a!) xpool, Tensor(b!) xphase, Tensor(c!) spool, Tensor(d!) sphase, Tensor ids, "
+      "int flags) -> (Tensor, Tensor)");
   m.def("launch_count() -> int", &launch_count);
 }
 
@@ -471,6 +599,9 @@ TORCH_LIBRARY_IMPL(pqmf_b200, CUDA, m) {
   m.impl("synthesis_bands", &synthesis_bands);
   m.impl("analysis_pcm16", &analysis_pcm16);
   m.impl("synthesis_pcm16", &synthesis_pcm16);
+  m.impl("stream_pool_analysis", &stream_pool_analysis);
+  m.impl("stream_pool_synthesis", &stream_pool_synthesis);
+  m.impl("stream_pool_step", &stream_pool_step);
 }
 
 // gradients w.r.t. the signal / the sub-bands only (the bank is a registered buffer in the reference, not a parameter)
@@ -480,4 +611,7 @@ TORCH_LIBRARY_IMPL(pqmf_b200, Autograd, m) {
   m.impl("analysis_stream", &analysis_stream_autograd);
   m.impl("synthesis_stream", &synthesis_stream_autograd);
   m.impl("stream_step", &stream_step_autograd);
+  m.impl("stream_pool_analysis", &stream_pool_analysis_autograd);
+  m.impl("stream_pool_synthesis", &stream_pool_synthesis_autograd);
+  m.impl("stream_pool_step", &stream_pool_step_autograd);
 }
