@@ -182,6 +182,37 @@ int pqmf_stream_pool_step_f32(const float* x, float* y, float* out, const float*
                               float* spool, int* sphase, int P, const int* ids, int n, long T, int M, int L, unsigned flags,
                               pqmf_stream_t stream);
 
+/* ---- int16 PCM blocks in the streaming calls (the PCM edge of pqmf_analysis_pcm16 / pqmf_synthesis_pcm16 on the streaming and pool entries
+ *      above): what the reference's block driver streams (PitchShifterPvoc/2-TestBlocks.py:26-30) and what a server's sessions receive and
+ *      return.  A PCM block is int16 interleaved WAV frames pcm [B, T, C]; widening is v / 32768 per channel, or with downmix != 0 the fp32
+ *      sum over the channels in channel order, then / C; quantising is clamp(rint(v * 32768), -32768, 32767).  Rows are B * C (row
+ *      b * C + c = channel c of clip b) or B with downmix.  Per row every entry is bit for bit its fp32 counterpart on the widened block,
+ *      followed by quantising, with the same state and phase-word updates: PCM and fp32 blocks continue one stream.
+ *        pqmf_analysis_stream_pcm16   pcm [B, T, C] -> y [rows, M, T/M]; state as pqmf_analysis_stream_f32 (rows streams)
+ *        pqmf_synthesis_stream_pcm16  s [B * C, M, n_frames] -> pcm [B, M * n_frames, C]; state as pqmf_synthesis_stream_f32
+ *        pqmf_stream_step_pcm16       pcm [B, T, C] -> y [rows, M, T/M] and pcm_out [B, T, C'] (C' = 1 with downmix, else C)
+ *        pqmf_stream_pool_*_pcm16     the pool entries with PCM blocks: ids [rows] (row r is the next block of stream ids[r]), rows <= P
+ *      Native kernels: the streaming Hankel-4 kernels (n_band 8 / 16 / 32), exactly where the fp32 call with the same rows, T, flags and
+ *      pool-ness runs them and the PCM buffer is aligned for them (32 bytes in, 16 bytes out); PCM output natively for one channel per clip
+ *      only.  Every other call (few streams, short or odd blocks, the fold / direct-form families, misaligned buffers, C' > 1 output)
+ *      returns PQMF_ERR_UNSUPPORTED before anything is launched, with state and phase words untouched; the caller widens, calls the fp32
+ *      entry and quantises (torch_ops.cpp does).  A step is native only when both directions are; a native step makes the launches of the
+ *      fp32 step (two lockstep, three in a pool).  Argument errors are checked on the host first (PQMF_ERR_ARG; B == 0 returns 0). ---- */
+int pqmf_analysis_stream_pcm16(const int16_t* pcm, float* y, const float* hk, const float* tables, const float* state_in, float* state_out, int B,
+                               long T, int C, int downmix, int M, int L, int frame_parity, unsigned flags, pqmf_stream_t stream);
+int pqmf_synthesis_stream_pcm16(const float* s, int16_t* pcm, const float* hk, const float* tables, const float* state_in, float* state_out, int B,
+                                int C, long n_frames, int M, int L, int frame_parity, unsigned flags, pqmf_stream_t stream);
+int pqmf_stream_step_pcm16(const int16_t* pcm, float* y, int16_t* pcm_out, const float* hk, const float* tables, const float* xstate_in,
+                           float* xstate_out, const float* sstate_in, float* sstate_out, int B, long T, int C, int downmix, int M, int L, int parity_in,
+                           int parity_out, unsigned flags, pqmf_stream_t stream);
+int pqmf_stream_pool_analysis_pcm16(const int16_t* pcm, float* y, const float* hk, const float* tables, float* xpool, int* xphase, int P,
+                                    const int* ids, int B, long T, int C, int downmix, int M, int L, unsigned flags, pqmf_stream_t stream);
+int pqmf_stream_pool_synthesis_pcm16(const float* s, int16_t* pcm, const float* hk, const float* tables, float* spool, int* sphase, int P,
+                                     const int* ids, int B, int C, long n_frames, int M, int L, unsigned flags, pqmf_stream_t stream);
+int pqmf_stream_pool_step_pcm16(const int16_t* pcm, float* y, int16_t* pcm_out, const float* hk, const float* tables, float* xpool, int* xphase,
+                                float* spool, int* sphase, int P, const int* ids, int B, long T, int C, int downmix, int M, int L, unsigned flags,
+                                pqmf_stream_t stream);
+
 /* ---- fused round trip on device buffers: PQMFWrapper.process (PQMFWrapper.py:81-92: forward, then inverse of the same
  *      sub-bands) and the Pvoc wrapper's forward (1-PitchShifterWrapper.py:303-316) ----
  * pqmf_analysis_f32 followed by pqmf_synthesis_f32 on the same stream, as one call; the synthesis kernels walk their tiles

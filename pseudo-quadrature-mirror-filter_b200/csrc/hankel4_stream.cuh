@@ -14,9 +14,14 @@
 // MMA row reads only its own stream's region, so which streams share a tile changes nothing: only the addresses of the history and
 // of the roll, and the sign, come from ids and the phase word, loaded per tile one tile ahead with the block.  A row whose id is
 // outside [0, P) is dead: zeros in, zeros out, no state touched.
+//
+// int16 PCM edge (IO = H4Io::PCM, pcm.cuh): the analysis reads its block from interleaved WAV frames (any channel count, optional
+// down-mix) and the synthesis of mono rows writes int16 samples.  The history is the fp32 state in both directions: the analysis rolls
+// the WIDENED block into it, so the state after a PCM block is the state after the fp32 block it stands for.
 #pragma once
 #include <type_traits>
 
+#include "half_io.cuh"
 #include "hankel4.cuh"
 #include "stream_pool.cuh"
 
@@ -55,12 +60,23 @@ struct H4AnalysisStreamParams {
 struct H4AnalysisStreamPoolParams : H4AnalysisStreamParams {
   StreamPoolIndex pool;
 };
+// PCM: the block rows come from interleaved int16 WAV frames (x unused); row b is channel b % C of clip b / C, or clip b when down-mixing
+struct H4AnalysisStreamPcmParams : H4AnalysisStreamParams {
+  PcmIn in;
+};
+struct H4AnalysisStreamPoolPcmParams : H4AnalysisStreamPoolParams {
+  PcmIn in;
+};
+template <bool POOL, H4Io IO>
+using H4AnalysisStreamArgs = std::conditional_t<POOL, std::conditional_t<IO == H4Io::PCM, H4AnalysisStreamPoolPcmParams, H4AnalysisStreamPoolParams>,
+                                                std::conditional_t<IO == H4Io::PCM, H4AnalysisStreamPcmParams, H4AnalysisStreamParams>>;
 
 // streaming analysis: tiles blockIdx.x, + gridDim.x, ... of spt streams each
-template <int M, bool POOL>
-__global__ void __launch_bounds__(kH4Threads, 1)
-    h4_analysis_stream_kernel(std::conditional_t<POOL, H4AnalysisStreamPoolParams, H4AnalysisStreamParams> p) {
+template <int M, bool POOL, H4Io IO>
+__global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_stream_kernel(H4AnalysisStreamArgs<POOL, IO> p) {
+  static_assert(IO == H4Io::F32 || IO == H4Io::PCM, "streaming blocks: fp32 rows or int16 PCM frames");
   h4_kernel<true, kH4Workers>(p.g, p.bank, p.n_tiles, 1u, p.pad_bytes, p.trim_lo, p.trim_hi, [&](const H4Smem& sm, uint32_t tmem, uint32_t pfull_leader, unsigned n_iter) {
+    constexpr bool PCM = IO == H4Io::PCM;
     constexpr int FR = 64 / M, HB = M / 2;  // frames per 64-sample row, bands per epilogue thread
     constexpr int NO = (kH4Rows * 8 + kH4Workers - 1) / kH4Workers;  // 4 x 8 samples per thread cover the 128 region rows of a tile
     const H4Shape& g = p.g;
@@ -82,6 +98,10 @@ __global__ void __launch_bounds__(kH4Threads, 1)
     size_t src_step[NO];
     float* roll[NO];  // where the group goes in hist_out (nullptr: it is not part of the last L samples)
     int hofs[NO], rofs[NO];  // POOL: offset of a history group in its stream's pool row / of a roll group in the next history (-1: neither)
+    // PCM: sample offset of a block group within its row (-1: not a block group).  The frames of row b sit in clip b / C (b when
+    // down-mixing), channel b % C: with C > 1 the step from one tile's row to the next need not keep the channel, so the address is made
+    // per tile from the row index (tile * spt + slot) instead of a running pointer.
+    [[maybe_unused]] int bofs[NO];
 #pragma unroll
     for (int r = 0; r < NO; ++r) {
       const int u = tid + kH4Workers * r;
@@ -90,6 +110,7 @@ __global__ void __launch_bounds__(kH4Threads, 1)
       src_step[r] = 0;
       roll[r] = nullptr;
       hofs[r] = rofs[r] = -1;
+      if constexpr (PCM) bofs[r] = -1;
       if (u < n_octs) {
         const int t = u / region_octs, w = u - t * region_octs, q = w >> 3, col = w & 7;
         const size_t stream0 = (size_t)blockIdx.x * sg.spt + t;  // the stream this group belongs to in this CTA's first tile
@@ -104,8 +125,12 @@ __global__ void __launch_bounds__(kH4Threads, 1)
         } else if (q - sg.hrows < sg.rows_b) {
           const long off = (q - sg.hrows) * 64 + 8 * col;
           q_slot[r] = t;
-          src[r] = p.x + stream0 * p.T + off;
-          src_step[r] = step_x;
+          if constexpr (PCM) {
+            bofs[r] = (int)off;
+          } else {
+            src[r] = p.x + stream0 * p.T + off;
+            src_step[r] = step_x;
+          }
           if (off >= p.T - p.L) {
             if constexpr (POOL) rofs[r] = (int)(off - (p.T - p.L));
             else roll[r] = p.hist_out + stream0 * p.L + (off - (p.T - p.L));
@@ -116,8 +141,10 @@ __global__ void __launch_bounds__(kH4Threads, 1)
     float xr[NO][8];
     int nlive = 0;  // live streams of the tile held in xr
     int par_ld = 0, par_cur = 0, par_prev = 0;  // POOL: frame parity of this thread's drain row in the loaded / converted / drained tile
+    [[maybe_unused]] int row_ld = 0;  // PCM: first row of the tile held in xr (convert runs before the next load, as for nlive)
     auto load_tile = [&](long tile) {
       nlive = (int)min((long)sg.spt, (long)p.B - tile * sg.spt);
+      if constexpr (PCM) row_ld = (int)(tile * sg.spt);
       if constexpr (POOL) {
         // the dependent index loads first (id, then its phase word); the data loads of history groups need both
         int id[NO], ph[NO];
@@ -140,6 +167,8 @@ __global__ void __launch_bounds__(kH4Threads, 1)
             for (int e = 0; e < 8; ++e) xr[r][e] = 0.f;
           } else if (hofs[r] >= 0) {
             ptx::ldg256_na(p.hist_in + ((size_t)(ph[r] & 1) * p.pool.P + row) * p.L + hofs[r], xr[r]);
+          } else if constexpr (PCM) {
+            pcm_load8_raw_row(p.in, row_ld + q_slot[r], bofs[r], (int)p.T, xr[r]);  // raw words: converted when the tile is consumed
           } else {
             ptx::ldg256_na(src[r], xr[r]);
           }
@@ -150,17 +179,27 @@ __global__ void __launch_bounds__(kH4Threads, 1)
 #pragma unroll
         for (int r = 0; r < NO; ++r) {
           if (q_slot[r] < nlive) {
-            ptx::ldg256_na(src[r], xr[r]);
+            if constexpr (PCM) {
+              if (bofs[r] >= 0) pcm_load8_raw_row(p.in, row_ld + q_slot[r], bofs[r], (int)p.T, xr[r]);
+              else ptx::ldg256_na(src[r], xr[r]);
+            } else {
+              ptx::ldg256_na(src[r], xr[r]);
+            }
           } else {
 #pragma unroll
             for (int e = 0; e < 8; ++e) xr[r][e] = 0.f;
           }
-          src[r] += src_step[r];
+          if constexpr (PCM) {
+            if (q_slot[r] != kDead && bofs[r] < 0) src[r] += step_h;  // only history groups have a source pointer (x is unused)
+          } else {
+            src[r] += src_step[r];
+          }
         }
       }
     };
     // fp32 -> fp16 planes; the threads that hold the last L samples of a block also roll the history (here, where the data is
-    // needed anyway: a store next to the load would make every prefetch wait for its own data)
+    // needed anyway: a store next to the load would make every prefetch wait for its own data).  PCM: the block groups' raw words are
+    // widened first (zeros of dead or missing rows widen to zeros), so planes and roll see the floats of the fp32 call.
     auto convert = [&](int pb) {
       unsigned char* p1 = sm.planes + (2 * pb) * g.plane;
       if constexpr (POOL) par_cur = par_ld;
@@ -168,6 +207,8 @@ __global__ void __launch_bounds__(kH4Threads, 1)
       for (int r = 0; r < NO; ++r) {
         const int u = tid + kH4Workers * r;
         if (u < n_octs) {
+          if constexpr (PCM)
+            if (bofs[r] >= 0) pcm_convert8(p.in, row_ld + q_slot[r], xr[r]);
           h4_split_store8(xr[r], p1, g.plane, sw128_offset((uint32_t)u * 16u));
           if (roll[r] != nullptr) {
             if (POOL || q_slot[r] < nlive) {  // POOL: load_tile set roll for live groups of this tile only
@@ -236,13 +277,25 @@ struct H4SynthesisStreamParams {
 struct H4SynthesisStreamPoolParams : H4SynthesisStreamParams {
   StreamPoolIndex pool;
 };
+// PCM: mono int16 output rows [B, M F] (out unused).  Two channels of one clip may sit in any two tiles (in a pool, any two streams), so an
+// interleaved store is not native here.
+struct H4SynthesisStreamPcmParams : H4SynthesisStreamParams {
+  int16_t* pcm_out;
+};
+struct H4SynthesisStreamPoolPcmParams : H4SynthesisStreamPoolParams {
+  int16_t* pcm_out;
+};
+template <bool POOL, H4Io IO>
+using H4SynthesisStreamArgs = std::conditional_t<POOL, std::conditional_t<IO == H4Io::PCM, H4SynthesisStreamPoolPcmParams, H4SynthesisStreamPoolParams>,
+                                                 std::conditional_t<IO == H4Io::PCM, H4SynthesisStreamPcmParams, H4SynthesisStreamParams>>;
 
 // streaming synthesis: tiles blockIdx.x, + gridDim.x, ... of spt streams each
-template <int M, bool POOL>
-__global__ void __launch_bounds__(kH4SynThreads, 1)
-    h4_synthesis_stream_kernel(std::conditional_t<POOL, H4SynthesisStreamPoolParams, H4SynthesisStreamParams> p) {
+template <int M, bool POOL, H4Io IO>
+__global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_stream_kernel(H4SynthesisStreamArgs<POOL, IO> p) {
   static_assert(M >= 8, "frame quads of 8-band groups (n_band 4 packs its chunks differently: offline kernels only)");
+  static_assert(IO == H4Io::F32 || IO == H4Io::PCM, "streaming blocks: fp32 rows or int16 PCM samples");
   h4_kernel<true, kH4SynWorkers>(p.g, p.bank, p.n_tiles, 1u, p.pad_bytes, p.trim_lo, p.trim_hi, [&](const H4Smem& sm, uint32_t tmem, uint32_t pfull_leader, unsigned n_iter) {
+    constexpr bool PCM = IO == H4Io::PCM;
     constexpr int FR = 64 / M, NBG = M / 8;  // frames per 128-byte plane row, 8-band groups
     const H4Shape& g = p.g;
     const H4StreamGeom& sg = p.sg;
@@ -341,11 +394,27 @@ __global__ void __launch_bounds__(kH4SynThreads, 1)
     const bool e_rows = et < sg.spt && eq0 < sg.rows_b;
     float* orun = p.out + ((size_t)blockIdx.x * sg.spt + et) * (size_t)(p.F * M) + 64 * eq0 + 32 * hb + 8 * (lane & 3);  // slot q: row eq0 + q of the block
     const size_t out_step = (size_t)gridDim.x * sg.spt * (size_t)(p.F * M);
+    [[maybe_unused]] int16_t* prun = nullptr;  // PCM: the same place in the int16 rows
+    if constexpr (PCM) prun = p.pcm_out + ((size_t)blockIdx.x * sg.spt + et) * (size_t)(p.F * M) + 64 * eq0 + 32 * hb + 8 * (lane & 3);
     long tile = blockIdx.x, prev_tile = 0;
     auto drain = [&](int dbuf) {
       if (warp >= 8) return;  // every worker waited for the MMAs; the ninth warp has no TMEM rows to drain
       float val[4][8];
       h4_drain_synthesis(tmem, dbuf, tid, val);
+      if constexpr (PCM) {  // quantised: eight samples = one 16-byte store per slot, a lane quad covers 64 contiguous bytes
+        int16_t* pp = prun;
+        prun += out_step;
+        if (!e_rows || prev_tile * sg.spt + et >= p.B) return;
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+          uint32_t w[4];
+#pragma unroll
+          for (int k = 0; k < 4; ++k)
+            w[k] = (uint32_t)(uint16_t)pcm_quantise(val[q][2 * k]) | ((uint32_t)(uint16_t)pcm_quantise(val[q][2 * k + 1]) << 16);
+          __stcs(reinterpret_cast<uint4*>(pp + (size_t)q * 64), make_uint4(w[0], w[1], w[2], w[3]));
+        }
+        return;
+      }
       float* op = orun;
       orun += out_step;
       if (!e_rows || prev_tile * sg.spt + et >= p.B) return;
@@ -362,21 +431,25 @@ __global__ void __launch_bounds__(kH4SynThreads, 1)
 }
 
 // launches (CTA pairs; on any error the caller runs other kernels: the fold kernels, or the direct form for pools)
-// Params: H4AnalysisStreamParams, or H4AnalysisStreamPoolParams for the POOL instantiation
+// Params: one of the H4AnalysisStream*Params above; it selects the instantiation (POOL, PCM)
 template <int M, typename Params>
 inline int h4_launch_analysis_stream(Params p, cudaStream_t st) {
-  constexpr bool POOL = std::is_same_v<Params, H4AnalysisStreamPoolParams>;
+  constexpr bool POOL = std::is_base_of_v<H4AnalysisStreamPoolParams, Params>;
+  constexpr H4Io IO = std::is_same_v<Params, H4AnalysisStreamArgs<POOL, H4Io::PCM>> ? H4Io::PCM : H4Io::F32;
+  static_assert(std::is_same_v<Params, H4AnalysisStreamArgs<POOL, IO>>, "params of a streaming analysis instantiation");
   static H4Configured configured;
   p.n_tiles = (p.B + p.s.spt - 1) / p.s.spt;
-  return h4_launch<true>(h4_analysis_stream_kernel<M, POOL>, p, kH4Threads, configured, st);
+  return h4_launch<true>(h4_analysis_stream_kernel<M, POOL, IO>, p, kH4Threads, configured, st);
 }
-// Params: H4SynthesisStreamParams, or H4SynthesisStreamPoolParams for the POOL instantiation
+// Params: one of the H4SynthesisStream*Params above
 template <int M, typename Params>
 inline int h4_launch_synthesis_stream(Params p, cudaStream_t st) {
-  constexpr bool POOL = std::is_same_v<Params, H4SynthesisStreamPoolParams>;
+  constexpr bool POOL = std::is_base_of_v<H4SynthesisStreamPoolParams, Params>;
+  constexpr H4Io IO = std::is_same_v<Params, H4SynthesisStreamArgs<POOL, H4Io::PCM>> ? H4Io::PCM : H4Io::F32;
+  static_assert(std::is_same_v<Params, H4SynthesisStreamArgs<POOL, IO>>, "params of a streaming synthesis instantiation");
   static H4Configured configured;
   p.n_tiles = (p.B + p.sg.spt - 1) / p.sg.spt;
-  return h4_launch<true>(h4_synthesis_stream_kernel<M, POOL>, p, kH4SynThreads, configured, st);
+  return h4_launch<true>(h4_synthesis_stream_kernel<M, POOL, IO>, p, kH4SynThreads, configured, st);
 }
 
 }  // namespace pqmf

@@ -76,6 +76,38 @@ __device__ __forceinline__ void pcm_convert8(const PcmIn& in, long b, float (&v)
   }
 }
 
+// pcm_load8_raw for the streaming kernels, whose rows and blocks stay below 2^31 (32-bit index arithmetic): the same 16-byte mono and
+// 32-byte stereo loads (raw words for pcm_convert8), and for more channels one pass over each frame's channels, converted on the spot
+// (pcm_sample's arithmetic: the down-mix sums in channel order, then divides by C)
+__device__ __forceinline__ void pcm_load8_raw_row(const PcmIn& in, int b, int s, int T, float (&v)[8]) {
+  int4 r0, r1;
+  if (in.C == 1) {
+    r0 = __ldg(reinterpret_cast<const int4*>(in.pcm + (size_t)b * T + s));
+    r1 = make_int4(0, 0, 0, 0);
+  } else if (in.C == 2) {
+    const int4* src = reinterpret_cast<const int4*>(in.pcm + ((size_t)(in.downmix ? b : (b >> 1)) * T + s) * 2);
+    r0 = __ldg(src);
+    r1 = __ldg(src + 1);
+  } else {
+    constexpr float kInv = 1.0f / 32768.0f;
+    const int clip = in.downmix ? b : b / in.C;
+    const int16_t* f = in.pcm + ((size_t)clip * T + s) * in.C + (in.downmix ? 0 : b - clip * in.C);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      if (in.downmix) {
+        float acc = 0.f;
+        for (int c = 0; c < in.C; ++c) acc += (float)__ldg(f + i * in.C + c) * kInv;
+        v[i] = acc / (float)in.C;
+      } else {
+        v[i] = (float)__ldg(f + i * in.C) * kInv;
+      }
+    }
+    return;
+  }
+  v[0] = __int_as_float(r0.x); v[1] = __int_as_float(r0.y); v[2] = __int_as_float(r0.z); v[3] = __int_as_float(r0.w);
+  v[4] = __int_as_float(r1.x); v[5] = __int_as_float(r1.y); v[6] = __int_as_float(r1.z); v[7] = __int_as_float(r1.w);
+}
+
 // eight consecutive output samples t .. t + 7 (t a multiple of 8) of row b -> interleaved int16 PCM [clips, total, C]
 __device__ __forceinline__ void pcm_store8(int16_t* pcm_out, int C, long b, long t, long total, const float (&v)[8]) {
   if (C == 1) {

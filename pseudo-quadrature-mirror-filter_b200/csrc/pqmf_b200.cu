@@ -311,93 +311,118 @@ int h4_synthesis(const void* s, void* out, const float* tables, int B, long F, i
   }
 }
 
-// ---- streaming blocks of n_band 16 on the Hankel kernels (hankel4_stream.cuh): several streams per MMA tile.  Any refusal
-//      (short blocks, few streams, odd sizes, a context without CTA pairs) returns UNSUPPORTED and the fold kernels run instead ----
-// pool != nullptr: the indexed (POOL) kernels, with state_in = state_out = the pool
-int h4_analysis_stream(const float* x, float* y, const float* tables, const float* state_in, float* state_out, int B, long T, int M, int L,
-                       int parity, unsigned flags, cudaStream_t st, const PoolRows* pool = nullptr) {
+// ---- streaming blocks on the Hankel-4 kernels (hankel4_stream.cuh): several streams per MMA tile.  ONE routing decision per direction
+//      for every streaming entry -- lockstep and pool, fp32 and int16 PCM: the kernels serve a call exactly where h4_stream_family holds
+//      and h4_*_stream_plan accepts its shape, flags and tile count, and its buffers meet the kernels' alignment (h4_*_stream_ok).
+//      Everywhere else (short blocks, few streams, odd sizes) an fp32 call runs other kernels -- the fold kernels for lockstep n_band 16,
+//      the direct form -- and a PCM call is refused with PQMF_ERR_UNSUPPORTED ----
+bool use_fast(int M, int L, const float* tables, unsigned flags);
+bool use_h4_family(int M, int L, const float* tables, unsigned flags);
+bool h4_stream_family(int M, int L, const float* tables, unsigned flags) {
+  if (use_fast(M, L, tables, flags)) return true;  // n_band 16 / L 512
+  return !pqmf::hankel16_supported(M, L) && use_h4_family(M, L, tables, flags) && (M == 8 || M == 32);
+}
+// p: everything but the buffers and the parity
+bool h4_analysis_stream_plan(int B, long T, int M, int L, const float* tables, unsigned flags, pqmf::H4AnalysisStreamParams& p) {
+  if (!h4_stream_family(M, L, tables, flags)) return false;
   int jlo, kt;
   h4_taps(flags, jlo, kt);
-  if (kt == 0 || (flags & (PQMF_FLAG_H4_SPLIT | PQMF_FLAG_NO_PAIR | PQMF_FLAG_FOLD))) return PQMF_ERR_UNSUPPORTED;
+  if (kt == 0 || (flags & (PQMF_FLAG_H4_SPLIT | PQMF_FLAG_NO_PAIR | PQMF_FLAG_FOLD))) return false;
   // the region of a stream starts with its history as WHOLE plane rows: where the taps need a fraction of a row (n_band 8: 224 samples)
   // the region carries the next multiple of 64 (the state holds L samples) and every window starts that much later (pad_bytes)
   const int hist = ((L - jlo + 63) / 64) * 64;
-  if (hist > L || T % 256 != 0 || T < L) return PQMF_ERR_UNSUPPORTED;
+  if (hist > L || T % 256 != 0 || T < L || L % 8 != 0) return false;
   const pqmf::H4StreamGeom sg = pqmf::h4_stream_geom(T, hist);
-  if (sg.pitch > pqmf::kH4Rows || sg.spt < 1 || (B + sg.spt - 1) / sg.spt < 96) return PQMF_ERR_UNSUPPORTED;
-  if (((uintptr_t)x | (uintptr_t)state_in) % 32 || ((uintptr_t)y | (uintptr_t)state_out) % 16 || L % 8 != 0) return PQMF_ERR_UNSUPPORTED;  // 256-bit loads
-  pqmf::H4AnalysisStreamParams p{};
-  p.x = x; p.hist_in = state_in; p.hist_out = state_out; p.y = y; p.T = T; p.B = B; p.L = L; p.parity = parity & 1;
+  if (sg.pitch > pqmf::kH4Rows || sg.spt < 1 || (B + sg.spt - 1) / sg.spt < 96) return false;
+  p.T = T; p.B = B; p.L = L;
   p.trim_lo = p.trim_hi = (flags & PQMF_FLAG_EXACT) ? 0 : (int)PQMF_FLAG_H4_TRIM_A(flags);
   p.pad_bytes = 2 * (hist - (L - jlo));
   p.g = pqmf::h4_shape(M, jlo, kt, true, false, p.pad_bytes);
   p.s = sg;
   p.bank = reinterpret_cast<const uint16_t*>(tables + h4_pair_offset(M, L));
-  int e = -2;
-  if (pool) {
-    const pqmf::H4AnalysisStreamPoolParams q{p, *pool};
-    switch (M) {
-      case 8: e = pqmf::h4_launch_analysis_stream<8>(q, st); break;
-      case 16: e = pqmf::h4_launch_analysis_stream<16>(q, st); break;
-      case 32: e = pqmf::h4_launch_analysis_stream<32>(q, st); break;
-      default: break;
-    }
-  } else {
-    switch (M) {
-      case 8: e = pqmf::h4_launch_analysis_stream<8>(p, st); break;
-      case 16: e = pqmf::h4_launch_analysis_stream<16>(p, st); break;
-      case 32: e = pqmf::h4_launch_analysis_stream<32>(p, st); break;
-      default: break;
-    }
-  }
-  if (e != 0) {
-    (void)cudaGetLastError();
-    return PQMF_ERR_UNSUPPORTED;
-  }
-  return 0;
+  return pqmf::h4_shape_fits(p.g);
 }
-int h4_synthesis_stream(const float* s, float* out, const float* tables, const float* state_in, float* state_out, int B, long F, int M, int L,
-                        int parity, unsigned flags, cudaStream_t st, const PoolRows* pool = nullptr) {
+// 256-bit signal loads (a PCM block: 16-byte mono, 32-byte stereo loads), 128-bit sub-band stores and state accesses
+bool h4_analysis_stream_ok(int B, long T, int M, int L, const float* tables, unsigned flags, const void* signal, const float* y, const float* state_in,
+                           const float* state_out, pqmf::H4AnalysisStreamParams& p) {
+  return h4_analysis_stream_plan(B, T, M, L, tables, flags, p) && ((uintptr_t)signal | (uintptr_t)state_in) % 32 == 0 &&
+         ((uintptr_t)y | (uintptr_t)state_out) % 16 == 0;
+}
+bool h4_synthesis_stream_plan(int B, long F, int M, int L, const float* tables, unsigned flags, pqmf::H4SynthesisStreamParams& p) {
+  if (!h4_stream_family(M, L, tables, flags)) return false;
   int jlo, kt;
   h4_taps(flags, jlo, kt);
-  if (kt == 0 || (flags & (PQMF_FLAG_H4_SPLIT | PQMF_FLAG_NO_PAIR | PQMF_FLAG_FOLD))) return PQMF_ERR_UNSUPPORTED;
+  if (kt == 0 || (flags & (PQMF_FLAG_H4_SPLIT | PQMF_FLAG_NO_PAIR | PQMF_FLAG_FOLD))) return false;
   const int K = L / M, taps_frames = (jlo + kt) / M;  // = ehi + 1: with o = -1 the window of output frame f starts at sub-band frame f - taps_frames
   // history and block are whole plane rows (64 / M frames each) and whole frame quads: the region carries the history rounded up to
   // rows (the state holds K frames) and the windows start that many frames later (pad_bytes)
   const int hist_frames = ((taps_frames * M + 63) / 64) * 64 / M;
-  if (hist_frames % 4 != 0 || hist_frames > K || (F * M) % 256 != 0 || F % 4 != 0 || F < K) return PQMF_ERR_UNSUPPORTED;
+  if (hist_frames % 4 != 0 || hist_frames > K || (F * M) % 256 != 0 || F % 4 != 0 || F < K) return false;
   const pqmf::H4StreamGeom sg = pqmf::h4_stream_geom(F * M, hist_frames * M);
-  if (sg.pitch > pqmf::kH4Rows || sg.spt < 1 || (B + sg.spt - 1) / sg.spt < 96) return PQMF_ERR_UNSUPPORTED;
-  if (((uintptr_t)s | (uintptr_t)state_in | (uintptr_t)state_out) % 16 || ((uintptr_t)out % 32)) return PQMF_ERR_UNSUPPORTED;
-  pqmf::H4SynthesisStreamParams p{};
-  p.s = s; p.state_in = state_in; p.state_out = state_out; p.out = out; p.F = F; p.B = B; p.K = K; p.parity = parity & 1;
+  if (sg.pitch > pqmf::kH4Rows || sg.spt < 1 || (B + sg.spt - 1) / sg.spt < 96) return false;
+  p.F = F; p.B = B; p.K = K;
   p.trim_lo = p.trim_hi = (flags & PQMF_FLAG_EXACT) ? 0 : (int)PQMF_FLAG_H4_TRIM_S(flags);
   p.pad_bytes = 2 * M * (hist_frames - taps_frames);
   p.g = pqmf::h4_shape(M, jlo, kt, true, true, p.pad_bytes);
   p.sg = sg;
   p.bank = reinterpret_cast<const uint16_t*>(tables + h4_pair_offset(M, L) + h4_pair_floats(M, L));
-  int e = -2;
-  if (pool) {
-    const pqmf::H4SynthesisStreamPoolParams q{p, *pool};
-    switch (M) {
-      case 8: e = pqmf::h4_launch_synthesis_stream<8>(q, st); break;
-      case 16: e = pqmf::h4_launch_synthesis_stream<16>(q, st); break;
-      case 32: e = pqmf::h4_launch_synthesis_stream<32>(q, st); break;
-      default: break;
-    }
-  } else {
-    switch (M) {
-      case 8: e = pqmf::h4_launch_synthesis_stream<8>(p, st); break;
-      case 16: e = pqmf::h4_launch_synthesis_stream<16>(p, st); break;
-      case 32: e = pqmf::h4_launch_synthesis_stream<32>(p, st); break;
-      default: break;
-    }
+  return pqmf::h4_shape_fits(p.g);
+}
+// 128-bit sub-band loads and state accesses; 256-bit fp32 output stores (PCM output: 128-bit int16 stores)
+bool h4_synthesis_stream_ok(int B, long F, int M, int L, const float* tables, unsigned flags, const float* s, const void* out, bool pcm_out,
+                            const float* state_in, const float* state_out, pqmf::H4SynthesisStreamParams& p) {
+  return h4_synthesis_stream_plan(B, F, M, L, tables, flags, p) && ((uintptr_t)s | (uintptr_t)state_in | (uintptr_t)state_out) % 16 == 0 &&
+         (uintptr_t)out % (pcm_out ? 16 : 32) == 0;
+}
+template <typename Params>
+int h4_analysis_stream_launch(const Params& p, int M, cudaStream_t st) {
+  switch (M) {
+    case 8: return pqmf::h4_launch_analysis_stream<8>(p, st);
+    case 16: return pqmf::h4_launch_analysis_stream<16>(p, st);
+    case 32: return pqmf::h4_launch_analysis_stream<32>(p, st);
+    default: return PQMF_ERR_UNSUPPORTED;
   }
-  if (e != 0) {
-    (void)cudaGetLastError();
+}
+template <typename Params>
+int h4_synthesis_stream_launch(const Params& p, int M, cudaStream_t st) {
+  switch (M) {
+    case 8: return pqmf::h4_launch_synthesis_stream<8>(p, st);
+    case 16: return pqmf::h4_launch_synthesis_stream<16>(p, st);
+    case 32: return pqmf::h4_launch_synthesis_stream<32>(p, st);
+    default: return PQMF_ERR_UNSUPPORTED;
+  }
+}
+// pool != nullptr: the indexed (POOL) kernels, with state_in = state_out = the pool.  pcm != nullptr: the block is int16 WAV frames (x
+// unused).  Returns 0, PQMF_ERR_UNSUPPORTED (refused: nothing launched) or the error of a launch that did not start (cleared).
+int h4_analysis_stream(const float* x, float* y, const float* tables, const float* state_in, float* state_out, int B, long T, int M, int L,
+                       int parity, unsigned flags, cudaStream_t st, const PoolRows* pool = nullptr, const pqmf::PcmIn* pcm = nullptr) {
+  pqmf::H4AnalysisStreamParams p{};
+  if (!h4_analysis_stream_ok(B, T, M, L, tables, flags, pcm ? static_cast<const void*>(pcm->pcm) : x, y, state_in, state_out, p))
     return PQMF_ERR_UNSUPPORTED;
-  }
-  return 0;
+  p.x = x; p.hist_in = state_in; p.hist_out = state_out; p.y = y; p.parity = parity & 1;
+  int e;
+  if (pcm && pool) e = h4_analysis_stream_launch(pqmf::H4AnalysisStreamPoolPcmParams{{p, *pool}, *pcm}, M, st);
+  else if (pcm) e = h4_analysis_stream_launch(pqmf::H4AnalysisStreamPcmParams{p, *pcm}, M, st);
+  else if (pool) e = h4_analysis_stream_launch(pqmf::H4AnalysisStreamPoolParams{p, *pool}, M, st);
+  else e = h4_analysis_stream_launch(p, M, st);
+  if (e != 0) (void)cudaGetLastError();
+  return e;
+}
+// pcm_out != nullptr: mono int16 output rows (out unused)
+int h4_synthesis_stream(const float* s, float* out, const float* tables, const float* state_in, float* state_out, int B, long F, int M, int L,
+                        int parity, unsigned flags, cudaStream_t st, const PoolRows* pool = nullptr, int16_t* pcm_out = nullptr) {
+  pqmf::H4SynthesisStreamParams p{};
+  if (!h4_synthesis_stream_ok(B, F, M, L, tables, flags, s, pcm_out ? static_cast<const void*>(pcm_out) : out, pcm_out != nullptr, state_in,
+                              state_out, p))
+    return PQMF_ERR_UNSUPPORTED;
+  p.s = s; p.state_in = state_in; p.state_out = state_out; p.out = out; p.parity = parity & 1;
+  int e;
+  if (pcm_out && pool) e = h4_synthesis_stream_launch(pqmf::H4SynthesisStreamPoolPcmParams{{p, *pool}, pcm_out}, M, st);
+  else if (pcm_out) e = h4_synthesis_stream_launch(pqmf::H4SynthesisStreamPcmParams{p, pcm_out}, M, st);
+  else if (pool) e = h4_synthesis_stream_launch(pqmf::H4SynthesisStreamPoolParams{p, *pool}, M, st);
+  else e = h4_synthesis_stream_launch(p, M, st);
+  if (e != 0) (void)cudaGetLastError();
+  return e;
 }
 
 // n_band 16 fast path: fold + tensor-core modulation (fast16*.cuh), or -- with PQMF_FLAG_EXACT -- the direct form as an
@@ -651,16 +676,12 @@ int roundtrip_host(const Sample* x_host, float* y_host, Sample* out_host, const 
   return rc;
 }
 
-// ---- stream pools.  One routing decision per direction: the indexed Hankel-4 kernels exactly where a lockstep call with B = n runs the
-//      Hankel-4 streaming kernels (the same family test as pqmf_*_stream_f32, and h4_*_stream's own shape, flag, alignment and tile-count
-//      checks); the indexed direct form everywhere else -- including few-stream n_band 16, where a lockstep call runs the fold kernels ----
-bool h4_stream_family(int M, int L, const float* tables, unsigned flags) {
-  if (use_fast(M, L, tables, flags)) return true;  // n_band 16 / L 512
-  return !pqmf::hankel16_supported(M, L) && use_h4_family(M, L, tables, flags) && (M == 8 || M == 32);
-}
+// ---- stream pools.  The indexed Hankel-4 kernels exactly where a lockstep call with B = n runs the Hankel-4 streaming kernels (the
+//      routing decision of h4_*_stream); the indexed direct form everywhere else -- including few-stream n_band 16, where a lockstep
+//      call runs the fold kernels ----
 int pool_analysis(const float* x, float* y, const float* hk, const float* tables, float* xpool, const PoolRows& pool, int n, long T, int M, int L,
                   unsigned flags, cudaStream_t st) {
-  if (h4_stream_family(M, L, tables, flags) && h4_analysis_stream(x, y, tables, xpool, xpool, n, T, M, L, 0, flags, st, &pool) == 0) {
+  if (h4_analysis_stream(x, y, tables, xpool, xpool, n, T, M, L, 0, flags, st, &pool) == 0) {
     ++g_launches;
     return 0;
   }
@@ -668,7 +689,7 @@ int pool_analysis(const float* x, float* y, const float* hk, const float* tables
 }
 int pool_synthesis(const float* s, float* out, const float* hk, const float* tables, float* spool, const PoolRows& pool, int n, long F, int M, int L,
                    unsigned flags, cudaStream_t st) {
-  if (h4_stream_family(M, L, tables, flags) && h4_synthesis_stream(s, out, tables, spool, spool, n, F, M, L, 0, flags, st, &pool) == 0) {
+  if (h4_synthesis_stream(s, out, tables, spool, spool, n, F, M, L, 0, flags, st, &pool) == 0) {
     ++g_launches;
     return 0;
   }
@@ -946,16 +967,11 @@ int pqmf_analysis_stream_f32(const float* x, float* y, const float* hk, const fl
   if (!x || !y) return PQMF_ERR_ARG;
   cudaStream_t st = (cudaStream_t)stream;
   const long F = T / M;
+  // many streams: the streaming Hankel-4 kernels (n_band 8 / 16 / 32); few n_band-16 streams: the fold kernels
+  if (h4_analysis_stream(x, y, tables, state_in, state_out, B, T, M, L, frame_parity, flags, st) == 0) { ++g_launches; return 0; }
   if (use_fast(M, L, tables, flags) && pqmf::hankel16_analysis_ok(x, y, T, F)) {
-    if (h4_analysis_stream(x, y, tables, state_in, state_out, B, T, 16, L, frame_parity, flags, st) == 0) { ++g_launches; return 0; }
     int e = fast_analysis(x, state_in, y, state_out, tables, B, T, F, L, frame_parity & 1, flags, st);
     if (e != PQMF_ERR_UNSUPPORTED) { g_launches += (e == 0); return e; }
-  }
-  // n_band 8 / 32 with many streams: the streaming Hankel kernels (same tiles-of-streams scheme as n_band 16)
-  if (!pqmf::hankel16_supported(M, L) && use_h4_family(M, L, tables, flags) && (M == 8 || M == 32) &&
-      h4_analysis_stream(x, y, tables, state_in, state_out, B, T, M, L, frame_parity, flags, st) == 0) {
-    ++g_launches;
-    return 0;
   }
   // fp32 direct form; the CTA of each row's last frame tile also rolls that row's history (no separate launch)
   return analysis_direct(x, state_in, y, hk, B, T, F, M, L, L, frame_parity, 0, st, pqmf::PcmIn{nullptr, 1, 0}, state_out);
@@ -971,15 +987,10 @@ int pqmf_synthesis_stream_f32(const float* s, float* out, const float* hk, const
   cudaStream_t st = (cudaStream_t)stream;
   const int K = L / M;
   // history frames sit K frames before frame 0 of the block: their parity offset is (frame_parity - K)
+  if (h4_synthesis_stream(s, out, tables, state_in, state_out, B, n_frames, M, L, frame_parity, flags, st) == 0) { ++g_launches; return 0; }
   if (use_fast(M, L, tables, flags) && pqmf::hankel16_synthesis_ok(s, out, n_frames)) {
-    if (h4_synthesis_stream(s, out, tables, state_in, state_out, B, n_frames, 16, L, frame_parity, flags, st) == 0) { ++g_launches; return 0; }
     int e = fast_synthesis(s, state_in, out, state_out, tables, B, n_frames, -M, frame_parity & 1, flags, st);
     if (e != PQMF_ERR_UNSUPPORTED) { g_launches += (e == 0); return e; }
-  }
-  if (!pqmf::hankel16_supported(M, L) && use_h4_family(M, L, tables, flags) && (M == 8 || M == 32) &&
-      h4_synthesis_stream(s, out, tables, state_in, state_out, B, n_frames, M, L, frame_parity, flags, st) == 0) {
-    ++g_launches;
-    return 0;
   }
   return synthesis_direct(s, state_in, out, hk, B, n_frames, M, L, -M, frame_parity, 0, st, nullptr, 1, nullptr, state_out);
 }
@@ -1031,6 +1042,115 @@ int pqmf_stream_pool_step_f32(const float* x, float* y, float* out, const float*
   if (int e = pool_analysis(x, y, hk, tables, xpool, xrows, n, T, M, L, flags, st)) return e;
   if (int e = pool_synthesis(y, out, hk, tables, spool, srows, n, T / M, M, L, flags, st)) return e;
   return pool_phase(xrows, n, xphase, T / M, sphase, T / M, st);
+}
+
+// ---- int16 PCM blocks in the streaming calls: the streaming Hankel-4 kernels with PCM loads (any channel count, optional down-mix) and
+//      mono PCM stores, exactly where the fp32 call with the same rows runs those kernels (h4_*_stream_ok, with the PCM buffer's alignment);
+//      every other call returns PQMF_ERR_UNSUPPORTED before anything is launched and the caller stages it through the fp32 entry ----
+static bool pcm_args_bad(int C, long rows) { return C < 1 || C > 64 || rows >= (1L << 31); }
+
+int pqmf_analysis_stream_pcm16(const int16_t* pcm, float* y, const float* hk, const float* tables, const float* state_in, float* state_out, int B,
+                               long T, int C, int downmix, int M, int L, int frame_parity, unsigned flags, pqmf_stream_t stream) {
+  const long rows = downmix ? (long)B : (long)B * C;
+  if (bad_dims(B, T, M, L) || (T % M) != 0 || pcm_args_bad(C, rows)) return PQMF_ERR_ARG;
+  if (B == 0) return PQMF_OK;
+  if (!hk || !state_in || !state_out || state_in == state_out || T == 0 || !pcm || !y) return PQMF_ERR_ARG;
+  const pqmf::PcmIn in{pcm, C, downmix ? 1 : 0};
+  if (h4_analysis_stream(nullptr, y, tables, state_in, state_out, (int)rows, T, M, L, frame_parity, flags, (cudaStream_t)stream, nullptr, &in) != 0)
+    return PQMF_ERR_UNSUPPORTED;  // nothing was launched
+  ++g_launches;
+  return PQMF_OK;
+}
+
+int pqmf_synthesis_stream_pcm16(const float* s, int16_t* pcm, const float* hk, const float* tables, const float* state_in, float* state_out, int B,
+                                int C, long n_frames, int M, int L, int frame_parity, unsigned flags, pqmf_stream_t stream) {
+  const long rows = (long)B * C;
+  if (bad_dims(B, n_frames, M, L) || (L % M) != 0 || pcm_args_bad(C, rows)) return PQMF_ERR_ARG;
+  if (B == 0) return PQMF_OK;
+  if (!hk || !state_in || !state_out || state_in == state_out || n_frames == 0 || !s || !pcm) return PQMF_ERR_ARG;
+  if (C != 1 ||
+      h4_synthesis_stream(s, nullptr, tables, state_in, state_out, (int)rows, n_frames, M, L, frame_parity, flags, (cudaStream_t)stream, nullptr, pcm) != 0)
+    return PQMF_ERR_UNSUPPORTED;
+  ++g_launches;
+  return PQMF_OK;
+}
+
+int pqmf_stream_step_pcm16(const int16_t* pcm, float* y, int16_t* pcm_out, const float* hk, const float* tables, const float* xstate_in,
+                           float* xstate_out, const float* sstate_in, float* sstate_out, int B, long T, int C, int downmix, int M, int L, int parity_in,
+                           int parity_out, unsigned flags, pqmf_stream_t stream) {
+  const long rows = downmix ? (long)B : (long)B * C;
+  if (bad_dims(B, T, M, L) || (T % M) != 0 || T == 0 || (L % M) != 0 || pcm_args_bad(C, rows)) return PQMF_ERR_ARG;
+  if (B == 0) return PQMF_OK;
+  if (!pcm || !y || !pcm_out || !hk || !xstate_in || !xstate_out || !sstate_in || !sstate_out || xstate_in == xstate_out ||
+      sstate_in == sstate_out)
+    return PQMF_ERR_ARG;
+  // both directions native, or nothing is launched
+  pqmf::H4AnalysisStreamParams pa{};
+  pqmf::H4SynthesisStreamParams ps{};
+  if ((downmix == 0 && C != 1) || !h4_analysis_stream_ok((int)rows, T, M, L, tables, flags, pcm, y, xstate_in, xstate_out, pa) ||
+      !h4_synthesis_stream_ok((int)rows, T / M, M, L, tables, flags, y, pcm_out, true, sstate_in, sstate_out, ps))
+    return PQMF_ERR_UNSUPPORTED;
+  cudaStream_t st = (cudaStream_t)stream;
+  const pqmf::PcmIn in{pcm, C, downmix ? 1 : 0};
+  if (h4_analysis_stream(nullptr, y, tables, xstate_in, xstate_out, (int)rows, T, M, L, parity_in, flags, st, nullptr, &in) != 0)
+    return PQMF_ERR_UNSUPPORTED;  // the launch did not start: nothing ran
+  ++g_launches;
+  // the analysis has run: a failed synthesis launch is an error, not a refusal (a staged retry would step the analysis state twice)
+  const int e = h4_synthesis_stream(y, nullptr, tables, sstate_in, sstate_out, (int)rows, T / M, M, L, parity_out, flags, st, nullptr, pcm_out);
+  if (e != 0) return e > 0 ? e : (int)cudaErrorLaunchFailure;
+  ++g_launches;
+  return PQMF_OK;
+}
+
+int pqmf_stream_pool_analysis_pcm16(const int16_t* pcm, float* y, const float* hk, const float* tables, float* xpool, int* xphase, int P,
+                                    const int* ids, int B, long T, int C, int downmix, int M, int L, unsigned flags, pqmf_stream_t stream) {
+  const long rows = downmix ? (long)B : (long)B * C;
+  if (bad_dims(B, T, M, L) || pcm_args_bad(C, rows) || bad_pool(P, (int)rows) || T <= 0 || (T % M) != 0) return PQMF_ERR_ARG;
+  if (B == 0) return PQMF_OK;
+  if (!pcm || !y || !hk || !xpool || !xphase || !ids) return PQMF_ERR_ARG;
+  cudaStream_t st = (cudaStream_t)stream;
+  const PoolRows pool{ids, xphase, P};
+  const pqmf::PcmIn in{pcm, C, downmix ? 1 : 0};
+  if (h4_analysis_stream(nullptr, y, tables, xpool, xpool, (int)rows, T, M, L, 0, flags, st, &pool, &in) != 0) return PQMF_ERR_UNSUPPORTED;
+  ++g_launches;
+  return pool_phase(pool, (int)rows, xphase, T / M, nullptr, 0, st);
+}
+
+int pqmf_stream_pool_synthesis_pcm16(const float* s, int16_t* pcm, const float* hk, const float* tables, float* spool, int* sphase, int P,
+                                     const int* ids, int B, int C, long n_frames, int M, int L, unsigned flags, pqmf_stream_t stream) {
+  const long rows = (long)B * C;
+  if (bad_dims(B, n_frames, M, L) || pcm_args_bad(C, rows) || bad_pool(P, (int)rows) || n_frames <= 0 || (L % M) != 0) return PQMF_ERR_ARG;
+  if (B == 0) return PQMF_OK;
+  if (!s || !pcm || !hk || !spool || !sphase || !ids) return PQMF_ERR_ARG;
+  cudaStream_t st = (cudaStream_t)stream;
+  const PoolRows pool{ids, sphase, P};
+  if (C != 1 || h4_synthesis_stream(s, nullptr, tables, spool, spool, (int)rows, n_frames, M, L, 0, flags, st, &pool, pcm) != 0)
+    return PQMF_ERR_UNSUPPORTED;
+  ++g_launches;
+  return pool_phase(pool, (int)rows, nullptr, 0, sphase, n_frames, st);
+}
+
+int pqmf_stream_pool_step_pcm16(const int16_t* pcm, float* y, int16_t* pcm_out, const float* hk, const float* tables, float* xpool, int* xphase,
+                                float* spool, int* sphase, int P, const int* ids, int B, long T, int C, int downmix, int M, int L, unsigned flags,
+                                pqmf_stream_t stream) {
+  const long rows = downmix ? (long)B : (long)B * C;
+  if (bad_dims(B, T, M, L) || pcm_args_bad(C, rows) || bad_pool(P, (int)rows) || T <= 0 || (T % M) != 0 || (L % M) != 0) return PQMF_ERR_ARG;
+  if (B == 0) return PQMF_OK;
+  if (!pcm || !y || !pcm_out || !hk || !xpool || !xphase || !spool || !sphase || !ids || xphase == sphase) return PQMF_ERR_ARG;
+  pqmf::H4AnalysisStreamParams pa{};
+  pqmf::H4SynthesisStreamParams ps{};
+  if ((downmix == 0 && C != 1) || !h4_analysis_stream_ok((int)rows, T, M, L, tables, flags, pcm, y, xpool, xpool, pa) ||
+      !h4_synthesis_stream_ok((int)rows, T / M, M, L, tables, flags, y, pcm_out, true, spool, spool, ps))
+    return PQMF_ERR_UNSUPPORTED;
+  cudaStream_t st = (cudaStream_t)stream;
+  const PoolRows xrows{ids, xphase, P}, srows{ids, sphase, P};
+  const pqmf::PcmIn in{pcm, C, downmix ? 1 : 0};
+  if (h4_analysis_stream(nullptr, y, tables, xpool, xpool, (int)rows, T, M, L, 0, flags, st, &xrows, &in) != 0) return PQMF_ERR_UNSUPPORTED;
+  ++g_launches;
+  const int e = h4_synthesis_stream(y, nullptr, tables, spool, spool, (int)rows, T / M, M, L, 0, flags, st, &srows, pcm_out);
+  if (e != 0) return e > 0 ? e : (int)cudaErrorLaunchFailure;  // see pqmf_stream_step_pcm16
+  ++g_launches;
+  return pool_phase(xrows, (int)rows, xphase, T / M, sphase, T / M, st);
 }
 
 int pqmf_roundtrip_f32(const float* x, float* y, float* out, const float* hk, const float* tables, int B, long T, long n_frames,

@@ -394,6 +394,191 @@ std::tuple<at::Tensor, at::Tensor> stream_pool_step(const at::Tensor& x, const a
   return {out, y};
 }
 
+// ---- int16 PCM blocks in the streaming ops (pqmf_*_stream_pcm16 / pqmf_stream_pool_*_pcm16): pcm [S, T, C] interleaved WAV frames, rows
+//      S * C' (C' = 1 with downmix, else C; row s * C' + c = channel c of block s).  Where the library has no native kernel (PQMF_ERR_UNSUPPORTED,
+//      nothing launched, no state touched) the op stages the call: widen, the fp32 op, quantise -- bit-identical to the native path by
+//      construction ----
+void check_pcm(const at::Tensor& pcm, const char* what) {
+  TORCH_CHECK(pcm.is_cuda(), "pcm must be a CUDA tensor (pqmf_b200 has no CPU fallback)");
+  TORCH_CHECK(pcm.scalar_type() == at::kShort, "pcm must be int16, got ", pcm.scalar_type());
+  TORCH_CHECK(pcm.dim() == 3, "pqmf ", what, " expects interleaved int16 WAV frames [blocks, time, channels], got ", pcm.dim(), " dims");
+  TORCH_CHECK(pcm.size(2) >= 1 && pcm.size(2) <= 64, "pqmf ", what, ": 1 to 64 channels, got ", pcm.size(2));
+}
+// [S, T, C] int16 -> [S, C', T] float32 with the kernels' arithmetic (pcm_sample): v / 32768, the down-mix summed in channel order, then / C
+// (a tensor divisor: torch divides by a host scalar through its reciprocal, which is not the same rounding for C = 3, 5, ...)
+at::Tensor pcm_widen(const at::Tensor& pcm, bool downmix) {
+  const at::Tensor f = pcm.to(at::kFloat).mul_(1.0 / 32768.0);
+  if (!downmix) return f.permute({0, 2, 1}).contiguous();
+  at::Tensor acc = f.select(2, 0).clone();
+  for (int64_t c = 1; c < f.size(2); ++c) acc.add_(f.select(2, c));
+  return acc.div_(at::full({}, (double)f.size(2), acc.options())).unsqueeze(1);
+}
+// [S, C, T] float32 -> [S, T, C] int16: clamp(rint(v * 32768), -32768, 32767) (pcm_quantise)
+at::Tensor pcm_quantise(const at::Tensor& v) {
+  return at::clamp(at::round(v * 32768.0), -32768.0, 32767.0).to(at::kShort).permute({0, 2, 1}).contiguous();
+}
+pqmf_stream_t cur_stream() { return (pqmf_stream_t)at::cuda::getCurrentCUDAStream().stream(); }
+
+// pcm [S, T, C] -> y [S, C' M, T / M]; state as analysis_stream (S C' streams)
+at::Tensor analysis_stream_pcm16(const at::Tensor& pcm, const at::Tensor& hk, const at::Tensor& tables, const at::Tensor& state_in, at::Tensor state_out,
+                                 int64_t frame_parity, bool downmix, int64_t flags) {
+  check_pcm(pcm, "analysis_stream_pcm16");
+  check_f32_cuda(state_in, "state_in");
+  check_f32_cuda(state_out, "state_out");
+  const Bank bank = bank_of(hk, pcm);
+  c10::cuda::CUDAGuard guard(pcm.device());
+  const at::Tensor pc = pcm.contiguous();
+  const int64_t S = pc.size(0), T = pc.size(1), C = pc.size(2), Cr = downmix ? 1 : C, rows = S * Cr;
+  TORCH_CHECK(rows < (1LL << 31), "bad sizes");
+  TORCH_CHECK(T > 0 && T % bank.M == 0, "streaming block length ", T, " must be a positive multiple of n_band=", bank.M);
+  TORCH_CHECK(state_in.is_contiguous() && state_out.is_contiguous() && state_in.numel() == rows * bank.L && state_out.numel() == rows * bank.L,
+              "analysis state must be two contiguous [streams, L] buffers (L=", bank.L, ", streams=", rows, ")");
+  TORCH_CHECK(state_in.data_ptr() != state_out.data_ptr(), "state_in and state_out must not alias");
+  at::Tensor y = at::empty({S, Cr * bank.M, T / bank.M}, pc.options().dtype(at::kFloat));
+  if (rows == 0) return y;
+  const int rc = pqmf_analysis_stream_pcm16(pc.data_ptr<int16_t>(), y.data_ptr<float>(), bank.ptr, tables_ptr(tables, pcm), state_in.data_ptr<float>(),
+                                            state_out.data_ptr<float>(), (int)S, (long)T, (int)C, downmix ? 1 : 0, (int)bank.M, (int)bank.L,
+                                            (int)(frame_parity & 1), (unsigned)flags, cur_stream());
+  if (rc == PQMF_ERR_UNSUPPORTED) return analysis_stream(pcm_widen(pc, downmix), hk, tables, state_in, state_out, frame_parity, flags);
+  check_rc(rc, "pqmf_analysis_stream_pcm16");
+  return y;
+}
+
+// s [S, C M, F] float32 -> pcm [S, M F, C] int16; state as synthesis_stream
+at::Tensor synthesis_stream_pcm16(const at::Tensor& s, const at::Tensor& hk, const at::Tensor& tables, const at::Tensor& state_in, at::Tensor state_out,
+                                  int64_t frame_parity, int64_t flags) {
+  check_f32_cuda(s, "s");
+  check_f32_cuda(state_in, "state_in");
+  check_f32_cuda(state_out, "state_out");
+  TORCH_CHECK(s.dim() == 3, "pqmf synthesis_stream_pcm16 expects [blocks, channels * n_band, frames], got ", s.dim(), " dims");
+  const Bank bank = bank_of(hk, s);
+  TORCH_CHECK(s.size(1) % bank.M == 0 && s.size(1) > 0, "sub-band tensor has ", s.size(1), " channels, expected a positive multiple of n_band=", bank.M);
+  c10::cuda::CUDAGuard guard(s.device());
+  const at::Tensor sc = s.contiguous();
+  const int64_t S = sc.size(0), C = sc.size(1) / bank.M, F = sc.size(2), rows = S * C;
+  TORCH_CHECK(C <= 64 && rows < (1LL << 31), "bad sizes");
+  TORCH_CHECK(state_in.is_contiguous() && state_out.is_contiguous() && state_in.numel() == rows * bank.L && state_out.numel() == rows * bank.L,
+              "synthesis state must be two contiguous [streams, n_band, L/n_band] buffers");
+  TORCH_CHECK(state_in.data_ptr() != state_out.data_ptr(), "state_in and state_out must not alias");
+  TORCH_CHECK(F > 0, "empty block");
+  at::Tensor pcm = at::empty({S, bank.M * F, C}, sc.options().dtype(at::kShort));
+  if (rows == 0) return pcm;
+  const int rc = pqmf_synthesis_stream_pcm16(sc.data_ptr<float>(), pcm.data_ptr<int16_t>(), bank.ptr, tables_ptr(tables, s), state_in.data_ptr<float>(),
+                                             state_out.data_ptr<float>(), (int)S, (int)C, (long)F, (int)bank.M, (int)bank.L, (int)(frame_parity & 1),
+                                             (unsigned)flags, cur_stream());
+  if (rc == PQMF_ERR_UNSUPPORTED) return pcm_quantise(synthesis_stream(sc, hk, tables, state_in, state_out, frame_parity, flags));
+  check_rc(rc, "pqmf_synthesis_stream_pcm16");
+  return pcm;
+}
+
+// one block step from PCM to PCM: (pcm_out [S, T, C'], y [S, C' M, T / M])
+std::tuple<at::Tensor, at::Tensor> stream_step_pcm16(const at::Tensor& pcm, const at::Tensor& hk, const at::Tensor& tables, const at::Tensor& xs_in,
+                                                     at::Tensor xs_out, const at::Tensor& ss_in, at::Tensor ss_out, int64_t parity_in, int64_t parity_out,
+                                                     bool downmix, int64_t flags) {
+  check_pcm(pcm, "stream_step_pcm16");
+  const at::Tensor* states[4] = {&xs_in, &xs_out, &ss_in, &ss_out};
+  for (const at::Tensor* t : states) check_f32_cuda(*t, "state");
+  const Bank bank = bank_of(hk, pcm);
+  c10::cuda::CUDAGuard guard(pcm.device());
+  const at::Tensor pc = pcm.contiguous();
+  const int64_t S = pc.size(0), T = pc.size(1), C = pc.size(2), Cr = downmix ? 1 : C, rows = S * Cr;
+  TORCH_CHECK(rows < (1LL << 31), "bad sizes");
+  TORCH_CHECK(T > 0 && T % bank.M == 0 && bank.L % bank.M == 0, "streaming block length ", T, " must be a positive multiple of n_band=", bank.M);
+  for (const at::Tensor* t : states)
+    TORCH_CHECK(t->is_contiguous() && t->numel() == rows * bank.L, "streaming state buffers must be contiguous with ", rows * bank.L, " elements");
+  TORCH_CHECK(xs_in.data_ptr() != xs_out.data_ptr() && ss_in.data_ptr() != ss_out.data_ptr(), "state_in and state_out must not alias");
+  at::Tensor y = at::empty({S, Cr * bank.M, T / bank.M}, pc.options().dtype(at::kFloat));
+  at::Tensor out = at::empty({S, T, Cr}, pc.options());
+  if (rows == 0) return {out, y};
+  const int rc = pqmf_stream_step_pcm16(pc.data_ptr<int16_t>(), y.data_ptr<float>(), out.data_ptr<int16_t>(), bank.ptr, tables_ptr(tables, pcm),
+                                        xs_in.data_ptr<float>(), xs_out.data_ptr<float>(), ss_in.data_ptr<float>(), ss_out.data_ptr<float>(), (int)S, (long)T,
+                                        (int)C, downmix ? 1 : 0, (int)bank.M, (int)bank.L, (int)(parity_in & 1), (int)(parity_out & 1), (unsigned)flags,
+                                        cur_stream());
+  if (rc == PQMF_ERR_UNSUPPORTED) {  // direction by direction, each native where it can be
+    at::Tensor ys = analysis_stream_pcm16(pc, hk, tables, xs_in, xs_out, parity_in, downmix, flags);
+    return {synthesis_stream_pcm16(ys, hk, tables, ss_in, ss_out, parity_out, flags), ys};
+  }
+  check_rc(rc, "pqmf_stream_step_pcm16");
+  return {out, y};
+}
+
+// pool: pcm [S, T, C] -> y [S, C' M, T / M]; ids [S C'] (row r is the next block of stream ids[r])
+at::Tensor stream_pool_analysis_pcm16(const at::Tensor& pcm, const at::Tensor& hk, const at::Tensor& tables, at::Tensor xpool, at::Tensor xphase,
+                                      const at::Tensor& ids, bool downmix, int64_t flags) {
+  check_pcm(pcm, "stream pool analysis_pcm16");
+  const Bank bank = bank_of(hk, pcm);
+  c10::cuda::CUDAGuard guard(pcm.device());
+  const at::Tensor pc = pcm.contiguous();
+  const int64_t S = pc.size(0), T = pc.size(1), C = pc.size(2), Cr = downmix ? 1 : C, rows = S * Cr;
+  TORCH_CHECK(T > 0 && T % bank.M == 0, "streaming block length ", T, " must be a positive multiple of n_band=", bank.M);
+  const Pool pool = pool_of(xpool, xphase, bank, pcm, "xpool");
+  const int* id = ids_of(ids, rows, pcm);
+  TORCH_CHECK(rows <= pool.P, "more rows (", rows, ") than streams in the pool (", pool.P, ")");
+  at::Tensor y = at::empty({S, Cr * bank.M, T / bank.M}, pc.options().dtype(at::kFloat));
+  if (rows == 0) return y;
+  const int rc = pqmf_stream_pool_analysis_pcm16(pc.data_ptr<int16_t>(), y.data_ptr<float>(), bank.ptr, tables_ptr(tables, pcm), pool.state, pool.phase,
+                                                 (int)pool.P, id, (int)S, (long)T, (int)C, downmix ? 1 : 0, (int)bank.M, (int)bank.L, (unsigned)flags,
+                                                 cur_stream());
+  if (rc == PQMF_ERR_UNSUPPORTED)
+    return stream_pool_analysis(pcm_widen(pc, downmix).view({rows, 1, T}), hk, tables, xpool, xphase, ids, flags).view({S, Cr * bank.M, T / bank.M});
+  check_rc(rc, "pqmf_stream_pool_analysis_pcm16");
+  return y;
+}
+
+// pool: s [S, C M, F] float32 -> pcm [S, M F, C] int16; ids [S C]
+at::Tensor stream_pool_synthesis_pcm16(const at::Tensor& s, const at::Tensor& hk, const at::Tensor& tables, at::Tensor spool, at::Tensor sphase,
+                                       const at::Tensor& ids, int64_t flags) {
+  check_f32_cuda(s, "s");
+  TORCH_CHECK(s.dim() == 3, "pqmf stream pool synthesis_pcm16 expects [blocks, channels * n_band, frames], got ", s.dim(), " dims");
+  const Bank bank = bank_of(hk, s);
+  TORCH_CHECK(s.size(1) % bank.M == 0 && s.size(1) > 0, "sub-band tensor has ", s.size(1), " channels, expected a positive multiple of n_band=", bank.M);
+  TORCH_CHECK(bank.L % bank.M == 0, "streaming synthesis needs L a multiple of n_band");
+  c10::cuda::CUDAGuard guard(s.device());
+  const at::Tensor sc = s.contiguous();
+  const int64_t S = sc.size(0), C = sc.size(1) / bank.M, F = sc.size(2), rows = S * C;
+  TORCH_CHECK(C <= 64, "bad sizes");
+  TORCH_CHECK(F > 0, "empty block");
+  const Pool pool = pool_of(spool, sphase, bank, s, "spool");
+  const int* id = ids_of(ids, rows, s);
+  TORCH_CHECK(rows <= pool.P, "more rows (", rows, ") than streams in the pool (", pool.P, ")");
+  at::Tensor pcm = at::empty({S, bank.M * F, C}, sc.options().dtype(at::kShort));
+  if (rows == 0) return pcm;
+  const int rc = pqmf_stream_pool_synthesis_pcm16(sc.data_ptr<float>(), pcm.data_ptr<int16_t>(), bank.ptr, tables_ptr(tables, s), pool.state, pool.phase,
+                                                  (int)pool.P, id, (int)S, (int)C, (long)F, (int)bank.M, (int)bank.L, (unsigned)flags, cur_stream());
+  if (rc == PQMF_ERR_UNSUPPORTED)
+    return pcm_quantise(stream_pool_synthesis(sc.view({rows, bank.M, F}), hk, tables, spool, sphase, ids, flags).view({S, C, bank.M * F}));
+  check_rc(rc, "pqmf_stream_pool_synthesis_pcm16");
+  return pcm;
+}
+
+// pool: one block step from PCM to PCM of the listed streams: (pcm_out [S, T, C'], y [S, C' M, T / M])
+std::tuple<at::Tensor, at::Tensor> stream_pool_step_pcm16(const at::Tensor& pcm, const at::Tensor& hk, const at::Tensor& tables, at::Tensor xpool,
+                                                          at::Tensor xphase, at::Tensor spool, at::Tensor sphase, const at::Tensor& ids, bool downmix,
+                                                          int64_t flags) {
+  check_pcm(pcm, "stream pool step_pcm16");
+  const Bank bank = bank_of(hk, pcm);
+  c10::cuda::CUDAGuard guard(pcm.device());
+  const at::Tensor pc = pcm.contiguous();
+  const int64_t S = pc.size(0), T = pc.size(1), C = pc.size(2), Cr = downmix ? 1 : C, rows = S * Cr;
+  TORCH_CHECK(T > 0 && T % bank.M == 0 && bank.L % bank.M == 0, "streaming block length ", T, " must be a positive multiple of n_band=", bank.M);
+  const Pool xp = pool_of(xpool, xphase, bank, pcm, "xpool"), sp = pool_of(spool, sphase, bank, pcm, "spool");
+  TORCH_CHECK(xp.P == sp.P, "the analysis and synthesis pools hold different numbers of streams");
+  const int* id = ids_of(ids, rows, pcm);
+  TORCH_CHECK(rows <= xp.P, "more rows (", rows, ") than streams in the pool (", xp.P, ")");
+  at::Tensor y = at::empty({S, Cr * bank.M, T / bank.M}, pc.options().dtype(at::kFloat));
+  at::Tensor out = at::empty({S, T, Cr}, pc.options());
+  if (rows == 0) return {out, y};
+  const int rc = pqmf_stream_pool_step_pcm16(pc.data_ptr<int16_t>(), y.data_ptr<float>(), out.data_ptr<int16_t>(), bank.ptr, tables_ptr(tables, pcm),
+                                             xp.state, xp.phase, sp.state, sp.phase, (int)xp.P, id, (int)S, (long)T, (int)C, downmix ? 1 : 0, (int)bank.M,
+                                             (int)bank.L, (unsigned)flags, cur_stream());
+  if (rc == PQMF_ERR_UNSUPPORTED) {  // direction by direction, each native where it can be
+    at::Tensor ys = stream_pool_analysis_pcm16(pc, hk, tables, xpool, xphase, ids, downmix, flags);
+    return {stream_pool_synthesis_pcm16(ys, hk, tables, spool, sphase, ids, flags), ys};
+  }
+  check_rc(rc, "pqmf_stream_pool_step_pcm16");
+  return {out, y};
+}
+
 int64_t launch_count() { return (int64_t)pqmf_launch_count(); }
 
 // ---- autograd (SURVEY 8f-2: the reference path is differentiable, upstream users train through PQMF) --------------------
@@ -554,6 +739,26 @@ std::tuple<at::Tensor, at::Tensor> stream_pool_step_autograd(const at::Tensor& x
   return op.call(x, hk, tables, xpool, xphase, spool, sphase, ids, flags);
 }
 
+at::Tensor synthesis_stream_pcm16_autograd(const at::Tensor& s, const at::Tensor& hk, const at::Tensor& tables, const at::Tensor& state_in,
+                                           at::Tensor state_out, int64_t frame_parity, int64_t flags) {
+  TORCH_CHECK(!(at::GradMode::is_enabled() && s.requires_grad()),
+              "pqmf_b200::synthesis_stream_pcm16 is not differentiable (streaming mode carries state across calls, and int16 output has no "
+              "gradient); use inverse() for training or wrap the call in torch.no_grad()");
+  at::AutoDispatchBelowADInplaceOrView guard;
+  static auto op = c10::Dispatcher::singleton().findSchemaOrThrow("pqmf_b200::synthesis_stream_pcm16", "").typed<decltype(synthesis_stream_pcm16)>();
+  return op.call(s, hk, tables, state_in, state_out, frame_parity, flags);
+}
+at::Tensor stream_pool_synthesis_pcm16_autograd(const at::Tensor& s, const at::Tensor& hk, const at::Tensor& tables, at::Tensor spool, at::Tensor sphase,
+                                                const at::Tensor& ids, int64_t flags) {
+  TORCH_CHECK(!(at::GradMode::is_enabled() && s.requires_grad()),
+              "pqmf_b200::stream_pool_synthesis_pcm16 is not differentiable (a stream pool carries state across calls, and int16 output has no "
+              "gradient); use inverse() for training or wrap the call in torch.no_grad()");
+  at::AutoDispatchBelowADInplaceOrView guard;
+  static auto op =
+      c10::Dispatcher::singleton().findSchemaOrThrow("pqmf_b200::stream_pool_synthesis_pcm16", "").typed<decltype(stream_pool_synthesis_pcm16)>();
+  return op.call(s, hk, tables, spool, sphase, ids, flags);
+}
+
 at::Tensor analysis_autograd(const at::Tensor& x, const at::Tensor& hk, const at::Tensor& tables, int64_t n_frames, int64_t flags) {
   return AnalysisFn::apply(x, hk, tables, n_frames, flags);
 }
@@ -585,6 +790,21 @@ TORCH_LIBRARY(pqmf_b200, m) {
   m.def(
       "stream_pool_step(Tensor x, Tensor hk, Tensor tables, Tensor(a!) xpool, Tensor(b!) xphase, Tensor(c!) spool, Tensor(d!) sphase, Tensor ids, "
       "int flags) -> (Tensor, Tensor)");
+  m.def(
+      "analysis_stream_pcm16(Tensor pcm, Tensor hk, Tensor tables, Tensor state_in, Tensor(a!) state_out, int frame_parity, bool downmix, int flags) "
+      "-> Tensor");
+  m.def(
+      "synthesis_stream_pcm16(Tensor s, Tensor hk, Tensor tables, Tensor state_in, Tensor(a!) state_out, int frame_parity, int flags) -> Tensor");
+  m.def(
+      "stream_step_pcm16(Tensor pcm, Tensor hk, Tensor tables, Tensor xs_in, Tensor(a!) xs_out, Tensor ss_in, Tensor(b!) ss_out, int parity_in, "
+      "int parity_out, bool downmix, int flags) -> (Tensor, Tensor)");
+  m.def(
+      "stream_pool_analysis_pcm16(Tensor pcm, Tensor hk, Tensor tables, Tensor(a!) xpool, Tensor(b!) xphase, Tensor ids, bool downmix, int flags) "
+      "-> Tensor");
+  m.def("stream_pool_synthesis_pcm16(Tensor s, Tensor hk, Tensor tables, Tensor(a!) spool, Tensor(b!) sphase, Tensor ids, int flags) -> Tensor");
+  m.def(
+      "stream_pool_step_pcm16(Tensor pcm, Tensor hk, Tensor tables, Tensor(a!) xpool, Tensor(b!) xphase, Tensor(c!) spool, Tensor(d!) sphase, "
+      "Tensor ids, bool downmix, int flags) -> (Tensor, Tensor)");
   m.def("launch_count() -> int", &launch_count);
 }
 
@@ -602,6 +822,12 @@ TORCH_LIBRARY_IMPL(pqmf_b200, CUDA, m) {
   m.impl("stream_pool_analysis", &stream_pool_analysis);
   m.impl("stream_pool_synthesis", &stream_pool_synthesis);
   m.impl("stream_pool_step", &stream_pool_step);
+  m.impl("analysis_stream_pcm16", &analysis_stream_pcm16);
+  m.impl("synthesis_stream_pcm16", &synthesis_stream_pcm16);
+  m.impl("stream_step_pcm16", &stream_step_pcm16);
+  m.impl("stream_pool_analysis_pcm16", &stream_pool_analysis_pcm16);
+  m.impl("stream_pool_synthesis_pcm16", &stream_pool_synthesis_pcm16);
+  m.impl("stream_pool_step_pcm16", &stream_pool_step_pcm16);
 }
 
 // gradients w.r.t. the signal / the sub-bands only (the bank is a registered buffer in the reference, not a parameter)
@@ -614,4 +840,6 @@ TORCH_LIBRARY_IMPL(pqmf_b200, Autograd, m) {
   m.impl("stream_pool_analysis", &stream_pool_analysis_autograd);
   m.impl("stream_pool_synthesis", &stream_pool_synthesis_autograd);
   m.impl("stream_pool_step", &stream_pool_step_autograd);
+  m.impl("synthesis_stream_pcm16", &synthesis_stream_pcm16_autograd);
+  m.impl("stream_pool_synthesis_pcm16", &stream_pool_synthesis_pcm16_autograd);
 }

@@ -19,7 +19,8 @@ signals and sub-bands and return the input's dtype: ``forward(x_d)`` is bit-equa
 fp32 accumulation, round-to-nearest-even output; the large offline calls run on half-precision kernels, the rest widen, run the
 fp32 kernels and round).  The input dtype and the module's dtype are independent: ``.half()`` / ``.to(torch.bfloat16)`` cast ``hk`` and
 ``h`` as the reference's module casts its buffers, and the arithmetic then uses that rounded bank, accumulated in fp32.  Other dtypes
-(float64 included) raise.  The streaming, int16-PCM and per-band entry points take float32 sub-bands / signals only.
+(float64 included) raise.  The streaming, int16-PCM and per-band entry points take float32 sub-bands / signals only (the streaming calls
+also take int16 PCM blocks: ``forward_stream_pcm16`` / ``inverse_stream_pcm16`` / ``process_stream_pcm16``).
 """
 from __future__ import annotations
 
@@ -389,6 +390,69 @@ class CachedPQMF(PQMF):
         self._frames_in += x.shape[-1] // self.n_band
         self._frames_out += x.shape[-1] // self.n_band
         return out, y
+
+    @torch.jit.export
+    def process_stream_pcm16(self, pcm: torch.Tensor, downmix: bool = False) -> Tuple[torch.Tensor, torch.Tensor]:
+        """``process_stream`` from 16-bit PCM to 16-bit PCM: ``pcm`` int16 ``[S, T_block, channels]`` (interleaved WAV frames) -> ``(pcm_out
+        int16 [S, T_block, C'], y float32 [S, C' * n_band, T_block / n_band])`` with ``C' = 1`` when down-mixing, else ``channels``.  Bit-equal
+        to ``process_stream`` on the widened block (``forward_pcm16``'s widening; row ``s * C' + c`` is channel ``c`` of block ``s``) followed by
+        ``inverse_pcm16``'s quantisation, with the same state updates: PCM and float32 blocks continue one stream."""
+        if pcm.dim() != 3:
+            raise RuntimeError("process_stream_pcm16 expects int16 WAV frames [blocks, time, channels]")
+        rows = pcm.shape[0] * (1 if downmix else pcm.shape[2])
+        length = self.hk.shape[1]
+        if self._x_state.shape[1] != rows or self._x_state.device != pcm.device:
+            self._x_state = torch.zeros(2, rows, length, device=pcm.device)
+            self._x_slot = 0
+            self._frames_in = 0
+        if self._s_state.shape[1] != rows or self._s_state.device != pcm.device:
+            self._s_state = torch.zeros(2, rows, length, device=pcm.device)
+            self._s_slot = 0
+            self._frames_out = 0
+        out, y = torch.ops.pqmf_b200.stream_step_pcm16(pcm, self.hk.float(), self._tables, self._x_state[self._x_slot],
+                                                       self._x_state[1 - self._x_slot], self._s_state[self._s_slot], self._s_state[1 - self._s_slot],
+                                                       self._frames_in % 2, self._frames_out % 2, downmix, self._flags)
+        self._x_slot = 1 - self._x_slot
+        self._s_slot = 1 - self._s_slot
+        self._frames_in += pcm.shape[1] // self.n_band
+        self._frames_out += pcm.shape[1] // self.n_band
+        return out, y
+
+    @torch.jit.export
+    def forward_stream_pcm16(self, pcm: torch.Tensor, downmix: bool = False) -> torch.Tensor:
+        """One block of streaming analysis from 16-bit PCM: int16 ``[S, T_block, channels]`` -> ``[S, C' * n_band, T_block / n_band]``,
+        bit-equal to ``forward_stream`` on the widened block (see ``process_stream_pcm16``); updates the same state."""
+        if pcm.dim() != 3:
+            raise RuntimeError("forward_stream_pcm16 expects int16 WAV frames [blocks, time, channels]")
+        rows = pcm.shape[0] * (1 if downmix else pcm.shape[2])
+        length = self.hk.shape[1]
+        if self._x_state.shape[1] != rows or self._x_state.device != pcm.device:
+            self._x_state = torch.zeros(2, rows, length, device=pcm.device)
+            self._x_slot = 0
+            self._frames_in = 0
+        y = torch.ops.pqmf_b200.analysis_stream_pcm16(pcm, self.hk.float(), self._tables, self._x_state[self._x_slot],
+                                                      self._x_state[1 - self._x_slot], self._frames_in % 2, downmix, self._flags)
+        self._x_slot = 1 - self._x_slot
+        self._frames_in += pcm.shape[1] // self.n_band
+        return y
+
+    @torch.jit.export
+    def inverse_stream_pcm16(self, s: torch.Tensor) -> torch.Tensor:
+        """One block of streaming synthesis to 16-bit PCM: float32 ``[S, C * n_band, F_block]`` -> int16 ``[S, n_band * F_block, C]``,
+        ``clamp(round(inverse_stream(s) * 32768), -32768, 32767)`` interleaved; updates the same state."""
+        if s.dim() != 3:
+            raise RuntimeError("inverse_stream_pcm16 expects a 3-D tensor [blocks, channels * n_band, frames]")
+        rows = s.shape[0] * (s.shape[1] // self.n_band)
+        length = self.hk.shape[1]
+        if self._s_state.shape[1] != rows or self._s_state.device != s.device:
+            self._s_state = torch.zeros(2, rows, length, device=s.device)
+            self._s_slot = 0
+            self._frames_out = 0
+        out = torch.ops.pqmf_b200.synthesis_stream_pcm16(s, self.hk.float(), self._tables, self._s_state[self._s_slot],
+                                                         self._s_state[1 - self._s_slot], self._frames_out % 2, self._flags)
+        self._s_slot = 1 - self._s_slot
+        self._frames_out += s.shape[-1]
+        return out
 
     @torch.jit.export
     def forward_stream(self, x: torch.Tensor) -> torch.Tensor:

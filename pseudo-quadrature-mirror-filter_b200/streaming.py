@@ -75,7 +75,8 @@ class StreamPool:
     the ``n`` distinct streams ``ids`` (in any order; streams not listed are left exactly as they are), and returns their signal
     ``[n, 1, T]`` and sub-bands ``[n, n_band, T / n_band]`` -- per row bit for bit what ``process_stream`` gives for that stream.
     ``forward`` / ``inverse`` run one direction, with its own state and parity as ``forward_stream`` / ``inverse_stream``; ``reset`` forgets
-    streams so that a new session can take their slots.
+    streams so that a new session can take their slots.  ``step_pcm16`` / ``forward_pcm16`` / ``inverse_pcm16`` are the same calls with
+    16-bit PCM blocks (interleaved WAV frames in, int16 samples out).
 
     ``ids`` is a list of ints or a CPU integer tensor (checked: in range and distinct, else ``ValueError``), or a CUDA integer tensor, which
     is trusted as it is and costs no host synchronisation.  With CUDA ids a step allocates nothing but its outputs, so it can be captured
@@ -139,6 +140,26 @@ class StreamPool:
         if mod.n_band == 1:
             return y
         return torch.ops.pqmf_b200.stream_pool_synthesis(y, mod.hk.float(), mod._tables, self.spool, self.sphase, self._ids(ids), mod._flags)
+
+    def step_pcm16(self, pcm: torch.Tensor, ids, downmix: bool = False) -> Tuple[torch.Tensor, torch.Tensor]:
+        """``step`` from 16-bit PCM to 16-bit PCM: ``pcm`` int16 ``[S, T, channels]`` -> ``(pcm_out int16 [S, T, C'], y [S, C' * n_band,
+        T / n_band])``, ``C' = 1`` when down-mixing, else ``channels``.  ``ids`` has one stream per row: row ``r * C' + c`` (channel ``c`` of
+        block ``r``) is stream ``ids[r * C' + c]``.  Per row bit-equal to ``step`` on the widened block (``CachedPQMF.forward_pcm16``'s
+        widening), then quantised (``inverse_pcm16``'s rounding); the same pool and phase-word updates."""
+        mod = self.mod
+        return torch.ops.pqmf_b200.stream_pool_step_pcm16(pcm, mod.hk.float(), mod._tables, self.xpool, self.xphase, self.spool, self.sphase,
+                                                          self._ids(ids), downmix, mod._flags)
+
+    def forward_pcm16(self, pcm: torch.Tensor, ids, downmix: bool = False) -> torch.Tensor:
+        """``forward`` from 16-bit PCM: int16 ``[S, T, channels]`` -> ``[S, C' * n_band, T / n_band]`` (rows and ids as ``step_pcm16``)."""
+        mod = self.mod
+        return torch.ops.pqmf_b200.stream_pool_analysis_pcm16(pcm, mod.hk.float(), mod._tables, self.xpool, self.xphase, self._ids(ids), downmix,
+                                                              mod._flags)
+
+    def inverse_pcm16(self, s: torch.Tensor, ids) -> torch.Tensor:
+        """``inverse`` to 16-bit PCM: ``[S, C * n_band, F]`` -> int16 ``[S, n_band * F, C]``; row ``r * C + c`` is stream ``ids[r * C + c]``."""
+        mod = self.mod
+        return torch.ops.pqmf_b200.stream_pool_synthesis_pcm16(s, mod.hk.float(), mod._tables, self.spool, self.sphase, self._ids(ids), mod._flags)
 
     def reset(self, ids=None) -> None:
         """Forget the listed streams (all when ``ids`` is None): zero history in both directions, parity 0; in place, on the device."""
