@@ -1,7 +1,8 @@
 """Differential fuzz: tensor-core Hankel kernels vs the register-tiled direct form (tables = empty) on random shapes with >= 96 tiles,
 offline (both delays) and streaming.  One-off robustness check (odd tile counts, partial last tiles, frame counts not a multiple of 4).
 Also the half-precision entry points against the fp32 ones (bit-identity) and the host-buffer entries against the device path.
-Arguments: seed, offline cases, host-entry cases, half-precision cases."""
+Also the n_band-16 fold / Hankel-16 kernels in their steady state against calls of one tile per CTA.
+Arguments: seed, offline cases, host-entry cases, half-precision cases, fold / Hankel-16 cases."""
 import sys, os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import random, torch
@@ -131,4 +132,45 @@ for case in range(int(sys.argv[4]) if len(sys.argv) > 4 else 40):
     if not (torch.equal(y.view(torch.int16), mod(x.float()).to(dt).view(torch.int16)) and
             torch.equal(o.view(torch.int16), mod.inverse(y.float()).to(dt).view(torch.int16)) and y.dtype == dt and o.dtype == dt):
         print("HALF MISMATCH", dict(m=m, att=att, dtype=str(dt), cls=cls.__name__, rows=rows, t=t, offset=offset)); sys.exit(1)
+# n_band 16 fold / Hankel-16 kernels (exact on / off) in the steady state of their persistent loops: lockstep streaming with blocks that
+# are not a multiple of 256 samples (the Hankel-4 streaming kernels refuse them) at 1000 - 5000 streams, and offline batches whose signal
+# sits 16 bytes past a 32-byte boundary and sub-bands 4 bytes past a 16-byte one (the Hankel-4 kernels refuse them).  Every row bit-equal
+# to calls of at most one tile per CTA (groups of 16 streams; offline row chunks of at most 2 x SMs tiles in any family) with the
+# family's forced flags -- a tile's output does not depend on which CTA runs it at which iteration.
+n_sm = torch.cuda.get_device_properties(0).multi_processor_count
+for case in range(int(sys.argv[5]) if len(sys.argv) > 5 else 12):
+    att = random.choice((80, 100, 110, 120, 130))
+    exact = random.random() < 0.5
+    cls = random.choice((pq.PQMF, pq.CachedPQMF))
+    mod = cls(att, 16, exact=exact).cuda()
+    f = mod._flags
+    forced = f | _lib.PQMF_FLAG_FOLD | (_lib.PQMF_FLAG_NO_FOLD if exact else 0)
+    hk, tab = mod.hk, mod._tables
+    if cls is pq.CachedPQMF and random.random() < 0.5:
+        streams = random.randint(1000, 5000)
+        plan = [random.choice((480, 960, 1920, 4800, 496, 48, 16)) for _ in range(4)]
+        for k, T in enumerate(plan):
+            x = (0.5 * torch.randn(streams, 1, T, device="cuda")).clamp_(-1, 1)
+            xs_in = mod._x_state[mod._x_slot].clone() if k else torch.zeros(streams, 512, device="cuda")
+            ss_in = mod._s_state[mod._s_slot].clone() if k else torch.zeros(streams, 512, device="cuda")
+            pin, pout = mod._frames_in % 2, mod._frames_out % 2
+            out, y = mod.process_stream(x)
+            for g in range(0, streams, 16):
+                xi, si = xs_in[g:g + 16], ss_in[g:g + 16]
+                o_r, y_r = torch.ops.pqmf_b200.stream_step(x[g:g + 16], hk, tab, xi, torch.empty_like(xi), si, torch.empty_like(si), pin, pout, forced)
+                if not (torch.equal(y[g:g + 16], y_r) and torch.equal(out[g:g + 16], o_r)):
+                    print("FOLD STREAM MISMATCH", dict(att=att, exact=exact, streams=streams, plan=plan, k=k, group=g)); sys.exit(1)
+    else:
+        rows, F = random.randint(100, 1500), random.randint(1, 2048)
+        delay = 1 if cls is pq.CachedPQMF else 0
+        x0 = (0.5 * torch.randn(rows, 1, 16 * F, device="cuda")).clamp_(-1, 1)
+        x = torch.empty(x0.numel() + 16, device="cuda")[4:4 + x0.numel()].view(x0.shape).copy_(x0)
+        y = mod(x)
+        s = torch.empty(y.numel() + 16, device="cuda")[1:1 + y.numel()].view(y.shape).copy_(y)
+        out = mod.inverse(s)
+        per = max(1, 2 * n_sm // -(-F // 64))  # rows per reference call: at most one tile per CTA in every family and direction
+        y_r = torch.cat([torch.ops.pqmf_b200.analysis(x0[i:i + per].clone(), hk, tab, F, forced) for i in range(0, rows, per)])
+        o_r = torch.cat([torch.ops.pqmf_b200.synthesis(y[i:i + per].clone(), hk, tab, delay, forced) for i in range(0, rows, per)])
+        if not (torch.equal(y, y_r) and torch.equal(out, o_r)):
+            print("FOLD OFFLINE MISMATCH", dict(att=att, exact=exact, cls=cls.__name__, rows=rows, F=F)); sys.exit(1)
 print("fuzz ok; worst |hankel - direct| per (n_band, attenuation):", {k: (f"{v[0]:.1e}", f"{v[1]:.1e}") for k, v in sorted(worst.items())})
