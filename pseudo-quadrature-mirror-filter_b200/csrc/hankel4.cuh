@@ -891,7 +891,6 @@ template <int M, bool PAIR>
 int h4_launch_analysis(H4AnalysisParams p, int B, cudaStream_t st, H4Io io = H4Io::F32) {
   static H4Configured configured[4];
   if (!h4_set_tiles(p, B, p.F * M)) return -2;
-  if (p.in.pcm != nullptr) io = H4Io::PCM;
   if (io != H4Io::F32) {
     if constexpr (PAIR) {
       switch (io) {
@@ -910,7 +909,7 @@ int h4_launch_analysis(H4AnalysisParams p, int B, cudaStream_t st, H4Io io = H4I
 template <int M, bool PAIR>
 int h4_launch_synthesis(H4SynthesisParams p, int B, cudaStream_t st, H4Io io = H4Io::F32) {
   static H4Configured configured[4];
-  if (p.pcm_out != nullptr) {
+  if (io == H4Io::PCM) {
     if constexpr (PAIR) {
       p.duo = (p.C == 2 && B % 2 == 0) ? 1 : 0;  // stereo: the tiles of a launch are (clip, chunk), each visited once per channel
       if (!h4_set_tiles(p, p.duo ? B / 2 : B, p.F * M)) return -2;

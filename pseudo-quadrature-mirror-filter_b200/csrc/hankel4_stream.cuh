@@ -430,26 +430,38 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_stream_kernel(H
   } H4_TRACE(nullptr));
 }
 
-// launches (CTA pairs; on any error the caller runs other kernels: the fold kernels, or the direct form for pools)
-// Params: one of the H4AnalysisStream*Params above; it selects the instantiation (POOL, PCM)
-template <int M, typename Params>
-inline int h4_launch_analysis_stream(Params p, cudaStream_t st) {
-  constexpr bool POOL = std::is_base_of_v<H4AnalysisStreamPoolParams, Params>;
-  constexpr H4Io IO = std::is_same_v<Params, H4AnalysisStreamArgs<POOL, H4Io::PCM>> ? H4Io::PCM : H4Io::F32;
-  static_assert(std::is_same_v<Params, H4AnalysisStreamArgs<POOL, IO>>, "params of a streaming analysis instantiation");
+// launches (CTA pairs; on any error the caller runs other kernels: the fold kernels, or the direct form for pools).  The instantiation
+// follows the call: POOL when pool != nullptr, and the sample format io, F32 or PCM (in: the WAV frames; pcm_out: the mono rows)
+template <int M, bool POOL, H4Io IO>
+inline int h4_launch_analysis_stream(const H4AnalysisStreamParams& base, const StreamPoolIndex* pool, const PcmIn& in, cudaStream_t st) {
   static H4Configured configured;
+  H4AnalysisStreamArgs<POOL, IO> p{};
+  static_cast<H4AnalysisStreamParams&>(p) = base;
+  if constexpr (POOL) p.pool = *pool;
+  if constexpr (IO == H4Io::PCM) p.in = in;
   p.n_tiles = (p.B + p.s.spt - 1) / p.s.spt;
   return h4_launch<true>(h4_analysis_stream_kernel<M, POOL, IO>, p, kH4Threads, configured, st);
 }
-// Params: one of the H4SynthesisStream*Params above
-template <int M, typename Params>
-inline int h4_launch_synthesis_stream(Params p, cudaStream_t st) {
-  constexpr bool POOL = std::is_base_of_v<H4SynthesisStreamPoolParams, Params>;
-  constexpr H4Io IO = std::is_same_v<Params, H4SynthesisStreamArgs<POOL, H4Io::PCM>> ? H4Io::PCM : H4Io::F32;
-  static_assert(std::is_same_v<Params, H4SynthesisStreamArgs<POOL, IO>>, "params of a streaming synthesis instantiation");
+template <int M>
+inline int h4_launch_analysis_stream(const H4AnalysisStreamParams& p, const StreamPoolIndex* pool, H4Io io, const PcmIn& in, cudaStream_t st) {
+  if (io == H4Io::PCM) return pool ? h4_launch_analysis_stream<M, true, H4Io::PCM>(p, pool, in, st) : h4_launch_analysis_stream<M, false, H4Io::PCM>(p, pool, in, st);
+  return pool ? h4_launch_analysis_stream<M, true, H4Io::F32>(p, pool, in, st) : h4_launch_analysis_stream<M, false, H4Io::F32>(p, pool, in, st);
+}
+template <int M, bool POOL, H4Io IO>
+inline int h4_launch_synthesis_stream(const H4SynthesisStreamParams& base, const StreamPoolIndex* pool, int16_t* pcm_out, cudaStream_t st) {
   static H4Configured configured;
+  H4SynthesisStreamArgs<POOL, IO> p{};
+  static_cast<H4SynthesisStreamParams&>(p) = base;
+  if constexpr (POOL) p.pool = *pool;
+  if constexpr (IO == H4Io::PCM) p.pcm_out = pcm_out;
   p.n_tiles = (p.B + p.sg.spt - 1) / p.sg.spt;
   return h4_launch<true>(h4_synthesis_stream_kernel<M, POOL, IO>, p, kH4SynThreads, configured, st);
+}
+template <int M>
+inline int h4_launch_synthesis_stream(const H4SynthesisStreamParams& p, const StreamPoolIndex* pool, H4Io io, int16_t* pcm_out, cudaStream_t st) {
+  if (io == H4Io::PCM)
+    return pool ? h4_launch_synthesis_stream<M, true, H4Io::PCM>(p, pool, pcm_out, st) : h4_launch_synthesis_stream<M, false, H4Io::PCM>(p, pool, pcm_out, st);
+  return pool ? h4_launch_synthesis_stream<M, true, H4Io::F32>(p, pool, pcm_out, st) : h4_launch_synthesis_stream<M, false, H4Io::F32>(p, pool, pcm_out, st);
 }
 
 }  // namespace pqmf

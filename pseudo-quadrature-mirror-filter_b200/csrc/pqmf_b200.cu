@@ -38,6 +38,12 @@ inline int cuda_status() {
   return (int)e;
 }
 
+// e: what a kernel launch returned.  Every launch that started counts once (pqmf_launch_count), wherever it is made.
+inline int counted(int e) {
+  g_launches += (e == 0);
+  return e;
+}
+
 template <typename K>
 int ensure_smem(K kernel, size_t bytes) {
   if (bytes <= 48 * 1024) return 0;
@@ -47,6 +53,28 @@ int ensure_smem(K kernel, size_t bytes) {
 
 // stream pools (stream_pool.cuh): the rows of a call are streams ids[0 .. n) of a pool of P
 using PoolRows = pqmf::StreamPoolIndex;
+
+// ---- what the dispatchers (run_analysis / run_synthesis) know of a call besides its shape and bank ----
+// Its sample side: analysis input, synthesis output.  The sub-bands are float32, or half bits when the signal is.
+struct Samples {
+  pqmf::H4Io io;
+  void* p;           // float32 rows, raw fp16 / bf16 bits or int16 WAV frames
+  pqmf::PcmIn pcm;   // PCM: {p, channels per frame, down-mix}; otherwise {nullptr, 1, 0}
+  void* rows() const { return io == pqmf::H4Io::PCM ? nullptr : p; }
+  int16_t* pcm_out() const { return io == pqmf::H4Io::PCM ? static_cast<int16_t*>(p) : nullptr; }
+};
+Samples samples(const void* p, pqmf::H4Io io = pqmf::H4Io::F32) { return {io, const_cast<void*>(p), {nullptr, 1, 0}}; }
+Samples pcm16(const int16_t* p, int C, int downmix = 0) { return {pqmf::H4Io::PCM, const_cast<int16_t*>(p), {p, C, downmix ? 1 : 0}}; }
+// Its carried history: none (offline: in == nullptr), lockstep, or a pool (in = out = the pool buffer, parity 0)
+struct History {
+  const float* in;
+  float* out;
+  int parity;
+  const PoolRows* pool;
+};
+constexpr History kOffline{nullptr, nullptr, 0, nullptr};
+History lockstep(const float* in, float* out, int parity) { return {in, out, parity, nullptr}; }
+History pooled(float* buf, const PoolRows& rows) { return {buf, buf, 0, &rows}; }
 
 // ------------------------------------------------------------------ direct-form launches
 // Params: AnalysisDirectParams, or AnalysisDirectPoolParams for the POOL instantiations
@@ -61,8 +89,7 @@ int launch_analysis_direct(Params p, int B, cudaStream_t st) {
   if (int e = ensure_smem(kern, smem)) return e;
   dim3 grid((unsigned)((p.n_frames + FT - 1) / FT), (unsigned)((p.M + NB - 1) / NB), (unsigned)B);
   kern<<<grid, pqmf::kDirectThreads, smem, st>>>(p);
-  ++g_launches;
-  return cuda_status();
+  return counted(cuda_status());
 }
 
 int analysis_direct(const float* x, const float* hist, float* y, const float* hk, int B, long T, long n_frames, int M, int L,
@@ -107,8 +134,7 @@ int launch_synthesis_direct(Params p, int B, cudaStream_t st) {
   if (int e = ensure_smem(kern, smem)) return e;
   dim3 grid((unsigned)((p.F + FT - 1) / FT), (unsigned)((p.M + NP - 1) / NP), (unsigned)B);
   kern<<<grid, pqmf::kDirectThreads, smem, st>>>(p);
-  ++g_launches;
-  return cuda_status();
+  return counted(cuda_status());
 }
 
 int synthesis_direct(const float* s, const float* hist, float* out, const float* hk, int B, long F, int M, int L, int off2,
@@ -209,7 +235,7 @@ int h4_analysis_m(pqmf::H4AnalysisParams p, const float* tables, int jlo, int kt
       p.trim_lo = half ? 0 : trim;
       p.trim_hi = half ? trim : 0;
       p.accumulate = half;
-      if (const int e = pqmf::h4_launch_analysis<M, true>(p, B, st, io)) {
+      if (const int e = counted(pqmf::h4_launch_analysis<M, true>(p, B, st, io))) {
         if (half) return e;
         (void)cudaGetLastError();  // nothing was launched: the caller falls back to the direct form, which must not see this error
         return PQMF_ERR_UNSUPPORTED;
@@ -221,7 +247,7 @@ int h4_analysis_m(pqmf::H4AnalysisParams p, const float* tables, int jlo, int kt
   if (!(flags & PQMF_FLAG_NO_PAIR)) {
     p.g = pqmf::h4_shape(M, jlo, kt, true, false);
     p.bank = reinterpret_cast<const uint16_t*>(tables + h4_pair_offset(M, L));
-    const int e = pqmf::h4_launch_analysis<M, true>(p, B, st, io);
+    const int e = counted(pqmf::h4_launch_analysis<M, true>(p, B, st, io));
     if (e == 0) return 0;
     (void)cudaGetLastError();  // a context that cannot co-schedule CTA pairs (e.g. an SM partition): same arithmetic, one CTA per SM
   }
@@ -231,23 +257,22 @@ int h4_analysis_m(pqmf::H4AnalysisParams p, const float* tables, int jlo, int kt
     if (!pqmf::hankel16_supported(M, L)) return PQMF_ERR_UNSUPPORTED;
     p.g = pqmf::h4_shape(M, jlo, kt, false, false);
     p.bank = reinterpret_cast<const uint16_t*>(tables + kH4TableOffset);
-    return pqmf::h4_launch_analysis<M, false>(p, B, st, io);
+    return counted(pqmf::h4_launch_analysis<M, false>(p, B, st, io));
   }
 }
-// x / y: float32 rows and sub-bands, or raw half bits when io is F16 / BF16 (x unused with PCM input)
-int h4_analysis(const void* x, void* y, const float* tables, int B, long T, long F, int M, int L, unsigned flags, cudaStream_t st,
-                pqmf::PcmIn pcm = pqmf::PcmIn{nullptr, 1, 0}, pqmf::H4Io io = pqmf::H4Io::F32) {
+// y: float32 sub-bands, or raw half bits when x is half
+int h4_analysis(const Samples& x, void* y, const float* tables, int B, long T, long F, int M, int L, unsigned flags, cudaStream_t st) {
   int jlo, kt;
   h4_taps(flags, jlo, kt);
   if (kt == 0) return PQMF_ERR_UNSUPPORTED;
   pqmf::H4AnalysisParams p{};
-  p.x = static_cast<const float*>(x); p.in = pcm; p.y = static_cast<float*>(y); p.T = T; p.F = F; p.off = L / 2; p.parity = 0; p.keep_in_l2 = 1;
+  p.x = static_cast<const float*>(x.rows()); p.in = x.pcm; p.y = static_cast<float*>(y); p.T = T; p.F = F; p.off = L / 2; p.parity = 0; p.keep_in_l2 = 1;
   switch (M) {
-    case 4: return h4_analysis_m<4>(p, tables, jlo, kt, B, L, flags, st, io);
-    case 8: return h4_analysis_m<8>(p, tables, jlo, kt, B, L, flags, st, io);
-    case 16: return h4_analysis_m<16>(p, tables, jlo, kt, B, L, flags, st, io);
-    case 32: return h4_analysis_m<32>(p, tables, jlo, kt, B, L, flags, st, io);
-    case 64: return h4_analysis_m<64>(p, tables, jlo, kt, B, L, flags, st, io);
+    case 4: return h4_analysis_m<4>(p, tables, jlo, kt, B, L, flags, st, x.io);
+    case 8: return h4_analysis_m<8>(p, tables, jlo, kt, B, L, flags, st, x.io);
+    case 16: return h4_analysis_m<16>(p, tables, jlo, kt, B, L, flags, st, x.io);
+    case 32: return h4_analysis_m<32>(p, tables, jlo, kt, B, L, flags, st, x.io);
+    case 64: return h4_analysis_m<64>(p, tables, jlo, kt, B, L, flags, st, x.io);
     default: return PQMF_ERR_UNSUPPORTED;
   }
 }
@@ -255,7 +280,6 @@ int h4_analysis(const void* x, void* y, const float* tables, int B, long T, long
 template <int M>
 int h4_synthesis_m(pqmf::H4SynthesisParams p, const float* tables, int jlo, int kt, int B, int L, unsigned flags, cudaStream_t st, pqmf::H4Io io) {
   const int trim = (flags & PQMF_FLAG_EXACT) ? 0 : (int)PQMF_FLAG_H4_TRIM_S(flags);
-  if ((flags & PQMF_FLAG_H4_SPLIT) && p.pcm_out != nullptr) return PQMF_ERR_UNSUPPORTED;  // the second launch accumulates: not in int16
   if (flags & PQMF_FLAG_H4_SPLIT) {
     for (int half = 0; half < 2; ++half) {
       p.g = pqmf::h4_shape(M, jlo + half * kt, kt, true, true);
@@ -264,7 +288,7 @@ int h4_synthesis_m(pqmf::H4SynthesisParams p, const float* tables, int jlo, int 
       p.trim_lo = half ? trim : 0;
       p.trim_hi = half ? 0 : trim;
       p.accumulate = half;
-      if (const int e = pqmf::h4_launch_synthesis<M, true>(p, B, st, io)) {
+      if (const int e = counted(pqmf::h4_launch_synthesis<M, true>(p, B, st, io))) {
         if (half) return e;
         (void)cudaGetLastError();
         return PQMF_ERR_UNSUPPORTED;
@@ -280,7 +304,7 @@ int h4_synthesis_m(pqmf::H4SynthesisParams p, const float* tables, int jlo, int 
     if (variant) p.trim_lo = p.trim_hi = trim > 0 ? trim - 1 : 0;
     p.g = pqmf::h4_shape(M, jlo, kt + variant * M, true, true);
     p.bank = reinterpret_cast<const uint16_t*>(tables + h4_pair_offset(M, L) + (1 + variant) * h4_pair_floats(M, L));
-    const int e = pqmf::h4_launch_synthesis<M, true>(p, B, st, io);
+    const int e = counted(pqmf::h4_launch_synthesis<M, true>(p, B, st, io));
     if (e == 0) return 0;
     (void)cudaGetLastError();
   }
@@ -290,34 +314,51 @@ int h4_synthesis_m(pqmf::H4SynthesisParams p, const float* tables, int jlo, int 
     if (!pqmf::hankel16_supported(M, L)) return PQMF_ERR_UNSUPPORTED;
     p.g = pqmf::h4_shape(M, jlo, kt, false, true);
     p.bank = reinterpret_cast<const uint16_t*>(tables + kH4TableOffset + kH4ImageFloats);
-    return pqmf::h4_launch_synthesis<M, false>(p, B, st, io);
+    return counted(pqmf::h4_launch_synthesis<M, false>(p, B, st, io));
   }
 }
-// s / out: float32 sub-bands and rows, or raw half bits when io is F16 / BF16 (out unused with PCM output)
-int h4_synthesis(const void* s, void* out, const float* tables, int B, long F, int off2, int M, int L, unsigned flags, cudaStream_t st,
-                 int16_t* pcm_out = nullptr, int C = 1, pqmf::H4Io io = pqmf::H4Io::F32) {
+// s: float32 sub-bands, or raw half bits when out is half
+int h4_synthesis(const void* s, const Samples& out, const float* tables, int B, long F, int off2, int M, int L, unsigned flags, cudaStream_t st) {
   int jlo, kt;
   h4_taps(flags, jlo, kt);
   if (kt == 0 || off2 % M != 0) return PQMF_ERR_UNSUPPORTED;
   pqmf::H4SynthesisParams p{};
-  p.s = static_cast<const float*>(s); p.out = static_cast<float*>(out); p.pcm_out = pcm_out; p.C = C; p.F = F; p.o = off2 / M; p.parity = 0; p.reverse = 1;
+  p.s = static_cast<const float*>(s); p.out = static_cast<float*>(out.rows()); p.pcm_out = out.pcm_out(); p.C = out.pcm.C; p.F = F; p.o = off2 / M; p.parity = 0; p.reverse = 1;
   switch (M) {
-    case 4: return h4_synthesis_m<4>(p, tables, jlo, kt, B, L, flags, st, io);
-    case 8: return h4_synthesis_m<8>(p, tables, jlo, kt, B, L, flags, st, io);
-    case 16: return h4_synthesis_m<16>(p, tables, jlo, kt, B, L, flags, st, io);
-    case 32: return h4_synthesis_m<32>(p, tables, jlo, kt, B, L, flags, st, io);
-    case 64: return h4_synthesis_m<64>(p, tables, jlo, kt, B, L, flags, st, io);
+    case 4: return h4_synthesis_m<4>(p, tables, jlo, kt, B, L, flags, st, out.io);
+    case 8: return h4_synthesis_m<8>(p, tables, jlo, kt, B, L, flags, st, out.io);
+    case 16: return h4_synthesis_m<16>(p, tables, jlo, kt, B, L, flags, st, out.io);
+    case 32: return h4_synthesis_m<32>(p, tables, jlo, kt, B, L, flags, st, out.io);
+    case 64: return h4_synthesis_m<64>(p, tables, jlo, kt, B, L, flags, st, out.io);
     default: return PQMF_ERR_UNSUPPORTED;
   }
 }
 
-// ---- streaming blocks on the Hankel-4 kernels (hankel4_stream.cuh): several streams per MMA tile.  ONE routing decision per direction
-//      for every streaming entry -- lockstep and pool, fp32 and int16 PCM: the kernels serve a call exactly where h4_stream_family holds
-//      and h4_*_stream_plan accepts its shape, flags and tile count, and its buffers meet the kernels' alignment (h4_*_stream_ok).
-//      Everywhere else (short blocks, few streams, odd sizes) an fp32 call runs other kernels -- the fold kernels for lockstep n_band 16,
-//      the direct form -- and a PCM call is refused with PQMF_ERR_UNSUPPORTED ----
-bool use_fast(int M, int L, const float* tables, unsigned flags);
-bool use_h4_family(int M, int L, const float* tables, unsigned flags);
+bool use_fast(int M, int L, const float* tables, unsigned flags) {
+  return tables != nullptr && !(flags & (PQMF_FLAG_NO_SIGN | PQMF_FLAG_FP32)) && pqmf::hankel16_supported(M, L);
+}
+// other band counts / prototype lengths: only the offline Hankel kernels exist (streaming, small batches and the sign-less free
+// functions use the direct form); PQMF_FLAG_EXACT keeps them but runs every correction term
+bool use_h4_family(int M, int L, const float* tables, unsigned flags) {
+  return tables != nullptr && !(flags & (PQMF_FLAG_NO_SIGN | PQMF_FLAG_FOLD | PQMF_FLAG_FP32)) && h4_family(M, L);
+}
+
+// ---- does an offline fp32 call with this shape and bank run the offline Hankel-4 kernels (h4_takes_* adds formats and alignment).
+//      (n_band 16 / L 512: fast_analysis's shape checks, hankel16_analysis_ok, are implied.) ----
+bool h4_route_analysis(int B, long T, long F, int M, int L, const float* tables, unsigned flags) {
+  const bool shape = T > 0 && (T % M) == 0 && (T % 8) == 0 && F == T / M && use_h4(B, F, M, nullptr);
+  if (use_fast(M, L, tables, flags)) return shape && !(flags & PQMF_FLAG_FOLD);
+  return !pqmf::hankel16_supported(M, L) && use_h4_family(M, L, tables, flags) && shape;
+}
+bool h4_route_synthesis(int B, long F, int M, int L, const float* tables, unsigned flags) {
+  const bool shape = F > 0 && (F & 3) == 0 && use_h4(B, F, M, nullptr);
+  if (use_fast(M, L, tables, flags)) return shape && !(flags & PQMF_FLAG_FOLD);
+  return !pqmf::hankel16_supported(M, L) && use_h4_family(M, L, tables, flags) && shape;
+}
+
+// ---- streaming blocks on the Hankel-4 kernels (hankel4_stream.cuh): several streams per MMA tile, wherever h4_stream_family holds
+//      and h4_*_stream_plan accepts the shape, flags and tile count.  Everywhere else (short blocks, few streams, odd sizes) the
+//      dispatchers go on to the fold kernels for lockstep n_band 16, or the direct form ----
 bool h4_stream_family(int M, int L, const float* tables, unsigned flags) {
   if (use_fast(M, L, tables, flags)) return true;  // n_band 16 / L 512
   return !pqmf::hankel16_supported(M, L) && use_h4_family(M, L, tables, flags) && (M == 8 || M == 32);
@@ -342,12 +383,6 @@ bool h4_analysis_stream_plan(int B, long T, int M, int L, const float* tables, u
   p.bank = reinterpret_cast<const uint16_t*>(tables + h4_pair_offset(M, L));
   return pqmf::h4_shape_fits(p.g);
 }
-// 256-bit signal loads (a PCM block: 16-byte mono, 32-byte stereo loads), 128-bit sub-band stores and state accesses
-bool h4_analysis_stream_ok(int B, long T, int M, int L, const float* tables, unsigned flags, const void* signal, const float* y, const float* state_in,
-                           const float* state_out, pqmf::H4AnalysisStreamParams& p) {
-  return h4_analysis_stream_plan(B, T, M, L, tables, flags, p) && ((uintptr_t)signal | (uintptr_t)state_in) % 32 == 0 &&
-         ((uintptr_t)y | (uintptr_t)state_out) % 16 == 0;
-}
 bool h4_synthesis_stream_plan(int B, long F, int M, int L, const float* tables, unsigned flags, pqmf::H4SynthesisStreamParams& p) {
   if (!h4_stream_family(M, L, tables, flags)) return false;
   int jlo, kt;
@@ -368,61 +403,29 @@ bool h4_synthesis_stream_plan(int B, long F, int M, int L, const float* tables, 
   p.bank = reinterpret_cast<const uint16_t*>(tables + h4_pair_offset(M, L) + h4_pair_floats(M, L));
   return pqmf::h4_shape_fits(p.g);
 }
-// 128-bit sub-band loads and state accesses; 256-bit fp32 output stores (PCM output: 128-bit int16 stores)
-bool h4_synthesis_stream_ok(int B, long F, int M, int L, const float* tables, unsigned flags, const float* s, const void* out, bool pcm_out,
-                            const float* state_in, const float* state_out, pqmf::H4SynthesisStreamParams& p) {
-  return h4_synthesis_stream_plan(B, F, M, L, tables, flags, p) && ((uintptr_t)s | (uintptr_t)state_in | (uintptr_t)state_out) % 16 == 0 &&
-         (uintptr_t)out % (pcm_out ? 16 : 32) == 0;
-}
-template <typename Params>
-int h4_analysis_stream_launch(const Params& p, int M, cudaStream_t st) {
+// the launch of a streaming call that h4_takes_* planned: lockstep or POOL instantiation by the history, fp32 or PCM by the samples.
+// Returns 0 or the error of a launch that did not start (cleared: the dispatcher goes on to other kernels).
+int h4_analysis_stream(pqmf::H4AnalysisStreamParams p, const Samples& x, void* y, const History& h, int M, cudaStream_t st) {
+  p.x = static_cast<const float*>(x.rows()); p.hist_in = h.in; p.hist_out = h.out; p.y = static_cast<float*>(y); p.parity = h.parity & 1;
+  int e = PQMF_ERR_UNSUPPORTED;
   switch (M) {
-    case 8: return pqmf::h4_launch_analysis_stream<8>(p, st);
-    case 16: return pqmf::h4_launch_analysis_stream<16>(p, st);
-    case 32: return pqmf::h4_launch_analysis_stream<32>(p, st);
-    default: return PQMF_ERR_UNSUPPORTED;
+    case 8: e = pqmf::h4_launch_analysis_stream<8>(p, h.pool, x.io, x.pcm, st); break;
+    case 16: e = pqmf::h4_launch_analysis_stream<16>(p, h.pool, x.io, x.pcm, st); break;
+    case 32: e = pqmf::h4_launch_analysis_stream<32>(p, h.pool, x.io, x.pcm, st); break;
   }
+  if (e != 0) (void)cudaGetLastError();
+  return counted(e);
 }
-template <typename Params>
-int h4_synthesis_stream_launch(const Params& p, int M, cudaStream_t st) {
+int h4_synthesis_stream(pqmf::H4SynthesisStreamParams p, const void* s, const Samples& out, const History& h, int M, cudaStream_t st) {
+  p.s = static_cast<const float*>(s); p.state_in = h.in; p.state_out = h.out; p.out = static_cast<float*>(out.rows()); p.parity = h.parity & 1;
+  int e = PQMF_ERR_UNSUPPORTED;
   switch (M) {
-    case 8: return pqmf::h4_launch_synthesis_stream<8>(p, st);
-    case 16: return pqmf::h4_launch_synthesis_stream<16>(p, st);
-    case 32: return pqmf::h4_launch_synthesis_stream<32>(p, st);
-    default: return PQMF_ERR_UNSUPPORTED;
+    case 8: e = pqmf::h4_launch_synthesis_stream<8>(p, h.pool, out.io, out.pcm_out(), st); break;
+    case 16: e = pqmf::h4_launch_synthesis_stream<16>(p, h.pool, out.io, out.pcm_out(), st); break;
+    case 32: e = pqmf::h4_launch_synthesis_stream<32>(p, h.pool, out.io, out.pcm_out(), st); break;
   }
-}
-// pool != nullptr: the indexed (POOL) kernels, with state_in = state_out = the pool.  pcm != nullptr: the block is int16 WAV frames (x
-// unused).  Returns 0, PQMF_ERR_UNSUPPORTED (refused: nothing launched) or the error of a launch that did not start (cleared).
-int h4_analysis_stream(const float* x, float* y, const float* tables, const float* state_in, float* state_out, int B, long T, int M, int L,
-                       int parity, unsigned flags, cudaStream_t st, const PoolRows* pool = nullptr, const pqmf::PcmIn* pcm = nullptr) {
-  pqmf::H4AnalysisStreamParams p{};
-  if (!h4_analysis_stream_ok(B, T, M, L, tables, flags, pcm ? static_cast<const void*>(pcm->pcm) : x, y, state_in, state_out, p))
-    return PQMF_ERR_UNSUPPORTED;
-  p.x = x; p.hist_in = state_in; p.hist_out = state_out; p.y = y; p.parity = parity & 1;
-  int e;
-  if (pcm && pool) e = h4_analysis_stream_launch(pqmf::H4AnalysisStreamPoolPcmParams{{p, *pool}, *pcm}, M, st);
-  else if (pcm) e = h4_analysis_stream_launch(pqmf::H4AnalysisStreamPcmParams{p, *pcm}, M, st);
-  else if (pool) e = h4_analysis_stream_launch(pqmf::H4AnalysisStreamPoolParams{p, *pool}, M, st);
-  else e = h4_analysis_stream_launch(p, M, st);
   if (e != 0) (void)cudaGetLastError();
-  return e;
-}
-// pcm_out != nullptr: mono int16 output rows (out unused)
-int h4_synthesis_stream(const float* s, float* out, const float* tables, const float* state_in, float* state_out, int B, long F, int M, int L,
-                        int parity, unsigned flags, cudaStream_t st, const PoolRows* pool = nullptr, int16_t* pcm_out = nullptr) {
-  pqmf::H4SynthesisStreamParams p{};
-  if (!h4_synthesis_stream_ok(B, F, M, L, tables, flags, s, pcm_out ? static_cast<const void*>(pcm_out) : out, pcm_out != nullptr, state_in,
-                              state_out, p))
-    return PQMF_ERR_UNSUPPORTED;
-  p.s = s; p.state_in = state_in; p.state_out = state_out; p.out = out; p.parity = parity & 1;
-  int e;
-  if (pcm_out && pool) e = h4_synthesis_stream_launch(pqmf::H4SynthesisStreamPoolPcmParams{{p, *pool}, pcm_out}, M, st);
-  else if (pcm_out) e = h4_synthesis_stream_launch(pqmf::H4SynthesisStreamPcmParams{p, pcm_out}, M, st);
-  else if (pool) e = h4_synthesis_stream_launch(pqmf::H4SynthesisStreamPoolParams{p, *pool}, M, st);
-  else e = h4_synthesis_stream_launch(p, M, st);
-  if (e != 0) (void)cudaGetLastError();
-  return e;
+  return counted(e);
 }
 
 // n_band 16 fast path: fold + tensor-core modulation (fast16*.cuh), or -- with PQMF_FLAG_EXACT -- the direct form as an
@@ -454,54 +457,101 @@ int exact_tc_synthesis(const float* s, const float* hist, float* out, float* his
   return trimmed ? pqmf::h16_launch_synthesis<64, 384>(p, st) : pqmf::h16_launch_synthesis<0, 512>(p, st);
 }
 
-// (offline calls try the Hankel-4 kernels before these: h4_route_analysis / h4_route_synthesis)
+// one launch each
 int fast_analysis(const float* x, const float* hist, float* y, float* hist_out, const float* tables, int B, long T, long F, int off,
                   int parity, unsigned flags, cudaStream_t st) {
-  if (flags & (PQMF_FLAG_EXACT | PQMF_FLAG_NO_FOLD)) return exact_tc_analysis(x, hist, y, hist_out, tables, B, T, F, off, parity, flags, st);
-  return pqmf::fast16_analysis(x, hist, y, hist_out, tables, B, T, F, off, parity, flags, st);
+  if (flags & (PQMF_FLAG_EXACT | PQMF_FLAG_NO_FOLD)) return counted(exact_tc_analysis(x, hist, y, hist_out, tables, B, T, F, off, parity, flags, st));
+  return counted(pqmf::fast16_analysis(x, hist, y, hist_out, tables, B, T, F, off, parity, flags, st));
 }
 
 int fast_synthesis(const float* s, const float* hist, float* out, float* hist_out, const float* tables, int B, long F, int off2,
                    int parity, unsigned flags, cudaStream_t st) {
-  if (flags & (PQMF_FLAG_EXACT | PQMF_FLAG_NO_FOLD)) return exact_tc_synthesis(s, hist, out, hist_out, tables, B, F, off2, parity, flags, st);
-  return pqmf::fast16_synthesis(s, hist, out, hist_out, tables, B, F, off2, parity, flags, st);
+  if (flags & (PQMF_FLAG_EXACT | PQMF_FLAG_NO_FOLD)) return counted(exact_tc_synthesis(s, hist, out, hist_out, tables, B, F, off2, parity, flags, st));
+  return counted(pqmf::fast16_synthesis(s, hist, out, hist_out, tables, B, F, off2, parity, flags, st));
 }
 
-bool use_fast(int M, int L, const float* tables, unsigned flags) {
-  return tables != nullptr && !(flags & (PQMF_FLAG_NO_SIGN | PQMF_FLAG_FP32)) && pqmf::hankel16_supported(M, L);
+// ---- which kernel family serves which sample format and history.  The dispatchers try them in this order.
+//        family                        | fp32                    | fp16 / bf16            | PCM
+//        Hankel-4                      | offline, lockstep, pool | offline, unsplit banks | all; output: unsplit banks, mono when streaming
+//        fold / Hankel-16 (n_band 16)  | offline, lockstep       | -                      | -
+//        direct form                   | offline, lockstep, pool | -                      | offline
+//      (the half-precision instantiations exist for the unsplit banks only; a split bank's second launch accumulates, not in int16;
+//      streaming PCM output is mono rows: the two channels of a clip may sit in any two tiles) ----
+bool h4_serves(const Samples& s, const History& h, unsigned flags, bool output) {
+  if (pqmf::h4_io_half(s.io)) return !h.in && !(flags & PQMF_FLAG_H4_SPLIT);
+  if (s.io == pqmf::H4Io::PCM && output) return !(flags & PQMF_FLAG_H4_SPLIT) && (!h.in || s.pcm.C == 1);
+  return true;
 }
-// other band counts / prototype lengths: only the offline Hankel kernels exist (streaming, small batches and the sign-less free
-// functions use the direct form); PQMF_FLAG_EXACT keeps them but runs every correction term
-bool use_h4_family(int M, int L, const float* tables, unsigned flags) {
-  return tables != nullptr && !(flags & (PQMF_FLAG_NO_SIGN | PQMF_FLAG_FOLD | PQMF_FLAG_FP32)) && h4_family(M, L);
+bool fold_serves(const Samples& s, const History& h) { return s.io == pqmf::H4Io::F32 && !h.pool; }
+bool direct_serves(const Samples& s, const History& h) { return s.io == pqmf::H4Io::F32 || (s.io == pqmf::H4Io::PCM && !h.in); }
+
+// ---- the Hankel-4 kernels take this call: the one decision per direction for every entry.  The history picks the offline route
+//      (h4_route_*) or the streaming plan (h4_*_stream_plan, returned in plan), then the format (h4_serves) and the buffers' alignment.
+//      So a PCM or half call runs natively exactly where the fp32 call with the same rows runs the same kernels with the same trims,
+//      which is what makes the two bit-identical. ----
+bool aligned(const void* p, int bytes) { return (uintptr_t)p % bytes == 0; }
+// 256-bit fp32 and PCM signal loads (PCM: 16-byte mono, 32-byte stereo loads), 128-bit half signal loads; 128-bit sub-band stores;
+// 256-bit loads of the streaming history, 128-bit rolls
+bool h4_takes_analysis(const Samples& x, const void* y, const History& h, int B, long T, long F, int M, int L, const float* tables, unsigned flags,
+                       pqmf::H4AnalysisStreamParams* plan = nullptr) {
+  pqmf::H4AnalysisStreamParams unused{};
+  if (!h4_serves(x, h, flags, false)) return false;
+  if (h.in ? !h4_analysis_stream_plan(B, T, M, L, tables, flags, plan ? *plan : unused) : !h4_route_analysis(B, T, F, M, L, tables, flags)) return false;
+  return aligned(x.p, pqmf::h4_io_half(x.io) ? 16 : 32) && aligned(y, 16) && aligned(h.in, 32) && aligned(h.out, 16);
+}
+// 256-bit fp32 output stores, 128-bit half and int16 stores; 128-bit sub-band loads and state accesses
+bool h4_takes_synthesis(const void* s, const Samples& out, const History& h, int B, long F, int M, int L, const float* tables, unsigned flags,
+                        pqmf::H4SynthesisStreamParams* plan = nullptr) {
+  pqmf::H4SynthesisStreamParams unused{};
+  if (!h4_serves(out, h, flags, true)) return false;
+  if (h.in ? !h4_synthesis_stream_plan(B, F, M, L, tables, flags, plan ? *plan : unused) : !h4_route_synthesis(B, F, M, L, tables, flags)) return false;
+  return aligned(out.p, out.io == pqmf::H4Io::F32 ? 32 : 16) && aligned(s, 16) && aligned(h.in, 16) && aligned(h.out, 16);
 }
 
-// ---- which kernels an offline call runs: the offline Hankel-4 kernels exactly when these say so and the buffers are aligned for
-//      them; everything else (n_band 16: the fold / Hankel-16 kernels; other band counts: the direct form) comes after.  The fp32 and
-//      the half-precision entry points both decide here, so a half-precision call runs natively exactly where the fp32 call on its
-//      widened input runs the same kernels with the same trims -- which is what makes the two bit-identical.
-//      (n_band 16 / L 512: fast_analysis's shape checks, hankel16_analysis_ok, are implied.) ----
-bool h4_route_analysis(int B, long T, long F, int M, int L, const float* tables, unsigned flags) {
-  const bool shape = T > 0 && (T % M) == 0 && (T % 8) == 0 && F == T / M && use_h4(B, F, M, nullptr);
-  if (use_fast(M, L, tables, flags)) return shape && !(flags & PQMF_FLAG_FOLD);
-  return !pqmf::hankel16_supported(M, L) && use_h4_family(M, L, tables, flags) && shape;
+// ---- one dispatcher per direction: the families in the order of the table above.  The offline Hankel-4 and the fold / Hankel-16
+//      kernels give way only on PQMF_ERR_UNSUPPORTED (nothing launched), the streaming Hankel-4 kernels on any launch that did not
+//      start (cleared).  No family left: PQMF_ERR_UNSUPPORTED, with nothing launched.  y and s: float32 sub-bands, or half bits with
+//      half samples ----
+int run_analysis(const Samples& x, void* y, const History& h, const float* hk, const float* tables, int B, long T, long F, int M, int L,
+                 unsigned flags, cudaStream_t st) {
+  pqmf::H4AnalysisStreamParams plan{};
+  if (h4_takes_analysis(x, y, h, B, T, F, M, L, tables, flags, &plan)) {
+    const int e = h.in ? h4_analysis_stream(plan, x, y, h, M, st) : h4_analysis(x, y, tables, B, T, F, M, L, flags, st);
+    if (e == 0 || (!h.in && e != PQMF_ERR_UNSUPPORTED)) return e;
+  }
+  const float* xf = static_cast<const float*>(x.rows());
+  float* yf = static_cast<float*>(y);
+  const int off = h.in ? L : L / 2;
+  if (fold_serves(x, h) && use_fast(M, L, tables, flags) && pqmf::hankel16_analysis_ok(xf, yf, T, F)) {
+    const int e = fast_analysis(xf, h.in, yf, h.out, tables, B, T, F, off, h.parity & 1, flags, st);
+    if (e != PQMF_ERR_UNSUPPORTED) return e;
+  }
+  if (!direct_serves(x, h)) return PQMF_ERR_UNSUPPORTED;
+  // streaming: the CTA of each row's last frame tile also rolls that row's history (no separate launch)
+  return analysis_direct(xf, h.in, yf, hk, B, T, F, M, L, off, h.parity, (!h.in && (flags & PQMF_FLAG_NO_SIGN)) ? 1 : 0, st, x.pcm, h.out,
+                         h.pool);
 }
-bool h4_route_synthesis(int B, long F, int M, int L, const float* tables, unsigned flags) {
-  const bool shape = F > 0 && (F & 3) == 0 && use_h4(B, F, M, nullptr);
-  if (use_fast(M, L, tables, flags)) return shape && !(flags & PQMF_FLAG_FOLD);
-  return !pqmf::hankel16_supported(M, L) && use_h4_family(M, L, tables, flags) && shape;
+
+// delay_frames: offline calls only
+int run_synthesis(const void* s, const Samples& out, const History& h, const float* hk, const float* tables, int B, long F, int M, int L,
+                  int delay_frames, unsigned flags, cudaStream_t st) {
+  pqmf::H4SynthesisStreamParams plan{};
+  const int off2 = h.in ? -M : L / 2 - delay_frames * M;
+  if (h4_takes_synthesis(s, out, h, B, F, M, L, tables, flags, &plan)) {
+    const int e = h.in ? h4_synthesis_stream(plan, s, out, h, M, st) : h4_synthesis(s, out, tables, B, F, off2, M, L, flags, st);
+    if (e == 0 || (!h.in && e != PQMF_ERR_UNSUPPORTED)) return e;
+  }
+  const float* sf = static_cast<const float*>(s);
+  float* of = static_cast<float*>(out.rows());
+  if (fold_serves(out, h) && use_fast(M, L, tables, flags) && pqmf::hankel16_synthesis_ok(sf, of, F)) {
+    const int e = fast_synthesis(sf, h.in, of, h.out, tables, B, F, off2, h.parity & 1, flags, st);
+    if (e != PQMF_ERR_UNSUPPORTED) return e;
+  }
+  if (!direct_serves(out, h)) return PQMF_ERR_UNSUPPORTED;
+  return synthesis_direct(sf, h.in, of, hk, B, F, M, L, off2, h.parity, (!h.in && (flags & PQMF_FLAG_NO_SIGN)) ? 1 : 0, st, out.pcm_out(),
+                          out.pcm.C, nullptr, h.out, h.pool);
 }
-// fp32 buffers: 256-bit signal loads / stores, 128-bit sub-band loads / stores
-bool h4_aligned_f32(const void* signal, const void* bands) { return ((uintptr_t)signal % 32) == 0 && ((uintptr_t)bands % 16) == 0; }
-// half-precision buffers: 128-bit signal loads / stores; 64-bit sub-band loads, up to 128-bit sub-band stores
-bool h4_aligned_half(const void* signal, const void* bands) { return (((uintptr_t)signal | (uintptr_t)bands) % 16) == 0; }
-// the half-precision instantiations exist for the unsplit banks, as CTA pairs
-bool half_analysis_native(const void* x, const void* y, int B, long T, long F, int M, int L, const float* tables, unsigned flags) {
-  return h4_route_analysis(B, T, F, M, L, tables, flags) && !(flags & PQMF_FLAG_H4_SPLIT) && h4_aligned_half(x, y);
-}
-bool half_synthesis_native(const void* s, const void* out, int B, long F, int M, int L, const float* tables, unsigned flags) {
-  return h4_route_synthesis(B, F, M, L, tables, flags) && !(flags & PQMF_FLAG_H4_SPLIT) && h4_aligned_half(out, s);
-}
+
 bool half_io_of(int dtype, pqmf::H4Io& io) {
   if (dtype == PQMF_DTYPE_F16) io = pqmf::H4Io::F16;
   else if (dtype == PQMF_DTYPE_BF16) io = pqmf::H4Io::BF16;
@@ -676,30 +726,10 @@ int roundtrip_host(const Sample* x_host, float* y_host, Sample* out_host, const 
   return rc;
 }
 
-// ---- stream pools.  The indexed Hankel-4 kernels exactly where a lockstep call with B = n runs the Hankel-4 streaming kernels (the
-//      routing decision of h4_*_stream); the indexed direct form everywhere else -- including few-stream n_band 16, where a lockstep
-//      call runs the fold kernels ----
-int pool_analysis(const float* x, float* y, const float* hk, const float* tables, float* xpool, const PoolRows& pool, int n, long T, int M, int L,
-                  unsigned flags, cudaStream_t st) {
-  if (h4_analysis_stream(x, y, tables, xpool, xpool, n, T, M, L, 0, flags, st, &pool) == 0) {
-    ++g_launches;
-    return 0;
-  }
-  return analysis_direct(x, xpool, y, hk, n, T, T / M, M, L, L, 0, 0, st, pqmf::PcmIn{nullptr, 1, 0}, xpool, &pool);
-}
-int pool_synthesis(const float* s, float* out, const float* hk, const float* tables, float* spool, const PoolRows& pool, int n, long F, int M, int L,
-                   unsigned flags, cudaStream_t st) {
-  if (h4_synthesis_stream(s, out, tables, spool, spool, n, F, M, L, 0, flags, st, &pool) == 0) {
-    ++g_launches;
-    return 0;
-  }
-  return synthesis_direct(s, spool, out, hk, n, F, M, L, -M, 0, 0, st, nullptr, 1, nullptr, spool, &pool);
-}
 // after the compute launches of a call: flip the half and advance the parity of every listed stream (one launch on the same stream)
 int pool_phase(const PoolRows& pool, int n, int* xphase, long x_frames, int* sphase, long s_frames, cudaStream_t st) {
   pqmf::stream_pool_phase_kernel<<<(n + 255) / 256, 256, 0, st>>>(pool.ids, n, pool.P, xphase, (int)(x_frames & 1), sphase, (int)(s_frames & 1));
-  ++g_launches;
-  return cuda_status();
+  return counted(cuda_status());
 }
 bool bad_pool(int P, int n) { return P < 1 || n < 0 || n > P; }
 
@@ -857,16 +887,7 @@ int pqmf_analysis_f32(const float* x, float* y, const float* hk, const float* ta
   if (bad_dims(B, T, M, L) || n_frames < 0) return PQMF_ERR_ARG;
   if (B == 0 || n_frames == 0) return PQMF_OK;
   if (!x || !y || !hk) return PQMF_ERR_ARG;
-  cudaStream_t st = (cudaStream_t)stream;
-  if (h4_route_analysis(B, T, n_frames, M, L, tables, flags) && h4_aligned_f32(x, y)) {
-    int e = h4_analysis(x, y, tables, B, T, n_frames, M, L, flags, st);
-    if (e != PQMF_ERR_UNSUPPORTED) { g_launches += (e == 0); return e; }
-  }
-  if (use_fast(M, L, tables, flags) && pqmf::hankel16_analysis_ok(x, y, T, n_frames)) {
-    int e = fast_analysis(x, nullptr, y, nullptr, tables, B, T, n_frames, L / 2, 0, flags, st);
-    if (e != PQMF_ERR_UNSUPPORTED) { g_launches += (e == 0); return e; }
-  }
-  return analysis_direct(x, nullptr, y, hk, B, T, n_frames, M, L, L / 2, 0, (flags & PQMF_FLAG_NO_SIGN) ? 1 : 0, st);
+  return run_analysis(samples(x), y, kOffline, hk, tables, B, T, n_frames, M, L, flags, (cudaStream_t)stream);
 }
 
 int pqmf_synthesis_f32(const float* s, float* out, const float* hk, const float* tables, int B, long n_frames, int M, int L,
@@ -874,17 +895,7 @@ int pqmf_synthesis_f32(const float* s, float* out, const float* hk, const float*
   if (bad_dims(B, n_frames, M, L) || delay_frames < 0 || delay_frames > 1) return PQMF_ERR_ARG;
   if (B == 0 || n_frames == 0) return PQMF_OK;
   if (!s || !out || !hk) return PQMF_ERR_ARG;
-  cudaStream_t st = (cudaStream_t)stream;
-  const int off2 = L / 2 - delay_frames * M;
-  if (h4_route_synthesis(B, n_frames, M, L, tables, flags) && h4_aligned_f32(out, s)) {
-    int e = h4_synthesis(s, out, tables, B, n_frames, off2, M, L, flags, st);
-    if (e != PQMF_ERR_UNSUPPORTED) { g_launches += (e == 0); return e; }
-  }
-  if (use_fast(M, L, tables, flags) && pqmf::hankel16_synthesis_ok(s, out, n_frames)) {
-    int e = fast_synthesis(s, nullptr, out, nullptr, tables, B, n_frames, off2, 0, flags, st);
-    if (e != PQMF_ERR_UNSUPPORTED) { g_launches += (e == 0); return e; }
-  }
-  return synthesis_direct(s, nullptr, out, hk, B, n_frames, M, L, off2, 0, (flags & PQMF_FLAG_NO_SIGN) ? 1 : 0, st);
+  return run_synthesis(s, samples(out), kOffline, hk, tables, B, n_frames, M, L, delay_frames, flags, (cudaStream_t)stream);
 }
 
 int pqmf_analysis_pcm16(const int16_t* pcm, float* y, const float* hk, const float* tables, int B, long T, int C, int downmix,
@@ -894,14 +905,7 @@ int pqmf_analysis_pcm16(const int16_t* pcm, float* y, const float* hk, const flo
   if (rows >= (1L << 31)) return PQMF_ERR_ARG;
   if (B == 0 || n_frames == 0) return PQMF_OK;
   if (!pcm || !y || !hk) return PQMF_ERR_ARG;
-  cudaStream_t st = (cudaStream_t)stream;
-  const pqmf::PcmIn in{pcm, C, downmix ? 1 : 0};
-  if (use_h4_family(M, L, tables, flags) && use_h4((int)rows, n_frames, M, nullptr) && T > 0 && (T % M) == 0 && (T % 8) == 0 && n_frames == T / M &&
-      ((uintptr_t)pcm % 32) == 0 && ((uintptr_t)y % 16) == 0) {
-    const int e = h4_analysis(nullptr, y, tables, (int)rows, T, n_frames, M, L, flags, st, in);
-    if (e != PQMF_ERR_UNSUPPORTED) { g_launches += (e == 0); return e; }
-  }
-  return analysis_direct(nullptr, nullptr, y, hk, (int)rows, T, n_frames, M, L, L / 2, 0, (flags & PQMF_FLAG_NO_SIGN) ? 1 : 0, st, in);
+  return run_analysis(pcm16(pcm, C, downmix), y, kOffline, hk, tables, (int)rows, T, n_frames, M, L, flags, (cudaStream_t)stream);
 }
 
 int pqmf_synthesis_pcm16(const float* s, int16_t* pcm, const float* hk, const float* tables, int B, int C, long n_frames, int M, int L,
@@ -911,14 +915,7 @@ int pqmf_synthesis_pcm16(const float* s, int16_t* pcm, const float* hk, const fl
   if (rows >= (1L << 31)) return PQMF_ERR_ARG;
   if (B == 0 || n_frames == 0) return PQMF_OK;
   if (!s || !pcm || !hk) return PQMF_ERR_ARG;
-  cudaStream_t st = (cudaStream_t)stream;
-  const int off2 = L / 2 - delay_frames * M;
-  if (use_h4_family(M, L, tables, flags) && use_h4((int)rows, n_frames, M, nullptr) && n_frames > 0 && (n_frames & 3) == 0 && ((uintptr_t)s % 16) == 0 &&
-      ((uintptr_t)pcm % 16) == 0) {
-    const int e = h4_synthesis(s, nullptr, tables, (int)rows, n_frames, off2, M, L, flags, st, pcm, C);
-    if (e != PQMF_ERR_UNSUPPORTED) { g_launches += (e == 0); return e; }
-  }
-  return synthesis_direct(s, nullptr, nullptr, hk, (int)rows, n_frames, M, L, off2, 0, (flags & PQMF_FLAG_NO_SIGN) ? 1 : 0, st, pcm, C);
+  return run_synthesis(s, pcm16(pcm, C), kOffline, hk, tables, (int)rows, n_frames, M, L, delay_frames, flags, (cudaStream_t)stream);
 }
 
 int pqmf_synthesis_bands_f32(const float* const* bands, const long* lens, float* out, const float* hk, int B, long n_frames, int M, int L,
@@ -946,8 +943,7 @@ int pqmf_synthesis_bands_f32(const float* const* bands, const long* lens, float*
     t.fade_in = fade_in;
     const int n = M * Lx;
     pqmf::band_tail_kernel<<<(n + 255) / 256, 256, 0, st>>>(t, M, tail_out);
-    ++g_launches;
-    if (int e = cuda_status()) return e;
+    if (int e = counted(cuda_status())) return e;
   } else if (fade) {
     cudaError_t e = cudaMemcpyAsync(tail_out, prev_tail, (size_t)M * Lx * sizeof(float), cudaMemcpyDeviceToDevice, st);
     if (e != cudaSuccess) return (int)e;
@@ -965,16 +961,8 @@ int pqmf_analysis_stream_f32(const float* x, float* y, const float* hk, const fl
   if (!hk || !state_in || !state_out || state_in == state_out) return PQMF_ERR_ARG;
   if (T == 0) return PQMF_ERR_ARG;
   if (!x || !y) return PQMF_ERR_ARG;
-  cudaStream_t st = (cudaStream_t)stream;
-  const long F = T / M;
   // many streams: the streaming Hankel-4 kernels (n_band 8 / 16 / 32); few n_band-16 streams: the fold kernels
-  if (h4_analysis_stream(x, y, tables, state_in, state_out, B, T, M, L, frame_parity, flags, st) == 0) { ++g_launches; return 0; }
-  if (use_fast(M, L, tables, flags) && pqmf::hankel16_analysis_ok(x, y, T, F)) {
-    int e = fast_analysis(x, state_in, y, state_out, tables, B, T, F, L, frame_parity & 1, flags, st);
-    if (e != PQMF_ERR_UNSUPPORTED) { g_launches += (e == 0); return e; }
-  }
-  // fp32 direct form; the CTA of each row's last frame tile also rolls that row's history (no separate launch)
-  return analysis_direct(x, state_in, y, hk, B, T, F, M, L, L, frame_parity, 0, st, pqmf::PcmIn{nullptr, 1, 0}, state_out);
+  return run_analysis(samples(x), y, lockstep(state_in, state_out, frame_parity), hk, tables, B, T, T / M, M, L, flags, (cudaStream_t)stream);
 }
 
 int pqmf_synthesis_stream_f32(const float* s, float* out, const float* hk, const float* tables, const float* state_in,
@@ -984,15 +972,8 @@ int pqmf_synthesis_stream_f32(const float* s, float* out, const float* hk, const
   if (B == 0) return PQMF_OK;
   if (!hk || !state_in || !state_out || state_in == state_out || n_frames == 0) return PQMF_ERR_ARG;
   if (!s || !out) return PQMF_ERR_ARG;
-  cudaStream_t st = (cudaStream_t)stream;
-  const int K = L / M;
   // history frames sit K frames before frame 0 of the block: their parity offset is (frame_parity - K)
-  if (h4_synthesis_stream(s, out, tables, state_in, state_out, B, n_frames, M, L, frame_parity, flags, st) == 0) { ++g_launches; return 0; }
-  if (use_fast(M, L, tables, flags) && pqmf::hankel16_synthesis_ok(s, out, n_frames)) {
-    int e = fast_synthesis(s, state_in, out, state_out, tables, B, n_frames, -M, frame_parity & 1, flags, st);
-    if (e != PQMF_ERR_UNSUPPORTED) { g_launches += (e == 0); return e; }
-  }
-  return synthesis_direct(s, state_in, out, hk, B, n_frames, M, L, -M, frame_parity, 0, st, nullptr, 1, nullptr, state_out);
+  return run_synthesis(s, samples(out), lockstep(state_in, state_out, frame_parity), hk, tables, B, n_frames, M, L, 0, flags, (cudaStream_t)stream);
 }
 
 int pqmf_stream_step_f32(const float* x, float* y, float* out, const float* hk, const float* tables, const float* xstate_in, float* xstate_out,
@@ -1016,7 +997,7 @@ int pqmf_stream_pool_analysis_f32(const float* x, float* y, const float* hk, con
   if (!x || !y || !hk || !xpool || !xphase || !ids) return PQMF_ERR_ARG;
   cudaStream_t st = (cudaStream_t)stream;
   const PoolRows pool{ids, xphase, P};
-  if (int e = pool_analysis(x, y, hk, tables, xpool, pool, n, T, M, L, flags, st)) return e;
+  if (int e = run_analysis(samples(x), y, pooled(xpool, pool), hk, tables, n, T, T / M, M, L, flags, st)) return e;
   return pool_phase(pool, n, xphase, T / M, nullptr, 0, st);
 }
 
@@ -1027,7 +1008,7 @@ int pqmf_stream_pool_synthesis_f32(const float* s, float* out, const float* hk, 
   if (!s || !out || !hk || !spool || !sphase || !ids) return PQMF_ERR_ARG;
   cudaStream_t st = (cudaStream_t)stream;
   const PoolRows pool{ids, sphase, P};
-  if (int e = pool_synthesis(s, out, hk, tables, spool, pool, n, n_frames, M, L, flags, st)) return e;
+  if (int e = run_synthesis(s, samples(out), pooled(spool, pool), hk, tables, n, n_frames, M, L, 0, flags, st)) return e;
   return pool_phase(pool, n, nullptr, 0, sphase, n_frames, st);
 }
 
@@ -1039,13 +1020,13 @@ int pqmf_stream_pool_step_f32(const float* x, float* y, float* out, const float*
   if (!x || !y || !out || !hk || !xpool || !xphase || !spool || !sphase || !ids || xphase == sphase) return PQMF_ERR_ARG;
   cudaStream_t st = (cudaStream_t)stream;
   const PoolRows xrows{ids, xphase, P}, srows{ids, sphase, P};
-  if (int e = pool_analysis(x, y, hk, tables, xpool, xrows, n, T, M, L, flags, st)) return e;
-  if (int e = pool_synthesis(y, out, hk, tables, spool, srows, n, T / M, M, L, flags, st)) return e;
+  if (int e = run_analysis(samples(x), y, pooled(xpool, xrows), hk, tables, n, T, T / M, M, L, flags, st)) return e;
+  if (int e = run_synthesis(y, samples(out), pooled(spool, srows), hk, tables, n, T / M, M, L, 0, flags, st)) return e;
   return pool_phase(xrows, n, xphase, T / M, sphase, T / M, st);
 }
 
 // ---- int16 PCM blocks in the streaming calls: the streaming Hankel-4 kernels with PCM loads (any channel count, optional down-mix) and
-//      mono PCM stores, exactly where the fp32 call with the same rows runs those kernels (h4_*_stream_ok, with the PCM buffer's alignment);
+//      mono PCM stores, exactly where the fp32 call with the same rows runs those kernels (h4_takes_*, with the PCM buffer's alignment);
 //      every other call returns PQMF_ERR_UNSUPPORTED before anything is launched and the caller stages it through the fp32 entry ----
 static bool pcm_args_bad(int C, long rows) { return C < 1 || C > 64 || rows >= (1L << 31); }
 
@@ -1055,11 +1036,8 @@ int pqmf_analysis_stream_pcm16(const int16_t* pcm, float* y, const float* hk, co
   if (bad_dims(B, T, M, L) || (T % M) != 0 || pcm_args_bad(C, rows)) return PQMF_ERR_ARG;
   if (B == 0) return PQMF_OK;
   if (!hk || !state_in || !state_out || state_in == state_out || T == 0 || !pcm || !y) return PQMF_ERR_ARG;
-  const pqmf::PcmIn in{pcm, C, downmix ? 1 : 0};
-  if (h4_analysis_stream(nullptr, y, tables, state_in, state_out, (int)rows, T, M, L, frame_parity, flags, (cudaStream_t)stream, nullptr, &in) != 0)
-    return PQMF_ERR_UNSUPPORTED;  // nothing was launched
-  ++g_launches;
-  return PQMF_OK;
+  return run_analysis(pcm16(pcm, C, downmix), y, lockstep(state_in, state_out, frame_parity), hk, tables, (int)rows, T, T / M, M, L, flags,
+                      (cudaStream_t)stream);
 }
 
 int pqmf_synthesis_stream_pcm16(const float* s, int16_t* pcm, const float* hk, const float* tables, const float* state_in, float* state_out, int B,
@@ -1068,11 +1046,8 @@ int pqmf_synthesis_stream_pcm16(const float* s, int16_t* pcm, const float* hk, c
   if (bad_dims(B, n_frames, M, L) || (L % M) != 0 || pcm_args_bad(C, rows)) return PQMF_ERR_ARG;
   if (B == 0) return PQMF_OK;
   if (!hk || !state_in || !state_out || state_in == state_out || n_frames == 0 || !s || !pcm) return PQMF_ERR_ARG;
-  if (C != 1 ||
-      h4_synthesis_stream(s, nullptr, tables, state_in, state_out, (int)rows, n_frames, M, L, frame_parity, flags, (cudaStream_t)stream, nullptr, pcm) != 0)
-    return PQMF_ERR_UNSUPPORTED;
-  ++g_launches;
-  return PQMF_OK;
+  return run_synthesis(s, pcm16(pcm, C), lockstep(state_in, state_out, frame_parity), hk, tables, (int)rows, n_frames, M, L, 0, flags,
+                       (cudaStream_t)stream);
 }
 
 int pqmf_stream_step_pcm16(const int16_t* pcm, float* y, int16_t* pcm_out, const float* hk, const float* tables, const float* xstate_in,
@@ -1084,21 +1059,15 @@ int pqmf_stream_step_pcm16(const int16_t* pcm, float* y, int16_t* pcm_out, const
   if (!pcm || !y || !pcm_out || !hk || !xstate_in || !xstate_out || !sstate_in || !sstate_out || xstate_in == xstate_out ||
       sstate_in == sstate_out)
     return PQMF_ERR_ARG;
-  // both directions native, or nothing is launched
-  pqmf::H4AnalysisStreamParams pa{};
-  pqmf::H4SynthesisStreamParams ps{};
-  if ((downmix == 0 && C != 1) || !h4_analysis_stream_ok((int)rows, T, M, L, tables, flags, pcm, y, xstate_in, xstate_out, pa) ||
-      !h4_synthesis_stream_ok((int)rows, T / M, M, L, tables, flags, y, pcm_out, true, sstate_in, sstate_out, ps))
+  // both directions native, or nothing is launched; the output rows are mono where the input is (one channel, or the down-mix)
+  const Samples in = pcm16(pcm, C, downmix), mono = pcm16(pcm_out, downmix ? 1 : C);
+  const History xh = lockstep(xstate_in, xstate_out, parity_in), sh = lockstep(sstate_in, sstate_out, parity_out);
+  if (!h4_takes_analysis(in, y, xh, (int)rows, T, T / M, M, L, tables, flags) || !h4_takes_synthesis(y, mono, sh, (int)rows, T / M, M, L, tables, flags))
     return PQMF_ERR_UNSUPPORTED;
   cudaStream_t st = (cudaStream_t)stream;
-  const pqmf::PcmIn in{pcm, C, downmix ? 1 : 0};
-  if (h4_analysis_stream(nullptr, y, tables, xstate_in, xstate_out, (int)rows, T, M, L, parity_in, flags, st, nullptr, &in) != 0)
-    return PQMF_ERR_UNSUPPORTED;  // the launch did not start: nothing ran
-  ++g_launches;
+  if (int e = run_analysis(in, y, xh, hk, tables, (int)rows, T, T / M, M, L, flags, st)) return e;  // the launch did not start: nothing ran
   // the analysis has run: a failed synthesis launch is an error, not a refusal (a staged retry would step the analysis state twice)
-  const int e = h4_synthesis_stream(y, nullptr, tables, sstate_in, sstate_out, (int)rows, T / M, M, L, parity_out, flags, st, nullptr, pcm_out);
-  if (e != 0) return e > 0 ? e : (int)cudaErrorLaunchFailure;
-  ++g_launches;
+  if (run_synthesis(y, mono, sh, hk, tables, (int)rows, T / M, M, L, 0, flags, st) != 0) return (int)cudaErrorLaunchFailure;
   return PQMF_OK;
 }
 
@@ -1110,9 +1079,7 @@ int pqmf_stream_pool_analysis_pcm16(const int16_t* pcm, float* y, const float* h
   if (!pcm || !y || !hk || !xpool || !xphase || !ids) return PQMF_ERR_ARG;
   cudaStream_t st = (cudaStream_t)stream;
   const PoolRows pool{ids, xphase, P};
-  const pqmf::PcmIn in{pcm, C, downmix ? 1 : 0};
-  if (h4_analysis_stream(nullptr, y, tables, xpool, xpool, (int)rows, T, M, L, 0, flags, st, &pool, &in) != 0) return PQMF_ERR_UNSUPPORTED;
-  ++g_launches;
+  if (int e = run_analysis(pcm16(pcm, C, downmix), y, pooled(xpool, pool), hk, tables, (int)rows, T, T / M, M, L, flags, st)) return e;
   return pool_phase(pool, (int)rows, xphase, T / M, nullptr, 0, st);
 }
 
@@ -1124,9 +1091,7 @@ int pqmf_stream_pool_synthesis_pcm16(const float* s, int16_t* pcm, const float* 
   if (!s || !pcm || !hk || !spool || !sphase || !ids) return PQMF_ERR_ARG;
   cudaStream_t st = (cudaStream_t)stream;
   const PoolRows pool{ids, sphase, P};
-  if (C != 1 || h4_synthesis_stream(s, nullptr, tables, spool, spool, (int)rows, n_frames, M, L, 0, flags, st, &pool, pcm) != 0)
-    return PQMF_ERR_UNSUPPORTED;
-  ++g_launches;
+  if (int e = run_synthesis(s, pcm16(pcm, C), pooled(spool, pool), hk, tables, (int)rows, n_frames, M, L, 0, flags, st)) return e;
   return pool_phase(pool, (int)rows, nullptr, 0, sphase, n_frames, st);
 }
 
@@ -1137,19 +1102,14 @@ int pqmf_stream_pool_step_pcm16(const int16_t* pcm, float* y, int16_t* pcm_out, 
   if (bad_dims(B, T, M, L) || pcm_args_bad(C, rows) || bad_pool(P, (int)rows) || T <= 0 || (T % M) != 0 || (L % M) != 0) return PQMF_ERR_ARG;
   if (B == 0) return PQMF_OK;
   if (!pcm || !y || !pcm_out || !hk || !xpool || !xphase || !spool || !sphase || !ids || xphase == sphase) return PQMF_ERR_ARG;
-  pqmf::H4AnalysisStreamParams pa{};
-  pqmf::H4SynthesisStreamParams ps{};
-  if ((downmix == 0 && C != 1) || !h4_analysis_stream_ok((int)rows, T, M, L, tables, flags, pcm, y, xpool, xpool, pa) ||
-      !h4_synthesis_stream_ok((int)rows, T / M, M, L, tables, flags, y, pcm_out, true, spool, spool, ps))
+  const PoolRows xrows{ids, xphase, P}, srows{ids, sphase, P};
+  const Samples in = pcm16(pcm, C, downmix), mono = pcm16(pcm_out, downmix ? 1 : C);
+  const History xh = pooled(xpool, xrows), sh = pooled(spool, srows);
+  if (!h4_takes_analysis(in, y, xh, (int)rows, T, T / M, M, L, tables, flags) || !h4_takes_synthesis(y, mono, sh, (int)rows, T / M, M, L, tables, flags))
     return PQMF_ERR_UNSUPPORTED;
   cudaStream_t st = (cudaStream_t)stream;
-  const PoolRows xrows{ids, xphase, P}, srows{ids, sphase, P};
-  const pqmf::PcmIn in{pcm, C, downmix ? 1 : 0};
-  if (h4_analysis_stream(nullptr, y, tables, xpool, xpool, (int)rows, T, M, L, 0, flags, st, &xrows, &in) != 0) return PQMF_ERR_UNSUPPORTED;
-  ++g_launches;
-  const int e = h4_synthesis_stream(y, nullptr, tables, spool, spool, (int)rows, T / M, M, L, 0, flags, st, &srows, pcm_out);
-  if (e != 0) return e > 0 ? e : (int)cudaErrorLaunchFailure;  // see pqmf_stream_step_pcm16
-  ++g_launches;
+  if (int e = run_analysis(in, y, xh, hk, tables, (int)rows, T, T / M, M, L, flags, st)) return e;
+  if (run_synthesis(y, mono, sh, hk, tables, (int)rows, T / M, M, L, 0, flags, st) != 0) return (int)cudaErrorLaunchFailure;  // see pqmf_stream_step_pcm16
   return pool_phase(xrows, (int)rows, xphase, T / M, sphase, T / M, st);
 }
 
@@ -1209,7 +1169,7 @@ int pqmf_reconstruct_f32(const float* x, float* out, float* scratch, size_t scra
 }
 
 // ---- half-precision I/O: the offline Hankel-4 kernels with fp16 / bf16 loads and stores (half_io.cuh), wherever the fp32 call
-//      would run them (h4_route_*); every other call is refused before anything is launched ----
+//      would run them (h4_takes_*); every other call is refused before anything is launched ----
 int pqmf_analysis_x(const void* x, void* y, const float* hk, const float* tables, int B, long T, long n_frames, int M, int L, unsigned flags,
                     int dtype, pqmf_stream_t stream) {
   if (dtype == PQMF_DTYPE_F32)
@@ -1218,10 +1178,7 @@ int pqmf_analysis_x(const void* x, void* y, const float* hk, const float* tables
   if (!half_io_of(dtype, io) || bad_dims(B, T, M, L) || n_frames < 0) return PQMF_ERR_ARG;
   if (B == 0 || n_frames == 0) return PQMF_OK;
   if (!x || !y || !hk) return PQMF_ERR_ARG;
-  if (!half_analysis_native(x, y, B, T, n_frames, M, L, tables, flags)) return PQMF_ERR_UNSUPPORTED;
-  const int e = h4_analysis(x, y, tables, B, T, n_frames, M, L, flags, (cudaStream_t)stream, pqmf::PcmIn{nullptr, 1, 0}, io);
-  g_launches += (e == 0);
-  return e;
+  return run_analysis(samples(x, io), y, kOffline, hk, tables, B, T, n_frames, M, L, flags, (cudaStream_t)stream);
 }
 
 int pqmf_synthesis_x(const void* s, void* out, const float* hk, const float* tables, int B, long n_frames, int M, int L, int delay_frames,
@@ -1232,10 +1189,7 @@ int pqmf_synthesis_x(const void* s, void* out, const float* hk, const float* tab
   if (!half_io_of(dtype, io) || bad_dims(B, n_frames, M, L) || delay_frames < 0 || delay_frames > 1) return PQMF_ERR_ARG;
   if (B == 0 || n_frames == 0) return PQMF_OK;
   if (!s || !out || !hk) return PQMF_ERR_ARG;
-  if (!half_synthesis_native(s, out, B, n_frames, M, L, tables, flags)) return PQMF_ERR_UNSUPPORTED;
-  const int e = h4_synthesis(s, out, tables, B, n_frames, L / 2 - delay_frames * M, M, L, flags, (cudaStream_t)stream, nullptr, 1, io);
-  g_launches += (e == 0);
-  return e;
+  return run_synthesis(s, samples(out, io), kOffline, hk, tables, B, n_frames, M, L, delay_frames, flags, (cudaStream_t)stream);
 }
 
 int pqmf_roundtrip_x(const void* x, void* y, void* out, const float* hk, const float* tables, int B, long T, long n_frames, int M, int L,
@@ -1248,7 +1202,8 @@ int pqmf_roundtrip_x(const void* x, void* y, void* out, const float* hk, const f
   if (B == 0 || n_frames == 0) return PQMF_OK;
   if (!x || !y || !out || !hk) return PQMF_ERR_ARG;
   // both directions native, or neither is launched
-  if (!half_analysis_native(x, y, B, T, n_frames, M, L, tables, flags) || !half_synthesis_native(y, out, B, n_frames, M, L, tables, flags))
+  if (!h4_takes_analysis(samples(x, io), y, kOffline, B, T, n_frames, M, L, tables, flags) ||
+      !h4_takes_synthesis(y, samples(out, io), kOffline, B, n_frames, M, L, tables, flags))
     return PQMF_ERR_UNSUPPORTED;
   const int e = pqmf_analysis_x(x, y, hk, tables, B, T, n_frames, M, L, flags, dtype, stream);
   if (e) return e;
@@ -1271,8 +1226,8 @@ int pqmf_reconstruct_x(const void* x, void* out, void* scratch, size_t scratch_b
   // every chunk native in both directions (a short last chunk may have too few tiles), or nothing is launched
   for (long r0 = 0; r0 < B; r0 += rows) {
     const int n = (int)(B - r0 < rows ? B - r0 : rows);
-    if (!half_analysis_native(xh + (size_t)r0 * T, scratch, n, T, n_frames, M, L, tables, flags) ||
-        !half_synthesis_native(scratch, oh + (size_t)r0 * M * n_frames, n, n_frames, M, L, tables, flags))
+    if (!h4_takes_analysis(samples(xh + (size_t)r0 * T, io), scratch, kOffline, n, T, n_frames, M, L, tables, flags) ||
+        !h4_takes_synthesis(scratch, samples(oh + (size_t)r0 * M * n_frames, io), kOffline, n, n_frames, M, L, tables, flags))
       return PQMF_ERR_UNSUPPORTED;
   }
   for (long r0 = 0; r0 < B; r0 += rows) {

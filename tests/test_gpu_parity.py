@@ -402,6 +402,38 @@ def test_hankel_other_prototype_lengths(pq, att, m):
     assert np.abs(oc[:, 0] - O.synthesis(s, hk, delay_frames=1)).max() <= tol
 
 
+@pytest.mark.parametrize("att,m,split", ((100, 64, True), (120, 32, True), (100, 32, False), (50, 64, False)))
+def test_launch_count_counts_both_tap_ranges_of_split_banks(lib, pq, att, m, split):
+    """pqmf_launch_count counts kernels: a split bank's two tap ranges are two launches per direction.  Its int16 synthesis stores
+    through the direct form (the second range accumulates, not in int16): one launch."""
+    mod = pq.PQMF(att, m).cuda()
+    assert bool(mod._flags & lib.PQMF_FLAG_H4_SPLIT) == split
+    hk, tab, L, fl = mod.hk.data_ptr(), mod._tables.data_ptr(), mod.hk.shape[1], mod._flags
+    b, t = 32, 32768  # 128 tiles of 8192 samples: the offline Hankel-4 kernels
+    f = t // m
+    torch.manual_seed(att + m)
+    x = (0.5 * torch.randn(b, t, device="cuda")).clamp_(-1, 1)
+    pcm = (x * 32767).to(torch.int16)
+    y = torch.empty(b, m, f, device="cuda")
+    out = torch.empty(b, t, device="cuda")
+    out16 = torch.empty(b, t, dtype=torch.int16, device="cuda")
+    c, st = lib.cabi, torch.cuda.current_stream().cuda_stream
+    calls = {
+        "analysis": lambda: c.pqmf_analysis_f32(x.data_ptr(), y.data_ptr(), hk, tab, b, t, f, m, L, fl, st),
+        "synthesis": lambda: c.pqmf_synthesis_f32(y.data_ptr(), out.data_ptr(), hk, tab, b, f, m, L, 0, fl, st),
+        "pcm_analysis": lambda: c.pqmf_analysis_pcm16(pcm.data_ptr(), y.data_ptr(), hk, tab, b, t, 1, 0, f, m, L, fl, st),
+        "pcm_synthesis": lambda: c.pqmf_synthesis_pcm16(y.data_ptr(), out16.data_ptr(), hk, tab, b, 1, f, m, L, 0, fl, st),
+    }
+    want = {"analysis": 2, "synthesis": 2, "pcm_analysis": 2, "pcm_synthesis": 1} if split else dict.fromkeys(calls, 1)
+    got = {}
+    for name, call in calls.items():
+        n0 = lib.launch_count()
+        rc = call()
+        got[name] = (rc, lib.launch_count() - n0)
+    torch.cuda.synchronize()
+    assert got == {name: (0, n) for name, n in want.items()}
+
+
 def test_cta_pair_and_single_cta_kernels_are_bit_identical(pq, lib):
     """PQMF_FLAG_NO_PAIR selects the one-CTA-per-SM launch of the same kernels: identical arithmetic, identical bits (odd tile
     counts exercise the pair's padding tile)."""
