@@ -499,13 +499,15 @@ bool h4_takes_analysis(const Samples& x, const void* y, const History& h, int B,
   if (h.in ? !h4_analysis_stream_plan(B, T, M, L, tables, flags, plan ? *plan : unused) : !h4_route_analysis(B, T, F, M, L, tables, flags)) return false;
   return aligned(x.p, pqmf::h4_io_half(x.io) ? 16 : 32) && aligned(y, 16) && aligned(h.in, 32) && aligned(h.out, 16);
 }
-// 256-bit fp32 output stores, 128-bit half and int16 stores; 128-bit sub-band loads and state accesses
+// 256-bit fp32 output stores, 128-bit half and mono int16 stores, 256-bit stores of interleaved stereo int16 frames (the offline duo
+// drain; h4_serves keeps stereo PCM output off the streaming kernels); 128-bit sub-band loads and state accesses
 bool h4_takes_synthesis(const void* s, const Samples& out, const History& h, int B, long F, int M, int L, const float* tables, unsigned flags,
                         pqmf::H4SynthesisStreamParams* plan = nullptr) {
   pqmf::H4SynthesisStreamParams unused{};
   if (!h4_serves(out, h, flags, true)) return false;
   if (h.in ? !h4_synthesis_stream_plan(B, F, M, L, tables, flags, plan ? *plan : unused) : !h4_route_synthesis(B, F, M, L, tables, flags)) return false;
-  return aligned(out.p, out.io == pqmf::H4Io::F32 ? 32 : 16) && aligned(s, 16) && aligned(h.in, 16) && aligned(h.out, 16);
+  const bool wide = out.io == pqmf::H4Io::F32 || (out.io == pqmf::H4Io::PCM && out.pcm.C == 2);
+  return aligned(out.p, wide ? 32 : 16) && aligned(s, 16) && aligned(h.in, 16) && aligned(h.out, 16);
 }
 
 // ---- one dispatcher per direction: the families in the order of the table above.  The offline Hankel-4 and the fold / Hankel-16
