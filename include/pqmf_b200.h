@@ -182,6 +182,33 @@ int pqmf_stream_pool_step_f32(const float* x, float* y, float* out, const float*
                               float* spool, int* sphase, int P, const int* ids, int n, long T, int M, int L, unsigned flags,
                               pqmf_stream_t stream);
 
+/* ---- grouped pool calls: sessions of different block lengths (a server whose clients choose their buffer sizes) stepped in one call.
+ *      A group is n rows of one block length T (samples): ids [n] (device int32), x [n, T], y [n, M, T/M], out [n, T].  The analysis reads
+ *      x and writes y, the synthesis reads y and writes out, the step does both; a pointer the direction does not use may be NULL.
+ *      Up to 8 groups per call; ids distinct across ALL groups, at most P rows in total; n == 0 groups are allowed; fp32 only.
+ *      Routing: the groups the streaming Hankel-4 kernels can plan (n_band 8 / 16 / 32, the block geometry, flags and alignment that a
+ *      single-group call would need, whatever their own tile count) run together in ONE launch per direction followed by one phase-word
+ *      launch, provided there are at least two of them and they make >= 96 tiles together (each direction, for a step).  Each of their rows
+ *      is what the streaming Hankel-4 POOL kernels give for it: pqmf_stream_pool_*_f32 of that group whenever that call runs those kernels.
+ *      Every other group runs through its pqmf_stream_pool_*_f32 entry with that entry's launches and bits.  G == 1 is that entry.  State
+ *      halves and phase words are updated as by the single-group entries, each group's parity advanced by its own T / M; streams not
+ *      listed are untouched.  All argument checks (PQMF_ERR_ARG) run on the host before anything is launched; G == 0 and all-empty
+ *      calls return 0. ---- */
+typedef struct pqmf_pool_group_f32 {
+  const int* ids;
+  int n;
+  long T;
+  const float* x;
+  float* y;
+  float* out;
+} pqmf_pool_group_f32;
+int pqmf_stream_pool_analysis_groups_f32(const pqmf_pool_group_f32* groups, int G, const float* hk, const float* tables, float* xpool, int* xphase,
+                                         int P, int M, int L, unsigned flags, pqmf_stream_t stream);
+int pqmf_stream_pool_synthesis_groups_f32(const pqmf_pool_group_f32* groups, int G, const float* hk, const float* tables, float* spool, int* sphase,
+                                          int P, int M, int L, unsigned flags, pqmf_stream_t stream);
+int pqmf_stream_pool_step_groups_f32(const pqmf_pool_group_f32* groups, int G, const float* hk, const float* tables, float* xpool, int* xphase,
+                                     float* spool, int* sphase, int P, int M, int L, unsigned flags, pqmf_stream_t stream);
+
 /* ---- int16 PCM blocks in the streaming calls (the PCM edge of pqmf_analysis_pcm16 / pqmf_synthesis_pcm16 on the streaming and pool entries
  *      above): what the reference's block driver streams (PitchShifterPvoc/2-TestBlocks.py:26-30) and what a server's sessions receive and
  *      return.  A PCM block is int16 interleaved WAV frames pcm [B, T, C]; widening is v / 32768 per channel, or with downmix != 0 the fp32

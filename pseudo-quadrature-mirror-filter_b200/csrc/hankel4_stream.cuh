@@ -13,7 +13,8 @@
 // is the next block of stream ids[r], whose phase word says which half holds its history and the parity of its next frame.  Each
 // MMA row reads only its own stream's region, so which streams share a tile changes nothing: only the addresses of the history and
 // of the roll, and the sign, come from ids and the phase word, loaded per tile one tile ahead with the block.  A row whose id is
-// outside [0, P) is dead: zeros in, zeros out, no state touched.
+// outside [0, P) is dead: zeros in, zeros out, no state touched.  The GROUPS kernels run a pool call of up to kPoolMaxGroups groups with
+// their own block lengths in one launch: each tile belongs to one group and has that group's region geometry (see below).
 //
 // int16 PCM edge (IO = H4Io::PCM, pcm.cuh): the analysis reads its block from interleaved WAV frames (any channel count, optional
 // down-mix) and the synthesis of mono rows writes int16 samples.  The history is the fp32 state in both directions: the analysis rolls
@@ -430,6 +431,285 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_stream_kernel(H
   } H4_TRACE(nullptr));
 }
 
+// ---- GROUPS: one pool launch over up to kPoolMaxGroups groups of rows with different block lengths (fp32, CTA pairs) ----
+// The tiles of the launch are the groups' tiles concatenated; every tile belongs to one group and has that group's region geometry
+// (the history rows are the same in every group: one bank, one H4Shape).  Each MMA row still reads only its own stream's region, so the
+// results of a group are those of the POOL instantiation on its rows.  A CTA's tile index only grows: a group cursor advances by
+// comparison, and the per-thread plan (the POOL kernels' tile-invariant plan) is rebuilt when a tile enters a new group -- at most G - 1
+// times per CTA.  Block addresses are made per tile from the row index.  The drain runs two tile loads behind the load, so the drained
+// tile's output row (pointer, frame stride, first frame, parity) travels through load -> convert -> drain with the tile.
+struct H4StreamGroup {
+  const int* ids;   // [n] stream of each row
+  const float* in;  // analysis: x [n, T]; synthesis: s [n, M, F]
+  float* out;       // analysis: y [n, M, F]; synthesis: out [n, M F]
+  long len;         // analysis: T; synthesis: F
+  int n;
+  int tile0;        // first tile of the group in the launch
+  H4StreamGeom s;
+};
+struct H4AnalysisStreamGroupsParams : H4AnalysisStreamPoolParams {
+  int G;
+  H4StreamGroup grp[kPoolMaxGroups];
+};
+struct H4SynthesisStreamGroupsParams : H4SynthesisStreamPoolParams {
+  int G;
+  H4StreamGroup grp[kPoolMaxGroups];
+};
+
+// the group of `tile`, from the group k of an earlier tile of the same CTA (tiles only grow); tiles past the last group (the second CTA
+// of a pair at the end) stay in the last group and have no live rows
+template <typename Params>
+__device__ __forceinline__ int h4_group_of(const Params& p, int k, long tile) {
+  while (k + 1 < p.G && tile >= p.grp[k + 1].tile0) ++k;
+  return k;
+}
+// region rows of the group with the fewest: rows past them are read only by MMA rows whose results are never stored
+template <typename Params>
+__device__ __forceinline__ int h4_groups_min_region_rows(const Params& p) {
+  int rows = kH4Rows;
+  for (int k = 0; k < p.G; ++k) rows = min(rows, p.grp[k].s.spt * p.grp[k].s.pitch);
+  return rows;
+}
+
+template <int M>
+__global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_stream_groups_kernel(H4AnalysisStreamGroupsParams p) {
+  h4_kernel<true, kH4Workers>(p.g, p.bank, p.n_tiles, 1u, p.pad_bytes, p.trim_lo, p.trim_hi, [&](const H4Smem& sm, uint32_t tmem, uint32_t pfull_leader, unsigned n_iter) {
+    constexpr int FR = 64 / M, HB = M / 2;
+    constexpr int NO = (kH4Rows * 8 + kH4Workers - 1) / kH4Workers;
+    const H4Shape& g = p.g;
+    const int tid = threadIdx.x;
+    // made finite once, below the smallest region span over the groups: a tile of a group with more region rows overwrites them with
+    // finite samples, which stay finite for the tiles after it
+    for (int u = h4_groups_min_region_rows(p) * 32 + tid; u < g.rows * 32; u += kH4Workers)
+#pragma unroll
+      for (int pl = 0; pl < 4; ++pl) reinterpret_cast<float*>(sm.planes + pl * g.plane)[u] = 0.f;
+    // the plan of the POOL kernel for group gi: slot, offset in the history row / in the block row / in the next history (-1: none)
+    constexpr int kDead = 1 << 20;
+    int gi = -1, n_octs = 0;
+    int q_slot[NO], hofs[NO], bofs[NO], rofs[NO];
+    auto plan = [&](int k) {
+      const H4StreamGeom sg = p.grp[k].s;
+      const long T = p.grp[k].len;
+      const int region_octs = sg.pitch * 8;
+      n_octs = sg.spt * region_octs;
+#pragma unroll
+      for (int r = 0; r < NO; ++r) {
+        const int u = tid + kH4Workers * r;
+        q_slot[r] = kDead;
+        hofs[r] = bofs[r] = rofs[r] = -1;
+        if (u < n_octs) {
+          const int t = u / region_octs, w = u - t * region_octs, q = w >> 3, col = w & 7;
+          if (q < sg.hrows) {
+            q_slot[r] = t;
+            hofs[r] = (p.L - sg.hrows * 64) + q * 64 + 8 * col;
+          } else if (q - sg.hrows < sg.rows_b) {
+            const long off = (q - sg.hrows) * 64 + 8 * col;
+            q_slot[r] = t;
+            bofs[r] = (int)off;
+            if (off >= T - p.L) rofs[r] = (int)(off - (T - p.L));
+          }
+        }
+      }
+    };
+    struct DrainRow {
+      float* y;  // this thread's first output of the tile (nullptr: not a stored row)
+      int F, eq, parity;
+    };
+    DrainRow d_ld{nullptr, 0, 0, 0}, d_cur = d_ld, d_prev = d_ld;  // of the loaded / converted / drained tile
+    float xr[NO][8];
+    float* roll[NO];
+    const int di = tid & 127, hb = tid >> 7;
+    auto load_tile = [&](long tile) {
+      const int k = h4_group_of(p, gi < 0 ? 0 : gi, tile);
+      if (k != gi) {
+        gi = k;
+        plan(k);
+      }
+      const H4StreamGroup& gr = p.grp[gi];
+      const H4StreamGeom sg = gr.s;
+      const long row0 = (tile - gr.tile0) * sg.spt;
+      const int nlive = (int)min((long)sg.spt, (long)gr.n - row0);
+      int id[NO], ph[NO];
+#pragma unroll
+      for (int r = 0; r < NO; ++r) {
+        id[r] = q_slot[r] < nlive ? __ldg(gr.ids + row0 + q_slot[r]) : -1;
+        if ((unsigned)id[r] >= (unsigned)p.pool.P) id[r] = -1;
+      }
+      const int dt = di / sg.pitch, dq = di - dt * sg.pitch;
+      const bool stored = dt < sg.spt && dq < sg.rows_b && dt < nlive;
+      int did = stored ? __ldg(gr.ids + row0 + dt) : -1;
+      if ((unsigned)did >= (unsigned)p.pool.P) did = -1;
+#pragma unroll
+      for (int r = 0; r < NO; ++r) ph[r] = id[r] >= 0 ? __ldg(p.pool.phase + id[r]) : 0;
+      const int F = (int)(gr.len / M);
+      d_ld.y = stored ? gr.out + ((size_t)(row0 + dt) * M + HB * hb) * F + FR * dq : nullptr;
+      d_ld.F = F;
+      d_ld.eq = dq;
+      d_ld.parity = did >= 0 ? (__ldg(p.pool.phase + did) >> 1) & 1 : 0;
+#pragma unroll
+      for (int r = 0; r < NO; ++r) {
+        const size_t row = (size_t)id[r];
+        if (id[r] < 0) {
+#pragma unroll
+          for (int e = 0; e < 8; ++e) xr[r][e] = 0.f;
+        } else if (hofs[r] >= 0) {
+          ptx::ldg256_na(p.hist_in + ((size_t)(ph[r] & 1) * p.pool.P + row) * p.L + hofs[r], xr[r]);
+        } else {
+          ptx::ldg256_na(gr.in + (size_t)(row0 + q_slot[r]) * gr.len + bofs[r], xr[r]);
+        }
+        roll[r] = (rofs[r] >= 0 && id[r] >= 0) ? p.hist_out + ((size_t)(~ph[r] & 1) * p.pool.P + row) * p.L + rofs[r] : nullptr;
+      }
+    };
+    auto convert = [&](int pb) {
+      unsigned char* p1 = sm.planes + (2 * pb) * g.plane;
+      d_cur = d_ld;
+#pragma unroll
+      for (int r = 0; r < NO; ++r) {
+        const int u = tid + kH4Workers * r;
+        if (u < n_octs) {
+          h4_split_store8(xr[r], p1, g.plane, sw128_offset((uint32_t)u * 16u));
+          if (roll[r] != nullptr) {
+            *reinterpret_cast<float4*>(roll[r]) = make_float4(xr[r][0], xr[r][1], xr[r][2], xr[r][3]);
+            *reinterpret_cast<float4*>(roll[r] + 4) = make_float4(xr[r][4], xr[r][5], xr[r][6], xr[r][7]);
+          }
+        }
+      }
+    };
+    auto drain = [&](int dbuf) {
+      float v[FR][HB];
+      h4_drain_analysis<M>(tmem, dbuf, tid, d_prev.eq, d_prev.parity, v);
+      if (d_prev.y == nullptr) return;
+#pragma unroll
+      for (int kk = 0; kk < HB; ++kk) {
+        float w[FR];
+#pragma unroll
+        for (int dl = 0; dl < FR; ++dl) w[dl] = v[dl][kk];
+        float* q = d_prev.y + (size_t)kk * d_prev.F;
+        if constexpr (FR >= 4) {
+#pragma unroll
+          for (int d4 = 0; d4 < FR; d4 += 4) __stcs(reinterpret_cast<float4*>(q + d4), make_float4(w[d4], w[d4 + 1], w[d4 + 2], w[d4 + 3]));
+        } else if constexpr (FR == 2) {
+          __stcs(reinterpret_cast<float2*>(q), make_float2(w[0], w[1]));
+        } else {
+          __stcs(q, w[0]);
+        }
+      }
+    };
+
+    long tile = blockIdx.x;
+    load_tile(tile);
+    h4_worker_loop<true>(sm, pfull_leader, n_iter, tid, convert, [&] { load_tile(tile + gridDim.x); }, drain, [&] {
+      tile += gridDim.x;
+      d_prev = d_cur;
+    } H4_TRACE(nullptr));
+  } H4_TRACE(nullptr));
+}
+
+template <int M>
+__global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_stream_groups_kernel(H4SynthesisStreamGroupsParams p) {
+  h4_kernel<true, kH4SynWorkers>(p.g, p.bank, p.n_tiles, 1u, p.pad_bytes, p.trim_lo, p.trim_hi, [&](const H4Smem& sm, uint32_t tmem, uint32_t pfull_leader, unsigned n_iter) {
+    constexpr int FR = 64 / M, NBG = M / 8;
+    const H4Shape& g = p.g;
+    const int tid = threadIdx.x, warp = tid >> 5;
+    for (int u = h4_groups_min_region_rows(p) * 32 + tid; u < g.rows * 32; u += kH4SynWorkers)
+#pragma unroll
+      for (int pl = 0; pl < 4; ++pl) reinterpret_cast<float*>(sm.planes + pl * g.plane)[u] = 0.f;
+    // the plan of the POOL kernel for group gi: item (frame quad wq, band group bg), its slot, and the offsets of its eight band rows in the
+    // history row / the block row / the next history (-1: none)
+    constexpr int kDead = 1 << 20;
+    int gi = -1, wq = 0, bg = 0, slot = kDead, hofs = -1, sofs = -1, rofs = -1;
+    bool has_item = false;
+    size_t src_pitch = 0;
+    auto plan = [&](int k) {
+      const H4StreamGeom sg = p.grp[k].s;
+      const long F = p.grp[k].len;
+      const int n_fq = sg.spt * sg.pitch * FR / 4;
+      bg = tid / n_fq;
+      wq = tid - bg * n_fq;
+      has_item = tid < NBG * n_fq;
+      const int region_frames = sg.pitch * FR, hist_fr = sg.hrows * FR, block_fr = sg.rows_b * FR;
+      const int lt = (4 * wq) / region_frames, lf = 4 * wq - lt * region_frames, fb = lf - hist_fr;
+      slot = kDead;
+      hofs = sofs = rofs = -1;
+      src_pitch = 0;
+      if (has_item) {
+        if (fb < 0) {
+          slot = lt;
+          hofs = 8 * bg * p.K + (p.K - hist_fr) + lf;
+          src_pitch = (size_t)p.K;
+        } else if (fb < block_fr) {
+          slot = lt;
+          sofs = (int)(8 * bg * F + fb);
+          src_pitch = (size_t)F;
+          if (fb >= F - p.K) rofs = (int)(8 * bg * p.K + (fb - (F - p.K)));
+        }
+      }
+    };
+    float4 v[8];
+    float* roll = nullptr;
+    uint32_t flip_ld = 0;
+    float* o_ld = nullptr;  // this thread's first output of the loaded / converted / drained tile (nullptr: not a stored row)
+    float* o_cur = nullptr;
+    float* o_prev = nullptr;
+    const int i0 = (tid & 127) & ~3, hb = tid >> 7, lane = tid & 31;
+    auto load_tile = [&](long tile) {
+      const int k = h4_group_of(p, gi < 0 ? 0 : gi, tile);
+      if (k != gi) {
+        gi = k;
+        plan(k);
+      }
+      const H4StreamGroup& gr = p.grp[gi];
+      const H4StreamGeom sg = gr.s;
+      const long row0 = (tile - gr.tile0) * sg.spt;
+      const int nlive = (int)min((long)sg.spt, (long)gr.n - row0);
+      int id = slot < nlive ? __ldg(gr.ids + row0 + slot) : -1;
+      if ((unsigned)id >= (unsigned)p.pool.P) id = -1;
+      const int ph = id >= 0 ? __ldg(p.pool.phase + id) : 0;
+      const float* from = hofs >= 0 ? p.state_in + ((size_t)(ph & 1) * p.pool.P + (size_t)id) * M * p.K + hofs
+                                    : gr.in + (size_t)(row0 + slot) * M * gr.len + sofs;
+#pragma unroll
+      for (int kk = 0; kk < 8; ++kk)
+        v[kk] = id >= 0 ? ptx::ldg128_na(reinterpret_cast<const float4*>(from + (size_t)kk * src_pitch)) : make_float4(0.f, 0.f, 0.f, 0.f);
+      roll = (rofs >= 0 && id >= 0) ? p.state_out + ((size_t)(~ph & 1) * p.pool.P + (size_t)id) * M * p.K + rofs : nullptr;
+      flip_ld = (ph & 2) ? 0u : 0x80000000u;
+      // pitch and rows_b are multiples of 4: the four rows of a lane quad belong to one region and are stored or not together
+      const int et = i0 / sg.pitch, eq0 = i0 - et * sg.pitch;
+      const bool stored = warp < 8 && et < sg.spt && eq0 < sg.rows_b && et < nlive;
+      o_ld = stored ? gr.out + (size_t)(row0 + et) * (size_t)(gr.len * M) + 64 * eq0 + 32 * hb + 8 * (lane & 3) : nullptr;
+    };
+    auto convert = [&](int pb) {
+      o_cur = o_ld;
+      if (!has_item) return;
+      unsigned char* p1 = sm.planes + (2 * pb) * g.plane;
+      if (roll != nullptr) {
+#pragma unroll
+        for (int kk = 0; kk < 8; ++kk) *reinterpret_cast<float4*>(roll + (size_t)kk * p.K) = v[kk];
+      }
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        float w[8];
+        h4_synthesis_chunk8(v, j, (j & 1) ? flip_ld ^ 0x80000000u : flip_ld, w);
+        h4_split_store8(w, p1, g.plane, sw128_offset((uint32_t)(4 * wq + j) * (2u * M) + 16u * bg));
+      }
+    };
+    auto drain = [&](int dbuf) {
+      if (warp >= 8) return;  // every worker waited for the MMAs; the ninth warp has no TMEM rows to drain
+      float val[4][8];
+      h4_drain_synthesis(tmem, dbuf, tid, val);
+      if (o_prev == nullptr) return;
+#pragma unroll
+      for (int q = 0; q < 4; ++q) ptx::stg256_cs(o_prev + (size_t)q * 64, val[q]);
+    };
+
+    long tile = blockIdx.x;
+    load_tile(tile);
+    h4_worker_loop<true>(sm, pfull_leader, n_iter, tid, convert, [&] { load_tile(tile + gridDim.x); }, drain, [&] {
+      tile += gridDim.x;
+      o_prev = o_cur;
+    } H4_TRACE(nullptr));
+  } H4_TRACE(nullptr));
+}
+
 // launches (CTA pairs; on any error the caller runs other kernels: the fold kernels, or the direct form for pools).  The instantiation
 // follows the call: POOL when pool != nullptr, and the sample format io, F32 or PCM (in: the WAV frames; pcm_out: the mono rows)
 template <int M, bool POOL, H4Io IO>
@@ -462,6 +742,17 @@ inline int h4_launch_synthesis_stream(const H4SynthesisStreamParams& p, const St
   if (io == H4Io::PCM)
     return pool ? h4_launch_synthesis_stream<M, true, H4Io::PCM>(p, pool, pcm_out, st) : h4_launch_synthesis_stream<M, false, H4Io::PCM>(p, pool, pcm_out, st);
   return pool ? h4_launch_synthesis_stream<M, true, H4Io::F32>(p, pool, pcm_out, st) : h4_launch_synthesis_stream<M, false, H4Io::F32>(p, pool, pcm_out, st);
+}
+// GROUPS: p.n_tiles, p.G and p.grp[] filled by the caller
+template <int M>
+inline int h4_launch_analysis_stream_groups(const H4AnalysisStreamGroupsParams& p, cudaStream_t st) {
+  static H4Configured configured;
+  return h4_launch<true>(h4_analysis_stream_groups_kernel<M>, p, kH4Threads, configured, st);
+}
+template <int M>
+inline int h4_launch_synthesis_stream_groups(const H4SynthesisStreamGroupsParams& p, cudaStream_t st) {
+  static H4Configured configured;
+  return h4_launch<true>(h4_synthesis_stream_groups_kernel<M>, p, kH4SynThreads, configured, st);
 }
 
 }  // namespace pqmf

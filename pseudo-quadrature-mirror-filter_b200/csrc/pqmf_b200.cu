@@ -363,8 +363,12 @@ bool h4_stream_family(int M, int L, const float* tables, unsigned flags) {
   if (use_fast(M, L, tables, flags)) return true;  // n_band 16 / L 512
   return !pqmf::hankel16_supported(M, L) && use_h4_family(M, L, tables, flags) && (M == 8 || M == 32);
 }
-// p: everything but the buffers and the parity
-bool h4_analysis_stream_plan(int B, long T, int M, int L, const float* tables, unsigned flags, pqmf::H4AnalysisStreamParams& p) {
+// the streaming Hankel-4 kernels take a call of at least this many tiles (a grouped pool call: its grouped groups together)
+constexpr long kH4StreamMinTiles = 96;
+long h4_stream_tiles(int B, const pqmf::H4StreamGeom& sg) { return (B + sg.spt - 1) / sg.spt; }
+// p: everything but the buffers and the parity.  min_tiles: the tile count the call must reach on its own
+bool h4_analysis_stream_plan(int B, long T, int M, int L, const float* tables, unsigned flags, pqmf::H4AnalysisStreamParams& p,
+                             long min_tiles = kH4StreamMinTiles) {
   if (!h4_stream_family(M, L, tables, flags)) return false;
   int jlo, kt;
   h4_taps(flags, jlo, kt);
@@ -374,7 +378,7 @@ bool h4_analysis_stream_plan(int B, long T, int M, int L, const float* tables, u
   const int hist = ((L - jlo + 63) / 64) * 64;
   if (hist > L || T % 256 != 0 || T < L || L % 8 != 0) return false;
   const pqmf::H4StreamGeom sg = pqmf::h4_stream_geom(T, hist);
-  if (sg.pitch > pqmf::kH4Rows || sg.spt < 1 || (B + sg.spt - 1) / sg.spt < 96) return false;
+  if (sg.pitch > pqmf::kH4Rows || sg.spt < 1 || h4_stream_tiles(B, sg) < min_tiles) return false;
   p.T = T; p.B = B; p.L = L;
   p.trim_lo = p.trim_hi = (flags & PQMF_FLAG_EXACT) ? 0 : (int)PQMF_FLAG_H4_TRIM_A(flags);
   p.pad_bytes = 2 * (hist - (L - jlo));
@@ -383,7 +387,8 @@ bool h4_analysis_stream_plan(int B, long T, int M, int L, const float* tables, u
   p.bank = reinterpret_cast<const uint16_t*>(tables + h4_pair_offset(M, L));
   return pqmf::h4_shape_fits(p.g);
 }
-bool h4_synthesis_stream_plan(int B, long F, int M, int L, const float* tables, unsigned flags, pqmf::H4SynthesisStreamParams& p) {
+bool h4_synthesis_stream_plan(int B, long F, int M, int L, const float* tables, unsigned flags, pqmf::H4SynthesisStreamParams& p,
+                              long min_tiles = kH4StreamMinTiles) {
   if (!h4_stream_family(M, L, tables, flags)) return false;
   int jlo, kt;
   h4_taps(flags, jlo, kt);
@@ -394,7 +399,7 @@ bool h4_synthesis_stream_plan(int B, long F, int M, int L, const float* tables, 
   const int hist_frames = ((taps_frames * M + 63) / 64) * 64 / M;
   if (hist_frames % 4 != 0 || hist_frames > K || (F * M) % 256 != 0 || F % 4 != 0 || F < K) return false;
   const pqmf::H4StreamGeom sg = pqmf::h4_stream_geom(F * M, hist_frames * M);
-  if (sg.pitch > pqmf::kH4Rows || sg.spt < 1 || (B + sg.spt - 1) / sg.spt < 96) return false;
+  if (sg.pitch > pqmf::kH4Rows || sg.spt < 1 || h4_stream_tiles(B, sg) < min_tiles) return false;
   p.F = F; p.B = B; p.K = K;
   p.trim_lo = p.trim_hi = (flags & PQMF_FLAG_EXACT) ? 0 : (int)PQMF_FLAG_H4_TRIM_S(flags);
   p.pad_bytes = 2 * M * (hist_frames - taps_frames);
@@ -493,19 +498,21 @@ bool aligned(const void* p, int bytes) { return (uintptr_t)p % bytes == 0; }
 // 256-bit fp32 and PCM signal loads (PCM: 16-byte mono, 32-byte stereo loads), 128-bit half signal loads; 128-bit sub-band stores;
 // 256-bit loads of the streaming history, 128-bit rolls
 bool h4_takes_analysis(const Samples& x, const void* y, const History& h, int B, long T, long F, int M, int L, const float* tables, unsigned flags,
-                       pqmf::H4AnalysisStreamParams* plan = nullptr) {
+                       pqmf::H4AnalysisStreamParams* plan = nullptr, long min_tiles = kH4StreamMinTiles) {
   pqmf::H4AnalysisStreamParams unused{};
   if (!h4_serves(x, h, flags, false)) return false;
-  if (h.in ? !h4_analysis_stream_plan(B, T, M, L, tables, flags, plan ? *plan : unused) : !h4_route_analysis(B, T, F, M, L, tables, flags)) return false;
+  if (h.in ? !h4_analysis_stream_plan(B, T, M, L, tables, flags, plan ? *plan : unused, min_tiles) : !h4_route_analysis(B, T, F, M, L, tables, flags))
+    return false;
   return aligned(x.p, pqmf::h4_io_half(x.io) ? 16 : 32) && aligned(y, 16) && aligned(h.in, 32) && aligned(h.out, 16);
 }
 // 256-bit fp32 output stores, 128-bit half and mono int16 stores, 256-bit stores of interleaved stereo int16 frames (the offline duo
 // drain; h4_serves keeps stereo PCM output off the streaming kernels); 128-bit sub-band loads and state accesses
 bool h4_takes_synthesis(const void* s, const Samples& out, const History& h, int B, long F, int M, int L, const float* tables, unsigned flags,
-                        pqmf::H4SynthesisStreamParams* plan = nullptr) {
+                        pqmf::H4SynthesisStreamParams* plan = nullptr, long min_tiles = kH4StreamMinTiles) {
   pqmf::H4SynthesisStreamParams unused{};
   if (!h4_serves(out, h, flags, true)) return false;
-  if (h.in ? !h4_synthesis_stream_plan(B, F, M, L, tables, flags, plan ? *plan : unused) : !h4_route_synthesis(B, F, M, L, tables, flags)) return false;
+  if (h.in ? !h4_synthesis_stream_plan(B, F, M, L, tables, flags, plan ? *plan : unused, min_tiles) : !h4_route_synthesis(B, F, M, L, tables, flags))
+    return false;
   const bool wide = out.io == pqmf::H4Io::F32 || (out.io == pqmf::H4Io::PCM && out.pcm.C == 2);
   return aligned(out.p, wide ? 32 : 16) && aligned(s, 16) && aligned(h.in, 16) && aligned(h.out, 16);
 }
@@ -734,6 +741,169 @@ int pool_phase(const PoolRows& pool, int n, int* xphase, long x_frames, int* sph
   return counted(cuda_status());
 }
 bool bad_pool(int P, int n) { return P < 1 || n < 0 || n > P; }
+
+// ---- grouped pool calls (pqmf_stream_pool_*_groups_f32): groups of rows with their own block lengths.  One rule: the groups the
+//      streaming Hankel-4 kernels can plan (h4_takes_*, family, plan and alignment, apart from the tile count) run together in one GROUPS
+//      launch per direction and one phase-word launch, when there are at least two of them and they reach kH4StreamMinTiles together
+//      (in both directions for a step).  Every other group runs through its single-group pool entry, with exactly that entry's launches ----
+enum class PoolDir { kAnalysis, kSynthesis, kStep };
+
+struct PoolGroupsCall {
+  PoolDir dir;
+  const pqmf_pool_group_f32* groups;
+  int G;
+  const float* hk;
+  const float* tables;
+  float *xpool, *spool;
+  int *xphase, *sphase;
+  int P, M, L;
+  unsigned flags;
+  cudaStream_t st;
+  bool analysis() const { return dir != PoolDir::kSynthesis; }
+  bool synthesis() const { return dir != PoolDir::kAnalysis; }
+};
+
+int pool_group_alone(const PoolGroupsCall& c, const pqmf_pool_group_f32& g) {
+  if (g.n == 0) return PQMF_OK;
+  pqmf_stream_t s = (pqmf_stream_t)c.st;
+  switch (c.dir) {
+    case PoolDir::kAnalysis:
+      return pqmf_stream_pool_analysis_f32(g.x, g.y, c.hk, c.tables, c.xpool, c.xphase, c.P, g.ids, g.n, g.T, c.M, c.L, c.flags, s);
+    case PoolDir::kSynthesis:
+      return pqmf_stream_pool_synthesis_f32(g.y, g.out, c.hk, c.tables, c.spool, c.sphase, c.P, g.ids, g.n, g.T / c.M, c.M, c.L, c.flags, s);
+    default:
+      return pqmf_stream_pool_step_f32(g.x, g.y, g.out, c.hk, c.tables, c.xpool, c.xphase, c.spool, c.sphase, c.P, g.ids, g.n, g.T, c.M, c.L,
+                                       c.flags, s);
+  }
+}
+
+template <typename Params>
+int h4_launch_stream_groups(const Params& p, int M, cudaStream_t st) {
+  int e = PQMF_ERR_UNSUPPORTED;
+  if constexpr (std::is_same_v<Params, pqmf::H4AnalysisStreamGroupsParams>) {
+    switch (M) {
+      case 8: e = pqmf::h4_launch_analysis_stream_groups<8>(p, st); break;
+      case 16: e = pqmf::h4_launch_analysis_stream_groups<16>(p, st); break;
+      case 32: e = pqmf::h4_launch_analysis_stream_groups<32>(p, st); break;
+    }
+  } else {
+    switch (M) {
+      case 8: e = pqmf::h4_launch_synthesis_stream_groups<8>(p, st); break;
+      case 16: e = pqmf::h4_launch_synthesis_stream_groups<16>(p, st); break;
+      case 32: e = pqmf::h4_launch_synthesis_stream_groups<32>(p, st); break;
+    }
+  }
+  if (e != 0) (void)cudaGetLastError();
+  return counted(e);
+}
+
+// the GROUPS launches of the groups in `joins`, planned in ap / sp, then one phase-word launch.  started: false when the first launch did
+// not start (nothing was launched: the caller runs the groups alone)
+int pool_groups_launch(const PoolGroupsCall& c, const bool* joins, const pqmf::H4AnalysisStreamParams* ap, const pqmf::H4SynthesisStreamParams* sp,
+                       bool& started) {
+  started = false;
+  pqmf::StreamPoolPhaseGroups phase{};
+  int first = -1;
+  for (int k = 0; k < c.G; ++k) {
+    if (!joins[k]) continue;
+    const pqmf_pool_group_f32& g = c.groups[k];
+    if (first < 0) first = k;
+    phase.ids[phase.G] = g.ids;
+    phase.adv[phase.G] = (int)((g.T / c.M) & 1);
+    phase.row0[phase.G + 1] = phase.row0[phase.G] + g.n;
+    ++phase.G;
+  }
+  // the bank, flags and history rows are the same for every group: the H4Shape, trims and pad of the first one hold for all
+  if (c.analysis()) {
+    pqmf::H4AnalysisStreamGroupsParams p{};
+    static_cast<pqmf::H4AnalysisStreamParams&>(p) = ap[first];
+    p.hist_in = p.hist_out = c.xpool;
+    p.pool = PoolRows{nullptr, c.xphase, c.P};
+    long tiles = 0;
+    for (int k = 0; k < c.G; ++k) {
+      if (!joins[k]) continue;
+      const pqmf_pool_group_f32& g = c.groups[k];
+      p.grp[p.G++] = pqmf::H4StreamGroup{g.ids, g.x, g.y, g.T, g.n, (int)tiles, ap[k].s};
+      tiles += h4_stream_tiles(g.n, ap[k].s);
+    }
+    p.n_tiles = tiles;
+    if (const int e = h4_launch_stream_groups(p, c.M, c.st)) return e;
+    started = true;
+  }
+  if (c.synthesis()) {
+    pqmf::H4SynthesisStreamGroupsParams p{};
+    static_cast<pqmf::H4SynthesisStreamParams&>(p) = sp[first];
+    p.state_in = p.state_out = c.spool;
+    p.pool = PoolRows{nullptr, c.sphase, c.P};
+    long tiles = 0;
+    for (int k = 0; k < c.G; ++k) {
+      if (!joins[k]) continue;
+      const pqmf_pool_group_f32& g = c.groups[k];
+      p.grp[p.G++] = pqmf::H4StreamGroup{g.ids, g.y, g.out, g.T / c.M, g.n, (int)tiles, sp[k].sg};
+      tiles += h4_stream_tiles(g.n, sp[k].sg);
+    }
+    p.n_tiles = tiles;
+    if (const int e = h4_launch_stream_groups(p, c.M, c.st)) {
+      if (!started) return e;
+      // the analysis has run: each group's synthesis goes through the single-group dispatcher (its own kernels), then the phase words
+      for (int k = 0; k < c.G; ++k) {
+        if (!joins[k]) continue;
+        const pqmf_pool_group_f32& g = c.groups[k];
+        const PoolRows rows{g.ids, c.sphase, c.P};
+        if (int e2 = run_synthesis(g.y, samples(g.out), pooled(c.spool, rows), c.hk, c.tables, g.n, g.T / c.M, c.M, c.L, 0, c.flags, c.st)) return e2;
+      }
+    }
+  }
+  started = true;
+  pqmf::stream_pool_phase_groups_kernel<<<(phase.row0[phase.G] + 255) / 256, 256, 0, c.st>>>(phase, c.P, c.analysis() ? c.xphase : nullptr,
+                                                                                            c.synthesis() ? c.sphase : nullptr);
+  return counted(cuda_status());
+}
+
+int pool_groups(const PoolGroupsCall& c) {
+  // every argument check before anything is launched: the single-group entries' rules per group, plus 0 <= G <= 8 and <= P rows in all
+  const bool ana = c.analysis(), syn = c.synthesis();
+  if (c.G < 0 || c.G > pqmf::kPoolMaxGroups || (c.G > 0 && !c.groups) || c.P < 1) return PQMF_ERR_ARG;
+  long rows = 0;
+  for (int k = 0; k < c.G; ++k) {
+    const pqmf_pool_group_f32& g = c.groups[k];
+    if (bad_dims(g.n, g.T, c.M, c.L) || g.T <= 0 || (g.T % c.M) != 0 || (syn && (c.L % c.M) != 0)) return PQMF_ERR_ARG;
+    if (g.n > 0 && (!g.ids || !g.y || (ana && !g.x) || (syn && !g.out))) return PQMF_ERR_ARG;
+    rows += g.n;
+  }
+  if (rows > c.P) return PQMF_ERR_ARG;
+  if (rows == 0) return PQMF_OK;
+  if (!c.hk || (ana && (!c.xpool || !c.xphase)) || (syn && (!c.spool || !c.sphase)) || (ana && syn && c.xphase == c.sphase)) return PQMF_ERR_ARG;
+  if (c.G == 1) return pool_group_alone(c, c.groups[0]);
+  // which groups the streaming Hankel-4 kernels plan, apart from the tile count, and how many tiles they make together
+  pqmf::H4AnalysisStreamParams ap[pqmf::kPoolMaxGroups];
+  pqmf::H4SynthesisStreamParams sp[pqmf::kPoolMaxGroups];
+  bool joins[pqmf::kPoolMaxGroups] = {};
+  long atiles = 0, stiles = 0;
+  int joined = 0;
+  for (int k = 0; k < c.G; ++k) {
+    const pqmf_pool_group_f32& g = c.groups[k];
+    if (g.n == 0) continue;
+    const PoolRows xrows{g.ids, c.xphase, c.P}, srows{g.ids, c.sphase, c.P};
+    ap[k] = pqmf::H4AnalysisStreamParams{};
+    sp[k] = pqmf::H4SynthesisStreamParams{};
+    if (ana && !h4_takes_analysis(samples(g.x), g.y, pooled(c.xpool, xrows), g.n, g.T, g.T / c.M, c.M, c.L, c.tables, c.flags, &ap[k], 1)) continue;
+    if (syn && !h4_takes_synthesis(g.y, samples(g.out), pooled(c.spool, srows), g.n, g.T / c.M, c.M, c.L, c.tables, c.flags, &sp[k], 1)) continue;
+    joins[k] = true;
+    ++joined;
+    if (ana) atiles += h4_stream_tiles(g.n, ap[k].s);
+    if (syn) stiles += h4_stream_tiles(g.n, sp[k].sg);
+  }
+  bool grouped = joined >= 2 && (!ana || atiles >= kH4StreamMinTiles) && (!syn || stiles >= kH4StreamMinTiles);
+  if (grouped) {
+    const int e = pool_groups_launch(c, joins, ap, sp, grouped);
+    if (grouped && e) return e;
+  }
+  for (int k = 0; k < c.G; ++k)
+    if (!(grouped && joins[k]))
+      if (int e = pool_group_alone(c, c.groups[k])) return e;
+  return PQMF_OK;
+}
 
 }  // namespace
 
@@ -1025,6 +1195,21 @@ int pqmf_stream_pool_step_f32(const float* x, float* y, float* out, const float*
   if (int e = run_analysis(samples(x), y, pooled(xpool, xrows), hk, tables, n, T, T / M, M, L, flags, st)) return e;
   if (int e = run_synthesis(y, samples(out), pooled(spool, srows), hk, tables, n, T / M, M, L, 0, flags, st)) return e;
   return pool_phase(xrows, n, xphase, T / M, sphase, T / M, st);
+}
+
+int pqmf_stream_pool_analysis_groups_f32(const pqmf_pool_group_f32* groups, int G, const float* hk, const float* tables, float* xpool, int* xphase,
+                                         int P, int M, int L, unsigned flags, pqmf_stream_t stream) {
+  return pool_groups({PoolDir::kAnalysis, groups, G, hk, tables, xpool, nullptr, xphase, nullptr, P, M, L, flags, (cudaStream_t)stream});
+}
+
+int pqmf_stream_pool_synthesis_groups_f32(const pqmf_pool_group_f32* groups, int G, const float* hk, const float* tables, float* spool, int* sphase,
+                                          int P, int M, int L, unsigned flags, pqmf_stream_t stream) {
+  return pool_groups({PoolDir::kSynthesis, groups, G, hk, tables, nullptr, spool, nullptr, sphase, P, M, L, flags, (cudaStream_t)stream});
+}
+
+int pqmf_stream_pool_step_groups_f32(const pqmf_pool_group_f32* groups, int G, const float* hk, const float* tables, float* xpool, int* xphase,
+                                     float* spool, int* sphase, int P, int M, int L, unsigned flags, pqmf_stream_t stream) {
+  return pool_groups({PoolDir::kStep, groups, G, hk, tables, xpool, spool, xphase, sphase, P, M, L, flags, (cudaStream_t)stream});
 }
 
 // ---- int16 PCM blocks in the streaming calls: the streaming Hankel-4 kernels with PCM loads (any channel count, optional down-mix) and

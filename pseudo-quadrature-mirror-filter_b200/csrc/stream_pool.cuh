@@ -45,4 +45,31 @@ __global__ void stream_pool_phase_kernel(const int* __restrict__ ids, int n, int
   }
 }
 
+// Grouped pool calls (pqmf_stream_pool_*_groups_f32): up to kPoolMaxGroups groups of rows, each with its own block length, in one call.
+// The phase words of every listed stream of the grouped launch are updated by one launch: the call's rows are the groups' rows
+// concatenated (group k holds rows row0[k] .. row0[k + 1] - 1), and each group advances its parity by its own frame count.
+constexpr int kPoolMaxGroups = 8;
+struct StreamPoolPhaseGroups {
+  const int* ids[kPoolMaxGroups];
+  int row0[kPoolMaxGroups + 1];
+  int adv[kPoolMaxGroups];  // frames per block of the group, & 1
+  int G;
+};
+__global__ void stream_pool_phase_groups_kernel(StreamPoolPhaseGroups t, int P, int* xphase, int* sphase) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= t.row0[t.G]) return;
+  int k = 0;
+  while (r >= t.row0[k + 1]) ++k;
+  const int id = t.ids[k][r - t.row0[k]];
+  if ((unsigned)id >= (unsigned)P) return;
+  if (xphase != nullptr) {
+    const int w = xphase[id];
+    xphase[id] = ((w & 1) ^ 1) | ((((w >> 1) + t.adv[k]) & 1) << 1);
+  }
+  if (sphase != nullptr) {
+    const int w = sphase[id];
+    sphase[id] = ((w & 1) ^ 1) | ((((w >> 1) + t.adv[k]) & 1) << 1);
+  }
+}
+
 }  // namespace pqmf

@@ -394,6 +394,109 @@ std::tuple<at::Tensor, at::Tensor> stream_pool_step(const at::Tensor& x, const a
   return {out, y};
 }
 
+// ---- grouped pool calls (pqmf_stream_pool_*_groups_f32): up to 8 groups of rows, each with its own block length.  Every group is
+//      checked before anything is launched; the ids stay one tensor per group (one device pointer each, nothing concatenated) ----
+enum class GroupsDir { kAnalysis, kSynthesis, kStep };
+
+// blocks: x [n, 1, T] (analysis, step) or s [n, M, F] (synthesis), one per group; returns the contiguous blocks and fills the descriptors
+std::vector<at::Tensor> groups_of(at::TensorList blocks, at::TensorList ids, const Bank& bank, const at::Tensor& like, int64_t P, GroupsDir dir,
+                                  std::vector<pqmf_pool_group_f32>& groups, const char* what) {
+  TORCH_CHECK(blocks.size() == ids.size(), what, ": ", blocks.size(), " block tensors but ", ids.size(), " id tensors");
+  TORCH_CHECK(blocks.size() <= 8, what, ": at most 8 groups per call, got ", blocks.size());
+  std::vector<at::Tensor> kept;
+  int64_t rows = 0;
+  for (size_t k = 0; k < blocks.size(); ++k) {
+    const at::Tensor& b = blocks[k];
+    check_f32_cuda(b, dir == GroupsDir::kSynthesis ? "s" : "x");
+    TORCH_CHECK(b.device() == like.device(), what, ": every group must be on the pool's device");
+    if (dir == GroupsDir::kSynthesis) {
+      TORCH_CHECK(b.dim() == 3 && b.size(1) == bank.M, what, " expects [streams, n_band, frames] per group, got ", b.sizes());
+      TORCH_CHECK(b.size(2) > 0, "empty block");
+    } else {
+      TORCH_CHECK(b.dim() == 3 && b.size(1) == 1, what, " expects [streams, 1, block] per group, got ", b.sizes());
+      TORCH_CHECK(b.size(2) > 0 && b.size(2) % bank.M == 0, "streaming block length ", b.size(2), " must be a positive multiple of n_band=", bank.M);
+    }
+    kept.push_back(b.contiguous());
+    const int64_t n = kept.back().size(0);
+    pqmf_pool_group_f32 g{};
+    g.ids = ids_of(ids[k], n, like);
+    g.n = (int)n;
+    g.T = (long)(dir == GroupsDir::kSynthesis ? kept.back().size(2) * bank.M : kept.back().size(2));
+    groups.push_back(g);
+    rows += n;
+  }
+  TORCH_CHECK(rows <= P, "more rows (", rows, ") than streams in the pool (", P, ")");
+  TORCH_CHECK(dir == GroupsDir::kAnalysis || bank.L % bank.M == 0, "streaming synthesis needs L a multiple of n_band");
+  return kept;
+}
+
+// xs[k] [n_k, 1, T_k] -> ys[k] [n_k, M, T_k / M]
+std::vector<at::Tensor> stream_pool_analysis_groups(at::TensorList xs, const at::Tensor& hk, const at::Tensor& tables, at::Tensor xpool,
+                                                    at::Tensor xphase, at::TensorList ids, int64_t flags) {
+  const Bank bank = bank_of(hk, xpool);
+  c10::cuda::CUDAGuard guard(xpool.device());
+  const Pool pool = pool_of(xpool, xphase, bank, xpool, "xpool");
+  std::vector<pqmf_pool_group_f32> groups;
+  const std::vector<at::Tensor> xc = groups_of(xs, ids, bank, xpool, pool.P, GroupsDir::kAnalysis, groups, "pqmf stream pool analysis_groups");
+  std::vector<at::Tensor> ys;
+  for (size_t k = 0; k < xc.size(); ++k) {
+    ys.push_back(at::empty({xc[k].size(0), bank.M, xc[k].size(2) / bank.M}, xc[k].options()));
+    groups[k].x = xc[k].data_ptr<float>();
+    groups[k].y = ys[k].data_ptr<float>();
+  }
+  check_rc(pqmf_stream_pool_analysis_groups_f32(groups.data(), (int)groups.size(), bank.ptr, tables_ptr(tables, xpool), pool.state, pool.phase,
+                                                (int)pool.P, (int)bank.M, (int)bank.L, (unsigned)flags,
+                                                (pqmf_stream_t)at::cuda::getCurrentCUDAStream().stream()),
+           "pqmf_stream_pool_analysis_groups_f32");
+  return ys;
+}
+
+// ss[k] [n_k, M, F_k] -> outs[k] [n_k, 1, M F_k]
+std::vector<at::Tensor> stream_pool_synthesis_groups(at::TensorList ss, const at::Tensor& hk, const at::Tensor& tables, at::Tensor spool,
+                                                     at::Tensor sphase, at::TensorList ids, int64_t flags) {
+  const Bank bank = bank_of(hk, spool);
+  c10::cuda::CUDAGuard guard(spool.device());
+  const Pool pool = pool_of(spool, sphase, bank, spool, "spool");
+  std::vector<pqmf_pool_group_f32> groups;
+  const std::vector<at::Tensor> sc = groups_of(ss, ids, bank, spool, pool.P, GroupsDir::kSynthesis, groups, "pqmf stream pool synthesis_groups");
+  std::vector<at::Tensor> outs;
+  for (size_t k = 0; k < sc.size(); ++k) {
+    outs.push_back(at::empty({sc[k].size(0), 1, bank.M * sc[k].size(2)}, sc[k].options()));
+    groups[k].y = sc[k].data_ptr<float>();
+    groups[k].out = outs[k].data_ptr<float>();
+  }
+  check_rc(pqmf_stream_pool_synthesis_groups_f32(groups.data(), (int)groups.size(), bank.ptr, tables_ptr(tables, spool), pool.state, pool.phase,
+                                                 (int)pool.P, (int)bank.M, (int)bank.L, (unsigned)flags,
+                                                 (pqmf_stream_t)at::cuda::getCurrentCUDAStream().stream()),
+           "pqmf_stream_pool_synthesis_groups_f32");
+  return outs;
+}
+
+// one block step of every group: (outs[k] [n_k, 1, T_k], ys[k] [n_k, M, T_k / M])
+std::tuple<std::vector<at::Tensor>, std::vector<at::Tensor>> stream_pool_step_groups(at::TensorList xs, const at::Tensor& hk, const at::Tensor& tables,
+                                                                                     at::Tensor xpool, at::Tensor xphase, at::Tensor spool,
+                                                                                     at::Tensor sphase, at::TensorList ids, int64_t flags) {
+  const Bank bank = bank_of(hk, xpool);
+  c10::cuda::CUDAGuard guard(xpool.device());
+  const Pool xp = pool_of(xpool, xphase, bank, xpool, "xpool"), sp = pool_of(spool, sphase, bank, xpool, "spool");
+  TORCH_CHECK(xp.P == sp.P, "the analysis and synthesis pools hold different numbers of streams");
+  std::vector<pqmf_pool_group_f32> groups;
+  const std::vector<at::Tensor> xc = groups_of(xs, ids, bank, xpool, xp.P, GroupsDir::kStep, groups, "pqmf stream pool step_groups");
+  std::vector<at::Tensor> ys, outs;
+  for (size_t k = 0; k < xc.size(); ++k) {
+    ys.push_back(at::empty({xc[k].size(0), bank.M, xc[k].size(2) / bank.M}, xc[k].options()));
+    outs.push_back(at::empty({xc[k].size(0), 1, xc[k].size(2)}, xc[k].options()));
+    groups[k].x = xc[k].data_ptr<float>();
+    groups[k].y = ys[k].data_ptr<float>();
+    groups[k].out = outs[k].data_ptr<float>();
+  }
+  check_rc(pqmf_stream_pool_step_groups_f32(groups.data(), (int)groups.size(), bank.ptr, tables_ptr(tables, xpool), xp.state, xp.phase, sp.state,
+                                            sp.phase, (int)xp.P, (int)bank.M, (int)bank.L, (unsigned)flags,
+                                            (pqmf_stream_t)at::cuda::getCurrentCUDAStream().stream()),
+           "pqmf_stream_pool_step_groups_f32");
+  return {outs, ys};
+}
+
 // ---- int16 PCM blocks in the streaming ops (pqmf_*_stream_pcm16 / pqmf_stream_pool_*_pcm16): pcm [S, T, C] interleaved WAV frames, rows
 //      S * C' (C' = 1 with downmix, else C; row s * C' + c = channel c of block s).  Where the library has no native kernel (PQMF_ERR_UNSUPPORTED,
 //      nothing launched, no state touched) the op stages the call: widen, the fp32 op, quantise -- bit-identical to the native path by
@@ -739,6 +842,43 @@ std::tuple<at::Tensor, at::Tensor> stream_pool_step_autograd(const at::Tensor& x
   return op.call(x, hk, tables, xpool, xphase, spool, sphase, ids, flags);
 }
 
+bool any_requires_grad(at::TensorList ts) {
+  for (const at::Tensor& t : ts)
+    if (t.requires_grad()) return true;
+  return false;
+}
+std::vector<at::Tensor> stream_pool_analysis_groups_autograd(at::TensorList xs, const at::Tensor& hk, const at::Tensor& tables, at::Tensor xpool,
+                                                             at::Tensor xphase, at::TensorList ids, int64_t flags) {
+  TORCH_CHECK(!(at::GradMode::is_enabled() && any_requires_grad(xs)),
+              "pqmf_b200::stream_pool_analysis_groups is not differentiable (a stream pool carries state across calls); use forward() for "
+              "training or wrap the call in torch.no_grad()");
+  at::AutoDispatchBelowADInplaceOrView guard;
+  static auto op =
+      c10::Dispatcher::singleton().findSchemaOrThrow("pqmf_b200::stream_pool_analysis_groups", "").typed<decltype(stream_pool_analysis_groups)>();
+  return op.call(xs, hk, tables, xpool, xphase, ids, flags);
+}
+std::vector<at::Tensor> stream_pool_synthesis_groups_autograd(at::TensorList ss, const at::Tensor& hk, const at::Tensor& tables, at::Tensor spool,
+                                                              at::Tensor sphase, at::TensorList ids, int64_t flags) {
+  TORCH_CHECK(!(at::GradMode::is_enabled() && any_requires_grad(ss)),
+              "pqmf_b200::stream_pool_synthesis_groups is not differentiable (a stream pool carries state across calls); use inverse() for "
+              "training or wrap the call in torch.no_grad()");
+  at::AutoDispatchBelowADInplaceOrView guard;
+  static auto op =
+      c10::Dispatcher::singleton().findSchemaOrThrow("pqmf_b200::stream_pool_synthesis_groups", "").typed<decltype(stream_pool_synthesis_groups)>();
+  return op.call(ss, hk, tables, spool, sphase, ids, flags);
+}
+std::tuple<std::vector<at::Tensor>, std::vector<at::Tensor>> stream_pool_step_groups_autograd(at::TensorList xs, const at::Tensor& hk,
+                                                                                              const at::Tensor& tables, at::Tensor xpool,
+                                                                                              at::Tensor xphase, at::Tensor spool, at::Tensor sphase,
+                                                                                              at::TensorList ids, int64_t flags) {
+  TORCH_CHECK(!(at::GradMode::is_enabled() && any_requires_grad(xs)),
+              "pqmf_b200::stream_pool_step_groups is not differentiable (a stream pool carries state across calls); use forward() / inverse() "
+              "for training or wrap the call in torch.no_grad()");
+  at::AutoDispatchBelowADInplaceOrView guard;
+  static auto op = c10::Dispatcher::singleton().findSchemaOrThrow("pqmf_b200::stream_pool_step_groups", "").typed<decltype(stream_pool_step_groups)>();
+  return op.call(xs, hk, tables, xpool, xphase, spool, sphase, ids, flags);
+}
+
 at::Tensor synthesis_stream_pcm16_autograd(const at::Tensor& s, const at::Tensor& hk, const at::Tensor& tables, const at::Tensor& state_in,
                                            at::Tensor state_out, int64_t frame_parity, int64_t flags) {
   TORCH_CHECK(!(at::GradMode::is_enabled() && s.requires_grad()),
@@ -805,6 +945,15 @@ TORCH_LIBRARY(pqmf_b200, m) {
   m.def(
       "stream_pool_step_pcm16(Tensor pcm, Tensor hk, Tensor tables, Tensor(a!) xpool, Tensor(b!) xphase, Tensor(c!) spool, Tensor(d!) sphase, "
       "Tensor ids, bool downmix, int flags) -> (Tensor, Tensor)");
+  m.def(
+      "stream_pool_analysis_groups(Tensor[] xs, Tensor hk, Tensor tables, Tensor(a!) xpool, Tensor(b!) xphase, Tensor[] ids, int flags) "
+      "-> Tensor[]");
+  m.def(
+      "stream_pool_synthesis_groups(Tensor[] ss, Tensor hk, Tensor tables, Tensor(a!) spool, Tensor(b!) sphase, Tensor[] ids, int flags) "
+      "-> Tensor[]");
+  m.def(
+      "stream_pool_step_groups(Tensor[] xs, Tensor hk, Tensor tables, Tensor(a!) xpool, Tensor(b!) xphase, Tensor(c!) spool, Tensor(d!) sphase, "
+      "Tensor[] ids, int flags) -> (Tensor[], Tensor[])");
   m.def("launch_count() -> int", &launch_count);
 }
 
@@ -828,6 +977,9 @@ TORCH_LIBRARY_IMPL(pqmf_b200, CUDA, m) {
   m.impl("stream_pool_analysis_pcm16", &stream_pool_analysis_pcm16);
   m.impl("stream_pool_synthesis_pcm16", &stream_pool_synthesis_pcm16);
   m.impl("stream_pool_step_pcm16", &stream_pool_step_pcm16);
+  m.impl("stream_pool_analysis_groups", &stream_pool_analysis_groups);
+  m.impl("stream_pool_synthesis_groups", &stream_pool_synthesis_groups);
+  m.impl("stream_pool_step_groups", &stream_pool_step_groups);
 }
 
 // gradients w.r.t. the signal / the sub-bands only (the bank is a registered buffer in the reference, not a parameter)
@@ -842,4 +994,7 @@ TORCH_LIBRARY_IMPL(pqmf_b200, Autograd, m) {
   m.impl("stream_pool_step", &stream_pool_step_autograd);
   m.impl("synthesis_stream_pcm16", &synthesis_stream_pcm16_autograd);
   m.impl("stream_pool_synthesis_pcm16", &stream_pool_synthesis_pcm16_autograd);
+  m.impl("stream_pool_analysis_groups", &stream_pool_analysis_groups_autograd);
+  m.impl("stream_pool_synthesis_groups", &stream_pool_synthesis_groups_autograd);
+  m.impl("stream_pool_step_groups", &stream_pool_step_groups_autograd);
 }

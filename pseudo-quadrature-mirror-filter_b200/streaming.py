@@ -13,7 +13,7 @@ from __future__ import annotations
 
 import operator
 
-from typing import Optional, Sequence, Tuple, Union
+from typing import List, Optional, Sequence, Tuple, Union
 
 import torch
 
@@ -76,7 +76,8 @@ class StreamPool:
     ``[n, 1, T]`` and sub-bands ``[n, n_band, T / n_band]`` -- per row bit for bit what ``process_stream`` gives for that stream.
     ``forward`` / ``inverse`` run one direction, with its own state and parity as ``forward_stream`` / ``inverse_stream``; ``reset`` forgets
     streams so that a new session can take their slots.  ``step_pcm16`` / ``forward_pcm16`` / ``inverse_pcm16`` are the same calls with
-    16-bit PCM blocks (interleaved WAV frames in, int16 samples out).
+    16-bit PCM blocks (interleaved WAV frames in, int16 samples out).  ``step_groups`` / ``forward_groups`` / ``inverse_groups`` take up
+    to 8 groups of streams with their own block lengths in one call.
 
     ``ids`` is a list of ints or a CPU integer tensor (checked: in range and distinct, else ``ValueError``), or a CUDA integer tensor, which
     is trusted as it is and costs no host synchronisation.  With CUDA ids a step allocates nothing but its outputs, so it can be captured
@@ -140,6 +141,56 @@ class StreamPool:
         if mod.n_band == 1:
             return y
         return torch.ops.pqmf_b200.stream_pool_synthesis(y, mod.hk.float(), mod._tables, self.spool, self.sphase, self._ids(ids), mod._flags)
+
+    MAX_GROUPS = 8
+
+    def _group_ids(self, groups) -> Tuple[List[torch.Tensor], List[torch.Tensor]]:
+        """Blocks and ids of ``(block, ids)`` pairs; CPU ids are checked as in ``step``, and distinct across all groups."""
+        groups = list(groups)
+        if len(groups) > self.MAX_GROUPS:
+            raise ValueError(f"at most {self.MAX_GROUPS} groups per call, got {len(groups)}")
+        blocks, ids, seen = [], [], set()
+        for block, gids in groups:
+            t = self._ids(gids)
+            if not (isinstance(gids, torch.Tensor) and gids.is_cuda):
+                host = [operator.index(i) for i in (gids.tolist() if isinstance(gids, torch.Tensor) else gids)]
+                if seen.intersection(host):
+                    raise ValueError("stream ids must be distinct across all groups")
+                seen.update(host)
+            blocks.append(block)
+            ids.append(t)
+        return blocks, ids
+
+    def step_groups(self, groups) -> List[Tuple[torch.Tensor, torch.Tensor]]:
+        """``step`` of up to 8 groups ``(x_g [n_g, 1, T_g], ids_g)`` with their own block lengths, in one call: returns ``[(out_g, y_g)]``.
+
+        The groups the streaming Hankel-4 kernels can take run together in one launch per direction when they make enough tiles together
+        (so small groups of several block lengths reach the tensor cores); each of their rows is what those kernels give it in a pool
+        call.  Every other group gives exactly what ``step(x_g, ids_g)`` gives; one group is ``step``.  ids follow ``step``'s rules and must
+        be distinct across all groups."""
+        blocks, ids = self._group_ids(groups)
+        mod = self.mod
+        if mod.n_band == 1:
+            return [(x, x) for x in blocks]
+        outs, ys = torch.ops.pqmf_b200.stream_pool_step_groups(blocks, mod.hk.float(), mod._tables, self.xpool, self.xphase, self.spool,
+                                                               self.sphase, ids, mod._flags)
+        return list(zip(outs, ys))
+
+    def forward_groups(self, groups) -> List[torch.Tensor]:
+        """``forward`` of up to 8 groups ``(x_g [n_g, 1, T_g], ids_g)`` in one call (routed as ``step_groups``): returns ``[y_g]``."""
+        blocks, ids = self._group_ids(groups)
+        mod = self.mod
+        if mod.n_band == 1:
+            return blocks
+        return list(torch.ops.pqmf_b200.stream_pool_analysis_groups(blocks, mod.hk.float(), mod._tables, self.xpool, self.xphase, ids, mod._flags))
+
+    def inverse_groups(self, groups) -> List[torch.Tensor]:
+        """``inverse`` of up to 8 groups ``(y_g [n_g, n_band, F_g], ids_g)`` in one call (routed as ``step_groups``): returns ``[out_g]``."""
+        blocks, ids = self._group_ids(groups)
+        mod = self.mod
+        if mod.n_band == 1:
+            return blocks
+        return list(torch.ops.pqmf_b200.stream_pool_synthesis_groups(blocks, mod.hk.float(), mod._tables, self.spool, self.sphase, ids, mod._flags))
 
     def step_pcm16(self, pcm: torch.Tensor, ids, downmix: bool = False) -> Tuple[torch.Tensor, torch.Tensor]:
         """``step`` from 16-bit PCM to 16-bit PCM: ``pcm`` int16 ``[S, T, channels]`` -> ``(pcm_out int16 [S, T, C'], y [S, C' * n_band,
