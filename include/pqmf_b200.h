@@ -240,6 +240,43 @@ int pqmf_stream_pool_step_pcm16(const int16_t* pcm, float* y, int16_t* pcm_out, 
                                 float* spool, int* sphase, int P, const int* ids, int B, long T, int C, int downmix, int M, int L, unsigned flags,
                                 pqmf_stream_t stream);
 
+/* ---- grouped pool calls with int16 PCM blocks: the grouped entries above (pqmf_stream_pool_*_groups_f32) with the PCM edge of the pool
+ *      entries.  A group is n clips of C channels and T samples: ids [rows] (device int32; rows = n, or n * C without downmix; row s * C' + c
+ *      is stream ids[s * C' + c]), pcm [n, T, C] interleaved WAV frames, y [n, C' M, T/M] and pcm_out [n, T, C'].  The analysis reads pcm and
+ *      writes y, the synthesis reads y ([n, C M, T/M], rows n * C, no downmix) and writes pcm_out [n, T, C], the step does both; a pointer
+ *      the direction does not use may be NULL.  downmix applies to the whole call; each group has its own T and C.  Per row the result is
+ *      bit for bit pqmf_stream_pool_*_groups_f32 on the widened blocks followed by quantising, with the same pool and phase-word updates.
+ *      Rule:
+ *        1. All argument checks on the host first (PQMF_ERR_ARG): the single-group PCM pool entries' checks per group, 0 <= G <= 8, at most
+ *           P rows in all, staged != NULL.  G == 0 and all-empty calls return 0.
+ *        2. The joined groups are those the fp32 grouped call would join on freshly allocated widened blocks (the PCM buffers' alignment
+ *           does not decide it).
+ *        3. If a joined group cannot run natively (a PCM input not 32-byte aligned, C' > 1 output in a synthesis or step) or the first
+ *           grouped launch does not start, the call returns PQMF_ERR_UNSUPPORTED with nothing launched: the caller widens every group,
+ *           calls the fp32 grouped entry and quantises.  A step whose synthesis launch fails after its analysis ran returns
+ *           cudaErrorLaunchFailure (a staged retry would step the analysis state twice).
+ *        4. Otherwise one GROUPS PCM launch per direction and one phase-word launch for the joined groups, then every other group through
+ *           its pqmf_stream_pool_*_pcm16 entry.  Where that entry refuses (PQMF_ERR_UNSUPPORTED, nothing launched), bit k of *staged is set
+ *           and the call goes on; the caller then runs group k through the single-group pool calls on the widened block -- what the fp32
+ *           grouped call does for a group it does not join.  *staged is 0 otherwise.  Returns 0.
+ *      G == 1 is the group's pqmf_stream_pool_*_pcm16 entry (a refusal sets bit 0). ---- */
+typedef struct pqmf_pool_group_pcm16 {
+  const int* ids;
+  int n;
+  long T;
+  int C;
+  const int16_t* pcm;
+  float* y;
+  int16_t* pcm_out;
+} pqmf_pool_group_pcm16;
+int pqmf_stream_pool_analysis_groups_pcm16(const pqmf_pool_group_pcm16* groups, int G, int downmix, const float* hk, const float* tables,
+                                           float* xpool, int* xphase, int P, int M, int L, unsigned flags, unsigned* staged, pqmf_stream_t stream);
+int pqmf_stream_pool_synthesis_groups_pcm16(const pqmf_pool_group_pcm16* groups, int G, const float* hk, const float* tables, float* spool,
+                                            int* sphase, int P, int M, int L, unsigned flags, unsigned* staged, pqmf_stream_t stream);
+int pqmf_stream_pool_step_groups_pcm16(const pqmf_pool_group_pcm16* groups, int G, int downmix, const float* hk, const float* tables, float* xpool,
+                                       int* xphase, float* spool, int* sphase, int P, int M, int L, unsigned flags, unsigned* staged,
+                                       pqmf_stream_t stream);
+
 /* ---- fused round trip on device buffers: PQMFWrapper.process (PQMFWrapper.py:81-92: forward, then inverse of the same
  *      sub-bands) and the Pvoc wrapper's forward (1-PitchShifterWrapper.py:303-316) ----
  * pqmf_analysis_f32 followed by pqmf_synthesis_f32 on the same stream, as one call; the synthesis kernels walk their tiles

@@ -431,13 +431,14 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_stream_kernel(H
   } H4_TRACE(nullptr));
 }
 
-// ---- GROUPS: one pool launch over up to kPoolMaxGroups groups of rows with different block lengths (fp32, CTA pairs) ----
+// ---- GROUPS: one pool launch over up to kPoolMaxGroups groups of rows with different block lengths (fp32 or PCM, CTA pairs) ----
 // The tiles of the launch are the groups' tiles concatenated; every tile belongs to one group and has that group's region geometry
 // (the history rows are the same in every group: one bank, one H4Shape).  Each MMA row still reads only its own stream's region, so the
 // results of a group are those of the POOL instantiation on its rows.  A CTA's tile index only grows: a group cursor advances by
 // comparison, and the per-thread plan (the POOL kernels' tile-invariant plan) is rebuilt when a tile enters a new group -- at most G - 1
 // times per CTA.  Block addresses are made per tile from the row index.  The drain runs two tile loads behind the load, so the drained
 // tile's output row (pointer, frame stride, first frame, parity) travels through load -> convert -> drain with the tile.
+// PCM (the POOL PCM kernels' edge, per group): each group has its own WAV frames (channel count, down-mix) and mono int16 output rows.
 struct H4StreamGroup {
   const int* ids;   // [n] stream of each row
   const float* in;  // analysis: x [n, T]; synthesis: s [n, M, F]
@@ -455,6 +456,17 @@ struct H4SynthesisStreamGroupsParams : H4SynthesisStreamPoolParams {
   int G;
   H4StreamGroup grp[kPoolMaxGroups];
 };
+// PCM: group k's block rows come from the WAV frames in[k] (grp[k].in unused), its mono output rows go to pcm_out[k] (grp[k].out unused)
+struct H4AnalysisStreamGroupsPcmParams : H4AnalysisStreamGroupsParams {
+  PcmIn in[kPoolMaxGroups];
+};
+struct H4SynthesisStreamGroupsPcmParams : H4SynthesisStreamGroupsParams {
+  int16_t* pcm_out[kPoolMaxGroups];
+};
+template <H4Io IO>
+using H4AnalysisStreamGroupsArgs = std::conditional_t<IO == H4Io::PCM, H4AnalysisStreamGroupsPcmParams, H4AnalysisStreamGroupsParams>;
+template <H4Io IO>
+using H4SynthesisStreamGroupsArgs = std::conditional_t<IO == H4Io::PCM, H4SynthesisStreamGroupsPcmParams, H4SynthesisStreamGroupsParams>;
 
 // the group of `tile`, from the group k of an earlier tile of the same CTA (tiles only grow); tiles past the last group (the second CTA
 // of a pair at the end) stay in the last group and have no live rows
@@ -471,9 +483,11 @@ __device__ __forceinline__ int h4_groups_min_region_rows(const Params& p) {
   return rows;
 }
 
-template <int M>
-__global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_stream_groups_kernel(H4AnalysisStreamGroupsParams p) {
+template <int M, H4Io IO>
+__global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_stream_groups_kernel(H4AnalysisStreamGroupsArgs<IO> p) {
+  static_assert(IO == H4Io::F32 || IO == H4Io::PCM, "streaming blocks: fp32 rows or int16 PCM frames");
   h4_kernel<true, kH4Workers>(p.g, p.bank, p.n_tiles, 1u, p.pad_bytes, p.trim_lo, p.trim_hi, [&](const H4Smem& sm, uint32_t tmem, uint32_t pfull_leader, unsigned n_iter) {
+    constexpr bool PCM = IO == H4Io::PCM;
     constexpr int FR = 64 / M, HB = M / 2;
     constexpr int NO = (kH4Rows * 8 + kH4Workers - 1) / kH4Workers;
     const H4Shape& g = p.g;
@@ -518,6 +532,9 @@ __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_stream_groups_kerne
     DrainRow d_ld{nullptr, 0, 0, 0}, d_cur = d_ld, d_prev = d_ld;  // of the loaded / converted / drained tile
     float xr[NO][8];
     float* roll[NO];
+    // PCM: first row of the tile held in xr, in its group gi.  convert runs before the next load_tile (h4_worker_loop), so gi, row_ld and
+    // the plan are still the loaded tile's when its raw words are widened
+    [[maybe_unused]] int row_ld = 0;
     const int di = tid & 127, hb = tid >> 7;
     auto load_tile = [&](long tile) {
       const int k = h4_group_of(p, gi < 0 ? 0 : gi, tile);
@@ -529,6 +546,7 @@ __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_stream_groups_kerne
       const H4StreamGeom sg = gr.s;
       const long row0 = (tile - gr.tile0) * sg.spt;
       const int nlive = (int)min((long)sg.spt, (long)gr.n - row0);
+      if constexpr (PCM) row_ld = (int)row0;
       int id[NO], ph[NO];
 #pragma unroll
       for (int r = 0; r < NO; ++r) {
@@ -554,12 +572,15 @@ __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_stream_groups_kerne
           for (int e = 0; e < 8; ++e) xr[r][e] = 0.f;
         } else if (hofs[r] >= 0) {
           ptx::ldg256_na(p.hist_in + ((size_t)(ph[r] & 1) * p.pool.P + row) * p.L + hofs[r], xr[r]);
+        } else if constexpr (PCM) {
+          pcm_load8_raw_row(p.in[gi], row_ld + q_slot[r], bofs[r], (int)gr.len, xr[r]);  // raw words: converted when the tile is consumed
         } else {
           ptx::ldg256_na(gr.in + (size_t)(row0 + q_slot[r]) * gr.len + bofs[r], xr[r]);
         }
         roll[r] = (rofs[r] >= 0 && id[r] >= 0) ? p.hist_out + ((size_t)(~ph[r] & 1) * p.pool.P + row) * p.L + rofs[r] : nullptr;
       }
     };
+    // PCM: the block groups' raw words are widened first (zeros of dead rows widen to zeros), so planes and roll see the fp32 call's floats
     auto convert = [&](int pb) {
       unsigned char* p1 = sm.planes + (2 * pb) * g.plane;
       d_cur = d_ld;
@@ -567,6 +588,8 @@ __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_stream_groups_kerne
       for (int r = 0; r < NO; ++r) {
         const int u = tid + kH4Workers * r;
         if (u < n_octs) {
+          if constexpr (PCM)
+            if (bofs[r] >= 0) pcm_convert8(p.in[gi], row_ld + q_slot[r], xr[r]);
           h4_split_store8(xr[r], p1, g.plane, sw128_offset((uint32_t)u * 16u));
           if (roll[r] != nullptr) {
             *reinterpret_cast<float4*>(roll[r]) = make_float4(xr[r][0], xr[r][1], xr[r][2], xr[r][3]);
@@ -605,9 +628,12 @@ __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_stream_groups_kerne
   } H4_TRACE(nullptr));
 }
 
-template <int M>
-__global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_stream_groups_kernel(H4SynthesisStreamGroupsParams p) {
+template <int M, H4Io IO>
+__global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_stream_groups_kernel(H4SynthesisStreamGroupsArgs<IO> p) {
+  static_assert(IO == H4Io::F32 || IO == H4Io::PCM, "streaming blocks: fp32 rows or int16 PCM samples");
   h4_kernel<true, kH4SynWorkers>(p.g, p.bank, p.n_tiles, 1u, p.pad_bytes, p.trim_lo, p.trim_hi, [&](const H4Smem& sm, uint32_t tmem, uint32_t pfull_leader, unsigned n_iter) {
+    constexpr bool PCM = IO == H4Io::PCM;
+    using Out = std::conditional_t<PCM, int16_t, float>;
     constexpr int FR = 64 / M, NBG = M / 8;
     const H4Shape& g = p.g;
     const int tid = threadIdx.x, warp = tid >> 5;
@@ -648,9 +674,9 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_stream_groups_k
     float4 v[8];
     float* roll = nullptr;
     uint32_t flip_ld = 0;
-    float* o_ld = nullptr;  // this thread's first output of the loaded / converted / drained tile (nullptr: not a stored row)
-    float* o_cur = nullptr;
-    float* o_prev = nullptr;
+    Out* o_ld = nullptr;  // this thread's first output of the loaded / converted / drained tile (nullptr: not a stored row); PCM: int16
+    Out* o_cur = nullptr;
+    Out* o_prev = nullptr;
     const int i0 = (tid & 127) & ~3, hb = tid >> 7, lane = tid & 31;
     auto load_tile = [&](long tile) {
       const int k = h4_group_of(p, gi < 0 ? 0 : gi, tile);
@@ -675,7 +701,10 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_stream_groups_k
       // pitch and rows_b are multiples of 4: the four rows of a lane quad belong to one region and are stored or not together
       const int et = i0 / sg.pitch, eq0 = i0 - et * sg.pitch;
       const bool stored = warp < 8 && et < sg.spt && eq0 < sg.rows_b && et < nlive;
-      o_ld = stored ? gr.out + (size_t)(row0 + et) * (size_t)(gr.len * M) + 64 * eq0 + 32 * hb + 8 * (lane & 3) : nullptr;
+      Out* base;
+      if constexpr (PCM) base = p.pcm_out[gi];
+      else base = gr.out;
+      o_ld = stored ? base + (size_t)(row0 + et) * (size_t)(gr.len * M) + 64 * eq0 + 32 * hb + 8 * (lane & 3) : nullptr;
     };
     auto convert = [&](int pb) {
       o_cur = o_ld;
@@ -697,8 +726,19 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_stream_groups_k
       float val[4][8];
       h4_drain_synthesis(tmem, dbuf, tid, val);
       if (o_prev == nullptr) return;
+      if constexpr (PCM) {  // quantised: eight samples = one 16-byte store per slot, as the POOL PCM kernel
 #pragma unroll
-      for (int q = 0; q < 4; ++q) ptx::stg256_cs(o_prev + (size_t)q * 64, val[q]);
+        for (int q = 0; q < 4; ++q) {
+          uint32_t w[4];
+#pragma unroll
+          for (int k = 0; k < 4; ++k)
+            w[k] = (uint32_t)(uint16_t)pcm_quantise(val[q][2 * k]) | ((uint32_t)(uint16_t)pcm_quantise(val[q][2 * k + 1]) << 16);
+          __stcs(reinterpret_cast<uint4*>(o_prev + (size_t)q * 64), make_uint4(w[0], w[1], w[2], w[3]));
+        }
+      } else {
+#pragma unroll
+        for (int q = 0; q < 4; ++q) ptx::stg256_cs(o_prev + (size_t)q * 64, val[q]);
+      }
     };
 
     long tile = blockIdx.x;
@@ -743,16 +783,33 @@ inline int h4_launch_synthesis_stream(const H4SynthesisStreamParams& p, const St
     return pool ? h4_launch_synthesis_stream<M, true, H4Io::PCM>(p, pool, pcm_out, st) : h4_launch_synthesis_stream<M, false, H4Io::PCM>(p, pool, pcm_out, st);
   return pool ? h4_launch_synthesis_stream<M, true, H4Io::F32>(p, pool, pcm_out, st) : h4_launch_synthesis_stream<M, false, H4Io::F32>(p, pool, pcm_out, st);
 }
-// GROUPS: p.n_tiles, p.G and p.grp[] filled by the caller
-template <int M>
-inline int h4_launch_analysis_stream_groups(const H4AnalysisStreamGroupsParams& p, cudaStream_t st) {
+// GROUPS: p.n_tiles, p.G and p.grp[] filled by the caller; the instantiation follows the sample format io (PCM: in[] / pcm_out[] per group)
+template <int M, H4Io IO>
+inline int h4_launch_analysis_stream_groups(const H4AnalysisStreamGroupsParams& base, const PcmIn* in, cudaStream_t st) {
   static H4Configured configured;
-  return h4_launch<true>(h4_analysis_stream_groups_kernel<M>, p, kH4Threads, configured, st);
+  H4AnalysisStreamGroupsArgs<IO> p{};
+  static_cast<H4AnalysisStreamGroupsParams&>(p) = base;
+  if constexpr (IO == H4Io::PCM)
+    for (int k = 0; k < p.G; ++k) p.in[k] = in[k];
+  return h4_launch<true>(h4_analysis_stream_groups_kernel<M, IO>, p, kH4Threads, configured, st);
 }
 template <int M>
-inline int h4_launch_synthesis_stream_groups(const H4SynthesisStreamGroupsParams& p, cudaStream_t st) {
+inline int h4_launch_analysis_stream_groups(const H4AnalysisStreamGroupsParams& p, H4Io io, const PcmIn* in, cudaStream_t st) {
+  return io == H4Io::PCM ? h4_launch_analysis_stream_groups<M, H4Io::PCM>(p, in, st) : h4_launch_analysis_stream_groups<M, H4Io::F32>(p, in, st);
+}
+template <int M, H4Io IO>
+inline int h4_launch_synthesis_stream_groups(const H4SynthesisStreamGroupsParams& base, int16_t* const* pcm_out, cudaStream_t st) {
   static H4Configured configured;
-  return h4_launch<true>(h4_synthesis_stream_groups_kernel<M>, p, kH4SynThreads, configured, st);
+  H4SynthesisStreamGroupsArgs<IO> p{};
+  static_cast<H4SynthesisStreamGroupsParams&>(p) = base;
+  if constexpr (IO == H4Io::PCM)
+    for (int k = 0; k < p.G; ++k) p.pcm_out[k] = pcm_out[k];
+  return h4_launch<true>(h4_synthesis_stream_groups_kernel<M, IO>, p, kH4SynThreads, configured, st);
+}
+template <int M>
+inline int h4_launch_synthesis_stream_groups(const H4SynthesisStreamGroupsParams& p, H4Io io, int16_t* const* pcm_out, cudaStream_t st) {
+  return io == H4Io::PCM ? h4_launch_synthesis_stream_groups<M, H4Io::PCM>(p, pcm_out, st)
+                         : h4_launch_synthesis_stream_groups<M, H4Io::F32>(p, pcm_out, st);
 }
 
 }  // namespace pqmf

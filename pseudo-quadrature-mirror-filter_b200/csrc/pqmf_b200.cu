@@ -742,10 +742,12 @@ int pool_phase(const PoolRows& pool, int n, int* xphase, long x_frames, int* sph
 }
 bool bad_pool(int P, int n) { return P < 1 || n < 0 || n > P; }
 
-// ---- grouped pool calls (pqmf_stream_pool_*_groups_f32): groups of rows with their own block lengths.  One rule: the groups the
-//      streaming Hankel-4 kernels can plan (h4_takes_*, family, plan and alignment, apart from the tile count) run together in one GROUPS
-//      launch per direction and one phase-word launch, when there are at least two of them and they reach kH4StreamMinTiles together
-//      (in both directions for a step).  Every other group runs through its single-group pool entry, with exactly that entry's launches ----
+// ---- grouped pool calls (pqmf_stream_pool_*_groups_f32 / _pcm16): groups of rows with their own block lengths.  One rule: the groups
+//      the streaming Hankel-4 kernels can plan (h4_takes_*, family, plan and alignment, apart from the tile count) run together in one
+//      GROUPS launch per direction and one phase-word launch, when there are at least two of them and they reach kH4StreamMinTiles together
+//      (in both directions for a step).  Every other group runs through its single-group pool entry, with exactly that entry's launches.
+//      A PCM call joins exactly the groups the fp32 call on the widened blocks would join (fresh, aligned fp32 rows: the PCM buffers'
+//      alignment does not decide it); it then runs natively or launches nothing ----
 enum class PoolDir { kAnalysis, kSynthesis, kStep };
 
 struct PoolGroupsCall {
@@ -759,13 +761,63 @@ struct PoolGroupsCall {
   int P, M, L;
   unsigned flags;
   cudaStream_t st;
+  // the sample format: PCM calls have pcm_groups (groups unused), one down-mix for the whole call, and the mask of staged groups
+  pqmf::H4Io io = pqmf::H4Io::F32;
+  const pqmf_pool_group_pcm16* pcm_groups = nullptr;
+  int downmix = 0;
+  unsigned* staged = nullptr;
   bool analysis() const { return dir != PoolDir::kSynthesis; }
   bool synthesis() const { return dir != PoolDir::kAnalysis; }
+  bool pcm() const { return io == pqmf::H4Io::PCM; }
 };
 
-int pool_group_alone(const PoolGroupsCall& c, const pqmf_pool_group_f32& g) {
-  if (g.n == 0) return PQMF_OK;
+// group k of either format: its rows (PCM: clips x C', C' = 1 with the down-mix, else C; a synthesis has no down-mix), the analysis input
+// and the synthesis output
+struct PoolGroup {
+  const int* ids;
+  int rows;
+  long T;
+  Samples x;
+  float* y;
+  Samples out;
+};
+PoolGroup pool_group(const PoolGroupsCall& c, int k) {
+  if (!c.pcm()) {
+    const pqmf_pool_group_f32& g = c.groups[k];
+    return {g.ids, g.n, g.T, samples(g.x), g.y, samples(g.out)};
+  }
+  const pqmf_pool_group_pcm16& g = c.pcm_groups[k];
+  return {g.ids, c.downmix ? g.n : g.n * g.C, g.T, pcm16(g.pcm, g.C, c.downmix), g.y, pcm16(g.pcm_out, c.downmix ? 1 : g.C)};
+}
+// the fp32 call's sample side of a group: PCM blocks stand for freshly allocated fp32 rows (null passes every alignment check)
+Samples fp32_view(const Samples& s) { return s.io == pqmf::H4Io::F32 ? s : samples(nullptr); }
+
+int pool_group_alone(const PoolGroupsCall& c, int k) {
   pqmf_stream_t s = (pqmf_stream_t)c.st;
+  if (c.pcm()) {
+    const pqmf_pool_group_pcm16& g = c.pcm_groups[k];
+    if (g.n == 0) return PQMF_OK;
+    int e;
+    switch (c.dir) {
+      case PoolDir::kAnalysis:
+        e = pqmf_stream_pool_analysis_pcm16(g.pcm, g.y, c.hk, c.tables, c.xpool, c.xphase, c.P, g.ids, g.n, g.T, g.C, c.downmix, c.M, c.L, c.flags, s);
+        break;
+      case PoolDir::kSynthesis:
+        e = pqmf_stream_pool_synthesis_pcm16(g.y, g.pcm_out, c.hk, c.tables, c.spool, c.sphase, c.P, g.ids, g.n, g.C, g.T / c.M, c.M, c.L, c.flags, s);
+        break;
+      default:
+        e = pqmf_stream_pool_step_pcm16(g.pcm, g.y, g.pcm_out, c.hk, c.tables, c.xpool, c.xphase, c.spool, c.sphase, c.P, g.ids, g.n, g.T, g.C,
+                                        c.downmix, c.M, c.L, c.flags, s);
+    }
+    // refused (nothing launched): the caller stages this group through the single-group calls on the widened block
+    if (e == PQMF_ERR_UNSUPPORTED) {
+      *c.staged |= 1u << k;
+      return PQMF_OK;
+    }
+    return e;
+  }
+  const pqmf_pool_group_f32& g = c.groups[k];
+  if (g.n == 0) return PQMF_OK;
   switch (c.dir) {
     case PoolDir::kAnalysis:
       return pqmf_stream_pool_analysis_f32(g.x, g.y, c.hk, c.tables, c.xpool, c.xphase, c.P, g.ids, g.n, g.T, c.M, c.L, c.flags, s);
@@ -777,20 +829,21 @@ int pool_group_alone(const PoolGroupsCall& c, const pqmf_pool_group_f32& g) {
   }
 }
 
+// the GROUPS launch of one direction, fp32 or PCM by io (PCM: in[] / pcm_out[] per group of the launch)
 template <typename Params>
-int h4_launch_stream_groups(const Params& p, int M, cudaStream_t st) {
+int h4_launch_stream_groups(const Params& p, int M, pqmf::H4Io io, const pqmf::PcmIn* in, int16_t* const* pcm_out, cudaStream_t st) {
   int e = PQMF_ERR_UNSUPPORTED;
   if constexpr (std::is_same_v<Params, pqmf::H4AnalysisStreamGroupsParams>) {
     switch (M) {
-      case 8: e = pqmf::h4_launch_analysis_stream_groups<8>(p, st); break;
-      case 16: e = pqmf::h4_launch_analysis_stream_groups<16>(p, st); break;
-      case 32: e = pqmf::h4_launch_analysis_stream_groups<32>(p, st); break;
+      case 8: e = pqmf::h4_launch_analysis_stream_groups<8>(p, io, in, st); break;
+      case 16: e = pqmf::h4_launch_analysis_stream_groups<16>(p, io, in, st); break;
+      case 32: e = pqmf::h4_launch_analysis_stream_groups<32>(p, io, in, st); break;
     }
   } else {
     switch (M) {
-      case 8: e = pqmf::h4_launch_synthesis_stream_groups<8>(p, st); break;
-      case 16: e = pqmf::h4_launch_synthesis_stream_groups<16>(p, st); break;
-      case 32: e = pqmf::h4_launch_synthesis_stream_groups<32>(p, st); break;
+      case 8: e = pqmf::h4_launch_synthesis_stream_groups<8>(p, io, pcm_out, st); break;
+      case 16: e = pqmf::h4_launch_synthesis_stream_groups<16>(p, io, pcm_out, st); break;
+      case 32: e = pqmf::h4_launch_synthesis_stream_groups<32>(p, io, pcm_out, st); break;
     }
   }
   if (e != 0) (void)cudaGetLastError();
@@ -798,19 +851,23 @@ int h4_launch_stream_groups(const Params& p, int M, cudaStream_t st) {
 }
 
 // the GROUPS launches of the groups in `joins`, planned in ap / sp, then one phase-word launch.  started: false when the first launch did
-// not start (nothing was launched: the caller runs the groups alone)
-int pool_groups_launch(const PoolGroupsCall& c, const bool* joins, const pqmf::H4AnalysisStreamParams* ap, const pqmf::H4SynthesisStreamParams* sp,
-                       bool& started) {
+// not start (nothing was launched: the caller runs the groups alone, or -- PCM -- refuses the call)
+int pool_groups_launch(const PoolGroupsCall& c, const PoolGroup* grp, const bool* joins, const pqmf::H4AnalysisStreamParams* ap,
+                       const pqmf::H4SynthesisStreamParams* sp, bool& started) {
   started = false;
   pqmf::StreamPoolPhaseGroups phase{};
+  pqmf::PcmIn in[pqmf::kPoolMaxGroups] = {};
+  int16_t* pcm_out[pqmf::kPoolMaxGroups] = {};
   int first = -1;
   for (int k = 0; k < c.G; ++k) {
     if (!joins[k]) continue;
-    const pqmf_pool_group_f32& g = c.groups[k];
+    const PoolGroup& g = grp[k];
     if (first < 0) first = k;
+    in[phase.G] = g.x.pcm;
+    pcm_out[phase.G] = g.out.pcm_out();
     phase.ids[phase.G] = g.ids;
     phase.adv[phase.G] = (int)((g.T / c.M) & 1);
-    phase.row0[phase.G + 1] = phase.row0[phase.G] + g.n;
+    phase.row0[phase.G + 1] = phase.row0[phase.G] + g.rows;
     ++phase.G;
   }
   // the bank, flags and history rows are the same for every group: the H4Shape, trims and pad of the first one hold for all
@@ -822,12 +879,12 @@ int pool_groups_launch(const PoolGroupsCall& c, const bool* joins, const pqmf::H
     long tiles = 0;
     for (int k = 0; k < c.G; ++k) {
       if (!joins[k]) continue;
-      const pqmf_pool_group_f32& g = c.groups[k];
-      p.grp[p.G++] = pqmf::H4StreamGroup{g.ids, g.x, g.y, g.T, g.n, (int)tiles, ap[k].s};
-      tiles += h4_stream_tiles(g.n, ap[k].s);
+      const PoolGroup& g = grp[k];
+      p.grp[p.G++] = pqmf::H4StreamGroup{g.ids, static_cast<const float*>(g.x.rows()), g.y, g.T, g.rows, (int)tiles, ap[k].s};
+      tiles += h4_stream_tiles(g.rows, ap[k].s);
     }
     p.n_tiles = tiles;
-    if (const int e = h4_launch_stream_groups(p, c.M, c.st)) return e;
+    if (const int e = h4_launch_stream_groups(p, c.M, c.io, in, pcm_out, c.st)) return e;
     started = true;
   }
   if (c.synthesis()) {
@@ -838,19 +895,21 @@ int pool_groups_launch(const PoolGroupsCall& c, const bool* joins, const pqmf::H
     long tiles = 0;
     for (int k = 0; k < c.G; ++k) {
       if (!joins[k]) continue;
-      const pqmf_pool_group_f32& g = c.groups[k];
-      p.grp[p.G++] = pqmf::H4StreamGroup{g.ids, g.y, g.out, g.T / c.M, g.n, (int)tiles, sp[k].sg};
-      tiles += h4_stream_tiles(g.n, sp[k].sg);
+      const PoolGroup& g = grp[k];
+      p.grp[p.G++] = pqmf::H4StreamGroup{g.ids, g.y, static_cast<float*>(g.out.rows()), g.T / c.M, g.rows, (int)tiles, sp[k].sg};
+      tiles += h4_stream_tiles(g.rows, sp[k].sg);
     }
     p.n_tiles = tiles;
-    if (const int e = h4_launch_stream_groups(p, c.M, c.st)) {
+    if (const int e = h4_launch_stream_groups(p, c.M, c.io, in, pcm_out, c.st)) {
       if (!started) return e;
-      // the analysis has run: each group's synthesis goes through the single-group dispatcher (its own kernels), then the phase words
+      // the analysis has run.  PCM: an error, not a refusal (a staged retry would step the analysis state twice; see
+      // pqmf_stream_step_pcm16).  fp32: each group's synthesis goes through the single-group dispatcher (its own kernels), then the phase words
+      if (c.pcm()) return (int)cudaErrorLaunchFailure;
       for (int k = 0; k < c.G; ++k) {
         if (!joins[k]) continue;
-        const pqmf_pool_group_f32& g = c.groups[k];
+        const PoolGroup& g = grp[k];
         const PoolRows rows{g.ids, c.sphase, c.P};
-        if (int e2 = run_synthesis(g.y, samples(g.out), pooled(c.spool, rows), c.hk, c.tables, g.n, g.T / c.M, c.M, c.L, 0, c.flags, c.st)) return e2;
+        if (int e2 = run_synthesis(g.y, g.out, pooled(c.spool, rows), c.hk, c.tables, g.rows, g.T / c.M, c.M, c.L, 0, c.flags, c.st)) return e2;
       }
     }
   }
@@ -860,48 +919,73 @@ int pool_groups_launch(const PoolGroupsCall& c, const bool* joins, const pqmf::H
   return counted(cuda_status());
 }
 
+bool pcm_args_bad(int C, long rows) { return C < 1 || C > 64 || rows >= (1L << 31); }
+
 int pool_groups(const PoolGroupsCall& c) {
   // every argument check before anything is launched: the single-group entries' rules per group, plus 0 <= G <= 8 and <= P rows in all
   const bool ana = c.analysis(), syn = c.synthesis();
-  if (c.G < 0 || c.G > pqmf::kPoolMaxGroups || (c.G > 0 && !c.groups) || c.P < 1) return PQMF_ERR_ARG;
+  if (c.G < 0 || c.G > pqmf::kPoolMaxGroups || (c.G > 0 && !(c.pcm() ? (const void*)c.pcm_groups : (const void*)c.groups)) || c.P < 1)
+    return PQMF_ERR_ARG;
   long rows = 0;
   for (int k = 0; k < c.G; ++k) {
-    const pqmf_pool_group_f32& g = c.groups[k];
-    if (bad_dims(g.n, g.T, c.M, c.L) || g.T <= 0 || (g.T % c.M) != 0 || (syn && (c.L % c.M) != 0)) return PQMF_ERR_ARG;
-    if (g.n > 0 && (!g.ids || !g.y || (ana && !g.x) || (syn && !g.out))) return PQMF_ERR_ARG;
-    rows += g.n;
+    if (c.pcm()) {
+      const pqmf_pool_group_pcm16& g = c.pcm_groups[k];
+      const long grows = c.downmix ? (long)g.n : (long)g.n * g.C;
+      if (bad_dims(g.n, g.T, c.M, c.L) || pcm_args_bad(g.C, grows) || g.T <= 0 || (g.T % c.M) != 0 || (syn && (c.L % c.M) != 0)) return PQMF_ERR_ARG;
+      if (g.n > 0 && (!g.ids || !g.y || (ana && !g.pcm) || (syn && !g.pcm_out))) return PQMF_ERR_ARG;
+      rows += grows;
+    } else {
+      const pqmf_pool_group_f32& g = c.groups[k];
+      if (bad_dims(g.n, g.T, c.M, c.L) || g.T <= 0 || (g.T % c.M) != 0 || (syn && (c.L % c.M) != 0)) return PQMF_ERR_ARG;
+      if (g.n > 0 && (!g.ids || !g.y || (ana && !g.x) || (syn && !g.out))) return PQMF_ERR_ARG;
+      rows += g.n;
+    }
   }
-  if (rows > c.P) return PQMF_ERR_ARG;
+  if (rows > c.P || (c.pcm() && !c.staged)) return PQMF_ERR_ARG;
+  if (c.pcm()) *c.staged = 0;
   if (rows == 0) return PQMF_OK;
   if (!c.hk || (ana && (!c.xpool || !c.xphase)) || (syn && (!c.spool || !c.sphase)) || (ana && syn && c.xphase == c.sphase)) return PQMF_ERR_ARG;
-  if (c.G == 1) return pool_group_alone(c, c.groups[0]);
+  if (c.G == 1) return pool_group_alone(c, 0);
   // which groups the streaming Hankel-4 kernels plan, apart from the tile count, and how many tiles they make together
+  PoolGroup grp[pqmf::kPoolMaxGroups];
   pqmf::H4AnalysisStreamParams ap[pqmf::kPoolMaxGroups];
   pqmf::H4SynthesisStreamParams sp[pqmf::kPoolMaxGroups];
   bool joins[pqmf::kPoolMaxGroups] = {};
   long atiles = 0, stiles = 0;
   int joined = 0;
   for (int k = 0; k < c.G; ++k) {
-    const pqmf_pool_group_f32& g = c.groups[k];
-    if (g.n == 0) continue;
+    const PoolGroup& g = grp[k] = pool_group(c, k);
+    if (g.rows == 0) continue;
     const PoolRows xrows{g.ids, c.xphase, c.P}, srows{g.ids, c.sphase, c.P};
     ap[k] = pqmf::H4AnalysisStreamParams{};
     sp[k] = pqmf::H4SynthesisStreamParams{};
-    if (ana && !h4_takes_analysis(samples(g.x), g.y, pooled(c.xpool, xrows), g.n, g.T, g.T / c.M, c.M, c.L, c.tables, c.flags, &ap[k], 1)) continue;
-    if (syn && !h4_takes_synthesis(g.y, samples(g.out), pooled(c.spool, srows), g.n, g.T / c.M, c.M, c.L, c.tables, c.flags, &sp[k], 1)) continue;
+    if (ana && !h4_takes_analysis(fp32_view(g.x), g.y, pooled(c.xpool, xrows), g.rows, g.T, g.T / c.M, c.M, c.L, c.tables, c.flags, &ap[k], 1)) continue;
+    if (syn && !h4_takes_synthesis(g.y, fp32_view(g.out), pooled(c.spool, srows), g.rows, g.T / c.M, c.M, c.L, c.tables, c.flags, &sp[k], 1)) continue;
     joins[k] = true;
     ++joined;
-    if (ana) atiles += h4_stream_tiles(g.n, ap[k].s);
-    if (syn) stiles += h4_stream_tiles(g.n, sp[k].sg);
+    if (ana) atiles += h4_stream_tiles(g.rows, ap[k].s);
+    if (syn) stiles += h4_stream_tiles(g.rows, sp[k].sg);
   }
   bool grouped = joined >= 2 && (!ana || atiles >= kH4StreamMinTiles) && (!syn || stiles >= kH4StreamMinTiles);
+  if (grouped && c.pcm()) {
+    // the joined groups run natively, or nothing is launched: their PCM buffers' alignment, and mono output rows
+    for (int k = 0; k < c.G; ++k) {
+      if (!joins[k]) continue;
+      const PoolGroup& g = grp[k];
+      const PoolRows xrows{g.ids, c.xphase, c.P}, srows{g.ids, c.sphase, c.P};
+      if ((ana && !h4_takes_analysis(g.x, g.y, pooled(c.xpool, xrows), g.rows, g.T, g.T / c.M, c.M, c.L, c.tables, c.flags, nullptr, 1)) ||
+          (syn && !h4_takes_synthesis(g.y, g.out, pooled(c.spool, srows), g.rows, g.T / c.M, c.M, c.L, c.tables, c.flags, nullptr, 1)))
+        return PQMF_ERR_UNSUPPORTED;
+    }
+  }
   if (grouped) {
-    const int e = pool_groups_launch(c, joins, ap, sp, grouped);
+    const int e = pool_groups_launch(c, grp, joins, ap, sp, grouped);
+    if (c.pcm() && !grouped) return PQMF_ERR_UNSUPPORTED;  // the first launch did not start: nothing ran
     if (grouped && e) return e;
   }
   for (int k = 0; k < c.G; ++k)
     if (!(grouped && joins[k]))
-      if (int e = pool_group_alone(c, c.groups[k])) return e;
+      if (int e = pool_group_alone(c, k)) return e;
   return PQMF_OK;
 }
 
@@ -1212,10 +1296,28 @@ int pqmf_stream_pool_step_groups_f32(const pqmf_pool_group_f32* groups, int G, c
   return pool_groups({PoolDir::kStep, groups, G, hk, tables, xpool, spool, xphase, sphase, P, M, L, flags, (cudaStream_t)stream});
 }
 
+int pqmf_stream_pool_analysis_groups_pcm16(const pqmf_pool_group_pcm16* groups, int G, int downmix, const float* hk, const float* tables,
+                                           float* xpool, int* xphase, int P, int M, int L, unsigned flags, unsigned* staged, pqmf_stream_t stream) {
+  return pool_groups({PoolDir::kAnalysis, nullptr, G, hk, tables, xpool, nullptr, xphase, nullptr, P, M, L, flags, (cudaStream_t)stream,
+                      pqmf::H4Io::PCM, groups, downmix ? 1 : 0, staged});
+}
+
+int pqmf_stream_pool_synthesis_groups_pcm16(const pqmf_pool_group_pcm16* groups, int G, const float* hk, const float* tables, float* spool,
+                                            int* sphase, int P, int M, int L, unsigned flags, unsigned* staged, pqmf_stream_t stream) {
+  return pool_groups({PoolDir::kSynthesis, nullptr, G, hk, tables, nullptr, spool, nullptr, sphase, P, M, L, flags, (cudaStream_t)stream,
+                      pqmf::H4Io::PCM, groups, 0, staged});
+}
+
+int pqmf_stream_pool_step_groups_pcm16(const pqmf_pool_group_pcm16* groups, int G, int downmix, const float* hk, const float* tables, float* xpool,
+                                       int* xphase, float* spool, int* sphase, int P, int M, int L, unsigned flags, unsigned* staged,
+                                       pqmf_stream_t stream) {
+  return pool_groups({PoolDir::kStep, nullptr, G, hk, tables, xpool, spool, xphase, sphase, P, M, L, flags, (cudaStream_t)stream, pqmf::H4Io::PCM,
+                      groups, downmix ? 1 : 0, staged});
+}
+
 // ---- int16 PCM blocks in the streaming calls: the streaming Hankel-4 kernels with PCM loads (any channel count, optional down-mix) and
 //      mono PCM stores, exactly where the fp32 call with the same rows runs those kernels (h4_takes_*, with the PCM buffer's alignment);
 //      every other call returns PQMF_ERR_UNSUPPORTED before anything is launched and the caller stages it through the fp32 entry ----
-static bool pcm_args_bad(int C, long rows) { return C < 1 || C > 64 || rows >= (1L << 31); }
 
 int pqmf_analysis_stream_pcm16(const int16_t* pcm, float* y, const float* hk, const float* tables, const float* state_in, float* state_out, int B,
                                long T, int C, int downmix, int M, int L, int frame_parity, unsigned flags, pqmf_stream_t stream) {

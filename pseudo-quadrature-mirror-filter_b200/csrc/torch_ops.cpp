@@ -398,15 +398,45 @@ std::tuple<at::Tensor, at::Tensor> stream_pool_step(const at::Tensor& x, const a
 //      checked before anything is launched; the ids stay one tensor per group (one device pointer each, nothing concatenated) ----
 enum class GroupsDir { kAnalysis, kSynthesis, kStep };
 
-// blocks: x [n, 1, T] (analysis, step) or s [n, M, F] (synthesis), one per group; returns the contiguous blocks and fills the descriptors
+void check_pcm(const at::Tensor& pcm, const char* what);
+
+// blocks: x [n, 1, T] (analysis, step) or s [n, M, F] (synthesis), one per group; returns the contiguous blocks and fills the descriptors.
+// pcm != nullptr: PCM groups, filled into *pcm instead -- pcm [S, T, C] int16 (analysis, step; rows S C', C' = 1 with downmix, else C) or
+// s [S, C M, F] float32 (synthesis; rows S C)
 std::vector<at::Tensor> groups_of(at::TensorList blocks, at::TensorList ids, const Bank& bank, const at::Tensor& like, int64_t P, GroupsDir dir,
-                                  std::vector<pqmf_pool_group_f32>& groups, const char* what) {
+                                  std::vector<pqmf_pool_group_f32>& groups, const char* what,
+                                  std::vector<pqmf_pool_group_pcm16>* pcm = nullptr, bool downmix = false) {
   TORCH_CHECK(blocks.size() == ids.size(), what, ": ", blocks.size(), " block tensors but ", ids.size(), " id tensors");
   TORCH_CHECK(blocks.size() <= 8, what, ": at most 8 groups per call, got ", blocks.size());
   std::vector<at::Tensor> kept;
   int64_t rows = 0;
   for (size_t k = 0; k < blocks.size(); ++k) {
     const at::Tensor& b = blocks[k];
+    if (pcm != nullptr) {
+      const bool syn = dir == GroupsDir::kSynthesis;
+      if (syn) {
+        check_f32_cuda(b, "s");
+        TORCH_CHECK(b.dim() == 3 && b.size(1) % bank.M == 0 && b.size(1) > 0, what, " expects [blocks, channels * n_band, frames] per group, got ",
+                    b.sizes());
+        TORCH_CHECK(b.size(1) / bank.M <= 64, what, ": 1 to 64 channels, got ", b.size(1) / bank.M);
+        TORCH_CHECK(b.size(2) > 0, "empty block");
+      } else {
+        check_pcm(b, "stream pool groups_pcm16");
+        TORCH_CHECK(b.size(1) > 0 && b.size(1) % bank.M == 0, "streaming block length ", b.size(1), " must be a positive multiple of n_band=", bank.M);
+      }
+      TORCH_CHECK(b.device() == like.device(), what, ": every group must be on the pool's device");
+      kept.push_back(b.contiguous());
+      const at::Tensor& c = kept.back();
+      pqmf_pool_group_pcm16 g{};
+      g.n = (int)c.size(0);
+      g.C = (int)(syn ? c.size(1) / bank.M : c.size(2));
+      g.T = (long)(syn ? c.size(2) * bank.M : c.size(1));
+      const int64_t n = (int64_t)g.n * (downmix && !syn ? 1 : g.C);
+      g.ids = ids_of(ids[k], n, like);
+      pcm->push_back(g);
+      rows += n;
+      continue;
+    }
     check_f32_cuda(b, dir == GroupsDir::kSynthesis ? "s" : "x");
     TORCH_CHECK(b.device() == like.device(), what, ": every group must be on the pool's device");
     if (dir == GroupsDir::kSynthesis) {
@@ -682,6 +712,120 @@ std::tuple<at::Tensor, at::Tensor> stream_pool_step_pcm16(const at::Tensor& pcm,
   return {out, y};
 }
 
+// ---- grouped pool calls with PCM blocks (pqmf_stream_pool_*_groups_pcm16): groups_of's PCM groups, one down-mix for the call.  Where the
+//      library refuses the whole call (PQMF_ERR_UNSUPPORTED, nothing launched) the op stages it: widen every group, the fp32 grouped op,
+//      quantise.  The groups it marks in `staged` (nothing launched for them) go through the single-group PCM pool op, which stages
+//      direction by direction ----
+bool staged_bit(unsigned staged, size_t k) { return (staged >> k) & 1u; }
+
+// pcms[k] int16 [S_k, T_k, C_k] -> ys[k] [S_k, C'_k M, T_k / M]
+std::vector<at::Tensor> stream_pool_analysis_groups_pcm16(at::TensorList pcms, const at::Tensor& hk, const at::Tensor& tables, at::Tensor xpool,
+                                                          at::Tensor xphase, at::TensorList ids, bool downmix, int64_t flags) {
+  const Bank bank = bank_of(hk, xpool);
+  c10::cuda::CUDAGuard guard(xpool.device());
+  const Pool pool = pool_of(xpool, xphase, bank, xpool, "xpool");
+  std::vector<pqmf_pool_group_f32> unused;
+  std::vector<pqmf_pool_group_pcm16> groups;
+  const std::vector<at::Tensor> pc =
+      groups_of(pcms, ids, bank, xpool, pool.P, GroupsDir::kAnalysis, unused, "pqmf stream pool analysis_groups_pcm16", &groups, downmix);
+  std::vector<at::Tensor> ys;
+  for (size_t k = 0; k < pc.size(); ++k) {
+    const int64_t Cr = downmix ? 1 : groups[k].C;
+    ys.push_back(at::empty({pc[k].size(0), Cr * bank.M, pc[k].size(1) / bank.M}, pc[k].options().dtype(at::kFloat)));
+    groups[k].pcm = pc[k].data_ptr<int16_t>();
+    groups[k].y = ys[k].data_ptr<float>();
+  }
+  unsigned staged = 0;
+  const int rc = pqmf_stream_pool_analysis_groups_pcm16(groups.data(), (int)groups.size(), downmix ? 1 : 0, bank.ptr, tables_ptr(tables, xpool),
+                                                        pool.state, pool.phase, (int)pool.P, (int)bank.M, (int)bank.L, (unsigned)flags, &staged,
+                                                        cur_stream());
+  if (rc == PQMF_ERR_UNSUPPORTED) {
+    std::vector<at::Tensor> xs;
+    for (size_t k = 0; k < pc.size(); ++k) xs.push_back(pcm_widen(pc[k], downmix).view({-1, 1, pc[k].size(1)}));
+    const std::vector<at::Tensor> yf = stream_pool_analysis_groups(xs, hk, tables, xpool, xphase, ids, flags);
+    for (size_t k = 0; k < pc.size(); ++k) ys[k] = yf[k].view(ys[k].sizes());
+    return ys;
+  }
+  check_rc(rc, "pqmf_stream_pool_analysis_groups_pcm16");
+  for (size_t k = 0; k < pc.size(); ++k)
+    if (staged_bit(staged, k)) ys[k] = stream_pool_analysis_pcm16(pc[k], hk, tables, xpool, xphase, ids[k], downmix, flags);
+  return ys;
+}
+
+// ss[k] float32 [S_k, C_k M, F_k] -> pcms[k] int16 [S_k, M F_k, C_k]
+std::vector<at::Tensor> stream_pool_synthesis_groups_pcm16(at::TensorList ss, const at::Tensor& hk, const at::Tensor& tables, at::Tensor spool,
+                                                           at::Tensor sphase, at::TensorList ids, int64_t flags) {
+  const Bank bank = bank_of(hk, spool);
+  c10::cuda::CUDAGuard guard(spool.device());
+  const Pool pool = pool_of(spool, sphase, bank, spool, "spool");
+  std::vector<pqmf_pool_group_f32> unused;
+  std::vector<pqmf_pool_group_pcm16> groups;
+  const std::vector<at::Tensor> sc =
+      groups_of(ss, ids, bank, spool, pool.P, GroupsDir::kSynthesis, unused, "pqmf stream pool synthesis_groups_pcm16", &groups);
+  std::vector<at::Tensor> outs;
+  for (size_t k = 0; k < sc.size(); ++k) {
+    outs.push_back(at::empty({sc[k].size(0), bank.M * sc[k].size(2), groups[k].C}, sc[k].options().dtype(at::kShort)));
+    groups[k].y = sc[k].data_ptr<float>();
+    groups[k].pcm_out = outs[k].data_ptr<int16_t>();
+  }
+  unsigned staged = 0;
+  const int rc = pqmf_stream_pool_synthesis_groups_pcm16(groups.data(), (int)groups.size(), bank.ptr, tables_ptr(tables, spool), pool.state,
+                                                         pool.phase, (int)pool.P, (int)bank.M, (int)bank.L, (unsigned)flags, &staged, cur_stream());
+  if (rc == PQMF_ERR_UNSUPPORTED) {
+    std::vector<at::Tensor> sv;
+    for (size_t k = 0; k < sc.size(); ++k) sv.push_back(sc[k].view({-1, bank.M, sc[k].size(2)}));
+    const std::vector<at::Tensor> of = stream_pool_synthesis_groups(sv, hk, tables, spool, sphase, ids, flags);
+    for (size_t k = 0; k < sc.size(); ++k) outs[k] = pcm_quantise(of[k].view({sc[k].size(0), groups[k].C, bank.M * sc[k].size(2)}));
+    return outs;
+  }
+  check_rc(rc, "pqmf_stream_pool_synthesis_groups_pcm16");
+  for (size_t k = 0; k < sc.size(); ++k)
+    if (staged_bit(staged, k)) outs[k] = stream_pool_synthesis_pcm16(sc[k], hk, tables, spool, sphase, ids[k], flags);
+  return outs;
+}
+
+// one block step of every group from PCM to PCM: (outs[k] int16 [S_k, T_k, C'_k], ys[k] [S_k, C'_k M, T_k / M])
+std::tuple<std::vector<at::Tensor>, std::vector<at::Tensor>> stream_pool_step_groups_pcm16(at::TensorList pcms, const at::Tensor& hk,
+                                                                                           const at::Tensor& tables, at::Tensor xpool,
+                                                                                           at::Tensor xphase, at::Tensor spool, at::Tensor sphase,
+                                                                                           at::TensorList ids, bool downmix, int64_t flags) {
+  const Bank bank = bank_of(hk, xpool);
+  c10::cuda::CUDAGuard guard(xpool.device());
+  const Pool xp = pool_of(xpool, xphase, bank, xpool, "xpool"), sp = pool_of(spool, sphase, bank, xpool, "spool");
+  TORCH_CHECK(xp.P == sp.P, "the analysis and synthesis pools hold different numbers of streams");
+  std::vector<pqmf_pool_group_f32> unused;
+  std::vector<pqmf_pool_group_pcm16> groups;
+  const std::vector<at::Tensor> pc =
+      groups_of(pcms, ids, bank, xpool, xp.P, GroupsDir::kStep, unused, "pqmf stream pool step_groups_pcm16", &groups, downmix);
+  std::vector<at::Tensor> ys, outs;
+  for (size_t k = 0; k < pc.size(); ++k) {
+    const int64_t Cr = downmix ? 1 : groups[k].C, S = pc[k].size(0), T = pc[k].size(1);
+    ys.push_back(at::empty({S, Cr * bank.M, T / bank.M}, pc[k].options().dtype(at::kFloat)));
+    outs.push_back(at::empty({S, T, Cr}, pc[k].options()));
+    groups[k].pcm = pc[k].data_ptr<int16_t>();
+    groups[k].y = ys[k].data_ptr<float>();
+    groups[k].pcm_out = outs[k].data_ptr<int16_t>();
+  }
+  unsigned staged = 0;
+  const int rc = pqmf_stream_pool_step_groups_pcm16(groups.data(), (int)groups.size(), downmix ? 1 : 0, bank.ptr, tables_ptr(tables, xpool), xp.state,
+                                                    xp.phase, sp.state, sp.phase, (int)xp.P, (int)bank.M, (int)bank.L, (unsigned)flags, &staged,
+                                                    cur_stream());
+  if (rc == PQMF_ERR_UNSUPPORTED) {
+    std::vector<at::Tensor> xs;
+    for (size_t k = 0; k < pc.size(); ++k) xs.push_back(pcm_widen(pc[k], downmix).view({-1, 1, pc[k].size(1)}));
+    const auto res = stream_pool_step_groups(xs, hk, tables, xpool, xphase, spool, sphase, ids, flags);
+    for (size_t k = 0; k < pc.size(); ++k) {
+      outs[k] = pcm_quantise(std::get<0>(res)[k].view({outs[k].size(0), outs[k].size(2), outs[k].size(1)}));
+      ys[k] = std::get<1>(res)[k].view(ys[k].sizes());
+    }
+    return {outs, ys};
+  }
+  check_rc(rc, "pqmf_stream_pool_step_groups_pcm16");
+  for (size_t k = 0; k < pc.size(); ++k)
+    if (staged_bit(staged, k)) std::tie(outs[k], ys[k]) = stream_pool_step_pcm16(pc[k], hk, tables, xpool, xphase, spool, sphase, ids[k], downmix, flags);
+  return {outs, ys};
+}
+
 int64_t launch_count() { return (int64_t)pqmf_launch_count(); }
 
 // ---- autograd (SURVEY 8f-2: the reference path is differentiable, upstream users train through PQMF) --------------------
@@ -899,6 +1043,45 @@ at::Tensor stream_pool_synthesis_pcm16_autograd(const at::Tensor& s, const at::T
   return op.call(s, hk, tables, spool, sphase, ids, flags);
 }
 
+// the grouped PCM ops: int16 blocks carry no gradient; float sub-bands that require grad are refused like the other streaming ops'
+std::vector<at::Tensor> stream_pool_analysis_groups_pcm16_autograd(at::TensorList pcms, const at::Tensor& hk, const at::Tensor& tables,
+                                                                   at::Tensor xpool, at::Tensor xphase, at::TensorList ids, bool downmix,
+                                                                   int64_t flags) {
+  TORCH_CHECK(!(at::GradMode::is_enabled() && any_requires_grad(pcms)),
+              "pqmf_b200::stream_pool_analysis_groups_pcm16 is not differentiable (a stream pool carries state across calls); use forward() for "
+              "training or wrap the call in torch.no_grad()");
+  at::AutoDispatchBelowADInplaceOrView guard;
+  static auto op = c10::Dispatcher::singleton()
+                       .findSchemaOrThrow("pqmf_b200::stream_pool_analysis_groups_pcm16", "")
+                       .typed<decltype(stream_pool_analysis_groups_pcm16)>();
+  return op.call(pcms, hk, tables, xpool, xphase, ids, downmix, flags);
+}
+std::vector<at::Tensor> stream_pool_synthesis_groups_pcm16_autograd(at::TensorList ss, const at::Tensor& hk, const at::Tensor& tables,
+                                                                    at::Tensor spool, at::Tensor sphase, at::TensorList ids, int64_t flags) {
+  TORCH_CHECK(!(at::GradMode::is_enabled() && any_requires_grad(ss)),
+              "pqmf_b200::stream_pool_synthesis_groups_pcm16 is not differentiable (a stream pool carries state across calls, and int16 output has "
+              "no gradient); use inverse() for training or wrap the call in torch.no_grad()");
+  at::AutoDispatchBelowADInplaceOrView guard;
+  static auto op = c10::Dispatcher::singleton()
+                       .findSchemaOrThrow("pqmf_b200::stream_pool_synthesis_groups_pcm16", "")
+                       .typed<decltype(stream_pool_synthesis_groups_pcm16)>();
+  return op.call(ss, hk, tables, spool, sphase, ids, flags);
+}
+std::tuple<std::vector<at::Tensor>, std::vector<at::Tensor>> stream_pool_step_groups_pcm16_autograd(at::TensorList pcms, const at::Tensor& hk,
+                                                                                                    const at::Tensor& tables, at::Tensor xpool,
+                                                                                                    at::Tensor xphase, at::Tensor spool,
+                                                                                                    at::Tensor sphase, at::TensorList ids,
+                                                                                                    bool downmix, int64_t flags) {
+  TORCH_CHECK(!(at::GradMode::is_enabled() && any_requires_grad(pcms)),
+              "pqmf_b200::stream_pool_step_groups_pcm16 is not differentiable (a stream pool carries state across calls); use forward() / "
+              "inverse() for training or wrap the call in torch.no_grad()");
+  at::AutoDispatchBelowADInplaceOrView guard;
+  static auto op = c10::Dispatcher::singleton()
+                       .findSchemaOrThrow("pqmf_b200::stream_pool_step_groups_pcm16", "")
+                       .typed<decltype(stream_pool_step_groups_pcm16)>();
+  return op.call(pcms, hk, tables, xpool, xphase, spool, sphase, ids, downmix, flags);
+}
+
 at::Tensor analysis_autograd(const at::Tensor& x, const at::Tensor& hk, const at::Tensor& tables, int64_t n_frames, int64_t flags) {
   return AnalysisFn::apply(x, hk, tables, n_frames, flags);
 }
@@ -954,6 +1137,15 @@ TORCH_LIBRARY(pqmf_b200, m) {
   m.def(
       "stream_pool_step_groups(Tensor[] xs, Tensor hk, Tensor tables, Tensor(a!) xpool, Tensor(b!) xphase, Tensor(c!) spool, Tensor(d!) sphase, "
       "Tensor[] ids, int flags) -> (Tensor[], Tensor[])");
+  m.def(
+      "stream_pool_analysis_groups_pcm16(Tensor[] pcms, Tensor hk, Tensor tables, Tensor(a!) xpool, Tensor(b!) xphase, Tensor[] ids, "
+      "bool downmix, int flags) -> Tensor[]");
+  m.def(
+      "stream_pool_synthesis_groups_pcm16(Tensor[] ss, Tensor hk, Tensor tables, Tensor(a!) spool, Tensor(b!) sphase, Tensor[] ids, int flags) "
+      "-> Tensor[]");
+  m.def(
+      "stream_pool_step_groups_pcm16(Tensor[] pcms, Tensor hk, Tensor tables, Tensor(a!) xpool, Tensor(b!) xphase, Tensor(c!) spool, "
+      "Tensor(d!) sphase, Tensor[] ids, bool downmix, int flags) -> (Tensor[], Tensor[])");
   m.def("launch_count() -> int", &launch_count);
 }
 
@@ -980,6 +1172,9 @@ TORCH_LIBRARY_IMPL(pqmf_b200, CUDA, m) {
   m.impl("stream_pool_analysis_groups", &stream_pool_analysis_groups);
   m.impl("stream_pool_synthesis_groups", &stream_pool_synthesis_groups);
   m.impl("stream_pool_step_groups", &stream_pool_step_groups);
+  m.impl("stream_pool_analysis_groups_pcm16", &stream_pool_analysis_groups_pcm16);
+  m.impl("stream_pool_synthesis_groups_pcm16", &stream_pool_synthesis_groups_pcm16);
+  m.impl("stream_pool_step_groups_pcm16", &stream_pool_step_groups_pcm16);
 }
 
 // gradients w.r.t. the signal / the sub-bands only (the bank is a registered buffer in the reference, not a parameter)
@@ -997,4 +1192,7 @@ TORCH_LIBRARY_IMPL(pqmf_b200, Autograd, m) {
   m.impl("stream_pool_analysis_groups", &stream_pool_analysis_groups_autograd);
   m.impl("stream_pool_synthesis_groups", &stream_pool_synthesis_groups_autograd);
   m.impl("stream_pool_step_groups", &stream_pool_step_groups_autograd);
+  m.impl("stream_pool_analysis_groups_pcm16", &stream_pool_analysis_groups_pcm16_autograd);
+  m.impl("stream_pool_synthesis_groups_pcm16", &stream_pool_synthesis_groups_pcm16_autograd);
+  m.impl("stream_pool_step_groups_pcm16", &stream_pool_step_groups_pcm16_autograd);
 }

@@ -18,6 +18,22 @@ from typing import List, Optional, Sequence, Tuple, Union
 import torch
 
 
+def _widen(pcm: torch.Tensor, downmix: bool) -> torch.Tensor:
+    """int16 ``[S, T, C]`` -> float32 ``[S, C', T]`` with the PCM ops' arithmetic: v / 32768, the down-mix summed in channel order, then / C."""
+    f = pcm.float().mul_(1.0 / 32768.0)
+    if not downmix:
+        return f.permute(0, 2, 1).contiguous()
+    acc = f[..., 0].clone()
+    for c in range(1, f.shape[-1]):
+        acc.add_(f[..., c])
+    return acc.div_(torch.full((), float(f.shape[-1]), device=acc.device)).unsqueeze(1)
+
+
+def _quantise(v: torch.Tensor) -> torch.Tensor:
+    """float32 ``[S, C, T]`` -> int16 ``[S, T, C]``: clamp(rint(v * 32768), -32768, 32767), the PCM ops' rounding."""
+    return torch.clamp(torch.round(v * 32768.0), -32768.0, 32767.0).to(torch.int16).permute(0, 2, 1).contiguous()
+
+
 class StreamGraph:
     """``g = StreamGraph(cached_pqmf, streams, block)``; then per block ``y, out = g.step(x_block)``.
 
@@ -77,7 +93,8 @@ class StreamPool:
     ``forward`` / ``inverse`` run one direction, with its own state and parity as ``forward_stream`` / ``inverse_stream``; ``reset`` forgets
     streams so that a new session can take their slots.  ``step_pcm16`` / ``forward_pcm16`` / ``inverse_pcm16`` are the same calls with
     16-bit PCM blocks (interleaved WAV frames in, int16 samples out).  ``step_groups`` / ``forward_groups`` / ``inverse_groups`` take up
-    to 8 groups of streams with their own block lengths in one call.
+    to 8 groups of streams with their own block lengths in one call, ``step_groups_pcm16`` / ``forward_groups_pcm16`` /
+    ``inverse_groups_pcm16`` the same with 16-bit PCM blocks.
 
     ``ids`` is a list of ints or a CPU integer tensor (checked: in range and distinct, else ``ValueError``), or a CUDA integer tensor, which
     is trusted as it is and costs no host synchronisation.  With CUDA ids a step allocates nothing but its outputs, so it can be captured
@@ -211,6 +228,41 @@ class StreamPool:
         """``inverse`` to 16-bit PCM: ``[S, C * n_band, F]`` -> int16 ``[S, n_band * F, C]``; row ``r * C + c`` is stream ``ids[r * C + c]``."""
         mod = self.mod
         return torch.ops.pqmf_b200.stream_pool_synthesis_pcm16(s, mod.hk.float(), mod._tables, self.spool, self.sphase, self._ids(ids), mod._flags)
+
+    def step_groups_pcm16(self, groups, downmix: bool = False) -> List[Tuple[torch.Tensor, torch.Tensor]]:
+        """``step_pcm16`` of up to 8 groups ``(pcm_g int16 [S_g, T_g, C_g], ids_g)`` with their own block lengths and channel counts, in one
+        call: returns ``[(pcm_out_g int16 [S_g, T_g, C'_g], y_g [S_g, C'_g * n_band, T_g / n_band])]``; ``downmix`` applies to every group.
+
+        Rows and ids of a group follow ``step_pcm16``; ids follow ``step_groups`` (distinct across all groups).  Per row bit-equal to
+        ``step_groups`` on the widened blocks, then quantised, with the same pool and phase-word updates: the groups ``step_groups`` would
+        run together run together here, with PCM loads and stores in the kernels.  One group is ``step_pcm16``."""
+        blocks, ids = self._group_ids(groups)
+        mod = self.mod
+        if mod.n_band == 1:
+            return [(_quantise(w), w) for w in (_widen(b, downmix) for b in blocks)]
+        outs, ys = torch.ops.pqmf_b200.stream_pool_step_groups_pcm16(blocks, mod.hk.float(), mod._tables, self.xpool, self.xphase, self.spool,
+                                                                     self.sphase, ids, downmix, mod._flags)
+        return list(zip(outs, ys))
+
+    def forward_groups_pcm16(self, groups, downmix: bool = False) -> List[torch.Tensor]:
+        """``forward_pcm16`` of up to 8 groups ``(pcm_g int16 [S_g, T_g, C_g], ids_g)`` in one call (routed as ``step_groups_pcm16``):
+        returns ``[y_g [S_g, C'_g * n_band, T_g / n_band]]``."""
+        blocks, ids = self._group_ids(groups)
+        mod = self.mod
+        if mod.n_band == 1:
+            return [_widen(b, downmix) for b in blocks]
+        return list(torch.ops.pqmf_b200.stream_pool_analysis_groups_pcm16(blocks, mod.hk.float(), mod._tables, self.xpool, self.xphase, ids,
+                                                                          downmix, mod._flags))
+
+    def inverse_groups_pcm16(self, groups) -> List[torch.Tensor]:
+        """``inverse_pcm16`` of up to 8 groups ``(s_g [S_g, C_g * n_band, F_g], ids_g)`` in one call (routed as ``step_groups_pcm16``):
+        returns ``[pcm_out_g int16 [S_g, n_band * F_g, C_g]]``; row ``r * C_g + c`` of a group is stream ``ids_g[r * C_g + c]``."""
+        blocks, ids = self._group_ids(groups)
+        mod = self.mod
+        if mod.n_band == 1:
+            return [_quantise(s) for s in blocks]
+        return list(torch.ops.pqmf_b200.stream_pool_synthesis_groups_pcm16(blocks, mod.hk.float(), mod._tables, self.spool, self.sphase, ids,
+                                                                           mod._flags))
 
     def reset(self, ids=None) -> None:
         """Forget the listed streams (all when ``ids`` is None): zero history in both directions, parity 0; in place, on the device."""
