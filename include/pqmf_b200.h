@@ -319,6 +319,25 @@ int pqmf_roundtrip_x(const void* x, void* y, void* out, const float* hk, const f
 int pqmf_reconstruct_x(const void* x, void* out, void* scratch, size_t scratch_bytes, const float* hk, const float* tables, int B, long T,
                        long n_frames, int M, int L, int delay_frames, unsigned flags, int dtype, pqmf_stream_t stream);
 
+/* ---- half-precision stream pools: pqmf_stream_pool_analysis_x / _synthesis_x / _step_x are the pool entries above
+ *      (pqmf_stream_pool_*_f32) with `void*` blocks, sub-bands and outputs whose element type is `dtype`.  The pool (xpool, spool) and the
+ *      phase words stay fp32 / int32 exactly as for the _f32 entries, so half, fp32 and PCM blocks continue one stream.  With
+ *      PQMF_DTYPE_F32 each one IS the _f32 entry.  With PQMF_DTYPE_F16 / PQMF_DTYPE_BF16 per row the analysis is bit for bit the _f32
+ *      analysis of the widened block followed by a round-to-nearest-even cast of y, the synthesis the _f32 synthesis of the widened
+ *      sub-bands followed by the cast of out, and the step is the analysis followed by the synthesis of the ROUNDED y; pool halves and
+ *      phase words are updated as by the _f32 entries.  Native kernels: the streaming Hankel-4 POOL kernels (n_band 8 / 16 / 32) with half
+ *      loads and stores, exactly where the _f32 pool call with the same rows, T and flags runs them and the half buffers are 16-byte
+ *      aligned.  Every other call (few streams, short or odd blocks, the direct form, split banks, misaligned buffers) returns
+ *      PQMF_ERR_UNSUPPORTED before anything is launched, with pool and phase words untouched; the caller then widens, calls the _f32 entry
+ *      and rounds, one direction at a time (torch_ops.cpp does).  The step is native only when both directions are (three launches, as the
+ *      _f32 step).  Argument errors are checked on the host first (PQMF_ERR_ARG, also for an unknown dtype; n == 0 returns 0). ---- */
+int pqmf_stream_pool_analysis_x(const void* x, void* y, const float* hk, const float* tables, float* xpool, int* xphase, int P, const int* ids,
+                                int n, long T, int M, int L, unsigned flags, int dtype, pqmf_stream_t stream);
+int pqmf_stream_pool_synthesis_x(const void* s, void* out, const float* hk, const float* tables, float* spool, int* sphase, int P, const int* ids,
+                                 int n, long n_frames, int M, int L, unsigned flags, int dtype, pqmf_stream_t stream);
+int pqmf_stream_pool_step_x(const void* x, void* y, void* out, const float* hk, const float* tables, float* xpool, int* xphase, float* spool,
+                            int* sphase, int P, const int* ids, int n, long T, int M, int L, unsigned flags, int dtype, pqmf_stream_t stream);
+
 /* ---- end-to-end host entry (what a non-torch host -- e.g. the Pure Data external that loads the
  *      reference's .ts, README.md:16 -- would call): host buffers in, host buffers out.
  * Pipelines H2D copy, analysis, synthesis and D2H copy over row chunks on internal streams and

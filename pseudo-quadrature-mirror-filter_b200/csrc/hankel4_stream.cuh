@@ -19,6 +19,11 @@
 // int16 PCM edge (IO = H4Io::PCM, pcm.cuh): the analysis reads its block from interleaved WAV frames (any channel count, optional
 // down-mix) and the synthesis of mono rows writes int16 samples.  The history is the fp32 state in both directions: the analysis rolls
 // the WIDENED block into it, so the state after a PCM block is the state after the fp32 block it stands for.
+//
+// Half-precision pools (POOL with IO = H4Io::F16 / BF16, half_io.cuh): blocks, sub-bands and outputs are raw fp16 / bf16 bits behind the
+// same pointers (a launch-time reinterpretation, no new fields), the pool stays fp32.  Block groups load half words one tile ahead and widen
+// them exactly before the fp16 split and the roll, so the pool receives the floats of the fp32 call on the widened block; the drains
+// round to nearest even.  Lockstep calls have no half instantiation.
 #pragma once
 #include <type_traits>
 
@@ -75,9 +80,9 @@ using H4AnalysisStreamArgs = std::conditional_t<POOL, std::conditional_t<IO == H
 // streaming analysis: tiles blockIdx.x, + gridDim.x, ... of spt streams each
 template <int M, bool POOL, H4Io IO>
 __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_stream_kernel(H4AnalysisStreamArgs<POOL, IO> p) {
-  static_assert(IO == H4Io::F32 || IO == H4Io::PCM, "streaming blocks: fp32 rows or int16 PCM frames");
+  static_assert(IO == H4Io::F32 || IO == H4Io::PCM || (POOL && h4_io_half(IO)), "streaming blocks: fp32 rows, int16 PCM frames or half pool rows");
   h4_kernel<true, kH4Workers>(p.g, p.bank, p.n_tiles, 1u, p.pad_bytes, p.trim_lo, p.trim_hi, [&](const H4Smem& sm, uint32_t tmem, uint32_t pfull_leader, unsigned n_iter) {
-    constexpr bool PCM = IO == H4Io::PCM;
+    constexpr bool PCM = IO == H4Io::PCM, HALF = h4_io_half(IO);
     constexpr int FR = 64 / M, HB = M / 2;  // frames per 64-sample row, bands per epilogue thread
     constexpr int NO = (kH4Rows * 8 + kH4Workers - 1) / kH4Workers;  // 4 x 8 samples per thread cover the 128 region rows of a tile
     const H4Shape& g = p.g;
@@ -128,6 +133,9 @@ __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_stream_kernel(H4Ana
           q_slot[r] = t;
           if constexpr (PCM) {
             bofs[r] = (int)off;
+          } else if constexpr (HALF) {  // the running pointer over 2-byte samples: T is a multiple of 256, so steps are whole floats
+            src[r] = reinterpret_cast<const float*>(reinterpret_cast<const uint16_t*>(p.x) + stream0 * p.T + off);
+            src_step[r] = step_x / 2;
           } else {
             src[r] = p.x + stream0 * p.T + off;
             src_step[r] = step_x;
@@ -170,6 +178,9 @@ __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_stream_kernel(H4Ana
             ptx::ldg256_na(p.hist_in + ((size_t)(ph[r] & 1) * p.pool.P + row) * p.L + hofs[r], xr[r]);
           } else if constexpr (PCM) {
             pcm_load8_raw_row(p.in, row_ld + q_slot[r], bofs[r], (int)p.T, xr[r]);  // raw words: converted when the tile is consumed
+          } else if constexpr (HALF) {  // eight half samples = 16 bytes, kept raw in xr[r][0..3] until the tile is consumed
+            const float4 raw = ptx::ldg128_na(reinterpret_cast<const float4*>(src[r]));
+            xr[r][0] = raw.x; xr[r][1] = raw.y; xr[r][2] = raw.z; xr[r][3] = raw.w;
           } else {
             ptx::ldg256_na(src[r], xr[r]);
           }
@@ -199,8 +210,8 @@ __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_stream_kernel(H4Ana
       }
     };
     // fp32 -> fp16 planes; the threads that hold the last L samples of a block also roll the history (here, where the data is
-    // needed anyway: a store next to the load would make every prefetch wait for its own data).  PCM: the block groups' raw words are
-    // widened first (zeros of dead or missing rows widen to zeros), so planes and roll see the floats of the fp32 call.
+    // needed anyway: a store next to the load would make every prefetch wait for its own data).  PCM and half: the block groups' raw words
+    // are widened first (zeros of dead or missing rows widen to zeros), so planes and roll see the floats of the fp32 call.
     auto convert = [&](int pb) {
       unsigned char* p1 = sm.planes + (2 * pb) * g.plane;
       if constexpr (POOL) par_cur = par_ld;
@@ -210,6 +221,8 @@ __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_stream_kernel(H4Ana
         if (u < n_octs) {
           if constexpr (PCM)
             if (bofs[r] >= 0) pcm_convert8(p.in, row_ld + q_slot[r], xr[r]);
+          if constexpr (HALF)
+            if (hofs[r] < 0) h4_widen8<IO>(xr[r]);  // block and padding groups (padding holds zeros); history groups are fp32
           h4_split_store8(xr[r], p1, g.plane, sw128_offset((uint32_t)u * 16u));
           if (roll[r] != nullptr) {
             if (POOL || q_slot[r] < nlive) {  // POOL: load_tile set roll for live groups of this tile only
@@ -227,10 +240,33 @@ __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_stream_kernel(H4Ana
     const bool e_row = et < sg.spt && eq < sg.rows_b;
     float* yrun = p.y + (((size_t)blockIdx.x * sg.spt + et) * M + HB * hb) * F + FR * eq;  // this thread's rows of the CTA's first tile
     const size_t y_step = (size_t)gridDim.x * sg.spt * M * F;
+    [[maybe_unused]] uint16_t* hrun = nullptr;  // half: the same place in the half sub-bands
+    if constexpr (HALF) hrun = reinterpret_cast<uint16_t*>(p.y) + (((size_t)blockIdx.x * sg.spt + et) * M + HB * hb) * F + FR * eq;
     long tile = blockIdx.x, prev_tile = 0;
     auto drain = [&](int dbuf) {
       float v[FR][HB];
       h4_drain_analysis<M>(tmem, dbuf, tid, eq, POOL ? par_prev : p.parity, v);  // the first frame of block row eq is FR eq
+      if constexpr (HALF) {  // round to nearest even; FR consecutive frames = 2 FR bytes per band (16 / 8 / 4 at n_band 8 / 16 / 32)
+        uint16_t* yp = hrun;
+        hrun += y_step;
+        if (!e_row || prev_tile * sg.spt + et >= p.B) return;
+#pragma unroll
+        for (int kk = 0; kk < HB; ++kk) {
+          uint16_t* q = yp + (size_t)kk * F;
+          if constexpr (FR >= 8) {
+#pragma unroll
+            for (int d8 = 0; d8 < FR; d8 += 8)
+              __stcs(reinterpret_cast<uint4*>(q + d8), make_uint4(h4_narrow2<IO>(v[d8][kk], v[d8 + 1][kk]), h4_narrow2<IO>(v[d8 + 2][kk], v[d8 + 3][kk]),
+                                                                h4_narrow2<IO>(v[d8 + 4][kk], v[d8 + 5][kk]), h4_narrow2<IO>(v[d8 + 6][kk], v[d8 + 7][kk])));
+          } else if constexpr (FR == 4) {
+            __stcs(reinterpret_cast<uint2*>(q), make_uint2(h4_narrow2<IO>(v[0][kk], v[1][kk]), h4_narrow2<IO>(v[2][kk], v[3][kk])));
+          } else {
+            static_assert(FR == 2, "n_band 8 / 16 / 32");
+            __stcs(reinterpret_cast<unsigned int*>(q), h4_narrow2<IO>(v[0][kk], v[1][kk]));
+          }
+        }
+        return;
+      }
       float* yp = yrun;
       yrun += y_step;
       if (!e_row || prev_tile * sg.spt + et >= p.B) return;
@@ -294,9 +330,9 @@ using H4SynthesisStreamArgs = std::conditional_t<POOL, std::conditional_t<IO == 
 template <int M, bool POOL, H4Io IO>
 __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_stream_kernel(H4SynthesisStreamArgs<POOL, IO> p) {
   static_assert(M >= 8, "frame quads of 8-band groups (n_band 4 packs its chunks differently: offline kernels only)");
-  static_assert(IO == H4Io::F32 || IO == H4Io::PCM, "streaming blocks: fp32 rows or int16 PCM samples");
+  static_assert(IO == H4Io::F32 || IO == H4Io::PCM || (POOL && h4_io_half(IO)), "streaming blocks: fp32 rows, int16 PCM samples or half pool rows");
   h4_kernel<true, kH4SynWorkers>(p.g, p.bank, p.n_tiles, 1u, p.pad_bytes, p.trim_lo, p.trim_hi, [&](const H4Smem& sm, uint32_t tmem, uint32_t pfull_leader, unsigned n_iter) {
-    constexpr bool PCM = IO == H4Io::PCM;
+    constexpr bool PCM = IO == H4Io::PCM, HALF = h4_io_half(IO);
     constexpr int FR = 64 / M, NBG = M / 8;  // frames per 128-byte plane row, 8-band groups
     const H4Shape& g = p.g;
     const H4StreamGeom& sg = p.sg;
@@ -334,9 +370,15 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_stream_kernel(H
         src_pitch = (size_t)p.K;
       } else if (fb < block_fr) {
         slot = lt;
-        src = p.s + band0 * p.F + fb;
-        src_step = (size_t)gridDim.x * sg.spt * M * p.F;
-        src_pitch = (size_t)p.F;
+        if constexpr (HALF) {  // the running pointer over 2-byte frames: F and fb are multiples of 4, so offsets and steps are whole floats
+          src = reinterpret_cast<const float*>(reinterpret_cast<const uint16_t*>(p.s) + band0 * p.F + fb);
+          src_step = (size_t)gridDim.x * sg.spt * M * p.F / 2;
+          src_pitch = (size_t)p.F / 2;
+        } else {
+          src = p.s + band0 * p.F + fb;
+          src_step = (size_t)gridDim.x * sg.spt * M * p.F;
+          src_pitch = (size_t)p.F;
+        }
         if (fb >= p.F - p.K) {  // the last K frames of the block become the next history
           if constexpr (POOL) rofs = 8 * bg * p.K + (fb - (p.F - p.K));
           else roll = p.state_out + band0 * p.K + (fb - (p.F - p.K));
@@ -354,9 +396,24 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_stream_kernel(H
         const int ph = id >= 0 ? __ldg(p.pool.phase + id) : 0;
         const size_t row = ((size_t)(ph & 1) * p.pool.P + (size_t)id) * M * p.K;  // the stream's current pool row; the next one is (ph & 1) ^ 1
         const float* from = hofs >= 0 ? p.state_in + row + hofs : src;
+        if constexpr (HALF) {  // block items: four half frames per 8-byte load, raw in .x / .y until the tile is consumed
+          const bool raw = hofs < 0;
 #pragma unroll
-        for (int kk = 0; kk < 8; ++kk)
-          v[kk] = id >= 0 ? ptx::ldg128_na(reinterpret_cast<const float4*>(from + (size_t)kk * src_pitch)) : make_float4(0.f, 0.f, 0.f, 0.f);
+          for (int kk = 0; kk < 8; ++kk) {
+            if (id < 0) {
+              v[kk] = make_float4(0.f, 0.f, 0.f, 0.f);
+            } else if (raw) {
+              const float2 h = ptx::ldg64_na(from + (size_t)kk * src_pitch);
+              v[kk] = make_float4(h.x, h.y, 0.f, 0.f);
+            } else {
+              v[kk] = ptx::ldg128_na(reinterpret_cast<const float4*>(from + (size_t)kk * src_pitch));
+            }
+          }
+        } else {
+#pragma unroll
+          for (int kk = 0; kk < 8; ++kk)
+            v[kk] = id >= 0 ? ptx::ldg128_na(reinterpret_cast<const float4*>(from + (size_t)kk * src_pitch)) : make_float4(0.f, 0.f, 0.f, 0.f);
+        }
         src += src_step;
         roll = (rofs >= 0 && id >= 0) ? p.state_out + ((size_t)(~ph & 1) * p.pool.P + (size_t)id) * M * p.K + rofs : nullptr;
         flip_ld = (ph & 2) ? 0u : 0x80000000u;
@@ -374,6 +431,10 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_stream_kernel(H
       if (!has_item) return;
       unsigned char* p1 = sm.planes + (2 * pb) * g.plane;
       const uint32_t fe = POOL ? flip_ld : flip_even, fo = POOL ? flip_ld ^ 0x80000000u : flip_odd;
+      if constexpr (HALF)  // exact, before the roll: the pool receives the widened frames (zeros of dead rows widen to zeros)
+        if (hofs < 0)
+#pragma unroll
+          for (int kk = 0; kk < 8; ++kk) v[kk] = h4_widen4<IO>(v[kk]);
       if (roll != nullptr) {
         if (POOL || slot < nlive) {  // POOL: load_tile set roll for a live item of this tile only
 #pragma unroll
@@ -397,6 +458,8 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_stream_kernel(H
     const size_t out_step = (size_t)gridDim.x * sg.spt * (size_t)(p.F * M);
     [[maybe_unused]] int16_t* prun = nullptr;  // PCM: the same place in the int16 rows
     if constexpr (PCM) prun = p.pcm_out + ((size_t)blockIdx.x * sg.spt + et) * (size_t)(p.F * M) + 64 * eq0 + 32 * hb + 8 * (lane & 3);
+    [[maybe_unused]] uint16_t* hrun = nullptr;  // half: the same place in the half rows
+    if constexpr (HALF) hrun = reinterpret_cast<uint16_t*>(p.out) + ((size_t)blockIdx.x * sg.spt + et) * (size_t)(p.F * M) + 64 * eq0 + 32 * hb + 8 * (lane & 3);
     long tile = blockIdx.x, prev_tile = 0;
     auto drain = [&](int dbuf) {
       if (warp >= 8) return;  // every worker waited for the MMAs; the ninth warp has no TMEM rows to drain
@@ -414,6 +477,16 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_stream_kernel(H
             w[k] = (uint32_t)(uint16_t)pcm_quantise(val[q][2 * k]) | ((uint32_t)(uint16_t)pcm_quantise(val[q][2 * k + 1]) << 16);
           __stcs(reinterpret_cast<uint4*>(pp + (size_t)q * 64), make_uint4(w[0], w[1], w[2], w[3]));
         }
+        return;
+      }
+      if constexpr (HALF) {  // round to nearest even: eight samples = one 16-byte store per slot, as the PCM drain
+        uint16_t* hp = hrun;
+        hrun += out_step;
+        if (!e_rows || prev_tile * sg.spt + et >= p.B) return;
+#pragma unroll
+        for (int q = 0; q < 4; ++q)
+          __stcs(reinterpret_cast<uint4*>(hp + (size_t)q * 64), make_uint4(h4_narrow2<IO>(val[q][0], val[q][1]), h4_narrow2<IO>(val[q][2], val[q][3]),
+                                                                          h4_narrow2<IO>(val[q][4], val[q][5]), h4_narrow2<IO>(val[q][6], val[q][7])));
         return;
       }
       float* op = orun;
@@ -751,7 +824,8 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_stream_groups_k
 }
 
 // launches (CTA pairs; on any error the caller runs other kernels: the fold kernels, or the direct form for pools).  The instantiation
-// follows the call: POOL when pool != nullptr, and the sample format io, F32 or PCM (in: the WAV frames; pcm_out: the mono rows)
+// follows the call: POOL when pool != nullptr, and the sample format io, F32, PCM (in: the WAV frames; pcm_out: the mono rows) or, for pools
+// only, F16 / BF16 (x, y, s and out hold half bits)
 template <int M, bool POOL, H4Io IO>
 inline int h4_launch_analysis_stream(const H4AnalysisStreamParams& base, const StreamPoolIndex* pool, const PcmIn& in, cudaStream_t st) {
   static H4Configured configured;
@@ -764,6 +838,10 @@ inline int h4_launch_analysis_stream(const H4AnalysisStreamParams& base, const S
 }
 template <int M>
 inline int h4_launch_analysis_stream(const H4AnalysisStreamParams& p, const StreamPoolIndex* pool, H4Io io, const PcmIn& in, cudaStream_t st) {
+  if (h4_io_half(io)) {  // pools only (x and y hold half bits)
+    if (!pool) return -2;
+    return io == H4Io::F16 ? h4_launch_analysis_stream<M, true, H4Io::F16>(p, pool, in, st) : h4_launch_analysis_stream<M, true, H4Io::BF16>(p, pool, in, st);
+  }
   if (io == H4Io::PCM) return pool ? h4_launch_analysis_stream<M, true, H4Io::PCM>(p, pool, in, st) : h4_launch_analysis_stream<M, false, H4Io::PCM>(p, pool, in, st);
   return pool ? h4_launch_analysis_stream<M, true, H4Io::F32>(p, pool, in, st) : h4_launch_analysis_stream<M, false, H4Io::F32>(p, pool, in, st);
 }
@@ -779,6 +857,11 @@ inline int h4_launch_synthesis_stream(const H4SynthesisStreamParams& base, const
 }
 template <int M>
 inline int h4_launch_synthesis_stream(const H4SynthesisStreamParams& p, const StreamPoolIndex* pool, H4Io io, int16_t* pcm_out, cudaStream_t st) {
+  if (h4_io_half(io)) {  // pools only (s and out hold half bits)
+    if (!pool) return -2;
+    return io == H4Io::F16 ? h4_launch_synthesis_stream<M, true, H4Io::F16>(p, pool, pcm_out, st)
+                           : h4_launch_synthesis_stream<M, true, H4Io::BF16>(p, pool, pcm_out, st);
+  }
   if (io == H4Io::PCM)
     return pool ? h4_launch_synthesis_stream<M, true, H4Io::PCM>(p, pool, pcm_out, st) : h4_launch_synthesis_stream<M, false, H4Io::PCM>(p, pool, pcm_out, st);
   return pool ? h4_launch_synthesis_stream<M, true, H4Io::F32>(p, pool, pcm_out, st) : h4_launch_synthesis_stream<M, false, H4Io::F32>(p, pool, pcm_out, st);

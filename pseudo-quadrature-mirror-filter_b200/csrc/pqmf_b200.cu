@@ -476,14 +476,14 @@ int fast_synthesis(const float* s, const float* hist, float* out, float* hist_ou
 }
 
 // ---- which kernel family serves which sample format and history.  The dispatchers try them in this order.
-//        family                        | fp32                    | fp16 / bf16            | PCM
-//        Hankel-4                      | offline, lockstep, pool | offline, unsplit banks | all; output: unsplit banks, mono when streaming
-//        fold / Hankel-16 (n_band 16)  | offline, lockstep       | -                      | -
-//        direct form                   | offline, lockstep, pool | -                      | offline
+//        family                        | fp32                    | fp16 / bf16                  | PCM
+//        Hankel-4                      | offline, lockstep, pool | offline, pool; unsplit banks | all; output: unsplit banks, mono when streaming
+//        fold / Hankel-16 (n_band 16)  | offline, lockstep       | -                            | -
+//        direct form                   | offline, lockstep, pool | -                            | offline
 //      (the half-precision instantiations exist for the unsplit banks only; a split bank's second launch accumulates, not in int16;
-//      streaming PCM output is mono rows: the two channels of a clip may sit in any two tiles) ----
+//      streaming PCM output is mono rows: the two channels of a clip may sit in any two tiles; lockstep streaming stays fp32 and PCM) ----
 bool h4_serves(const Samples& s, const History& h, unsigned flags, bool output) {
-  if (pqmf::h4_io_half(s.io)) return !h.in && !(flags & PQMF_FLAG_H4_SPLIT);
+  if (pqmf::h4_io_half(s.io)) return (!h.in || h.pool) && !(flags & PQMF_FLAG_H4_SPLIT);
   if (s.io == pqmf::H4Io::PCM && output) return !(flags & PQMF_FLAG_H4_SPLIT) && (!h.in || s.pcm.C == 1);
   return true;
 }
@@ -1313,6 +1313,60 @@ int pqmf_stream_pool_step_groups_pcm16(const pqmf_pool_group_pcm16* groups, int 
                                        pqmf_stream_t stream) {
   return pool_groups({PoolDir::kStep, nullptr, G, hk, tables, xpool, spool, xphase, sphase, P, M, L, flags, (cudaStream_t)stream, pqmf::H4Io::PCM,
                       groups, downmix ? 1 : 0, staged});
+}
+
+// ---- half-precision pools: the streaming Hankel-4 POOL kernels with fp16 / bf16 loads and stores, exactly where the fp32 pool call with the
+//      same rows runs those kernels (h4_takes_*, with 16-byte aligned half buffers); every other call returns PQMF_ERR_UNSUPPORTED before
+//      anything is launched and the caller stages it direction by direction through the fp32 entries ----
+int pqmf_stream_pool_analysis_x(const void* x, void* y, const float* hk, const float* tables, float* xpool, int* xphase, int P, const int* ids,
+                                int n, long T, int M, int L, unsigned flags, int dtype, pqmf_stream_t stream) {
+  if (dtype == PQMF_DTYPE_F32)
+    return pqmf_stream_pool_analysis_f32(static_cast<const float*>(x), static_cast<float*>(y), hk, tables, xpool, xphase, P, ids, n, T, M, L, flags,
+                                         stream);
+  pqmf::H4Io io;
+  if (!half_io_of(dtype, io) || bad_dims(n, T, M, L) || bad_pool(P, n) || T <= 0 || (T % M) != 0) return PQMF_ERR_ARG;
+  if (n == 0) return PQMF_OK;
+  if (!x || !y || !hk || !xpool || !xphase || !ids) return PQMF_ERR_ARG;
+  cudaStream_t st = (cudaStream_t)stream;
+  const PoolRows pool{ids, xphase, P};
+  if (int e = run_analysis(samples(x, io), y, pooled(xpool, pool), hk, tables, n, T, T / M, M, L, flags, st)) return e;
+  return pool_phase(pool, n, xphase, T / M, nullptr, 0, st);
+}
+
+int pqmf_stream_pool_synthesis_x(const void* s, void* out, const float* hk, const float* tables, float* spool, int* sphase, int P, const int* ids,
+                                 int n, long n_frames, int M, int L, unsigned flags, int dtype, pqmf_stream_t stream) {
+  if (dtype == PQMF_DTYPE_F32)
+    return pqmf_stream_pool_synthesis_f32(static_cast<const float*>(s), static_cast<float*>(out), hk, tables, spool, sphase, P, ids, n, n_frames, M, L,
+                                          flags, stream);
+  pqmf::H4Io io;
+  if (!half_io_of(dtype, io) || bad_dims(n, n_frames, M, L) || bad_pool(P, n) || n_frames <= 0 || (L % M) != 0) return PQMF_ERR_ARG;
+  if (n == 0) return PQMF_OK;
+  if (!s || !out || !hk || !spool || !sphase || !ids) return PQMF_ERR_ARG;
+  cudaStream_t st = (cudaStream_t)stream;
+  const PoolRows pool{ids, sphase, P};
+  if (int e = run_synthesis(s, samples(out, io), pooled(spool, pool), hk, tables, n, n_frames, M, L, 0, flags, st)) return e;
+  return pool_phase(pool, n, nullptr, 0, sphase, n_frames, st);
+}
+
+int pqmf_stream_pool_step_x(const void* x, void* y, void* out, const float* hk, const float* tables, float* xpool, int* xphase, float* spool,
+                            int* sphase, int P, const int* ids, int n, long T, int M, int L, unsigned flags, int dtype, pqmf_stream_t stream) {
+  if (dtype == PQMF_DTYPE_F32)
+    return pqmf_stream_pool_step_f32(static_cast<const float*>(x), static_cast<float*>(y), static_cast<float*>(out), hk, tables, xpool, xphase, spool,
+                                     sphase, P, ids, n, T, M, L, flags, stream);
+  pqmf::H4Io io;
+  if (!half_io_of(dtype, io) || bad_dims(n, T, M, L) || bad_pool(P, n) || T <= 0 || (T % M) != 0 || (L % M) != 0) return PQMF_ERR_ARG;
+  if (n == 0) return PQMF_OK;
+  if (!x || !y || !out || !hk || !xpool || !xphase || !spool || !sphase || !ids || xphase == sphase) return PQMF_ERR_ARG;
+  const PoolRows xrows{ids, xphase, P}, srows{ids, sphase, P};
+  const Samples in = samples(x, io), res = samples(out, io);
+  const History xh = pooled(xpool, xrows), sh = pooled(spool, srows);
+  // both directions native, or nothing is launched; the synthesis reads the rounded sub-bands the analysis wrote
+  if (!h4_takes_analysis(in, y, xh, n, T, T / M, M, L, tables, flags) || !h4_takes_synthesis(y, res, sh, n, T / M, M, L, tables, flags))
+    return PQMF_ERR_UNSUPPORTED;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (int e = run_analysis(in, y, xh, hk, tables, n, T, T / M, M, L, flags, st)) return e;
+  if (run_synthesis(y, res, sh, hk, tables, n, T / M, M, L, 0, flags, st) != 0) return (int)cudaErrorLaunchFailure;  // see pqmf_stream_step_pcm16
+  return pool_phase(xrows, n, xphase, T / M, sphase, T / M, st);
 }
 
 // ---- int16 PCM blocks in the streaming calls: the streaming Hankel-4 kernels with PCM loads (any channel count, optional down-mix) and

@@ -394,6 +394,94 @@ std::tuple<at::Tensor, at::Tensor> stream_pool_step(const at::Tensor& x, const a
   return {out, y};
 }
 
+// ---- half-precision pools (pqmf_stream_pool_*_x): blocks, sub-bands and outputs of the pool's dtype (float32, float16 or bfloat16), the
+//      pool itself fp32.  A tensor of another dtype is refused.  Where the library has no native kernel (PQMF_ERR_UNSUPPORTED, nothing
+//      launched) the op stages the call one direction at a time: widen, the fp32 pool op, round -- so a staged step's synthesis reads the
+//      rounded sub-bands, as the native step's does ----
+int pool_dtype(const at::Tensor& t, at::ScalarType dtype, const char* name) {
+  TORCH_CHECK(t.is_cuda(), name, " must be a CUDA tensor (pqmf_b200 has no CPU fallback)");
+  TORCH_CHECK(dtype == at::kFloat || dtype == at::kHalf || dtype == at::kBFloat16, "a stream pool's dtype must be float32, float16 or bfloat16, got ",
+              dtype);
+  TORCH_CHECK(t.scalar_type() == dtype, name, " must be ", dtype, " (the pool's dtype), got ", t.scalar_type());
+  return dtype == at::kFloat ? PQMF_DTYPE_F32 : dtype == at::kHalf ? PQMF_DTYPE_F16 : PQMF_DTYPE_BF16;
+}
+
+// x [n, 1, T] -> y [n, M, T / M], both of dtype
+at::Tensor stream_pool_analysis_x(const at::Tensor& x, const at::Tensor& hk, const at::Tensor& tables, at::Tensor xpool, at::Tensor xphase,
+                                  const at::Tensor& ids, at::ScalarType dtype, int64_t flags) {
+  const int code = pool_dtype(x, dtype, "x");
+  TORCH_CHECK(x.dim() == 3 && x.size(1) == 1, "pqmf stream pool analysis expects [streams, 1, block], got ", x.sizes());
+  const Bank bank = bank_of(hk, x);
+  c10::cuda::CUDAGuard guard(x.device());
+  const at::Tensor xc = x.contiguous();
+  const int64_t n = xc.size(0), T = xc.size(2);
+  TORCH_CHECK(T > 0 && T % bank.M == 0, "streaming block length ", T, " must be a positive multiple of n_band=", bank.M);
+  const Pool pool = pool_of(xpool, xphase, bank, x, "xpool");
+  const int* id = ids_of(ids, n, x);
+  TORCH_CHECK(n <= pool.P, "more rows (", n, ") than streams in the pool (", pool.P, ")");
+  at::Tensor y = at::empty({n, bank.M, T / bank.M}, xc.options());
+  if (n == 0) return y;
+  const int rc = pqmf_stream_pool_analysis_x(xc.data_ptr(), y.data_ptr(), bank.ptr, tables_ptr(tables, x), pool.state, pool.phase, (int)pool.P, id,
+                                             (int)n, (long)T, (int)bank.M, (int)bank.L, (unsigned)flags, code,
+                                             (pqmf_stream_t)at::cuda::getCurrentCUDAStream().stream());
+  if (staged(rc, code)) return stream_pool_analysis(xc.to(at::kFloat), hk, tables, xpool, xphase, ids, flags).to(dtype);
+  check_rc(rc, "pqmf_stream_pool_analysis_x");
+  return y;
+}
+
+// s [n, M, F] -> out [n, 1, M F], both of dtype
+at::Tensor stream_pool_synthesis_x(const at::Tensor& s, const at::Tensor& hk, const at::Tensor& tables, at::Tensor spool, at::Tensor sphase,
+                                   const at::Tensor& ids, at::ScalarType dtype, int64_t flags) {
+  const int code = pool_dtype(s, dtype, "s");
+  const Bank bank = bank_of(hk, s);
+  TORCH_CHECK(s.dim() == 3 && s.size(1) == bank.M, "pqmf stream pool synthesis expects [streams, n_band, frames], got ", s.sizes());
+  TORCH_CHECK(bank.L % bank.M == 0, "streaming synthesis needs L a multiple of n_band");
+  c10::cuda::CUDAGuard guard(s.device());
+  const at::Tensor sc = s.contiguous();
+  const int64_t n = sc.size(0), F = sc.size(2);
+  TORCH_CHECK(F > 0, "empty block");
+  const Pool pool = pool_of(spool, sphase, bank, s, "spool");
+  const int* id = ids_of(ids, n, s);
+  TORCH_CHECK(n <= pool.P, "more rows (", n, ") than streams in the pool (", pool.P, ")");
+  at::Tensor out = at::empty({n, 1, bank.M * F}, sc.options());
+  if (n == 0) return out;
+  const int rc = pqmf_stream_pool_synthesis_x(sc.data_ptr(), out.data_ptr(), bank.ptr, tables_ptr(tables, s), pool.state, pool.phase, (int)pool.P, id,
+                                              (int)n, (long)F, (int)bank.M, (int)bank.L, (unsigned)flags, code,
+                                             (pqmf_stream_t)at::cuda::getCurrentCUDAStream().stream());
+  if (staged(rc, code)) return stream_pool_synthesis(sc.to(at::kFloat), hk, tables, spool, sphase, ids, flags).to(dtype);
+  check_rc(rc, "pqmf_stream_pool_synthesis_x");
+  return out;
+}
+
+// one block step of the listed streams: (out [n, 1, T], y [n, M, T / M]), both of dtype; the synthesis reads the rounded y
+std::tuple<at::Tensor, at::Tensor> stream_pool_step_x(const at::Tensor& x, const at::Tensor& hk, const at::Tensor& tables, at::Tensor xpool,
+                                                       at::Tensor xphase, at::Tensor spool, at::Tensor sphase, const at::Tensor& ids,
+                                                       at::ScalarType dtype, int64_t flags) {
+  const int code = pool_dtype(x, dtype, "x");
+  TORCH_CHECK(x.dim() == 3 && x.size(1) == 1, "pqmf stream pool step expects [streams, 1, block], got ", x.sizes());
+  const Bank bank = bank_of(hk, x);
+  c10::cuda::CUDAGuard guard(x.device());
+  const at::Tensor xc = x.contiguous();
+  const int64_t n = xc.size(0), T = xc.size(2);
+  TORCH_CHECK(T > 0 && T % bank.M == 0 && bank.L % bank.M == 0, "streaming block length ", T, " must be a positive multiple of n_band=", bank.M);
+  const Pool xp = pool_of(xpool, xphase, bank, x, "xpool"), sp = pool_of(spool, sphase, bank, x, "spool");
+  TORCH_CHECK(xp.P == sp.P, "the analysis and synthesis pools hold different numbers of streams");
+  const int* id = ids_of(ids, n, x);
+  TORCH_CHECK(n <= xp.P, "more rows (", n, ") than streams in the pool (", xp.P, ")");
+  at::Tensor y = at::empty({n, bank.M, T / bank.M}, xc.options());
+  at::Tensor out = at::empty({n, 1, T}, xc.options());
+  if (n == 0) return {out, y};
+  const int rc = pqmf_stream_pool_step_x(xc.data_ptr(), y.data_ptr(), out.data_ptr(), bank.ptr, tables_ptr(tables, x), xp.state, xp.phase, sp.state,
+                                         sp.phase, (int)xp.P, id, (int)n, (long)T, (int)bank.M, (int)bank.L, (unsigned)flags, code,
+                                             (pqmf_stream_t)at::cuda::getCurrentCUDAStream().stream());
+  if (staged(rc, code)) {  // direction by direction, each native where it can be (never the fp32 step on the widened block)
+    at::Tensor ys = stream_pool_analysis_x(xc, hk, tables, xpool, xphase, ids, dtype, flags);
+    return {stream_pool_synthesis_x(ys, hk, tables, spool, sphase, ids, dtype, flags), ys};
+  }
+  check_rc(rc, "pqmf_stream_pool_step_x");
+  return {out, y};
+}
+
 // ---- grouped pool calls (pqmf_stream_pool_*_groups_f32): up to 8 groups of rows, each with its own block length.  Every group is
 //      checked before anything is launched; the ids stay one tensor per group (one device pointer each, nothing concatenated) ----
 enum class GroupsDir { kAnalysis, kSynthesis, kStep };
@@ -986,6 +1074,35 @@ std::tuple<at::Tensor, at::Tensor> stream_pool_step_autograd(const at::Tensor& x
   return op.call(x, hk, tables, xpool, xphase, spool, sphase, ids, flags);
 }
 
+at::Tensor stream_pool_analysis_x_autograd(const at::Tensor& x, const at::Tensor& hk, const at::Tensor& tables, at::Tensor xpool, at::Tensor xphase,
+                                           const at::Tensor& ids, at::ScalarType dtype, int64_t flags) {
+  TORCH_CHECK(!(at::GradMode::is_enabled() && x.requires_grad()),
+              "pqmf_b200::stream_pool_analysis_x is not differentiable (a stream pool carries state across calls); use forward() for training "
+              "or wrap the call in torch.no_grad()");
+  at::AutoDispatchBelowADInplaceOrView guard;
+  static auto op = c10::Dispatcher::singleton().findSchemaOrThrow("pqmf_b200::stream_pool_analysis_x", "").typed<decltype(stream_pool_analysis_x)>();
+  return op.call(x, hk, tables, xpool, xphase, ids, dtype, flags);
+}
+at::Tensor stream_pool_synthesis_x_autograd(const at::Tensor& s, const at::Tensor& hk, const at::Tensor& tables, at::Tensor spool, at::Tensor sphase,
+                                            const at::Tensor& ids, at::ScalarType dtype, int64_t flags) {
+  TORCH_CHECK(!(at::GradMode::is_enabled() && s.requires_grad()),
+              "pqmf_b200::stream_pool_synthesis_x is not differentiable (a stream pool carries state across calls); use inverse() for training "
+              "or wrap the call in torch.no_grad()");
+  at::AutoDispatchBelowADInplaceOrView guard;
+  static auto op = c10::Dispatcher::singleton().findSchemaOrThrow("pqmf_b200::stream_pool_synthesis_x", "").typed<decltype(stream_pool_synthesis_x)>();
+  return op.call(s, hk, tables, spool, sphase, ids, dtype, flags);
+}
+std::tuple<at::Tensor, at::Tensor> stream_pool_step_x_autograd(const at::Tensor& x, const at::Tensor& hk, const at::Tensor& tables, at::Tensor xpool,
+                                                               at::Tensor xphase, at::Tensor spool, at::Tensor sphase, const at::Tensor& ids,
+                                                               at::ScalarType dtype, int64_t flags) {
+  TORCH_CHECK(!(at::GradMode::is_enabled() && x.requires_grad()),
+              "pqmf_b200::stream_pool_step_x is not differentiable (a stream pool carries state across calls); use forward() / inverse() for "
+              "training or wrap the call in torch.no_grad()");
+  at::AutoDispatchBelowADInplaceOrView guard;
+  static auto op = c10::Dispatcher::singleton().findSchemaOrThrow("pqmf_b200::stream_pool_step_x", "").typed<decltype(stream_pool_step_x)>();
+  return op.call(x, hk, tables, xpool, xphase, spool, sphase, ids, dtype, flags);
+}
+
 bool any_requires_grad(at::TensorList ts) {
   for (const at::Tensor& t : ts)
     if (t.requires_grad()) return true;
@@ -1146,6 +1263,15 @@ TORCH_LIBRARY(pqmf_b200, m) {
   m.def(
       "stream_pool_step_groups_pcm16(Tensor[] pcms, Tensor hk, Tensor tables, Tensor(a!) xpool, Tensor(b!) xphase, Tensor(c!) spool, "
       "Tensor(d!) sphase, Tensor[] ids, bool downmix, int flags) -> (Tensor[], Tensor[])");
+  m.def(
+      "stream_pool_analysis_x(Tensor x, Tensor hk, Tensor tables, Tensor(a!) xpool, Tensor(b!) xphase, Tensor ids, ScalarType dtype, int flags) "
+      "-> Tensor");
+  m.def(
+      "stream_pool_synthesis_x(Tensor s, Tensor hk, Tensor tables, Tensor(a!) spool, Tensor(b!) sphase, Tensor ids, ScalarType dtype, int flags) "
+      "-> Tensor");
+  m.def(
+      "stream_pool_step_x(Tensor x, Tensor hk, Tensor tables, Tensor(a!) xpool, Tensor(b!) xphase, Tensor(c!) spool, Tensor(d!) sphase, "
+      "Tensor ids, ScalarType dtype, int flags) -> (Tensor, Tensor)");
   m.def("launch_count() -> int", &launch_count);
 }
 
@@ -1175,6 +1301,9 @@ TORCH_LIBRARY_IMPL(pqmf_b200, CUDA, m) {
   m.impl("stream_pool_analysis_groups_pcm16", &stream_pool_analysis_groups_pcm16);
   m.impl("stream_pool_synthesis_groups_pcm16", &stream_pool_synthesis_groups_pcm16);
   m.impl("stream_pool_step_groups_pcm16", &stream_pool_step_groups_pcm16);
+  m.impl("stream_pool_analysis_x", &stream_pool_analysis_x);
+  m.impl("stream_pool_synthesis_x", &stream_pool_synthesis_x);
+  m.impl("stream_pool_step_x", &stream_pool_step_x);
 }
 
 // gradients w.r.t. the signal / the sub-bands only (the bank is a registered buffer in the reference, not a parameter)
@@ -1195,4 +1324,7 @@ TORCH_LIBRARY_IMPL(pqmf_b200, Autograd, m) {
   m.impl("stream_pool_analysis_groups_pcm16", &stream_pool_analysis_groups_pcm16_autograd);
   m.impl("stream_pool_synthesis_groups_pcm16", &stream_pool_synthesis_groups_pcm16_autograd);
   m.impl("stream_pool_step_groups_pcm16", &stream_pool_step_groups_pcm16_autograd);
+  m.impl("stream_pool_analysis_x", &stream_pool_analysis_x_autograd);
+  m.impl("stream_pool_synthesis_x", &stream_pool_synthesis_x_autograd);
+  m.impl("stream_pool_step_x", &stream_pool_step_x_autograd);
 }

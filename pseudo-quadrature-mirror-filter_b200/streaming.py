@@ -7,7 +7,7 @@ history from one buffer and write the new history to another (ping-pong), so a s
 captures TWO graphs -- even and odd steps -- over fixed input / state / output buffers and alternates between them.
 
 ``StreamPool`` serves many independent sessions instead of one lockstep batch: each call steps any subset of the pool's streams, each
-with its own history, ping-pong half and frame parity kept on the device.
+with its own history, ping-pong half and frame parity kept on the device.  A pool may take float32, float16 or bfloat16 blocks.
 """
 from __future__ import annotations
 
@@ -27,6 +27,17 @@ def _widen(pcm: torch.Tensor, downmix: bool) -> torch.Tensor:
     for c in range(1, f.shape[-1]):
         acc.add_(f[..., c])
     return acc.div_(torch.full((), float(f.shape[-1]), device=acc.device)).unsqueeze(1)
+
+
+# the names torch's C++ side gives dtypes in its errors ("x must be BFloat16 (the pool's dtype), got Float")
+_ATEN_NAMES = {torch.float32: "Float", torch.float16: "Half", torch.bfloat16: "BFloat16", torch.float64: "Double", torch.int16: "Short",
+               torch.int32: "Int", torch.int64: "Long"}
+POOL_DTYPES = (torch.float32, torch.float16, torch.bfloat16)
+
+
+def _check_dtype(t: torch.Tensor, dtype: torch.dtype, name: str) -> None:
+    if t.dtype != dtype:
+        raise RuntimeError(f"{name} must be {_ATEN_NAMES[dtype]} (the pool's dtype), got {_ATEN_NAMES.get(t.dtype, str(t.dtype))}")
 
 
 def _quantise(v: torch.Tensor) -> torch.Tensor:
@@ -85,7 +96,7 @@ class StreamGraph:
 
 
 class StreamPool:
-    """Device-resident streaming state for ``capacity`` independent streams of one ``CachedPQMF`` (fp32).
+    """Device-resident streaming state for ``capacity`` independent streams of one ``CachedPQMF``.
 
     ``pool = StreamPool(mod, capacity)``; then per call ``out, y = pool.step(x, ids)``: ``x`` ``[n, 1, T]`` holds the next block of each of
     the ``n`` distinct streams ``ids`` (in any order; streams not listed are left exactly as they are), and returns their signal
@@ -102,16 +113,27 @@ class StreamPool:
     number of frames per block.
 
     The pool reads ``mod.hk``, ``mod._tables`` and ``mod._flags`` at every call (``load_state_dict``, casts and ``refresh_tables`` carry
-    through) and uses none of ``mod``'s own streaming state.  One pool is stepped from one CUDA stream at a time."""
+    through) and uses none of ``mod``'s own streaming state.  One pool is stepped from one CUDA stream at a time.
 
-    def __init__(self, mod, capacity: int):
+    ``dtype`` (float32, float16 or bfloat16; independent of the module's dtype) is the element type of the float blocks and sub-bands
+    that ``step`` / ``forward`` / ``inverse`` and the grouped float calls take and return; a block of another dtype raises.  The pool's state
+    stays float32 whatever the dtype.  On a half pool, per row ``forward(x)`` is bit for bit ``forward(x.float())`` of a float32 pool
+    rounded to ``dtype``, ``inverse(y)`` likewise, and ``step(x)`` is ``forward`` followed by ``inverse`` of the ROUNDED sub-bands, with the
+    state and phase words of that float32 pool.  ``step`` / ``forward`` / ``inverse`` run the streaming Hankel-4 kernels with half loads
+    and stores where the float32 pool would run those kernels; other calls and the grouped float calls are staged (widen, float32 call,
+    round) direction by direction.  The PCM calls are those of a float32 pool."""
+
+    def __init__(self, mod, capacity: int, dtype: torch.dtype = torch.float32):
         if capacity < 1:
             raise ValueError(f"StreamPool needs a capacity of at least 1, got {capacity}")
+        if dtype not in POOL_DTYPES:
+            raise ValueError(f"StreamPool dtype must be torch.float32, torch.float16 or torch.bfloat16, got {dtype}")
         dev = mod.hk.device
         if dev.type != "cuda":
             raise RuntimeError("StreamPool needs the module on a CUDA device")
         self.mod = mod
         self.capacity = int(capacity)
+        self.dtype = dtype
         m, length = mod.hk.shape
         self.xpool = torch.zeros(2, capacity, length, device=dev)
         self.spool = torch.zeros(2, capacity, m, max(length // m, 1), device=dev)
@@ -137,11 +159,20 @@ class StreamPool:
             raise ValueError("stream ids must be distinct")
         return torch.tensor(host, dtype=torch.int32).to(dev)
 
+    @property
+    def _half(self) -> bool:
+        return self.dtype != torch.float32
+
     def step(self, x: torch.Tensor, ids) -> Tuple[torch.Tensor, torch.Tensor]:
         """One block of the listed streams through analysis and synthesis: returns ``(out, y)``."""
         mod = self.mod
         if mod.n_band == 1:
+            if self._half:
+                _check_dtype(x, self.dtype, "x")
             return x, x
+        if self._half:
+            return torch.ops.pqmf_b200.stream_pool_step_x(x, mod.hk.float(), mod._tables, self.xpool, self.xphase, self.spool, self.sphase,
+                                                          self._ids(ids), self.dtype, mod._flags)
         return torch.ops.pqmf_b200.stream_pool_step(x, mod.hk.float(), mod._tables, self.xpool, self.xphase, self.spool, self.sphase,
                                                     self._ids(ids), mod._flags)
 
@@ -149,14 +180,24 @@ class StreamPool:
         """Streaming analysis of one block of the listed streams: ``[n, 1, T]`` -> ``[n, n_band, T / n_band]``."""
         mod = self.mod
         if mod.n_band == 1:
+            if self._half:
+                _check_dtype(x, self.dtype, "x")
             return x
+        if self._half:
+            return torch.ops.pqmf_b200.stream_pool_analysis_x(x, mod.hk.float(), mod._tables, self.xpool, self.xphase, self._ids(ids), self.dtype,
+                                                              mod._flags)
         return torch.ops.pqmf_b200.stream_pool_analysis(x, mod.hk.float(), mod._tables, self.xpool, self.xphase, self._ids(ids), mod._flags)
 
     def inverse(self, y: torch.Tensor, ids) -> torch.Tensor:
         """Streaming synthesis of one block of the listed streams: ``[n, n_band, F]`` -> ``[n, 1, n_band * F]``."""
         mod = self.mod
         if mod.n_band == 1:
+            if self._half:
+                _check_dtype(y, self.dtype, "s")
             return y
+        if self._half:
+            return torch.ops.pqmf_b200.stream_pool_synthesis_x(y, mod.hk.float(), mod._tables, self.spool, self.sphase, self._ids(ids), self.dtype,
+                                                               mod._flags)
         return torch.ops.pqmf_b200.stream_pool_synthesis(y, mod.hk.float(), mod._tables, self.spool, self.sphase, self._ids(ids), mod._flags)
 
     MAX_GROUPS = 8
@@ -184,7 +225,13 @@ class StreamPool:
         The groups the streaming Hankel-4 kernels can take run together in one launch per direction when they make enough tiles together
         (so small groups of several block lengths reach the tensor cores); each of their rows is what those kernels give it in a pool
         call.  Every other group gives exactly what ``step(x_g, ids_g)`` gives; one group is ``step``.  ids follow ``step``'s rules and must
-        be distinct across all groups."""
+        be distinct across all groups.  On a half pool the call is staged direction by direction: ``forward_groups`` then ``inverse_groups``
+        of the rounded sub-bands."""
+        if self._half:
+            groups = list(groups)
+            ys = self.forward_groups(groups)
+            outs = self.inverse_groups([(y, gids) for y, (_, gids) in zip(ys, groups)])
+            return list(zip(outs, ys))
         blocks, ids = self._group_ids(groups)
         mod = self.mod
         if mod.n_band == 1:
@@ -193,21 +240,33 @@ class StreamPool:
                                                                self.sphase, ids, mod._flags)
         return list(zip(outs, ys))
 
+    def _widened(self, blocks: List[torch.Tensor], name: str) -> List[torch.Tensor]:
+        """Half pool: the groups' blocks, checked against the pool's dtype, as float32 (exact)."""
+        for b in blocks:
+            _check_dtype(b, self.dtype, name)
+        return [b.float() for b in blocks]
+
     def forward_groups(self, groups) -> List[torch.Tensor]:
         """``forward`` of up to 8 groups ``(x_g [n_g, 1, T_g], ids_g)`` in one call (routed as ``step_groups``): returns ``[y_g]``."""
         blocks, ids = self._group_ids(groups)
         mod = self.mod
+        if self._half:
+            blocks = self._widened(blocks, "x")
         if mod.n_band == 1:
-            return blocks
-        return list(torch.ops.pqmf_b200.stream_pool_analysis_groups(blocks, mod.hk.float(), mod._tables, self.xpool, self.xphase, ids, mod._flags))
+            return [b.to(self.dtype) for b in blocks] if self._half else blocks
+        ys = torch.ops.pqmf_b200.stream_pool_analysis_groups(blocks, mod.hk.float(), mod._tables, self.xpool, self.xphase, ids, mod._flags)
+        return [y.to(self.dtype) for y in ys] if self._half else list(ys)
 
     def inverse_groups(self, groups) -> List[torch.Tensor]:
         """``inverse`` of up to 8 groups ``(y_g [n_g, n_band, F_g], ids_g)`` in one call (routed as ``step_groups``): returns ``[out_g]``."""
         blocks, ids = self._group_ids(groups)
         mod = self.mod
+        if self._half:
+            blocks = self._widened(blocks, "s")
         if mod.n_band == 1:
-            return blocks
-        return list(torch.ops.pqmf_b200.stream_pool_synthesis_groups(blocks, mod.hk.float(), mod._tables, self.spool, self.sphase, ids, mod._flags))
+            return [b.to(self.dtype) for b in blocks] if self._half else blocks
+        outs = torch.ops.pqmf_b200.stream_pool_synthesis_groups(blocks, mod.hk.float(), mod._tables, self.spool, self.sphase, ids, mod._flags)
+        return [o.to(self.dtype) for o in outs] if self._half else list(outs)
 
     def step_pcm16(self, pcm: torch.Tensor, ids, downmix: bool = False) -> Tuple[torch.Tensor, torch.Tensor]:
         """``step`` from 16-bit PCM to 16-bit PCM: ``pcm`` int16 ``[S, T, channels]`` -> ``(pcm_out int16 [S, T, C'], y [S, C' * n_band,
