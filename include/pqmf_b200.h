@@ -185,7 +185,8 @@ int pqmf_stream_pool_step_f32(const float* x, float* y, float* out, const float*
 /* ---- grouped pool calls: sessions of different block lengths (a server whose clients choose their buffer sizes) stepped in one call.
  *      A group is n rows of one block length T (samples): ids [n] (device int32), x [n, T], y [n, M, T/M], out [n, T].  The analysis reads
  *      x and writes y, the synthesis reads y and writes out, the step does both; a pointer the direction does not use may be NULL.
- *      Up to 8 groups per call; ids distinct across ALL groups, at most P rows in total; n == 0 groups are allowed; fp32 only.
+ *      Up to 8 groups per call; ids distinct across ALL groups, at most P rows in total; n == 0 groups are allowed.  fp32 blocks here;
+ *      int16 PCM and half-precision blocks in the _pcm16 and _x grouped entries below.
  *      Routing: the groups the streaming Hankel-4 kernels can plan (n_band 8 / 16 / 32, the block geometry, flags and alignment that a
  *      single-group call would need, whatever their own tile count) run together in ONE launch per direction followed by one phase-word
  *      launch, provided there are at least two of them and they make >= 96 tiles together (each direction, for a step).  Each of their rows
@@ -276,6 +277,36 @@ int pqmf_stream_pool_synthesis_groups_pcm16(const pqmf_pool_group_pcm16* groups,
 int pqmf_stream_pool_step_groups_pcm16(const pqmf_pool_group_pcm16* groups, int G, int downmix, const float* hk, const float* tables, float* xpool,
                                        int* xphase, float* spool, int* sphase, int P, int M, int L, unsigned flags, unsigned* staged,
                                        pqmf_stream_t stream);
+
+/* ---- grouped pool calls with half-precision blocks: the grouped entries above (pqmf_stream_pool_*_groups_f32) with `void*` x, y and out
+ *      whose element type is `dtype` (PQMF_DTYPE_*, see the half-precision pools below); the pool and phase words stay fp32 / int32.  With
+ *      PQMF_DTYPE_F32 each one IS the _f32 grouped entry (and sets *staged = 0).  With PQMF_DTYPE_F16 / PQMF_DTYPE_BF16 per row the analysis
+ *      is bit for bit pqmf_stream_pool_analysis_groups_f32 on the widened blocks followed by a round-to-nearest-even cast of y, the synthesis
+ *      likewise on the widened sub-bands; pool halves and phase words are updated as by the fp32 call.  There is no grouped half step: a
+ *      half step is the analysis followed by the synthesis of the ROUNDED sub-bands, and the two directions may join different groups.
+ *      Rule, as for the PCM groups:
+ *        1. All argument checks on the host first (PQMF_ERR_ARG): an unknown dtype, the single-group _x entries' checks per group,
+ *           0 <= G <= 8, at most P rows in all, staged != NULL.  G == 0 and all-empty calls return 0.
+ *        2. The joined groups are those the fp32 grouped call of the same direction would join on freshly allocated fp32 blocks and
+ *           sub-bands (the half buffers' alignment does not decide it).
+ *        3. If a joined group cannot run natively (a half x, y or out not 16-byte aligned) or the grouped launch does not start, the call
+ *           returns PQMF_ERR_UNSUPPORTED with nothing launched: the caller widens every group, calls the fp32 grouped entry and rounds.
+ *        4. Otherwise one GROUPS half launch and one phase-word launch for the joined groups, then every other group through its
+ *           pqmf_stream_pool_*_x entry.  Where that entry refuses, bit k of *staged is set and the call goes on; the caller then runs group k
+ *           through the single-group pool calls on the widened block.  *staged is 0 otherwise.  Returns 0.
+ *      G == 1 is the group's pqmf_stream_pool_*_x entry (a refusal sets bit 0). ---- */
+typedef struct pqmf_pool_group_x {
+  const int* ids;
+  int n;
+  long T;
+  const void* x;
+  void* y;
+  void* out;
+} pqmf_pool_group_x;
+int pqmf_stream_pool_analysis_groups_x(const pqmf_pool_group_x* groups, int G, const float* hk, const float* tables, float* xpool, int* xphase,
+                                       int P, int M, int L, unsigned flags, int dtype, unsigned* staged, pqmf_stream_t stream);
+int pqmf_stream_pool_synthesis_groups_x(const pqmf_pool_group_x* groups, int G, const float* hk, const float* tables, float* spool, int* sphase,
+                                        int P, int M, int L, unsigned flags, int dtype, unsigned* staged, pqmf_stream_t stream);
 
 /* ---- fused round trip on device buffers: PQMFWrapper.process (PQMFWrapper.py:81-92: forward, then inverse of the same
  *      sub-bands) and the Pvoc wrapper's forward (1-PitchShifterWrapper.py:303-316) ----

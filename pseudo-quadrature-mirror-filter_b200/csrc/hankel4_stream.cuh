@@ -23,7 +23,7 @@
 // Half-precision pools (POOL with IO = H4Io::F16 / BF16, half_io.cuh): blocks, sub-bands and outputs are raw fp16 / bf16 bits behind the
 // same pointers (a launch-time reinterpretation, no new fields), the pool stays fp32.  Block groups load half words one tile ahead and widen
 // them exactly before the fp16 split and the roll, so the pool receives the floats of the fp32 call on the widened block; the drains
-// round to nearest even.  Lockstep calls have no half instantiation.
+// round to nearest even.  The GROUPS kernels have the same half instantiations.  Lockstep calls have no half instantiation.
 #pragma once
 #include <type_traits>
 
@@ -512,6 +512,7 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_stream_kernel(H
 // times per CTA.  Block addresses are made per tile from the row index.  The drain runs two tile loads behind the load, so the drained
 // tile's output row (pointer, frame stride, first frame, parity) travels through load -> convert -> drain with the tile.
 // PCM (the POOL PCM kernels' edge, per group): each group has its own WAV frames (channel count, down-mix) and mono int16 output rows.
+// Half (the POOL half kernels' edge): grp[k].in / grp[k].out hold fp16 / bf16 bits; block addresses are made per tile in 2-byte elements.
 struct H4StreamGroup {
   const int* ids;   // [n] stream of each row
   const float* in;  // analysis: x [n, T]; synthesis: s [n, M, F]
@@ -558,9 +559,10 @@ __device__ __forceinline__ int h4_groups_min_region_rows(const Params& p) {
 
 template <int M, H4Io IO>
 __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_stream_groups_kernel(H4AnalysisStreamGroupsArgs<IO> p) {
-  static_assert(IO == H4Io::F32 || IO == H4Io::PCM, "streaming blocks: fp32 rows or int16 PCM frames");
+  static_assert(IO == H4Io::F32 || IO == H4Io::PCM || h4_io_half(IO), "streaming blocks: fp32 rows, int16 PCM frames or half rows");
   h4_kernel<true, kH4Workers>(p.g, p.bank, p.n_tiles, 1u, p.pad_bytes, p.trim_lo, p.trim_hi, [&](const H4Smem& sm, uint32_t tmem, uint32_t pfull_leader, unsigned n_iter) {
-    constexpr bool PCM = IO == H4Io::PCM;
+    constexpr bool PCM = IO == H4Io::PCM, HALF = h4_io_half(IO);
+    using Y = std::conditional_t<HALF, uint16_t, float>;  // sub-band element: half bits behind grp[k].out
     constexpr int FR = 64 / M, HB = M / 2;
     constexpr int NO = (kH4Rows * 8 + kH4Workers - 1) / kH4Workers;
     const H4Shape& g = p.g;
@@ -599,7 +601,7 @@ __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_stream_groups_kerne
       }
     };
     struct DrainRow {
-      float* y;  // this thread's first output of the tile (nullptr: not a stored row)
+      Y* y;  // this thread's first output of the tile (nullptr: not a stored row)
       int F, eq, parity;
     };
     DrainRow d_ld{nullptr, 0, 0, 0}, d_cur = d_ld, d_prev = d_ld;  // of the loaded / converted / drained tile
@@ -633,7 +635,7 @@ __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_stream_groups_kerne
 #pragma unroll
       for (int r = 0; r < NO; ++r) ph[r] = id[r] >= 0 ? __ldg(p.pool.phase + id[r]) : 0;
       const int F = (int)(gr.len / M);
-      d_ld.y = stored ? gr.out + ((size_t)(row0 + dt) * M + HB * hb) * F + FR * dq : nullptr;
+      d_ld.y = stored ? reinterpret_cast<Y*>(gr.out) + ((size_t)(row0 + dt) * M + HB * hb) * F + FR * dq : nullptr;
       d_ld.F = F;
       d_ld.eq = dq;
       d_ld.parity = did >= 0 ? (__ldg(p.pool.phase + did) >> 1) & 1 : 0;
@@ -647,13 +649,18 @@ __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_stream_groups_kerne
           ptx::ldg256_na(p.hist_in + ((size_t)(ph[r] & 1) * p.pool.P + row) * p.L + hofs[r], xr[r]);
         } else if constexpr (PCM) {
           pcm_load8_raw_row(p.in[gi], row_ld + q_slot[r], bofs[r], (int)gr.len, xr[r]);  // raw words: converted when the tile is consumed
+        } else if constexpr (HALF) {  // eight half samples = 16 bytes, kept raw in xr[r][0..3] until the tile is consumed
+          const float4 raw =
+              ptx::ldg128_na(reinterpret_cast<const float4*>(reinterpret_cast<const uint16_t*>(gr.in) + (size_t)(row0 + q_slot[r]) * gr.len + bofs[r]));
+          xr[r][0] = raw.x; xr[r][1] = raw.y; xr[r][2] = raw.z; xr[r][3] = raw.w;
         } else {
           ptx::ldg256_na(gr.in + (size_t)(row0 + q_slot[r]) * gr.len + bofs[r], xr[r]);
         }
         roll[r] = (rofs[r] >= 0 && id[r] >= 0) ? p.hist_out + ((size_t)(~ph[r] & 1) * p.pool.P + row) * p.L + rofs[r] : nullptr;
       }
     };
-    // PCM: the block groups' raw words are widened first (zeros of dead rows widen to zeros), so planes and roll see the fp32 call's floats
+    // PCM and half: the block groups' raw words are widened first (zeros of dead rows widen to zeros), so planes and roll see the fp32
+    // call's floats.  gi and the plan are still the loaded tile's (see row_ld), also on the first tile after a group switch
     auto convert = [&](int pb) {
       unsigned char* p1 = sm.planes + (2 * pb) * g.plane;
       d_cur = d_ld;
@@ -663,6 +670,8 @@ __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_stream_groups_kerne
         if (u < n_octs) {
           if constexpr (PCM)
             if (bofs[r] >= 0) pcm_convert8(p.in[gi], row_ld + q_slot[r], xr[r]);
+          if constexpr (HALF)
+            if (hofs[r] < 0) h4_widen8<IO>(xr[r]);  // block and padding groups (padding holds zeros); history groups are fp32
           h4_split_store8(xr[r], p1, g.plane, sw128_offset((uint32_t)u * 16u));
           if (roll[r] != nullptr) {
             *reinterpret_cast<float4*>(roll[r]) = make_float4(xr[r][0], xr[r][1], xr[r][2], xr[r][3]);
@@ -675,19 +684,37 @@ __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_stream_groups_kerne
       float v[FR][HB];
       h4_drain_analysis<M>(tmem, dbuf, tid, d_prev.eq, d_prev.parity, v);
       if (d_prev.y == nullptr) return;
+      if constexpr (HALF) {  // round to nearest even; 2 FR bytes per band, as the POOL half drain
 #pragma unroll
-      for (int kk = 0; kk < HB; ++kk) {
-        float w[FR];
+        for (int kk = 0; kk < HB; ++kk) {
+          uint16_t* q = d_prev.y + (size_t)kk * d_prev.F;
+          if constexpr (FR >= 8) {
 #pragma unroll
-        for (int dl = 0; dl < FR; ++dl) w[dl] = v[dl][kk];
-        float* q = d_prev.y + (size_t)kk * d_prev.F;
-        if constexpr (FR >= 4) {
+            for (int d8 = 0; d8 < FR; d8 += 8)
+              __stcs(reinterpret_cast<uint4*>(q + d8), make_uint4(h4_narrow2<IO>(v[d8][kk], v[d8 + 1][kk]), h4_narrow2<IO>(v[d8 + 2][kk], v[d8 + 3][kk]),
+                                                                h4_narrow2<IO>(v[d8 + 4][kk], v[d8 + 5][kk]), h4_narrow2<IO>(v[d8 + 6][kk], v[d8 + 7][kk])));
+          } else if constexpr (FR == 4) {
+            __stcs(reinterpret_cast<uint2*>(q), make_uint2(h4_narrow2<IO>(v[0][kk], v[1][kk]), h4_narrow2<IO>(v[2][kk], v[3][kk])));
+          } else {
+            static_assert(FR == 2, "n_band 8 / 16 / 32");
+            __stcs(reinterpret_cast<unsigned int*>(q), h4_narrow2<IO>(v[0][kk], v[1][kk]));
+          }
+        }
+      } else {
 #pragma unroll
-          for (int d4 = 0; d4 < FR; d4 += 4) __stcs(reinterpret_cast<float4*>(q + d4), make_float4(w[d4], w[d4 + 1], w[d4 + 2], w[d4 + 3]));
-        } else if constexpr (FR == 2) {
-          __stcs(reinterpret_cast<float2*>(q), make_float2(w[0], w[1]));
-        } else {
-          __stcs(q, w[0]);
+        for (int kk = 0; kk < HB; ++kk) {
+          float w[FR];
+#pragma unroll
+          for (int dl = 0; dl < FR; ++dl) w[dl] = v[dl][kk];
+          float* q = d_prev.y + (size_t)kk * d_prev.F;
+          if constexpr (FR >= 4) {
+#pragma unroll
+            for (int d4 = 0; d4 < FR; d4 += 4) __stcs(reinterpret_cast<float4*>(q + d4), make_float4(w[d4], w[d4 + 1], w[d4 + 2], w[d4 + 3]));
+          } else if constexpr (FR == 2) {
+            __stcs(reinterpret_cast<float2*>(q), make_float2(w[0], w[1]));
+          } else {
+            __stcs(q, w[0]);
+          }
         }
       }
     };
@@ -703,10 +730,10 @@ __global__ void __launch_bounds__(kH4Threads, 1) h4_analysis_stream_groups_kerne
 
 template <int M, H4Io IO>
 __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_stream_groups_kernel(H4SynthesisStreamGroupsArgs<IO> p) {
-  static_assert(IO == H4Io::F32 || IO == H4Io::PCM, "streaming blocks: fp32 rows or int16 PCM samples");
+  static_assert(IO == H4Io::F32 || IO == H4Io::PCM || h4_io_half(IO), "streaming blocks: fp32 rows, int16 PCM samples or half rows");
   h4_kernel<true, kH4SynWorkers>(p.g, p.bank, p.n_tiles, 1u, p.pad_bytes, p.trim_lo, p.trim_hi, [&](const H4Smem& sm, uint32_t tmem, uint32_t pfull_leader, unsigned n_iter) {
-    constexpr bool PCM = IO == H4Io::PCM;
-    using Out = std::conditional_t<PCM, int16_t, float>;
+    constexpr bool PCM = IO == H4Io::PCM, HALF = h4_io_half(IO);
+    using Out = std::conditional_t<PCM, int16_t, std::conditional_t<HALF, uint16_t, float>>;
     constexpr int FR = 64 / M, NBG = M / 8;
     const H4Shape& g = p.g;
     const int tid = threadIdx.x, warp = tid >> 5;
@@ -739,7 +766,7 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_stream_groups_k
         } else if (fb < block_fr) {
           slot = lt;
           sofs = (int)(8 * bg * F + fb);
-          src_pitch = (size_t)F;
+          src_pitch = HALF ? (size_t)F / 2 : (size_t)F;  // half: in whole floats (F and fb are multiples of 4)
           if (fb >= F - p.K) rofs = (int)(8 * bg * p.K + (fb - (F - p.K)));
         }
       }
@@ -765,24 +792,43 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_stream_groups_k
       if ((unsigned)id >= (unsigned)p.pool.P) id = -1;
       const int ph = id >= 0 ? __ldg(p.pool.phase + id) : 0;
       const float* from = hofs >= 0 ? p.state_in + ((size_t)(ph & 1) * p.pool.P + (size_t)id) * M * p.K + hofs
+                          : HALF    ? reinterpret_cast<const float*>(reinterpret_cast<const uint16_t*>(gr.in) + (size_t)(row0 + slot) * M * gr.len + sofs)
                                     : gr.in + (size_t)(row0 + slot) * M * gr.len + sofs;
+      if constexpr (HALF) {  // block items: four half frames per 8-byte load, raw in .x / .y until the tile is consumed
 #pragma unroll
-      for (int kk = 0; kk < 8; ++kk)
-        v[kk] = id >= 0 ? ptx::ldg128_na(reinterpret_cast<const float4*>(from + (size_t)kk * src_pitch)) : make_float4(0.f, 0.f, 0.f, 0.f);
-      roll = (rofs >= 0 && id >= 0) ? p.state_out + ((size_t)(~ph & 1) * p.pool.P + (size_t)id) * M * p.K + rofs : nullptr;
+        for (int kk = 0; kk < 8; ++kk) {
+          if (id < 0) {
+            v[kk] = make_float4(0.f, 0.f, 0.f, 0.f);
+          } else if (hofs < 0) {
+            const float2 h = ptx::ldg64_na(from + (size_t)kk * src_pitch);
+            v[kk] = make_float4(h.x, h.y, 0.f, 0.f);
+          } else {
+            v[kk] = ptx::ldg128_na(reinterpret_cast<const float4*>(from + (size_t)kk * src_pitch));
+          }
+        }
+      } else {
+#pragma unroll
+        for (int kk = 0; kk < 8; ++kk)
+          v[kk] = id >= 0 ? ptx::ldg128_na(reinterpret_cast<const float4*>(from + (size_t)kk * src_pitch)) : make_float4(0.f, 0.f, 0.f, 0.f);
+      }
+      roll =(rofs >= 0 && id >= 0) ? p.state_out + ((size_t)(~ph & 1) * p.pool.P + (size_t)id) * M * p.K + rofs : nullptr;
       flip_ld = (ph & 2) ? 0u : 0x80000000u;
       // pitch and rows_b are multiples of 4: the four rows of a lane quad belong to one region and are stored or not together
       const int et = i0 / sg.pitch, eq0 = i0 - et * sg.pitch;
       const bool stored = warp < 8 && et < sg.spt && eq0 < sg.rows_b && et < nlive;
       Out* base;
       if constexpr (PCM) base = p.pcm_out[gi];
-      else base = gr.out;
+      else base = reinterpret_cast<Out*>(gr.out);
       o_ld = stored ? base + (size_t)(row0 + et) * (size_t)(gr.len * M) + 64 * eq0 + 32 * hb + 8 * (lane & 3) : nullptr;
     };
     auto convert = [&](int pb) {
       o_cur = o_ld;
       if (!has_item) return;
       unsigned char* p1 = sm.planes + (2 * pb) * g.plane;
+      if constexpr (HALF)  // exact, before the roll (hofs: the loaded tile's plan); zeros of dead rows widen to zeros
+        if (hofs < 0)
+#pragma unroll
+          for (int kk = 0; kk < 8; ++kk) v[kk] = h4_widen4<IO>(v[kk]);
       if (roll != nullptr) {
 #pragma unroll
         for (int kk = 0; kk < 8; ++kk) *reinterpret_cast<float4*>(roll + (size_t)kk * p.K) = v[kk];
@@ -808,6 +854,11 @@ __global__ void __launch_bounds__(kH4SynThreads, 1) h4_synthesis_stream_groups_k
             w[k] = (uint32_t)(uint16_t)pcm_quantise(val[q][2 * k]) | ((uint32_t)(uint16_t)pcm_quantise(val[q][2 * k + 1]) << 16);
           __stcs(reinterpret_cast<uint4*>(o_prev + (size_t)q * 64), make_uint4(w[0], w[1], w[2], w[3]));
         }
+      } else if constexpr (HALF) {  // round to nearest even: eight samples = one 16-byte store per slot, as the POOL half kernel
+#pragma unroll
+        for (int q = 0; q < 4; ++q)
+          __stcs(reinterpret_cast<uint4*>(o_prev + (size_t)q * 64), make_uint4(h4_narrow2<IO>(val[q][0], val[q][1]), h4_narrow2<IO>(val[q][2], val[q][3]),
+                                                                              h4_narrow2<IO>(val[q][4], val[q][5]), h4_narrow2<IO>(val[q][6], val[q][7])));
       } else {
 #pragma unroll
         for (int q = 0; q < 4; ++q) ptx::stg256_cs(o_prev + (size_t)q * 64, val[q]);
@@ -866,7 +917,8 @@ inline int h4_launch_synthesis_stream(const H4SynthesisStreamParams& p, const St
     return pool ? h4_launch_synthesis_stream<M, true, H4Io::PCM>(p, pool, pcm_out, st) : h4_launch_synthesis_stream<M, false, H4Io::PCM>(p, pool, pcm_out, st);
   return pool ? h4_launch_synthesis_stream<M, true, H4Io::F32>(p, pool, pcm_out, st) : h4_launch_synthesis_stream<M, false, H4Io::F32>(p, pool, pcm_out, st);
 }
-// GROUPS: p.n_tiles, p.G and p.grp[] filled by the caller; the instantiation follows the sample format io (PCM: in[] / pcm_out[] per group)
+// GROUPS: p.n_tiles, p.G and p.grp[] filled by the caller; the instantiation follows the sample format io (PCM: in[] / pcm_out[] per group;
+// F16 / BF16: grp[k].in and grp[k].out hold half bits)
 template <int M, H4Io IO>
 inline int h4_launch_analysis_stream_groups(const H4AnalysisStreamGroupsParams& base, const PcmIn* in, cudaStream_t st) {
   static H4Configured configured;
@@ -878,7 +930,12 @@ inline int h4_launch_analysis_stream_groups(const H4AnalysisStreamGroupsParams& 
 }
 template <int M>
 inline int h4_launch_analysis_stream_groups(const H4AnalysisStreamGroupsParams& p, H4Io io, const PcmIn* in, cudaStream_t st) {
-  return io == H4Io::PCM ? h4_launch_analysis_stream_groups<M, H4Io::PCM>(p, in, st) : h4_launch_analysis_stream_groups<M, H4Io::F32>(p, in, st);
+  switch (io) {
+    case H4Io::PCM: return h4_launch_analysis_stream_groups<M, H4Io::PCM>(p, in, st);
+    case H4Io::F16: return h4_launch_analysis_stream_groups<M, H4Io::F16>(p, in, st);
+    case H4Io::BF16: return h4_launch_analysis_stream_groups<M, H4Io::BF16>(p, in, st);
+    default: return h4_launch_analysis_stream_groups<M, H4Io::F32>(p, in, st);
+  }
 }
 template <int M, H4Io IO>
 inline int h4_launch_synthesis_stream_groups(const H4SynthesisStreamGroupsParams& base, int16_t* const* pcm_out, cudaStream_t st) {
@@ -891,8 +948,12 @@ inline int h4_launch_synthesis_stream_groups(const H4SynthesisStreamGroupsParams
 }
 template <int M>
 inline int h4_launch_synthesis_stream_groups(const H4SynthesisStreamGroupsParams& p, H4Io io, int16_t* const* pcm_out, cudaStream_t st) {
-  return io == H4Io::PCM ? h4_launch_synthesis_stream_groups<M, H4Io::PCM>(p, pcm_out, st)
-                         : h4_launch_synthesis_stream_groups<M, H4Io::F32>(p, pcm_out, st);
+  switch (io) {
+    case H4Io::PCM: return h4_launch_synthesis_stream_groups<M, H4Io::PCM>(p, pcm_out, st);
+    case H4Io::F16: return h4_launch_synthesis_stream_groups<M, H4Io::F16>(p, pcm_out, st);
+    case H4Io::BF16: return h4_launch_synthesis_stream_groups<M, H4Io::BF16>(p, pcm_out, st);
+    default: return h4_launch_synthesis_stream_groups<M, H4Io::F32>(p, pcm_out, st);
+  }
 }
 
 }  // namespace pqmf

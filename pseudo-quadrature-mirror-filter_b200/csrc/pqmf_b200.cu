@@ -480,7 +480,8 @@ int fast_synthesis(const float* s, const float* hist, float* out, float* hist_ou
 //        Hankel-4                      | offline, lockstep, pool | offline, pool; unsplit banks | all; output: unsplit banks, mono when streaming
 //        fold / Hankel-16 (n_band 16)  | offline, lockstep       | -                            | -
 //        direct form                   | offline, lockstep, pool | -                            | offline
-//      (the half-precision instantiations exist for the unsplit banks only; a split bank's second launch accumulates, not in int16;
+//      (pool: single-group and grouped calls, in every format; the half-precision instantiations exist for the unsplit banks only; a split
+//      bank's second launch accumulates, not in int16;
 //      streaming PCM output is mono rows: the two channels of a clip may sit in any two tiles; lockstep streaming stays fp32 and PCM) ----
 bool h4_serves(const Samples& s, const History& h, unsigned flags, bool output) {
   if (pqmf::h4_io_half(s.io)) return (!h.in || h.pool) && !(flags & PQMF_FLAG_H4_SPLIT);
@@ -742,12 +743,12 @@ int pool_phase(const PoolRows& pool, int n, int* xphase, long x_frames, int* sph
 }
 bool bad_pool(int P, int n) { return P < 1 || n < 0 || n > P; }
 
-// ---- grouped pool calls (pqmf_stream_pool_*_groups_f32 / _pcm16): groups of rows with their own block lengths.  One rule: the groups
+// ---- grouped pool calls (pqmf_stream_pool_*_groups_f32 / _pcm16 / _x): groups of rows with their own block lengths.  One rule: the groups
 //      the streaming Hankel-4 kernels can plan (h4_takes_*, family, plan and alignment, apart from the tile count) run together in one
 //      GROUPS launch per direction and one phase-word launch, when there are at least two of them and they reach kH4StreamMinTiles together
 //      (in both directions for a step).  Every other group runs through its single-group pool entry, with exactly that entry's launches.
-//      A PCM call joins exactly the groups the fp32 call on the widened blocks would join (fresh, aligned fp32 rows: the PCM buffers'
-//      alignment does not decide it); it then runs natively or launches nothing ----
+//      A PCM or half call joins exactly the groups the fp32 call on the widened blocks would join (fresh, aligned fp32 rows: the PCM or
+//      half buffers' alignment does not decide it); it then runs natively or launches nothing ----
 enum class PoolDir { kAnalysis, kSynthesis, kStep };
 
 struct PoolGroupsCall {
@@ -761,14 +762,20 @@ struct PoolGroupsCall {
   int P, M, L;
   unsigned flags;
   cudaStream_t st;
-  // the sample format: PCM calls have pcm_groups (groups unused), one down-mix for the whole call, and the mask of staged groups
+  // the sample format: PCM calls have pcm_groups (groups unused) and one down-mix for the whole call, half calls (one direction) have
+  // half_groups (groups unused); both have the mask of staged groups
   pqmf::H4Io io = pqmf::H4Io::F32;
   const pqmf_pool_group_pcm16* pcm_groups = nullptr;
   int downmix = 0;
   unsigned* staged = nullptr;
+  const pqmf_pool_group_x* half_groups = nullptr;
+  int dtype = PQMF_DTYPE_F32;
   bool analysis() const { return dir != PoolDir::kSynthesis; }
   bool synthesis() const { return dir != PoolDir::kAnalysis; }
   bool pcm() const { return io == pqmf::H4Io::PCM; }
+  bool half() const { return pqmf::h4_io_half(io); }
+  bool widened() const { return io != pqmf::H4Io::F32; }  // the call stands for the fp32 call on the widened blocks
+  const void* descriptors() const { return pcm() ? (const void*)pcm_groups : half() ? (const void*)half_groups : (const void*)groups; }
 };
 
 // group k of either format: its rows (PCM: clips x C', C' = 1 with the down-mix, else C; a synthesis has no down-mix), the analysis input
@@ -782,6 +789,10 @@ struct PoolGroup {
   Samples out;
 };
 PoolGroup pool_group(const PoolGroupsCall& c, int k) {
+  if (c.half()) {  // y holds half bits as well
+    const pqmf_pool_group_x& g = c.half_groups[k];
+    return {g.ids, g.n, g.T, samples(g.x, c.io), static_cast<float*>(g.y), samples(g.out, c.io)};
+  }
   if (!c.pcm()) {
     const pqmf_pool_group_f32& g = c.groups[k];
     return {g.ids, g.n, g.T, samples(g.x), g.y, samples(g.out)};
@@ -789,11 +800,26 @@ PoolGroup pool_group(const PoolGroupsCall& c, int k) {
   const pqmf_pool_group_pcm16& g = c.pcm_groups[k];
   return {g.ids, c.downmix ? g.n : g.n * g.C, g.T, pcm16(g.pcm, g.C, c.downmix), g.y, pcm16(g.pcm_out, c.downmix ? 1 : g.C)};
 }
-// the fp32 call's sample side of a group: PCM blocks stand for freshly allocated fp32 rows (null passes every alignment check)
+// the fp32 call's sample side of a group: PCM and half blocks stand for freshly allocated fp32 rows (null passes every alignment check)
 Samples fp32_view(const Samples& s) { return s.io == pqmf::H4Io::F32 ? s : samples(nullptr); }
+// and its sub-bands: half sub-bands stand for fresh fp32 ones too
+const void* fp32_view(const PoolGroupsCall& c, const float* y) { return c.half() ? nullptr : y; }
 
 int pool_group_alone(const PoolGroupsCall& c, int k) {
   pqmf_stream_t s = (pqmf_stream_t)c.st;
+  if (c.half()) {  // one direction (there is no grouped half step)
+    const pqmf_pool_group_x& g = c.half_groups[k];
+    if (g.n == 0) return PQMF_OK;
+    const int e = c.analysis()
+                      ? pqmf_stream_pool_analysis_x(g.x, g.y, c.hk, c.tables, c.xpool, c.xphase, c.P, g.ids, g.n, g.T, c.M, c.L, c.flags, c.dtype, s)
+                      : pqmf_stream_pool_synthesis_x(g.y, g.out, c.hk, c.tables, c.spool, c.sphase, c.P, g.ids, g.n, g.T / c.M, c.M, c.L, c.flags,
+                                                     c.dtype, s);
+    if (e == PQMF_ERR_UNSUPPORTED) {  // refused (nothing launched): the caller stages this group
+      *c.staged |= 1u << k;
+      return PQMF_OK;
+    }
+    return e;
+  }
   if (c.pcm()) {
     const pqmf_pool_group_pcm16& g = c.pcm_groups[k];
     if (g.n == 0) return PQMF_OK;
@@ -829,7 +855,7 @@ int pool_group_alone(const PoolGroupsCall& c, int k) {
   }
 }
 
-// the GROUPS launch of one direction, fp32 or PCM by io (PCM: in[] / pcm_out[] per group of the launch)
+// the GROUPS launch of one direction, fp32, PCM or half by io (PCM: in[] / pcm_out[] per group of the launch)
 template <typename Params>
 int h4_launch_stream_groups(const Params& p, int M, pqmf::H4Io io, const pqmf::PcmIn* in, int16_t* const* pcm_out, cudaStream_t st) {
   int e = PQMF_ERR_UNSUPPORTED;
@@ -851,7 +877,7 @@ int h4_launch_stream_groups(const Params& p, int M, pqmf::H4Io io, const pqmf::P
 }
 
 // the GROUPS launches of the groups in `joins`, planned in ap / sp, then one phase-word launch.  started: false when the first launch did
-// not start (nothing was launched: the caller runs the groups alone, or -- PCM -- refuses the call)
+// not start (nothing was launched: the caller runs the groups alone, or -- PCM, half -- refuses the call)
 int pool_groups_launch(const PoolGroupsCall& c, const PoolGroup* grp, const bool* joins, const pqmf::H4AnalysisStreamParams* ap,
                        const pqmf::H4SynthesisStreamParams* sp, bool& started) {
   started = false;
@@ -902,9 +928,9 @@ int pool_groups_launch(const PoolGroupsCall& c, const PoolGroup* grp, const bool
     p.n_tiles = tiles;
     if (const int e = h4_launch_stream_groups(p, c.M, c.io, in, pcm_out, c.st)) {
       if (!started) return e;
-      // the analysis has run.  PCM: an error, not a refusal (a staged retry would step the analysis state twice; see
-      // pqmf_stream_step_pcm16).  fp32: each group's synthesis goes through the single-group dispatcher (its own kernels), then the phase words
-      if (c.pcm()) return (int)cudaErrorLaunchFailure;
+      // the analysis has run (never in a half call, which has one direction).  PCM: an error, not a refusal (a staged retry would step
+      // the analysis state twice; see pqmf_stream_step_pcm16).  fp32: each group's synthesis goes through the single-group dispatcher (its own kernels), then the phase words
+      if (c.widened()) return (int)cudaErrorLaunchFailure;
       for (int k = 0; k < c.G; ++k) {
         if (!joins[k]) continue;
         const PoolGroup& g = grp[k];
@@ -924,8 +950,7 @@ bool pcm_args_bad(int C, long rows) { return C < 1 || C > 64 || rows >= (1L << 3
 int pool_groups(const PoolGroupsCall& c) {
   // every argument check before anything is launched: the single-group entries' rules per group, plus 0 <= G <= 8 and <= P rows in all
   const bool ana = c.analysis(), syn = c.synthesis();
-  if (c.G < 0 || c.G > pqmf::kPoolMaxGroups || (c.G > 0 && !(c.pcm() ? (const void*)c.pcm_groups : (const void*)c.groups)) || c.P < 1)
-    return PQMF_ERR_ARG;
+  if (c.G < 0 || c.G > pqmf::kPoolMaxGroups || (c.G > 0 && !c.descriptors()) || c.P < 1) return PQMF_ERR_ARG;
   long rows = 0;
   for (int k = 0; k < c.G; ++k) {
     if (c.pcm()) {
@@ -935,14 +960,14 @@ int pool_groups(const PoolGroupsCall& c) {
       if (g.n > 0 && (!g.ids || !g.y || (ana && !g.pcm) || (syn && !g.pcm_out))) return PQMF_ERR_ARG;
       rows += grows;
     } else {
-      const pqmf_pool_group_f32& g = c.groups[k];
-      if (bad_dims(g.n, g.T, c.M, c.L) || g.T <= 0 || (g.T % c.M) != 0 || (syn && (c.L % c.M) != 0)) return PQMF_ERR_ARG;
-      if (g.n > 0 && (!g.ids || !g.y || (ana && !g.x) || (syn && !g.out))) return PQMF_ERR_ARG;
-      rows += g.n;
+      const PoolGroup g = pool_group(c, k);
+      if (bad_dims(g.rows, g.T, c.M, c.L) || g.T <= 0 || (g.T % c.M) != 0 || (syn && (c.L % c.M) != 0)) return PQMF_ERR_ARG;
+      if (g.rows > 0 && (!g.ids || !g.y || (ana && !g.x.p) || (syn && !g.out.p))) return PQMF_ERR_ARG;
+      rows += g.rows;
     }
   }
-  if (rows > c.P || (c.pcm() && !c.staged)) return PQMF_ERR_ARG;
-  if (c.pcm()) *c.staged = 0;
+  if (rows > c.P || (c.widened() && !c.staged)) return PQMF_ERR_ARG;
+  if (c.widened()) *c.staged = 0;
   if (rows == 0) return PQMF_OK;
   if (!c.hk || (ana && (!c.xpool || !c.xphase)) || (syn && (!c.spool || !c.sphase)) || (ana && syn && c.xphase == c.sphase)) return PQMF_ERR_ARG;
   if (c.G == 1) return pool_group_alone(c, 0);
@@ -959,16 +984,17 @@ int pool_groups(const PoolGroupsCall& c) {
     const PoolRows xrows{g.ids, c.xphase, c.P}, srows{g.ids, c.sphase, c.P};
     ap[k] = pqmf::H4AnalysisStreamParams{};
     sp[k] = pqmf::H4SynthesisStreamParams{};
-    if (ana && !h4_takes_analysis(fp32_view(g.x), g.y, pooled(c.xpool, xrows), g.rows, g.T, g.T / c.M, c.M, c.L, c.tables, c.flags, &ap[k], 1)) continue;
-    if (syn && !h4_takes_synthesis(g.y, fp32_view(g.out), pooled(c.spool, srows), g.rows, g.T / c.M, c.M, c.L, c.tables, c.flags, &sp[k], 1)) continue;
+    const void* y = fp32_view(c, g.y);
+    if (ana && !h4_takes_analysis(fp32_view(g.x), y, pooled(c.xpool, xrows), g.rows, g.T, g.T / c.M, c.M, c.L, c.tables, c.flags, &ap[k], 1)) continue;
+    if (syn && !h4_takes_synthesis(y, fp32_view(g.out), pooled(c.spool, srows), g.rows, g.T / c.M, c.M, c.L, c.tables, c.flags, &sp[k], 1)) continue;
     joins[k] = true;
     ++joined;
     if (ana) atiles += h4_stream_tiles(g.rows, ap[k].s);
     if (syn) stiles += h4_stream_tiles(g.rows, sp[k].sg);
   }
   bool grouped = joined >= 2 && (!ana || atiles >= kH4StreamMinTiles) && (!syn || stiles >= kH4StreamMinTiles);
-  if (grouped && c.pcm()) {
-    // the joined groups run natively, or nothing is launched: their PCM buffers' alignment, and mono output rows
+  if (grouped && c.widened()) {
+    // the joined groups run natively, or nothing is launched: their PCM or half buffers' alignment, and mono PCM output rows
     for (int k = 0; k < c.G; ++k) {
       if (!joins[k]) continue;
       const PoolGroup& g = grp[k];
@@ -980,13 +1006,33 @@ int pool_groups(const PoolGroupsCall& c) {
   }
   if (grouped) {
     const int e = pool_groups_launch(c, grp, joins, ap, sp, grouped);
-    if (c.pcm() && !grouped) return PQMF_ERR_UNSUPPORTED;  // the first launch did not start: nothing ran
+    if (c.widened() && !grouped) return PQMF_ERR_UNSUPPORTED;  // the first launch did not start: nothing ran
     if (grouped && e) return e;
   }
   for (int k = 0; k < c.G; ++k)
     if (!(grouped && joins[k]))
       if (int e = pool_group_alone(c, k)) return e;
   return PQMF_OK;
+}
+
+// the _x grouped entries: PQMF_DTYPE_F32 is the _f32 grouped call (same descriptor fields), fp16 / bf16 the half call
+int pool_groups_x(PoolGroupsCall c, const pqmf_pool_group_x* groups, int dtype) {
+  if (dtype != PQMF_DTYPE_F32) {
+    if (!half_io_of(dtype, c.io)) return PQMF_ERR_ARG;
+    c.half_groups = groups;
+    c.dtype = dtype;
+    return pool_groups(c);
+  }
+  if (!c.staged || c.G < 0 || c.G > pqmf::kPoolMaxGroups) return PQMF_ERR_ARG;
+  *c.staged = 0;
+  pqmf_pool_group_f32 f32[pqmf::kPoolMaxGroups];
+  for (int k = 0; groups && k < c.G; ++k) {
+    const pqmf_pool_group_x& g = groups[k];
+    f32[k] = {g.ids, g.n, g.T, static_cast<const float*>(g.x), static_cast<float*>(g.y), static_cast<float*>(g.out)};
+  }
+  c.groups = groups ? f32 : nullptr;
+  c.staged = nullptr;
+  return pool_groups(c);
 }
 
 }  // namespace
@@ -1313,6 +1359,20 @@ int pqmf_stream_pool_step_groups_pcm16(const pqmf_pool_group_pcm16* groups, int 
                                        pqmf_stream_t stream) {
   return pool_groups({PoolDir::kStep, nullptr, G, hk, tables, xpool, spool, xphase, sphase, P, M, L, flags, (cudaStream_t)stream, pqmf::H4Io::PCM,
                       groups, downmix ? 1 : 0, staged});
+}
+
+int pqmf_stream_pool_analysis_groups_x(const pqmf_pool_group_x* groups, int G, const float* hk, const float* tables, float* xpool, int* xphase,
+                                       int P, int M, int L, unsigned flags, int dtype, unsigned* staged, pqmf_stream_t stream) {
+  return pool_groups_x({PoolDir::kAnalysis, nullptr, G, hk, tables, xpool, nullptr, xphase, nullptr, P, M, L, flags, (cudaStream_t)stream,
+                        pqmf::H4Io::F32, nullptr, 0, staged},
+                       groups, dtype);
+}
+
+int pqmf_stream_pool_synthesis_groups_x(const pqmf_pool_group_x* groups, int G, const float* hk, const float* tables, float* spool, int* sphase,
+                                        int P, int M, int L, unsigned flags, int dtype, unsigned* staged, pqmf_stream_t stream) {
+  return pool_groups_x({PoolDir::kSynthesis, nullptr, G, hk, tables, nullptr, spool, nullptr, sphase, P, M, L, flags, (cudaStream_t)stream,
+                        pqmf::H4Io::F32, nullptr, 0, staged},
+                       groups, dtype);
 }
 
 // ---- half-precision pools: the streaming Hankel-4 POOL kernels with fp16 / bf16 loads and stores, exactly where the fp32 pool call with the

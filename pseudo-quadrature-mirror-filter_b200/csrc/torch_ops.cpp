@@ -398,12 +398,16 @@ std::tuple<at::Tensor, at::Tensor> stream_pool_step(const at::Tensor& x, const a
 //      pool itself fp32.  A tensor of another dtype is refused.  Where the library has no native kernel (PQMF_ERR_UNSUPPORTED, nothing
 //      launched) the op stages the call one direction at a time: widen, the fp32 pool op, round -- so a staged step's synthesis reads the
 //      rounded sub-bands, as the native step's does ----
-int pool_dtype(const at::Tensor& t, at::ScalarType dtype, const char* name) {
-  TORCH_CHECK(t.is_cuda(), name, " must be a CUDA tensor (pqmf_b200 has no CPU fallback)");
+int pool_dtype_code(at::ScalarType dtype) {
   TORCH_CHECK(dtype == at::kFloat || dtype == at::kHalf || dtype == at::kBFloat16, "a stream pool's dtype must be float32, float16 or bfloat16, got ",
               dtype);
-  TORCH_CHECK(t.scalar_type() == dtype, name, " must be ", dtype, " (the pool's dtype), got ", t.scalar_type());
   return dtype == at::kFloat ? PQMF_DTYPE_F32 : dtype == at::kHalf ? PQMF_DTYPE_F16 : PQMF_DTYPE_BF16;
+}
+int pool_dtype(const at::Tensor& t, at::ScalarType dtype, const char* name) {
+  TORCH_CHECK(t.is_cuda(), name, " must be a CUDA tensor (pqmf_b200 has no CPU fallback)");
+  const int code = pool_dtype_code(dtype);
+  TORCH_CHECK(t.scalar_type() == dtype, name, " must be ", dtype, " (the pool's dtype), got ", t.scalar_type());
+  return code;
 }
 
 // x [n, 1, T] -> y [n, M, T / M], both of dtype
@@ -490,10 +494,10 @@ void check_pcm(const at::Tensor& pcm, const char* what);
 
 // blocks: x [n, 1, T] (analysis, step) or s [n, M, F] (synthesis), one per group; returns the contiguous blocks and fills the descriptors.
 // pcm != nullptr: PCM groups, filled into *pcm instead -- pcm [S, T, C] int16 (analysis, step; rows S C', C' = 1 with downmix, else C) or
-// s [S, C M, F] float32 (synthesis; rows S C)
+// s [S, C M, F] float32 (synthesis; rows S C).  dtype: the element type of x / s (a half pool's, checked by pool_dtype)
 std::vector<at::Tensor> groups_of(at::TensorList blocks, at::TensorList ids, const Bank& bank, const at::Tensor& like, int64_t P, GroupsDir dir,
                                   std::vector<pqmf_pool_group_f32>& groups, const char* what,
-                                  std::vector<pqmf_pool_group_pcm16>* pcm = nullptr, bool downmix = false) {
+                                  std::vector<pqmf_pool_group_pcm16>* pcm = nullptr, bool downmix = false, at::ScalarType dtype = at::kFloat) {
   TORCH_CHECK(blocks.size() == ids.size(), what, ": ", blocks.size(), " block tensors but ", ids.size(), " id tensors");
   TORCH_CHECK(blocks.size() <= 8, what, ": at most 8 groups per call, got ", blocks.size());
   std::vector<at::Tensor> kept;
@@ -525,7 +529,8 @@ std::vector<at::Tensor> groups_of(at::TensorList blocks, at::TensorList ids, con
       rows += n;
       continue;
     }
-    check_f32_cuda(b, dir == GroupsDir::kSynthesis ? "s" : "x");
+    if (dtype == at::kFloat) check_f32_cuda(b, dir == GroupsDir::kSynthesis ? "s" : "x");
+    else pool_dtype(b, dtype, dir == GroupsDir::kSynthesis ? "s" : "x");
     TORCH_CHECK(b.device() == like.device(), what, ": every group must be on the pool's device");
     if (dir == GroupsDir::kSynthesis) {
       TORCH_CHECK(b.dim() == 3 && b.size(1) == bank.M, what, " expects [streams, n_band, frames] per group, got ", b.sizes());
@@ -914,6 +919,81 @@ std::tuple<std::vector<at::Tensor>, std::vector<at::Tensor>> stream_pool_step_gr
   return {outs, ys};
 }
 
+// ---- grouped pool calls with half-precision blocks (pqmf_stream_pool_*_groups_x): groups_of's groups of the pool's dtype, outputs of that
+//      dtype.  Where the library refuses the whole call (PQMF_ERR_UNSUPPORTED, nothing launched) the op stages it: widen every group, the
+//      fp32 grouped op, round.  The groups it marks in `staged` go through the single-group half pool op, which stages them on its own ----
+std::vector<pqmf_pool_group_x> half_groups(const std::vector<pqmf_pool_group_f32>& groups) {
+  std::vector<pqmf_pool_group_x> hg;
+  for (const pqmf_pool_group_f32& g : groups) hg.push_back({g.ids, g.n, g.T, nullptr, nullptr, nullptr});
+  return hg;
+}
+
+// xs[k] [n_k, 1, T_k] -> ys[k] [n_k, M, T_k / M], all of dtype
+std::vector<at::Tensor> stream_pool_analysis_groups_x(at::TensorList xs, const at::Tensor& hk, const at::Tensor& tables, at::Tensor xpool,
+                                                      at::Tensor xphase, at::TensorList ids, at::ScalarType dtype, int64_t flags) {
+  const Bank bank = bank_of(hk, xpool);
+  c10::cuda::CUDAGuard guard(xpool.device());
+  const Pool pool = pool_of(xpool, xphase, bank, xpool, "xpool");
+  const int code = pool_dtype_code(dtype);
+  std::vector<pqmf_pool_group_f32> f32;
+  const std::vector<at::Tensor> xc =
+      groups_of(xs, ids, bank, xpool, pool.P, GroupsDir::kAnalysis, f32, "pqmf stream pool analysis_groups", nullptr, false, dtype);
+  std::vector<pqmf_pool_group_x> groups = half_groups(f32);
+  std::vector<at::Tensor> ys;
+  for (size_t k = 0; k < xc.size(); ++k) {
+    ys.push_back(at::empty({xc[k].size(0), bank.M, xc[k].size(2) / bank.M}, xc[k].options()));
+    groups[k].x = xc[k].data_ptr();
+    groups[k].y = ys[k].data_ptr();
+  }
+  unsigned staged = 0;
+  const int rc = pqmf_stream_pool_analysis_groups_x(groups.data(), (int)groups.size(), bank.ptr, tables_ptr(tables, xpool), pool.state, pool.phase,
+                                                    (int)pool.P, (int)bank.M, (int)bank.L, (unsigned)flags, code, &staged, cur_stream());
+  if (rc == PQMF_ERR_UNSUPPORTED) {
+    std::vector<at::Tensor> xf;
+    for (const at::Tensor& x : xc) xf.push_back(x.to(at::kFloat));
+    const std::vector<at::Tensor> yf = stream_pool_analysis_groups(xf, hk, tables, xpool, xphase, ids, flags);
+    for (size_t k = 0; k < xc.size(); ++k) ys[k] = yf[k].to(dtype);
+    return ys;
+  }
+  check_rc(rc, "pqmf_stream_pool_analysis_groups_x");
+  for (size_t k = 0; k < xc.size(); ++k)
+    if (staged_bit(staged, k)) ys[k] = stream_pool_analysis_x(xc[k], hk, tables, xpool, xphase, ids[k], dtype, flags);
+  return ys;
+}
+
+// ss[k] [n_k, M, F_k] -> outs[k] [n_k, 1, M F_k], all of dtype
+std::vector<at::Tensor> stream_pool_synthesis_groups_x(at::TensorList ss, const at::Tensor& hk, const at::Tensor& tables, at::Tensor spool,
+                                                       at::Tensor sphase, at::TensorList ids, at::ScalarType dtype, int64_t flags) {
+  const Bank bank = bank_of(hk, spool);
+  c10::cuda::CUDAGuard guard(spool.device());
+  const Pool pool = pool_of(spool, sphase, bank, spool, "spool");
+  const int code = pool_dtype_code(dtype);
+  std::vector<pqmf_pool_group_f32> f32;
+  const std::vector<at::Tensor> sc =
+      groups_of(ss, ids, bank, spool, pool.P, GroupsDir::kSynthesis, f32, "pqmf stream pool synthesis_groups", nullptr, false, dtype);
+  std::vector<pqmf_pool_group_x> groups = half_groups(f32);
+  std::vector<at::Tensor> outs;
+  for (size_t k = 0; k < sc.size(); ++k) {
+    outs.push_back(at::empty({sc[k].size(0), 1, bank.M * sc[k].size(2)}, sc[k].options()));
+    groups[k].y = sc[k].data_ptr();
+    groups[k].out = outs[k].data_ptr();
+  }
+  unsigned staged = 0;
+  const int rc = pqmf_stream_pool_synthesis_groups_x(groups.data(), (int)groups.size(), bank.ptr, tables_ptr(tables, spool), pool.state, pool.phase,
+                                                     (int)pool.P, (int)bank.M, (int)bank.L, (unsigned)flags, code, &staged, cur_stream());
+  if (rc == PQMF_ERR_UNSUPPORTED) {
+    std::vector<at::Tensor> sf;
+    for (const at::Tensor& s : sc) sf.push_back(s.to(at::kFloat));
+    const std::vector<at::Tensor> of = stream_pool_synthesis_groups(sf, hk, tables, spool, sphase, ids, flags);
+    for (size_t k = 0; k < sc.size(); ++k) outs[k] = of[k].to(dtype);
+    return outs;
+  }
+  check_rc(rc, "pqmf_stream_pool_synthesis_groups_x");
+  for (size_t k = 0; k < sc.size(); ++k)
+    if (staged_bit(staged, k)) outs[k] = stream_pool_synthesis_x(sc[k], hk, tables, spool, sphase, ids[k], dtype, flags);
+  return outs;
+}
+
 int64_t launch_count() { return (int64_t)pqmf_launch_count(); }
 
 // ---- autograd (SURVEY 8f-2: the reference path is differentiable, upstream users train through PQMF) --------------------
@@ -1128,6 +1208,27 @@ std::vector<at::Tensor> stream_pool_synthesis_groups_autograd(at::TensorList ss,
       c10::Dispatcher::singleton().findSchemaOrThrow("pqmf_b200::stream_pool_synthesis_groups", "").typed<decltype(stream_pool_synthesis_groups)>();
   return op.call(ss, hk, tables, spool, sphase, ids, flags);
 }
+std::vector<at::Tensor> stream_pool_analysis_groups_x_autograd(at::TensorList xs, const at::Tensor& hk, const at::Tensor& tables, at::Tensor xpool,
+                                                               at::Tensor xphase, at::TensorList ids, at::ScalarType dtype, int64_t flags) {
+  TORCH_CHECK(!(at::GradMode::is_enabled() && any_requires_grad(xs)),
+              "pqmf_b200::stream_pool_analysis_groups_x is not differentiable (a stream pool carries state across calls); use forward() for "
+              "training or wrap the call in torch.no_grad()");
+  at::AutoDispatchBelowADInplaceOrView guard;
+  static auto op =
+      c10::Dispatcher::singleton().findSchemaOrThrow("pqmf_b200::stream_pool_analysis_groups_x", "").typed<decltype(stream_pool_analysis_groups_x)>();
+  return op.call(xs, hk, tables, xpool, xphase, ids, dtype, flags);
+}
+std::vector<at::Tensor> stream_pool_synthesis_groups_x_autograd(at::TensorList ss, const at::Tensor& hk, const at::Tensor& tables, at::Tensor spool,
+                                                                at::Tensor sphase, at::TensorList ids, at::ScalarType dtype, int64_t flags) {
+  TORCH_CHECK(!(at::GradMode::is_enabled() && any_requires_grad(ss)),
+              "pqmf_b200::stream_pool_synthesis_groups_x is not differentiable (a stream pool carries state across calls); use inverse() for "
+              "training or wrap the call in torch.no_grad()");
+  at::AutoDispatchBelowADInplaceOrView guard;
+  static auto op = c10::Dispatcher::singleton()
+                       .findSchemaOrThrow("pqmf_b200::stream_pool_synthesis_groups_x", "")
+                       .typed<decltype(stream_pool_synthesis_groups_x)>();
+  return op.call(ss, hk, tables, spool, sphase, ids, dtype, flags);
+}
 std::tuple<std::vector<at::Tensor>, std::vector<at::Tensor>> stream_pool_step_groups_autograd(at::TensorList xs, const at::Tensor& hk,
                                                                                               const at::Tensor& tables, at::Tensor xpool,
                                                                                               at::Tensor xphase, at::Tensor spool, at::Tensor sphase,
@@ -1272,6 +1373,12 @@ TORCH_LIBRARY(pqmf_b200, m) {
   m.def(
       "stream_pool_step_x(Tensor x, Tensor hk, Tensor tables, Tensor(a!) xpool, Tensor(b!) xphase, Tensor(c!) spool, Tensor(d!) sphase, "
       "Tensor ids, ScalarType dtype, int flags) -> (Tensor, Tensor)");
+  m.def(
+      "stream_pool_analysis_groups_x(Tensor[] xs, Tensor hk, Tensor tables, Tensor(a!) xpool, Tensor(b!) xphase, Tensor[] ids, ScalarType dtype, "
+      "int flags) -> Tensor[]");
+  m.def(
+      "stream_pool_synthesis_groups_x(Tensor[] ss, Tensor hk, Tensor tables, Tensor(a!) spool, Tensor(b!) sphase, Tensor[] ids, ScalarType dtype, "
+      "int flags) -> Tensor[]");
   m.def("launch_count() -> int", &launch_count);
 }
 
@@ -1304,6 +1411,8 @@ TORCH_LIBRARY_IMPL(pqmf_b200, CUDA, m) {
   m.impl("stream_pool_analysis_x", &stream_pool_analysis_x);
   m.impl("stream_pool_synthesis_x", &stream_pool_synthesis_x);
   m.impl("stream_pool_step_x", &stream_pool_step_x);
+  m.impl("stream_pool_analysis_groups_x", &stream_pool_analysis_groups_x);
+  m.impl("stream_pool_synthesis_groups_x", &stream_pool_synthesis_groups_x);
 }
 
 // gradients w.r.t. the signal / the sub-bands only (the bank is a registered buffer in the reference, not a parameter)
@@ -1327,4 +1436,6 @@ TORCH_LIBRARY_IMPL(pqmf_b200, Autograd, m) {
   m.impl("stream_pool_analysis_x", &stream_pool_analysis_x_autograd);
   m.impl("stream_pool_synthesis_x", &stream_pool_synthesis_x_autograd);
   m.impl("stream_pool_step_x", &stream_pool_step_x_autograd);
+  m.impl("stream_pool_analysis_groups_x", &stream_pool_analysis_groups_x_autograd);
+  m.impl("stream_pool_synthesis_groups_x", &stream_pool_synthesis_groups_x_autograd);
 }

@@ -119,9 +119,10 @@ class StreamPool:
     that ``step`` / ``forward`` / ``inverse`` and the grouped float calls take and return; a block of another dtype raises.  The pool's state
     stays float32 whatever the dtype.  On a half pool, per row ``forward(x)`` is bit for bit ``forward(x.float())`` of a float32 pool
     rounded to ``dtype``, ``inverse(y)`` likewise, and ``step(x)`` is ``forward`` followed by ``inverse`` of the ROUNDED sub-bands, with the
-    state and phase words of that float32 pool.  ``step`` / ``forward`` / ``inverse`` run the streaming Hankel-4 kernels with half loads
-    and stores where the float32 pool would run those kernels; other calls and the grouped float calls are staged (widen, float32 call,
-    round) direction by direction.  The PCM calls are those of a float32 pool."""
+    state and phase words of that float32 pool.  ``step`` / ``forward`` / ``inverse`` and ``forward_groups`` / ``inverse_groups`` run the
+    streaming Hankel-4 kernels with half loads and stores where the float32 pool would run those kernels; other calls are staged (widen,
+    float32 call, round) direction by direction, and ``step_groups`` is ``forward_groups`` then ``inverse_groups``.  The PCM calls are those
+    of a float32 pool."""
 
     def __init__(self, mod, capacity: int, dtype: torch.dtype = torch.float32):
         if capacity < 1:
@@ -225,8 +226,8 @@ class StreamPool:
         The groups the streaming Hankel-4 kernels can take run together in one launch per direction when they make enough tiles together
         (so small groups of several block lengths reach the tensor cores); each of their rows is what those kernels give it in a pool
         call.  Every other group gives exactly what ``step(x_g, ids_g)`` gives; one group is ``step``.  ids follow ``step``'s rules and must
-        be distinct across all groups.  On a half pool the call is staged direction by direction: ``forward_groups`` then ``inverse_groups``
-        of the rounded sub-bands."""
+        be distinct across all groups.  On a half pool the call is ``forward_groups`` then ``inverse_groups`` of the rounded sub-bands: each
+        direction joins the groups the float32 call of that direction would join."""
         if self._half:
             groups = list(groups)
             ys = self.forward_groups(groups)
@@ -240,33 +241,35 @@ class StreamPool:
                                                                self.sphase, ids, mod._flags)
         return list(zip(outs, ys))
 
-    def _widened(self, blocks: List[torch.Tensor], name: str) -> List[torch.Tensor]:
-        """Half pool: the groups' blocks, checked against the pool's dtype, as float32 (exact)."""
-        for b in blocks:
-            _check_dtype(b, self.dtype, name)
-        return [b.float() for b in blocks]
-
     def forward_groups(self, groups) -> List[torch.Tensor]:
-        """``forward`` of up to 8 groups ``(x_g [n_g, 1, T_g], ids_g)`` in one call (routed as ``step_groups``): returns ``[y_g]``."""
+        """``forward`` of up to 8 groups ``(x_g [n_g, 1, T_g], ids_g)`` in one call (routed as ``step_groups``): returns ``[y_g]``.  On a
+        half pool per row the float32 call on the widened blocks, rounded; the joined groups run one half-precision launch."""
         blocks, ids = self._group_ids(groups)
         mod = self.mod
         if self._half:
-            blocks = self._widened(blocks, "x")
+            for b in blocks:
+                _check_dtype(b, self.dtype, "x")
         if mod.n_band == 1:
-            return [b.to(self.dtype) for b in blocks] if self._half else blocks
-        ys = torch.ops.pqmf_b200.stream_pool_analysis_groups(blocks, mod.hk.float(), mod._tables, self.xpool, self.xphase, ids, mod._flags)
-        return [y.to(self.dtype) for y in ys] if self._half else list(ys)
+            return [b.float().to(self.dtype) for b in blocks] if self._half else blocks
+        if self._half:
+            return list(torch.ops.pqmf_b200.stream_pool_analysis_groups_x(blocks, mod.hk.float(), mod._tables, self.xpool, self.xphase, ids,
+                                                                          self.dtype, mod._flags))
+        return list(torch.ops.pqmf_b200.stream_pool_analysis_groups(blocks, mod.hk.float(), mod._tables, self.xpool, self.xphase, ids, mod._flags))
 
     def inverse_groups(self, groups) -> List[torch.Tensor]:
-        """``inverse`` of up to 8 groups ``(y_g [n_g, n_band, F_g], ids_g)`` in one call (routed as ``step_groups``): returns ``[out_g]``."""
+        """``inverse`` of up to 8 groups ``(y_g [n_g, n_band, F_g], ids_g)`` in one call (routed as ``step_groups``): returns ``[out_g]``.  On
+        a half pool per row the float32 call on the widened sub-bands, rounded; the joined groups run one half-precision launch."""
         blocks, ids = self._group_ids(groups)
         mod = self.mod
         if self._half:
-            blocks = self._widened(blocks, "s")
+            for b in blocks:
+                _check_dtype(b, self.dtype, "s")
         if mod.n_band == 1:
-            return [b.to(self.dtype) for b in blocks] if self._half else blocks
-        outs = torch.ops.pqmf_b200.stream_pool_synthesis_groups(blocks, mod.hk.float(), mod._tables, self.spool, self.sphase, ids, mod._flags)
-        return [o.to(self.dtype) for o in outs] if self._half else list(outs)
+            return [b.float().to(self.dtype) for b in blocks] if self._half else blocks
+        if self._half:
+            return list(torch.ops.pqmf_b200.stream_pool_synthesis_groups_x(blocks, mod.hk.float(), mod._tables, self.spool, self.sphase, ids,
+                                                                           self.dtype, mod._flags))
+        return list(torch.ops.pqmf_b200.stream_pool_synthesis_groups(blocks, mod.hk.float(), mod._tables, self.spool, self.sphase, ids, mod._flags))
 
     def step_pcm16(self, pcm: torch.Tensor, ids, downmix: bool = False) -> Tuple[torch.Tensor, torch.Tensor]:
         """``step`` from 16-bit PCM to 16-bit PCM: ``pcm`` int16 ``[S, T, channels]`` -> ``(pcm_out int16 [S, T, C'], y [S, C' * n_band,
